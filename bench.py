@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- bins/sec for expected + scores on B200 (BASELINE.json metric), plus the CPU reference arm.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config ...] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one synthetic matrix that is already resident in HBM:
@@ -19,6 +19,9 @@ Beside it, in the same JSON line:
                 timed region (epi_single_host_packed: the matrix in the 4/5-bit packed transport layout; the int8 variant
                 beside it; S3 and paired configurations through epi_s3_host / epi_paired_host)
   cpu_baseline  N = 1 only: the UNMODIFIED reference (oracle/_ref, byte-compiled by __graft_entry__.build()) on the box's host cores
+
+`--dump-outputs DIR` writes what our arm's timed path computed in its last step as DIR/<name>.npy (dump_outputs below): the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times that reference -- expected.main -> expectedCombination.main -> scores.main with one worker
 process per core on a bounded TSV.gz sample of the workload, parse and gz write included (kind "reference"; the oracle's
@@ -49,7 +52,9 @@ CONFIGS = {
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps; with --impl reference each is one full pass of the reference (for S3 tens of "
+                         "seconds of set-up each, which the sample budget does not bound)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="s2_genome_833", choices=sorted(CONFIGS))
@@ -59,7 +64,59 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-target", action="store_true", help="skip the strong-scaling target sections (S2 / S1 genome, S3 chr1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (our arm only; with several GPUs, "
+                         "the tables and rank 0's bins)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+DUMP_SEED = 20261020
+DUMP_ROWS = 1 << 18                 # bins written from a longer per-bin output (19 MB of float32 scores at 18 states)
+DUMP_ENTRIES = 1 << 20              # entries written from a larger table (the S3 table holds C*C*K*K)
+
+
+def sample_rows(bins, n=DUMP_ROWS):
+    """A fixed, seeded, sorted sample of n of the bins (all bins when there are no more than n)."""
+    import numpy as np
+    if bins <= n:
+        return np.arange(bins)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(bins, n, replace=False))
+
+
+def take_rows(t, rows):
+    """Rows `rows` of the device tensor t (per-bin output, bins on dimension 0)."""
+    import torch
+    return t.index_select(0, torch.from_numpy(rows).to(t.device))
+
+
+def dump_outputs(directory, rows, per_bin, tables):
+    """--dump-outputs: every array as DIR/<name>.npy, float32 kept as float32 and every other type as float64 (exact for the
+    integer tables), with the sampled bin indices as rows.npy.  `per_bin` arrays arrive already taken at `rows` and are
+    written whole; a table of more than DUMP_ENTRIES entries is written at a fixed, seeded sample of its flat entries,
+    indices in <name>_entries.npy.  Everything stays within 64 MB."""
+    import numpy as np
+    d = Path(directory)
+    d.mkdir(parents=True, exist_ok=True)
+    out = {"rows": rows}
+    out.update({name: t.cpu().numpy() for name, t in per_bin.items()})
+    for name, t in tables.items():
+        a = t.cpu().numpy()
+        if a.size > DUMP_ENTRIES:
+            pick = np.sort(np.random.default_rng(DUMP_SEED).choice(a.size, DUMP_ENTRIES, replace=False))
+            out[name + "_entries"] = pick
+            a = a.reshape(-1)[pick]
+        out[name] = a
+    out = {name: a.astype(np.float32 if a.dtype == np.float32 else np.float64) for name, a in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > 64 << 20:
+        raise RuntimeError("--dump-outputs: %d bytes exceed 64 MB" % total)
+    for name, a in out.items():
+        np.save(d / (name + ".npy"), a)
 
 
 def peaks():
@@ -70,10 +127,10 @@ def peaks():
 
 
 # ------------------------------------------------------------------------------------------------
-# CPU arm.  kind "reference": the UNMODIFIED reference (oracle/_ref, byte-compiled by oracle/stage_reference.py from
-# /root/reference) runs its own expected.main -> expectedCombination.main -> scores.main on a TSV.gz sample of the
-# workload with one worker process per host core -- what `epilogos -l -c 0` executes before the ROI step (run.py:191-279),
-# TSV parse and gz write included; its own verbose timers give the compute-only share.  kind "port": the oracle's
+# CPU arm.  kind "reference": the UNMODIFIED reference (oracle/_ref, byte-compiled by oracle/stage_reference.py from the
+# checkout EPILOGOS_REFERENCE names) runs its own expected.main -> expectedCombination.main -> scores.main on a TSV.gz
+# sample of the workload with one worker process per host core -- what `epilogos -l -c 0` executes before the ROI step
+# (run.py:191-279), TSV parse and gz write included; its own verbose timers give the compute-only share.  kind "port": the oracle's
 # row-loop port (same algorithm and cost, I/O excluded), the fallback when the reference was not staged.
 # ------------------------------------------------------------------------------------------------
 def config_dict(args, world, bins, cols, k, desc, pitch=None):
@@ -269,9 +326,9 @@ def run_reference(args):
     bins, cols, k, desc = CONFIGS[args.config]
     paired = args.config.startswith("paired")
     saliency = 1 if paired else int(args.config[1])
-    steps, warmup = max(1, args.steps), args.warmup
+    steps, warmup = args.steps, args.warmup
     if saliency == 3:               # one pass costs tens of seconds of fixed set-up per worker (693k-tuple pair list, 0.9 GB tables)
-        steps, warmup = min(steps, 2), 0
+        warmup = 0
     base, times, n = cpu_arm(args, steps, warmup, budget_s=float(os.environ.get("EPI_BENCH_REF_BUDGET_S", "150")))
     sec = sum(times) / len(times)
     metric = ("bins/sec for paired expected+scores (S1)" if paired else "bins/sec for expected+scores (S%d)" % saliency)
@@ -595,6 +652,10 @@ def run_ours(args):
     value = bins * world / (ms_per_step * 1e-3)
     k1_ms = float(k1_ms.item())
     check, _ = _check_step(torch, dist, world, last, bins * world, cols, saliency, scores)
+    if args.dump_outputs and rank == 0:
+        rows = sample_rows(bins)
+        dump_outputs(args.dump_outputs, rows, {"scores": take_rows(scores, rows)},
+                     {"expected_counts": last["n"], "expected": last["e"]})
 
     # ---- the north-star target: ONE genome / ONE chr1 sharded over the GPUs (strong scaling), S2, S1 and S3 ----
     target = None
@@ -719,6 +780,7 @@ def run_ours_s3(args, engine, synth, dist, world, rank, local, bins, cols, k, de
     scores = torch.empty((bins, k), dtype=torch.float32, device="cuda")
     stream = torch.cuda.current_stream()
     gram_ev = []
+    keep = {}
 
     def step(timed):
         if timed:
@@ -733,8 +795,9 @@ def run_ours_s3(args, engine, synth, dist, world, rank, local, bins, cols, k, de
         _, exp3 = engine.s3_finalize(tiles, cols, k, plan["mp"], bins * world, want_counts=False, want_exp=True)
         terms = engine.s3_terms(exp3.reshape(-1), cols, k)
         engine.scores_s3(x, cols, k, terms, out32=scores)
+        keep["exp3"] = exp3
 
-    steps = min(args.steps, 3)
+    steps = args.steps
     sampler = ClockSampler(local) if rank == 0 else None
     step(False)
     torch.cuda.synchronize()
@@ -754,6 +817,9 @@ def run_ours_s3(args, engine, synth, dist, world, rank, local, bins, cols, k, de
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_per_step, gram_ms = float(ms[0]), float(ms[1])
+    if args.dump_outputs and rank == 0:
+        rows = sample_rows(bins)
+        dump_outputs(args.dump_outputs, rows, {"scores": take_rows(scores, rows)}, {"expected": keep["exp3"]})
     e2e = None
     if not args.no_e2e:
         # end to end through epi_s3_host: pinned host matrix in, float32 scores out (the 0.9 GB table stays on the device)
@@ -825,8 +891,10 @@ def run_ours_paired(args, engine, synth, dist, world, rank, local, bins, cols, k
     xa = synth.synth_states_device(bins, c1, k, seed=5 + 10 * rank)
     xb = synth.synth_states_device(bins, c2, k, seed=6 + 10 * rank)
     stream = torch.cuda.current_stream()
+    rows = sample_rows(bins, DUMP_ROWS // 64) if args.dump_outputs else None     # 1000 null distances per bin
+    last = {}
 
-    def step():
+    def step(nulls=None):
         ca = engine.bin_counts(xa, c1, k)
         cb = engine.bin_counts(xb, c2, k)
         comb = (ca + cb).contiguous()
@@ -836,18 +904,21 @@ def run_ours_paired(args, engine, synth, dist, world, rank, local, bins, cols, k
         e = engine.normalize(n1)
         sa, sb = engine.scores_s1(ca, c1, e), engine.scores_s1(cb, c2, e)
         delta, _ = engine.pairwise_combine(sa, sb, None, None)
-        engine.quiescent_mask(ca, c1, cb, c2, k - 1)
-        engine.pairwise_real_reduce(delta)
+        mask = engine.quiescent_mask(ca, c1, cb, c2, k - 1)
+        dist_real, max_diff = engine.pairwise_real_reduce(delta)
+        last.update(expected=e, delta=delta, quiescent=mask, distance=dist_real, max_diff_state=max_diff)
         done = 0
         while done < nperm:
             n = min(batch, nperm - done)
             oa, ob = engine.shuffled_counts_philox(ca, cb, c1, c2, 100 + done, n)
             na = engine.scores_s1(oa.reshape(-1, k), c1, e)
             nb = engine.scores_s1(ob.reshape(-1, k), c2, e)
-            engine.pairwise_combine(None, None, na, nb)
+            _, null = engine.pairwise_combine(None, None, na, nb)
+            if nulls is not None:
+                nulls.append(take_rows(null.view(n, bins).t(), rows))
             done += n
 
-    steps = min(args.steps, 3)
+    steps = args.steps
     sampler = ClockSampler(local) if rank == 0 else None
     step()
     torch.cuda.synchronize()
@@ -865,6 +936,20 @@ def run_ours_paired(args, engine, synth, dist, world, rank, local, bins, cols, k
     ms = torch.tensor([t0.elapsed_time(t1) / steps], device="cuda", dtype=torch.float64)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
+    if args.dump_outputs:
+        # The null distances of a step are dropped batch by batch, so the last timed step's are taken from one more pass,
+        # untimed: the step is deterministic (seeded inputs, null draws keyed by seed and bin).  That pass must reproduce
+        # the last timed step's other outputs bit for bit, or the dump would mix two different computations.
+        timed = dict(last)
+        nulls = []
+        step(nulls)
+        for name, t in timed.items():
+            if not torch.equal(t, last[name]):
+                raise RuntimeError("--dump-outputs: the paired step is not deterministic (%s differs between passes)" % name)
+        if rank == 0:
+            per_bin = {name: take_rows(timed[name], rows) for name in ("delta", "quiescent", "distance", "max_diff_state")}
+            per_bin["null_distances"] = torch.cat(nulls, dim=1)
+            dump_outputs(args.dump_outputs, rows, per_bin, {"expected": timed["expected"]})
     e2e = None
     if not args.no_e2e:
         # end to end through epi_paired_host with pinned host matrices: tables, delta, quiescence mask and null distances

@@ -1,10 +1,10 @@
 """Generate the golden fixtures in this directory by running the UNMODIFIED reference.
 
-Run once in the authoring container (needs /root/reference):   python tests/golden/make_golden.py
+Run once with a checkout of the reference:   EPILOGOS_REFERENCE=/path/to/epilogos python tests/golden/make_golden.py
 The reference ships no tests / golden vectors for the scoring path (SURVEY.md section 4), so the goldens
 are outputs of the reference itself (expected.main -> expectedCombination.main -> scores.main through
 oracle/reference_driver.py) on
-  * a real-data slice: 10 biosamples x 4000 bins of chr1 built from /root/reference/data/ChromHMM with the
+  * a real-data slice: 10 biosamples x 4000 bins of chr1 built from the reference's data/ChromHMM with the
     paste recipe of bin/preprocess_data_ChromHMM.sh:34-49 (rows 100000..103999, a varied region), and
   * small seeded synthetic matrices of the benchmark shapes (C=833/K=18, C=127/K=15).
 Each fixture is a compressed .npz holding the 0-based int8 input and the reference outputs.
@@ -85,7 +85,7 @@ def s3_big_case(name, bins=48, cols=833, k=18, seed=11):
 
 def real_full_case():
     """BASELINE configs[0] substitute: the whole real chr1 matrix (1,246,253 bins x 10 biosamples, 18 states) assembled
-    from /root/reference/data/ChromHMM, run through the reference's stages with 8 worker processes.  Outputs are too big to
+    from the reference's data/ChromHMM, run through the reference's stages with 8 worker processes.  Outputs are too big to
     commit: keep the input (0.6 MB compressed), the tables, sha256 digests of the float32 score arrays and of the
     scores text, and the reference's own top-100 regions of interest (helpers.maxMean on its scores)."""
     import warnings

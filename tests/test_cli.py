@@ -115,7 +115,7 @@ def test_cli_main_end_to_end_on_cpu_with_the_oracle_backend(tmp_path, golden, mo
 
 def test_bench_reference_arm_contract(tmp_path):
     """`bench.py --impl reference`: rank 0 prints ONE JSON line with the contract's keys (the unmodified reference staged under
-    oracle/_ref when /root/reference exists, else the oracle port), the same `config` object our arm prints, e2e = value;
+    oracle/_ref or named by EPILOGOS_REFERENCE, else the oracle port), the same `config` object our arm prints, e2e = value;
     every other rank exits 0 without output."""
     import json
     import os
@@ -141,3 +141,109 @@ def test_bench_reference_arm_contract(tmp_path):
     r = subprocess.run([sys.executable, str(root / "bench.py"), "--impl", "reference", "--gpus", "2"], capture_output=True,
                        text=True, timeout=120, env=dict(env, RANK="1", WORLD_SIZE="2"))
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_bench_dump_outputs_format(tmp_path):
+    """bench.dump_outputs: float32 stays float32, integer tables become exact float64, a large table is written at a seeded
+    sample of its entries, and the same call writes the same files."""
+    import sys
+    from pathlib import Path
+    import torch
+    sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
+    import bench
+    rows = bench.sample_rows(5_000_000)
+    assert len(rows) == bench.DUMP_ROWS and np.array_equal(rows, bench.sample_rows(5_000_000)) and (np.diff(rows) > 0).all()
+    assert np.array_equal(bench.sample_rows(100), np.arange(100))
+    scores = torch.arange(100 * 18, dtype=torch.float32).reshape(100, 18)
+    table = torch.arange(18 * 18, dtype=torch.int64).reshape(18, 18) + (1 << 40)
+    big = torch.arange(bench.DUMP_ENTRIES + 5, dtype=torch.float32)
+    wide = torch.arange((bench.DUMP_ENTRIES // 18 + 1) * 18, dtype=torch.float32).reshape(-1, 18)   # per-bin: written whole
+    for d in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(d, np.array([3, 50]), {"scores": bench.take_rows(scores, np.array([3, 50])), "wide": wide},
+                           {"expected_counts": table, "big": big})
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == ["big.npy", "big_entries.npy", "expected_counts.npy", "rows.npy", "scores.npy", "wide.npy"]
+    for n in names:
+        assert (tmp_path / "a" / n).read_bytes() == (tmp_path / "b" / n).read_bytes()
+    s = np.load(tmp_path / "a" / "scores.npy")
+    assert s.dtype == np.float32 and np.array_equal(s, scores.numpy()[[3, 50]])
+    t = np.load(tmp_path / "a" / "expected_counts.npy")
+    assert t.dtype == np.float64 and np.array_equal(t.astype(np.int64), table.numpy())
+    b, e = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "a" / "big_entries.npy")
+    assert b.shape == (bench.DUMP_ENTRIES,) and np.array_equal(b, e.astype(np.float32))
+    assert np.array_equal(np.load(tmp_path / "a" / "wide.npy"), wide.numpy())
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_repeat(tmp_path):
+    """`bench.py --dump-outputs`: two runs with the same arguments write the same outputs, and the dumped table has its
+    closed form (S2 counts sum to bins C (C-1))."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from pathlib import Path
+    root = Path(__file__).resolve().parent.parent
+    env = dict(os.environ, EPI_BENCH_NO_CLOCKS="1")
+    for run_dir in ("a", "b"):
+        r = subprocess.run([sys.executable, str(root / "bench.py"), "--steps", "2", "--warmup", "0", "--bins", "300000",
+                            "--no-e2e", "--no-target", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / run_dir)],
+                           capture_output=True, text=True, timeout=600, env=env)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert line["steps"] == 2 and line["check"] == "ok"
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == ["expected.npy", "expected_counts.npy", "rows.npy", "scores.npy"]
+    for n in names:
+        assert np.array_equal(np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n))
+    counts = np.load(tmp_path / "a" / "expected_counts.npy")
+    scores = np.load(tmp_path / "a" / "scores.npy")
+    assert counts.shape == (18, 18) and counts.sum() == 300000 * 833 * 832
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert rows.shape == (1 << 18,) and rows.max() < 300000 and scores.shape == (1 << 18, 18)
+    assert scores.dtype == np.float32 and np.isfinite(scores).all()
+
+
+# per configuration: the engine call made once per step, and the passes outside the timed loop (S2: 3 warm-up passes at
+# --warmup 0 and 3 more after the clock sampler starts; S3 and paired: 1 warm-up pass; paired: 1 untimed pass for the dump)
+STEP_CALLS = {"s2_genome_833": ("bin_counts", 6), "s3_chr1_833": ("s3_expected_tiles", 1), "paired_s1_chr1": ("quiescent_mask", 2)}
+DUMP_FILES = {"s2_genome_833": {"expected", "expected_counts", "rows", "scores"},
+              "s3_chr1_833": {"expected", "expected_entries", "rows", "scores"},
+              "paired_s1_chr1": {"delta", "distance", "expected", "max_diff_state", "null_distances", "quiescent", "rows"}}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("config", sorted(STEP_CALLS))
+def test_bench_steps_and_dump_per_config(tmp_path, monkeypatch, capsys, config):
+    """In process, so the engine's calls can be counted: `--steps 4` runs exactly 4 timed steps in every configuration (S3
+    and paired mode used to stop at 3), and each configuration's dump holds its outputs at the documented sizes."""
+    import json
+    import sys
+    from pathlib import Path
+    sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
+    import bench
+    from epilogos_b200 import engine
+    name, outside = STEP_CALLS[config]
+    calls = []
+    real = getattr(engine, name)
+    monkeypatch.setattr(engine, name, lambda *a, **k: (calls.append(1), real(*a, **k))[1])
+    monkeypatch.setenv("EPI_BENCH_NO_CLOCKS", "1")
+    steps, bins = 4, 20000
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--config", config, "--steps", str(steps), "--warmup", "0", "--bins",
+                                      str(bins), "--no-e2e", "--no-target", "--no-cpu-baseline", "--dump-outputs",
+                                      str(tmp_path)])
+    bench.main()
+    line = json.loads([ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")][-1])
+    assert line["steps"] == steps and len(calls) == steps + outside
+    out = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    assert set(out) == DUMP_FILES[config]
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    if config == "s3_chr1_833":
+        assert out["scores"].shape == (bins, 18) and np.array_equal(out["rows"], np.arange(bins))
+        assert out["expected"].shape == out["expected_entries"].shape == (bench.DUMP_ENTRIES,)
+        assert out["expected_entries"].max() < 833 * 833 * 18 * 18
+    if config == "paired_s1_chr1":
+        n = bench.DUMP_ROWS // 64
+        assert out["rows"].shape == (n,) and out["delta"].shape == (n, 18) and out["null_distances"].shape == (n, 1000)
+        assert out["expected"].shape == (18,) and abs(float(out["expected"].sum()) - 1.0) < 1e-5

@@ -317,7 +317,7 @@ try:
     session.load_shard({f!r}, "null", 18, OracleBackend())
     print("NO ERROR", flush=True)
 except Exception as exc:
-    print("RAISED", td.get_rank(), type(exc).__name__, str(exc)[:200], flush=True)
+    print("RAISED", td.get_rank(), type(exc).__name__, str(exc), flush=True)
 td.destroy_process_group()
 """
 

@@ -2,8 +2,8 @@
 
 tests/test_oracle_golden.py pins the oracle to committed outputs of the reference; this module draws fresh matrices (seeded,
 so a failure can be replayed) and runs the reference itself -- expected.main -> expectedCombination.main -> scores.main
-through oracle/reference_driver.py -- wherever it can be imported (/root/reference in the authoring container, or the
-byte-compiled oracle/_ref that __graft_entry__.build() stages).  Skipped where neither exists.  Same bar as the fixtures:
+through oracle/reference_driver.py -- wherever it can be imported (the checkout EPILOGOS_REFERENCE names, or the
+byte-compiled oracle/_ref that __graft_entry__.build() stages from it).  Skipped where neither exists.  Same bar as the fixtures:
 integer tables, float32 expected payload, float32 scores, formatted text and seeded null distances bit for bit.
 """
 import numpy as np
@@ -12,7 +12,7 @@ import pytest
 from oracle import epilogos_oracle as orc
 from oracle import reference_driver as ref
 
-pytestmark = [pytest.mark.skipif(not ref.available(), reason="the reference is neither at /root/reference nor staged in oracle/_ref"),
+pytestmark = [pytest.mark.skipif(not ref.available(), reason="the reference is neither named by EPILOGOS_REFERENCE nor staged in oracle/_ref"),
               pytest.mark.filterwarnings("ignore:This process .* is multi-threaded, use of fork:DeprecationWarning")]   # its Pool
 
 

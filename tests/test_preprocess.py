@@ -1,6 +1,7 @@
 """ChromHMM state-by-line files -> input matrices (epilogos_b200.preprocess, the native form of the reference's
 bin/preprocess_data_ChromHMM.sh): byte-identical `matrix_<chr>.txt` files and messages, against a restatement of the
-script's paste / awk recipe everywhere and against the UNMODIFIED script and its example data where /root/reference exists."""
+script's paste / awk recipe everywhere and against the UNMODIFIED script and its example data where EPILOGOS_REFERENCE names a
+checkout of the reference."""
 import gzip
 import io
 import subprocess
@@ -11,9 +12,11 @@ import pytest
 
 from epilogos_b200 import helpers, preprocess
 from epilogos_b200._lib import EpilogosB200Error
+from oracle import stage_reference
 
-SCRIPT = Path("/root/reference/bin/preprocess_data_ChromHMM.sh")
-EXAMPLE = Path("/root/reference/data/ChromHMM")
+REFERENCE = stage_reference.SOURCE if stage_reference.source_available() else None
+SCRIPT = REFERENCE / "bin" / "preprocess_data_ChromHMM.sh" if REFERENCE else None
+EXAMPLE = REFERENCE / "data" / "ChromHMM" if REFERENCE else None
 
 
 def _statebyline(path, biosample, chrom, labels, gz):
@@ -71,7 +74,7 @@ def test_matrices_equal_the_scripts_recipe(tmp_path):
     files = preprocess.find_files(data, preprocess.biosamples(tmp_path / "meta.tsv"), "chr1")
     direct, chrom = preprocess.read_chromosome(files, num_states=25)
     assert chrom == "chr1" and direct.dtype == np.int8 and np.array_equal(direct, m)
-    if SCRIPT.is_file():                                            # the unmodified script on the same files
+    if SCRIPT and SCRIPT.is_file():                                 # the unmodified script on the same files
         ref = tmp_path / "ref"
         ref.mkdir()
         r = subprocess.run(["bash", str(SCRIPT), str(data), str(tmp_path / "meta.tsv"), str(tmp_path / "sizes.genome")], cwd=ref,
@@ -137,12 +140,13 @@ def test_matrix_writer_matches_python_formatting(tmp_path):
         assert f.read() == b""
 
 
-@pytest.mark.skipif(not (SCRIPT.is_file() and EXAMPLE.is_dir()), reason="needs the reference's script and example data")
+@pytest.mark.skipif(not (SCRIPT and SCRIPT.is_file() and EXAMPLE.is_dir()),
+                    reason="needs the reference's script and example data (EPILOGOS_REFERENCE)")
 def test_real_example_data_against_the_unmodified_script(tmp_path, golden):
     """The reference's own example (10 biosamples, chr1, 1,246,253 bins): the script's matrix_chr1.txt byte for byte, and the
     matrix read directly from the state-by-line files equals the matrix the goldens were generated from."""
     (tmp_path / "sizes.genome").write_text("chr1\t249250621\nchr2\t243199373\n")
-    meta = Path("/root/reference/data/metadata_Boix.txt")
+    meta = REFERENCE / "data" / "metadata_Boix.txt"
     ref = tmp_path / "ref"
     ref.mkdir()
     r = subprocess.run(["bash", str(SCRIPT), str(EXAMPLE), str(meta), str(tmp_path / "sizes.genome")], cwd=ref, capture_output=True,
