@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda.h>
+#include <stddef.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -34,7 +35,41 @@ int check_device();   // 0 if an sm_100 device is current, else sets the error a
 
 int sm_count();
 int persistent_grid(int64_t ntiles, int per_sm);   // min(ntiles, SMs * per_sm), at least 1
-void* device_scratch(size_t* bytes);                 // per-device scratch: 64 x 8-byte slots + 16 KB table area
+
+// ---- per-device workspace ---------------------------------------------------------------------
+constexpr int S1_TABLE_MAX_WIDTH = 4095;           // widest input whose S1 scores come from a value table
+
+struct PrepFlags {
+    int has_zero;       // some expected frequency is 0 -> masked terms -> DIRECT evaluation
+};
+
+// constants of the kind::i8 S2 score kernel (tc_tables.cu), written by its prepare kernel
+struct K5TcConsts {
+    double dg[EPI_MAX_STATES];                  // M_tt 2^-F / perms / 8: the [s==t] term of y_t (see `base` in the kernel)
+    double scale;                               // 2^-F / perms
+    double cst;                                 // (2^52 + 2^51) * scale
+    int has_zero;
+    uint32_t m1, m8, m16;                       // 1, 2^8, 2^16 (opaque to the compiler)
+    int fbits;                                  // F: M = round(-log2 E * 2^F)
+};
+
+// Small tables the score and normalise entry points stage on the device before a launch.  One per device, allocated on
+// first use; calls for one device are stream-ordered with respect to each other (include/epilogos_b200.h).
+struct DeviceWorkspace {
+    unsigned long long reduce_slots[64];                            // grand totals of epi_normalize_i64, round-robin
+    double log2e[EPI_MAX_STATES * EPI_MAX_STATES];                  // K5: log2 E, copied to constant memory
+    PrepFlags prep_flags;                                           // K5: zero flag of the expected table
+    int s3_symmetric;                                               // K6: the S3 terms table is symmetric
+    alignas(16) uint8_t k5tc_b_image[8 * EPI_MAX_STATES * 128];     // kind::i8 B operand: 8 rows x 128 B per state
+    K5TcConsts k5tc_consts;
+    alignas(8) double s1_v64[EPI_MAX_STATES * (S1_TABLE_MAX_WIDTH + 1)];   // S1 value table [K][width + 1]
+    alignas(8) float s1_v32[EPI_MAX_STATES * (S1_TABLE_MAX_WIDTH + 1)];    // its float32 rounding
+};
+static_assert(offsetof(DeviceWorkspace, k5tc_b_image) % 16 == 0, "the B operand image is a bulk-copy source");
+static_assert(offsetof(DeviceWorkspace, s1_v64) % 8 == 0 && offsetof(DeviceWorkspace, s1_v32) % 8 == 0,
+              "the S1 value tables need 8-byte alignment");
+
+DeviceWorkspace* device_workspace();   // the current device's workspace; nullptr if it could not be allocated
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time libcuda dependency)
 typedef CUresult (*tensor_map_encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -48,12 +83,8 @@ int launch_k2_tc(const uint16_t* cnt, int64_t bins, int K, int width, int64_t* n
 int scores_s2_tc(const uint16_t* cnt, int64_t bins, int K, int width, int64_t perms, const float* e, int* zero_flag,
                  float* o32, double* o64, cudaStream_t st);
 bool scores_s2_tc_eligible(int width);
-// kind::f16 form of the S2 score mat-vec (tc_scores_h.cu): counts as fp16 subnormals, width <= 1023
-int scores_s2_h(const uint16_t* cnt, int64_t bins, int K, int width, int64_t perms, const float* e, int* zero_flag,
-                float* o32, double* o64, cudaStream_t st);
-bool scores_s2_h_eligible(int width);
-int scores_s2_h_fixed_point(const float* e, int K, int64_t perms, unsigned long long* mfix_dev, int* fbits_host,
-                            cudaStream_t st);
+int scores_s2_tc_fixed_point(const float* e, int K, int64_t perms, unsigned long long* mfix_dev, int* fbits_host,
+                             cudaStream_t st);
 
 // ---- device-side PTX wrappers -----------------------------------------------------------------
 #ifdef __CUDACC__

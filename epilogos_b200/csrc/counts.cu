@@ -349,7 +349,7 @@ static K1Plan plan_k1(int cols, int num_states) {
     pl.nchunks = (nvec + best - 1) / best;
     pl.mode = num_states <= 16 ? MODE_F2 : (num_states <= 18 ? MODE_F2M : MODE_B1);
     pl.npad = pl.nchunks * best * 16 - cols;
-    pl.small = best == 9 && nvec <= 8 && pl.mode != MODE_B1 && getenv("EPI_K1_NO_SMALL") == nullptr;
+    pl.small = best == 9 && nvec <= 8 && pl.mode != MODE_B1;
     return pl;
 }
 

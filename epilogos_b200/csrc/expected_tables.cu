@@ -207,22 +207,20 @@ int persistent_grid(int64_t ntiles, int per_sm) {
     return (int)g;
 }
 
-// per-device scratch (allocated once; no stream-ordered malloc on the hot path).  64 eight-byte slots handed
-// out round-robin, followed by a 16 KB area used by the score kernels' table preparation.
-void* device_scratch(size_t* bytes) {
-    static void* base[64] = {nullptr};
-    constexpr size_t kBytes = 64 * 8 + 16384;
+// allocated once per device: no stream-ordered malloc on the hot path
+DeviceWorkspace* device_workspace() {
+    static DeviceWorkspace* base[64] = {nullptr};
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
-    if (base[dev] == nullptr && cudaMalloc(&base[dev], kBytes) != cudaSuccess) return nullptr;
-    if (bytes) *bytes = kBytes;
+    if (base[dev] == nullptr && cudaMalloc(reinterpret_cast<void**>(&base[dev]), sizeof(DeviceWorkspace)) != cudaSuccess)
+        return nullptr;
     return base[dev];
 }
 
 static unsigned long long* scratch_slot() {
     static unsigned next = 0;
-    void* b = device_scratch(nullptr);
-    return b ? reinterpret_cast<unsigned long long*>(b) + (next++ & 63) : nullptr;
+    DeviceWorkspace* ws = device_workspace();
+    return ws ? &ws->reduce_slots[next++ & 63] : nullptr;
 }
 
 template <int NBLK, bool FULL>

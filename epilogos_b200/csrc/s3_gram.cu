@@ -8,36 +8,31 @@
 //
 //  * epi_s3_onehot   writes the TRANSPOSED one-hot OHT[m][b] (m = j*K+s, bins contiguous), which makes both
 //                    GEMM operands K-major (the contraction index is the bin): the canonical TN layout.
-//  * epi_s3_gram     persistent warp-specialised tcgen05 kernel: 128x256 output tiles, UMMA 128x256x32
-//                    (kind::i8, unsigned 0/1 operands, int32 accumulators in TMEM), operands streamed by TMA
-//                    (128-byte swizzle) through a 4-stage mbarrier ring; warp 0 = TMA producer, warp 1 = TMEM
+//  * epi_s3_gram     persistent warp-specialised tcgen05 kernel on CTA pairs: 256x256 output blocks, UMMA 256x256x32
+//                    (kind::i8, cta_group::2, unsigned 0/1 operands, int32 accumulators in TMEM), operands streamed by
+//                    TMA (128-byte swizzle) through a 6-stage mbarrier ring; warp 0 = TMA producer, warp 1 = TMEM
 //                    allocator + single-thread MMA issuer, warps 2-5 = epilogue (tcgen05.ld -> global tiles).
-//                    Tiles are rasterised in column groups so the ~148 tiles in flight share operand panels in L2.
+//                    Blocks are rasterised in column groups so the blocks in flight share operand panels in L2.
 //  * epi_s3_finalize turns the (all-reduced) tile buffer into the reference's [C][C][K][K] table: int64 counts
 //                    and/or float32 frequencies (float64 divide by the grand total, expectedCombination.py:42),
 //                    mirroring the lower triangle and zeroing the i == j blocks.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tc05.cuh"
 
 namespace epi {
 
-constexpr int G_TM = 128;           // tile rows   (UMMA M)
-constexpr int G_TN = 256;           // tile cols   (UMMA N)
+constexpr int G_TM = 128;           // tile rows
+constexpr int G_TN = 256;           // tile cols
 constexpr int G_TK = 128;           // bins per pipeline stage (= one 128-byte swizzle atom of int8)
 constexpr int G_UK = 32;            // bins per tcgen05.mma (int8)
-constexpr int G_STAGES = 4;
 constexpr int G_THREADS = 192;
 constexpr int G_GROUP = 8;          // n-tiles per raster group
-constexpr int G_A_BYTES = G_TM * G_TK;          // 16 KB
-constexpr int G_B_BYTES = G_TN * G_TK;          // 32 KB
-constexpr int G_STAGE_BYTES = G_A_BYTES + G_B_BYTES;
 constexpr int G_MAX_GROUPS = 64;
 
 // The Gram matrix is cut into 256 x 256 blocks (Mi, nj), Mi <= nj (on or above the diagonal); block p of the schedule is
-// stored as TWO 128 x 256 tiles t = 2p (rows 256 Mi .. +127) and t = 2p + 1 (rows 256 Mi + 128 .. +255): the unit of the
-// one-CTA kernel is a tile, the unit of the two-CTA kernel a block (each CTA of the pair owns one of its tiles).
+// stored as TWO 128 x 256 tiles t = 2p (rows 256 Mi .. +127) and t = 2p + 1 (rows 256 Mi + 128 .. +255), one per CTA of
+// the pair that computes it.  This tile buffer is the all-reduce payload between ranks, and epi_s3_plan (its size) and
+// epi_s3_finalize (the (mi, nj) -> tile look-up) count in these tiles.
 struct TileSchedule {
     int mt, nt;                       // number of 128-row tiles / 256-col blocks per side
     int ngroups;
@@ -84,8 +79,6 @@ __device__ inline void decode_tile(const TileSchedule& sc, int t, int& mi, int& 
     mi = 2 * Mi + (t & 1);
 }
 
-constexpr uint32_t G_IDESC = umma_i8_idesc(G_TM, G_TN);
-
 // ================================================================================================
 // one-hot expansion, transposed:  OHT[(j*K+s)][b] = (x[b][j] == s)
 // CTA = 128 bins x 32 biosamples.  Labels are staged transposed in shared memory, then every thread
@@ -127,145 +120,11 @@ __global__ void __launch_bounds__(256) s3_onehot_kernel(const int8_t* __restrict
 }
 
 // ================================================================================================
-// Gram kernel
-// ================================================================================================
-__global__ void __launch_bounds__(G_THREADS, 1)
-s3_gram_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
-               const __grid_constant__ TileSchedule sched, int kblocks, int accumulate, int probe,
-               int32_t* __restrict__ tiles) {
-    extern __shared__ uint8_t smem_raw[];
-    // 128-byte-swizzled operand tiles need 1024-byte alignment (the launch reserves the slack)
-    uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    uint8_t* ring = smem;                                                            // G_STAGES * 48 KB
-    uint64_t* full = reinterpret_cast<uint64_t*>(smem + G_STAGES * G_STAGE_BYTES);   // TMA -> MMA
-    uint64_t* empty = full + G_STAGES;                                               // MMA -> TMA
-    uint64_t* tmem_full = empty + G_STAGES;                                          // MMA -> epilogue
-    uint64_t* tmem_empty = tmem_full + 1;                                            // epilogue -> MMA
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 1);
-
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < G_STAGES; ++s) {
-            mbar_init(&full[s], 1);
-            mbar_init(&empty[s], 1);
-        }
-        mbar_init(tmem_full, 1);
-        mbar_init(tmem_empty, 4);          // one arrive per epilogue warp
-        mbar_fence_init();
-    }
-    if (warp == 1) tmem_alloc(tmem_slot, G_TN);      // 256 columns x 128 lanes of int32 accumulators
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    if (warp == 0) {
-        // ------------------------------ TMA producer ------------------------------
-        if (lane == 0) {
-            tma_prefetch_desc(&map_a);
-            tma_prefetch_desc(&map_b);
-            int s = 0;
-            uint32_t ph = 0;
-            long long issued = 0;
-            for (int t = blockIdx.x; t < sched.total; t += gridDim.x) {
-                int mi, nj;
-                decode_tile(sched, t, mi, nj);
-                for (int kb = 0; kb < kblocks; ++kb) {
-                    mbar_wait(&empty[s], ph ^ 1);
-                    if (probe && issued >= G_STAGES) {
-                        // tensor-peak probe: operands stay whatever is in the ring, no memory traffic at all
-                        mbar_arrive(&full[s]);
-                    } else {
-                        mbar_expect_tx(&full[s], G_STAGE_BYTES);
-                        uint8_t* st = ring + s * G_STAGE_BYTES;
-                        tma_load_2d(st, &map_a, kb * G_TK, mi * G_TM, &full[s]);
-                        tma_load_2d(st + G_A_BYTES, &map_b, kb * G_TK, nj * G_TN, &full[s]);
-                    }
-                    ++issued;
-                    if (++s == G_STAGES) {
-                        s = 0;
-                        ph ^= 1;
-                    }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ------------------------------ MMA issuer (one thread) ------------------------------
-        if (lane == 0) {
-            int s = 0;
-            uint32_t ph = 0, acc_ph = 0;
-            for (int t = blockIdx.x; t < sched.total; t += gridDim.x) {
-                mbar_wait(tmem_empty, acc_ph ^ 1);           // epilogue has drained the previous tile
-                tc_fence_after();
-                for (int kb = 0; kb < kblocks; ++kb) {
-                    mbar_wait(&full[s], ph);
-                    tc_fence_after();
-                    const uint32_t a_addr = smem_u32(ring + s * G_STAGE_BYTES);
-                    const uint64_t a_desc = make_kmajor_sw128_desc(a_addr);
-                    const uint64_t b_desc = make_kmajor_sw128_desc(a_addr + G_A_BYTES);
-#pragma unroll
-                    for (int k = 0; k < G_TK / G_UK; ++k) {
-                        // advancing 32 bytes along K inside the swizzle atom = +2 in the (addr >> 4) field
-                        umma_i8(tmem_base, a_desc + 2 * k, b_desc + 2 * k, G_IDESC, (kb | k) != 0 ? 1u : 0u);
-                    }
-                    umma_commit(&empty[s]);                   // stage may be refilled once these MMAs are done
-                    if (++s == G_STAGES) {
-                        s = 0;
-                        ph ^= 1;
-                    }
-                }
-                umma_commit(tmem_full);                       // accumulator complete
-                acc_ph ^= 1;
-            }
-        }
-    } else {
-        // ------------------------------ epilogue: TMEM -> global tile buffer ------------------------------
-        const int quarter = warp & 3;                         // TMEM lane quarter this warp may access
-        uint32_t acc_ph = 0;
-        for (int t = blockIdx.x; t < sched.total; t += gridDim.x) {
-            mbar_wait(tmem_full, acc_ph);
-            acc_ph ^= 1;
-            tc_fence_after();
-            int32_t* dst = tiles + (long long)t * (G_TM * G_TN) + (long long)(quarter * 32 + lane) * G_TN;
-#pragma unroll 1
-            for (int c0 = 0; c0 < G_TN; c0 += 32) {
-                uint32_t v[32];
-                tmem_ld_32x32(tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)c0, v);
-                int4* d4 = reinterpret_cast<int4*>(dst + c0);
-                if (accumulate) {
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        int4 o = d4[i];
-                        o.x += (int)v[4 * i];
-                        o.y += (int)v[4 * i + 1];
-                        o.z += (int)v[4 * i + 2];
-                        o.w += (int)v[4 * i + 3];
-                        d4[i] = o;
-                    }
-                } else {
-#pragma unroll
-                    for (int i = 0; i < 8; ++i)
-                        d4[i] = make_int4((int)v[4 * i], (int)v[4 * i + 1], (int)v[4 * i + 2], (int)v[4 * i + 3]);
-                }
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(tmem_empty);
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc(tmem_base, G_TN);
-}
-
-// ================================================================================================
-// Gram kernel, two-CTA form (default): a CTA pair (cluster of 2 = one TPC) computes one 256 x 256 block with
+// Gram kernel: a CTA pair (cluster of 2 = one TPC) computes one 256 x 256 block with
 // tcgen05.mma.cta_group::2 (UMMA 256 x 256 x 32).  CTA r of the pair stages rows 256 Mi + 128 r .. +127 of the A operand
 // and rows 256 nj + 128 r .. +127 of the B operand -- 32 KB per 128-bin stage instead of the 48 KB (128 A rows + 256 B
-// rows) of the one-CTA kernel, whose 3.2 POP/s were bound by operand delivery from L2 (94 B/clk/SM at tensor peak), not by
-// the tensor pipe (the same kernel with operand loads disabled issues 4.47 POP/s).  Two 256-column accumulators per CTA
+// rows) of a one-CTA 128 x 256 tile.  A one-CTA kernel reached 3.2 POP/s, bound by operand delivery from L2 (94 B/clk/SM
+// at tensor peak), not by the tensor pipe (4.47 POP/s with operand loads disabled).  Two 256-column accumulators per CTA
 // (all 512 TMEM columns) let the epilogue of block p overlap the MMAs of block p + 1.
 //   warp 0: TMA producer (both CTAs; transaction bytes of both land on the LEADER's full barrier)
 //   warp 1: TMEM allocator (both CTAs) + single-thread MMA issuer (leader CTA only; commits are multicast to both CTAs)
@@ -577,28 +436,15 @@ extern "C" int epi_s3_gram(const int8_t* oht_dev, int64_t mp, int64_t bp, int32_
     EPI_REQUIRE(oht_dev != nullptr && tiles_dev != nullptr, "null pointer argument");
     EPI_REQUIRE((reinterpret_cast<uintptr_t>(tiles_dev) & 15) == 0, "tiles_dev must be 16-byte aligned");
     const TileSchedule sc = make_schedule(mp);
-    const int probe2 = (accumulate & 2) ? 1 : 0;
-    if (getenv("EPI_S3_GRAM1") == nullptr) {
-        // two-CTA kernel: one tensor map with 128-row boxes serves the A and the B halves
-        CUtensorMap map;
-        if (int rc = make_oht_map(&map, oht_dev, mp, bp, 128)) return rc;
-        const size_t smem2 = (size_t)G2_STAGES * G2_STAGE_BYTES + (2 * G2_STAGES + 4) * 8 + 16 + 1024;
-        EPI_CUDA(cudaFuncSetAttribute(s3_gram2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-        int grid2 = sm_count() & ~1;
-        if (grid2 > sc.total) grid2 = sc.total;              // total is even: two CTAs per block
-        s3_gram2_kernel<<<grid2, G_THREADS, smem2, st>>>(map, sc, (int)(bp / G_TK), accumulate & 1, probe2, tiles_dev);
-        EPI_CUDA(cudaGetLastError());
-        return 0;
-    }
-    CUtensorMap map_a, map_b;
-    if (int rc = make_oht_map(&map_a, oht_dev, mp, bp, G_TM)) return rc;
-    if (int rc = make_oht_map(&map_b, oht_dev, mp, bp, G_TN)) return rc;
-    const size_t smem = (size_t)G_STAGES * G_STAGE_BYTES + (2 * G_STAGES + 2) * 8 + 16 + 1024;
-    EPI_CUDA(cudaFuncSetAttribute(s3_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = sm_count();
-    if (grid > sc.total) grid = sc.total;
     const int probe = (accumulate & 2) ? 1 : 0;      // bit 1 of `accumulate`: tensor-peak probe (results are garbage)
-    s3_gram_kernel<<<grid, G_THREADS, smem, st>>>(map_a, map_b, sc, (int)(bp / G_TK), accumulate & 1, probe, tiles_dev);
+    // one tensor map with 128-row boxes serves the A and the B halves
+    CUtensorMap map;
+    if (int rc = make_oht_map(&map, oht_dev, mp, bp, 128)) return rc;
+    const size_t smem = (size_t)G2_STAGES * G2_STAGE_BYTES + (2 * G2_STAGES + 4) * 8 + 16 + 1024;
+    EPI_CUDA(cudaFuncSetAttribute(s3_gram2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int grid = sm_count() & ~1;
+    if (grid > sc.total) grid = sc.total;              // total is even: two CTAs per block
+    s3_gram2_kernel<<<grid, G_THREADS, smem, st>>>(map, sc, (int)(bp / G_TK), accumulate & 1, probe, tiles_dev);
     EPI_CUDA(cudaGetLastError());
     return 0;
 }

@@ -25,8 +25,6 @@
 // registers and, summed over the j-block, to the score row of x_i in shared memory: half the look-ups (the limiter) and
 // half the slab traffic.  s3_symmetry_kernel verifies the property on the device for every table it is given (a foreign
 // exp_freq file need not have it); both kernels are queued and the one that does not apply exits at once.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace epi {
@@ -340,6 +338,8 @@ extern "C" int epi_scores_s3(const int8_t* x_dev, int64_t bins, int32_t cols, in
     while (!fits(bpt, jc) && bpt > 1) bpt >>= 1;
     while (!fits(bpt, jc) && jc > 2) jc >>= 1;
     EPI_REQUIRE(fits(bpt, jc), "S3 score blocking does not fit shared memory for K=%d", K);
+    DeviceWorkspace* ws = device_workspace();
+    EPI_REQUIRE(ws != nullptr, "could not allocate the per-device workspace");
     const int64_t bc = (int64_t)S3S_THREADS * bpt;
     const int64_t bp = ((bins + bc - 1) / bc) * bc;
     uint8_t* xt = nullptr;
@@ -347,13 +347,9 @@ extern "C" int epi_scores_s3(const int8_t* x_dev, int64_t bins, int32_t cols, in
     dim3 tg((unsigned)((bp + 63) / 64), (unsigned)((cols + 63) / 64));
     s3_transpose_kernel<<<tg, 256, 0, st>>>(x_dev, bins, cols, pitch, xt, bp);
     // is the table symmetric (it is whenever it comes from s3Calc)?  decided on the device, no host round trip
-    int* gate = reinterpret_cast<int*>(static_cast<uint8_t*>(device_scratch(nullptr)) + 64 * 8 + 16384 - 64);
-    if (getenv("EPI_S3_FULL") != nullptr) {
-        EPI_CUDA(cudaMemsetAsync(gate, 0, 4, st));                  // A/B runs: force the ordered-pair kernel
-    } else {
-        EPI_CUDA(cudaMemsetAsync(gate, 1, 4, st));
-        s3_symmetry_kernel<<<sm_count() * 8, 256, 0, st>>>(terms_dev, cols, K, gate);
-    }
+    int* gate = &ws->s3_symmetric;
+    EPI_CUDA(cudaMemsetAsync(gate, 1, 4, st));
+    s3_symmetry_kernel<<<sm_count() * 8, 256, 0, st>>>(terms_dev, cols, K, gate);
     int rc = 0;
 #define EPI_S3S_CASE(B, J) if (bpt == B && jc == J) rc = launch_s3_score<B, J>(xt, bp, bins, cols, K, terms_dev, gate, out32_dev, out64_dev, st); else
     EPI_S3S_CASE(4, 8) EPI_S3S_CASE(2, 8) EPI_S3S_CASE(1, 8) EPI_S3S_CASE(4, 4) EPI_S3S_CASE(2, 4) EPI_S3S_CASE(1, 4)

@@ -41,11 +41,7 @@ constexpr int KT_MAX = EPI_MAX_STATES;
 
 __constant__ __align__(16) double c_log2e[KT_MAX * KT_MAX];     // S2: log2 E[s][t], row stride KT; S1: log2 E[s]
 
-struct PrepFlags {
-    int has_zero;       // some expected frequency is 0 -> masked terms -> DIRECT evaluation
-};
-
-// one CTA: expected table (float32) -> log2 table (float64, row stride kt) + zero flag, in device scratch
+// one CTA: expected table (float32) -> log2 table (float64, row stride kt) + zero flag, in the device workspace
 __global__ void k5_prepare_kernel(const float* __restrict__ e, int rows, int cols, int kt, double* __restrict__ out,
                                   PrepFlags* flags) {
     __shared__ int zero;
@@ -126,7 +122,6 @@ __device__ __forceinline__ void warp_store_scores(const float* slab, float* __re
 // and the per-bin work is a table look-up.  The float32 output is therefore the float32 rounding of exactly the
 // float64 expression the reference evaluates (no re-association: rankings downstream, e.g. the regions of interest,
 // see the same values), and the kernel is bound by its 6K bytes per bin of traffic.
-constexpr int S1_TABLE_MAX_WIDTH = 4095;
 constexpr int S1_SMEM_TABLE_BYTES = 96 * 1024;
 
 __global__ void k5_s1_table_kernel(const float* __restrict__ exp1, int K, int width, float* __restrict__ v32,
@@ -310,17 +305,14 @@ static int k5_ctas_per_sm(int dflt) {
     return dflt;
 }
 
-// builds the log2 table in device scratch, copies it into constant memory (device-to-device, stream ordered)
+// builds the log2 table in the device workspace, copies it into constant memory (device-to-device, stream ordered)
 static int prepare_tables(const float* e, int rows, int cols, int kt, cudaStream_t st, const PrepFlags** flags_out) {
-    size_t bytes = 0;
-    uint8_t* scratch = static_cast<uint8_t*>(device_scratch(&bytes));
-    EPI_REQUIRE(scratch != nullptr, "could not allocate the per-device scratch");
-    double* table = reinterpret_cast<double*>(scratch + 64 * 8);
-    PrepFlags* flags = reinterpret_cast<PrepFlags*>(scratch + 64 * 8 + KT_MAX * KT_MAX * 8);
-    k5_prepare_kernel<<<1, 256, 0, st>>>(e, rows, cols, kt, table, flags);
+    DeviceWorkspace* ws = device_workspace();
+    EPI_REQUIRE(ws != nullptr, "could not allocate the per-device workspace");
+    k5_prepare_kernel<<<1, 256, 0, st>>>(e, rows, cols, kt, ws->log2e, &ws->prep_flags);
     EPI_CUDA(cudaGetLastError());
-    EPI_CUDA(cudaMemcpyToSymbolAsync(c_log2e, table, (size_t)rows * kt * 8, 0, cudaMemcpyDeviceToDevice, st));
-    *flags_out = flags;
+    EPI_CUDA(cudaMemcpyToSymbolAsync(c_log2e, ws->log2e, (size_t)rows * kt * 8, 0, cudaMemcpyDeviceToDevice, st));
+    *flags_out = &ws->prep_flags;
     return 0;
 }
 
@@ -334,15 +326,11 @@ static int launch_s1(const uint16_t* cnt, int64_t bins, int K, int width, const 
         EPI_CUDA(cudaGetLastError());
         return 0;
     }
-    // value table: K x (width+1) float32 + float64, in a per-device workspace
-    static uint8_t* ws[64] = {nullptr};
-    int dev = 0;
-    EPI_CUDA(cudaGetDevice(&dev));
-    EPI_REQUIRE(dev >= 0 && dev < 64, "device index %d out of range", dev);
-    constexpr size_t kEntries = (size_t)EPI_MAX_STATES * (S1_TABLE_MAX_WIDTH + 1);
-    if (ws[dev] == nullptr) EPI_CUDA(cudaMalloc(reinterpret_cast<void**>(&ws[dev]), kEntries * 12));
-    double* v64 = reinterpret_cast<double*>(ws[dev]);
-    float* v32 = reinterpret_cast<float*>(ws[dev] + kEntries * 8);
+    // value table: K x (width+1) float32 + float64, in the device workspace
+    DeviceWorkspace* ws = device_workspace();
+    EPI_REQUIRE(ws != nullptr, "could not allocate the per-device workspace");
+    double* v64 = ws->s1_v64;
+    float* v32 = ws->s1_v32;
     const int n = K * (width + 1);
     k5_s1_table_kernel<<<(n + 255) / 256, 256, 0, st>>>(e, K, width, v32, v64);
     EPI_CUDA(cudaGetLastError());
@@ -351,7 +339,7 @@ static int launch_s1(const uint16_t* cnt, int64_t bins, int K, int width, const 
     const int64_t ntiles = (bins + K5_THREADS - 1) / K5_THREADS;
     const size_t base_big = (size_t)32 * 32 * K * 8 + 32 * 16;          // 1024-thread CTA
     if (table <= (size_t)S1_SMEM_TABLE_BYTES && 4 * (base + table + 1024) > (size_t)220 * 1024 &&
-        base_big + table + 1024 <= (size_t)226 * 1024 && getenv("EPI_K5_S1_SMALL_CTA") == nullptr) {
+        base_big + table + 1024 <= (size_t)226 * 1024) {
         // fewer than four 256-thread CTAs would fit next to their tables: one 1024-thread CTA per SM shares ONE table
         auto kern = k5_s1_kernel<true, 1024>;
         EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(base_big + table)));
@@ -390,9 +378,9 @@ static int dispatch_s2(const uint16_t* cnt, int64_t bins, int K, int width, int6
     const PrepFlags* flags = nullptr;
     if (mode == EPI_SCORE_TABLE && scores_s2_tc_eligible(width) && getenv("EPI_K5_ALU") == nullptr) {
         // tensor-core mat-vec (tc_tables.cu); a table with zero entries makes it a no-op and un-gates the DIRECT kernel
-        uint8_t* scratch = static_cast<uint8_t*>(device_scratch(nullptr));
-        EPI_REQUIRE(scratch != nullptr, "could not allocate the per-device scratch");
-        PrepFlags* fl = reinterpret_cast<PrepFlags*>(scratch + 64 * 8 + KT_MAX * KT_MAX * 8);
+        DeviceWorkspace* ws = device_workspace();
+        EPI_REQUIRE(ws != nullptr, "could not allocate the per-device workspace");
+        PrepFlags* fl = &ws->prep_flags;
         if (int rc = scores_s2_tc(cnt, bins, K, width, perms, e, &fl->has_zero, o32, o64, st)) return rc;
         return launch_s2<KT, true>(cnt, bins, K, width, perms, e, fl, 2, o32, o64, st);
     }
@@ -435,7 +423,7 @@ extern "C" int epi_scores_s2_fixed_point(const float* exp2_dev, int32_t K, int64
     EPI_REQUIRE(K >= 1 && K <= EPI_MAX_STATES, "num_states=%d out of range [1, %d]", K, EPI_MAX_STATES);
     EPI_REQUIRE(perms >= 1 && exp2_dev != nullptr && mfix_dev != nullptr, "bad argument");
     int fbits = 0;
-    if (int rc = scores_s2_h_fixed_point(exp2_dev, K, perms, reinterpret_cast<unsigned long long*>(mfix_dev), &fbits, st))
+    if (int rc = scores_s2_tc_fixed_point(exp2_dev, K, perms, reinterpret_cast<unsigned long long*>(mfix_dev), &fbits, st))
         return rc;
     if (fraction_bits_out) *fraction_bits_out = fbits;
     return 0;

@@ -1,7 +1,5 @@
 // tcgen05 / TMEM wrappers shared by the tensor-core kernels (S3 Gram, S2 expected table, S2 scores).  sm_100a only.
 #pragma once
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace epi {
@@ -51,19 +49,11 @@ __device__ __forceinline__ bool mbar_try_wait_hint(uint64_t* bar, uint32_t parit
         : "memory");
     return ok != 0;
 }
-// suspend-time hint of mbar_wait_wd in ns; one copy per translation unit (no relocatable device code in this build).
-// Tuning knob: EPI_WAIT_HINT_NS in the environment (0 = plain polling), applied by apply_wait_hint() before a launch.
-static __constant__ uint32_t c_wait_hint_ns = 200000u;
+// suspend-time hint of mbar_wait_wd in ns (K5-S2 ran within 1 % at 0 / 500 / 5000 / 200000 ns, profiles/README.md)
+constexpr uint32_t MBAR_WAIT_HINT_NS = 200000u;
 __device__ __forceinline__ void mbar_wait_wd(uint64_t* bar, uint32_t parity) {
     uint32_t spins = 0;
-    const uint32_t hint = c_wait_hint_ns;
-    if (hint == 0) {                          // plain polling
-        while (!mbar_try_wait(bar, parity)) {
-            if (++spins > (1u << 28)) __trap();
-        }
-        return;
-    }
-    while (!mbar_try_wait_hint(bar, parity, hint)) {
+    while (!mbar_try_wait_hint(bar, parity, MBAR_WAIT_HINT_NS)) {
         if (++spins > (1u << 22)) __trap();
     }
 }
@@ -138,18 +128,6 @@ __host__ __device__ __forceinline__ uint32_t sw128_offset(uint32_t row, uint32_t
 // instruction descriptor, kind::i8: D=S32 (2<<4), A=U8, B=U8 (format 0), both K-major, N>>3 at [17,23), M>>4 at [24,29)
 __host__ __device__ constexpr uint32_t umma_i8_idesc(uint32_t m, uint32_t n) {
     return (2u << 4) | ((n >> 3) << 17) | ((m >> 4) << 24);
-}
-
-static inline int apply_wait_hint(cudaStream_t st) {
-    static int applied = -1;
-    const char* e = getenv("EPI_WAIT_HINT_NS");
-    const int want = e ? atoi(e) : -1;
-    if (want < 0 || want == applied) return 0;
-    const uint32_t v = (uint32_t)want;
-    EPI_CUDA(cudaMemcpyToSymbolAsync(c_wait_hint_ns, &v, sizeof(v), 0, cudaMemcpyHostToDevice, st));
-    EPI_CUDA(cudaStreamSynchronize(st));
-    applied = want;
-    return 0;
 }
 
 #endif  // __CUDACC__

@@ -164,7 +164,6 @@ template <int KT, int KR>
 static int launch_k2_tc_impl(const uint16_t* cnt, int64_t bins, int K, int64_t* n1, int64_t* n2, cudaStream_t st) {
     const size_t smem = 1024 + (size_t)T2_OPS * T2_OP_BYTES + (size_t)T2_STAGES * T2_BINS * K * 2 +
                         (2 * T2_STAGES + 2 * T2_OPS + 2) * 8 + 16;
-    if (int rc = apply_wait_hint(st)) return rc;
     auto kern = k2_tc_kernel<KT, KR>;
     EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int64_t ntiles = (bins + T2_BINS - 1) / T2_BINS;
@@ -206,19 +205,14 @@ __device__ __forceinline__ uint32_t mad_lo(uint32_t a, uint32_t b, uint32_t c) {
     return d;
 }
 
-struct K5TcConsts {
-    double dg[EPI_MAX_STATES];                  // M_tt 2^-F / perms / 8: the [s==t] term of y_t (see `base` in the kernel)
-    double scale;                               // 2^-F / perms
-    double cst;                                 // (2^52 + 2^51) * scale
-    int has_zero;
-    uint32_t m1, m8, m16;                       // 1, 2^8, 2^16 (opaque to the compiler)
-};
 __constant__ K5TcConsts c_k5tc;
 
 // one CTA: float32 expected table -> fixed-point digits of -log2 E laid out as the 128-byte-swizzled B operand
-// (row n = 8t + d, byte k = 2s + h holds digit d-h of M_st), per-state constants, zero flag.
+// (row n = 8t + d, byte k = 2s + h holds digit d-h of M_st), per-state constants, zero flag; mfix_out (optional)
+// receives the fixed-point table itself (diagnostic / tests).
 __global__ void k5tc_prepare_kernel(const float* __restrict__ e, int K, double perms, int nrows,
-                                    uint8_t* __restrict__ b_image, K5TcConsts* __restrict__ out, int* __restrict__ zero_flag) {
+                                    uint8_t* __restrict__ b_image, K5TcConsts* __restrict__ out, int* __restrict__ zero_flag,
+                                    unsigned long long* __restrict__ mfix_out) {
     __shared__ unsigned long long mfix[EPI_MAX_STATES * EPI_MAX_STATES];
     __shared__ double mval[EPI_MAX_STATES * EPI_MAX_STATES];
     __shared__ unsigned long long maxbits;
@@ -250,6 +244,7 @@ __global__ void k5tc_prepare_kernel(const float* __restrict__ e, int K, double p
         unsigned long long v = (unsigned long long)llrint(ldexp(mval[i], F));
         if (v >= (1ull << 56)) v = (1ull << 56) - 1;
         mfix[i] = v;
+        if (mfix_out != nullptr) mfix_out[i] = v;
     }
     for (int i = threadIdx.x; i < nrows * 128 / 4; i += blockDim.x) reinterpret_cast<uint32_t*>(b_image)[i] = 0u;
     __syncthreads();
@@ -268,6 +263,7 @@ __global__ void k5tc_prepare_kernel(const float* __restrict__ e, int K, double p
         out->m1 = 1u;
         out->m8 = 1u << 8;
         out->m16 = 1u << 16;
+        out->fbits = F;
         *zero_flag = zero;
     }
 }
@@ -489,26 +485,18 @@ k5_s2_tc_kernel(const uint16_t* __restrict__ cnt, long long bins, int Krt, int w
     if (warp == 4 * NWG + 1) tmem_dealloc(tmem_base, 512);
 }
 
-static uint8_t* k5tc_workspace() {
-    static uint8_t* base[64] = {nullptr};
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
-    if (base[dev] == nullptr && cudaMalloc(reinterpret_cast<void**>(&base[dev]), 256 * 128 + 1024) != cudaSuccess) return nullptr;
-    return base[dev];
-}
-
 template <int KT, int KR, int NWG, bool WANT64>
-static int launch_k5_tc2(const uint16_t* cnt, int64_t bins, int K, int width, int64_t perms, const uint8_t* ws, float* o32,
-                         double* o64, cudaStream_t st) {
+static int launch_k5_tc2(const uint16_t* cnt, int64_t bins, int K, int width, int64_t perms, const uint8_t* b_image,
+                         float* o32, double* o64, cudaStream_t st) {
     constexpr int NPAD = ((8 * KT + 31) / 32) * 32;
-    if (int rc = apply_wait_hint(st)) return rc;
     auto kern = k5_s2_tc_kernel<KT, KR, NWG, WANT64>;
     const size_t smem = 1024 + (size_t)NWG * T5_A_BYTES + (size_t)NPAD * 128 + (size_t)NWG * 2 * T5_BINS * K * 2 +
                         (size_t)NWG * T5_BINS * K * 4 + (size_t)(width + 2) * 16 +
                         (size_t)(6 * NWG + 1) * 8 + 16;
     EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int64_t ntiles = (bins + T5_BINS - 1) / T5_BINS;
-    kern<<<persistent_grid(ntiles, 1), NWG * 128 + 64, smem, st>>>(cnt, (long long)bins, K, width, (double)perms, ws, o32, o64);
+    kern<<<persistent_grid(ntiles, 1), NWG * 128 + 64, smem, st>>>(cnt, (long long)bins, K, width, (double)perms, b_image,
+                                                                    o32, o64);
     EPI_CUDA(cudaGetLastError());
     return 0;
 }
@@ -517,22 +505,20 @@ template <int KT, int KR, int NWG>
 static int launch_k5_tc(const uint16_t* cnt, int64_t bins, int K, int width, int64_t perms, const float* e, int* zero_flag,
                         float* o32, double* o64, cudaStream_t st) {
     constexpr int NPAD = ((8 * KT + 31) / 32) * 32;
-    uint8_t* ws = k5tc_workspace();
-    EPI_REQUIRE(ws != nullptr, "could not allocate the score-table workspace");
-    K5TcConsts* consts = reinterpret_cast<K5TcConsts*>(ws + 256 * 128);
-    k5tc_prepare_kernel<<<1, 256, 0, st>>>(e, K, (double)perms, NPAD, ws, consts, zero_flag);
+    static_assert(NPAD * 128 <= sizeof(DeviceWorkspace::k5tc_b_image), "B operand image exceeds its workspace region");
+    DeviceWorkspace* ws = device_workspace();
+    EPI_REQUIRE(ws != nullptr, "could not allocate the per-device workspace");
+    k5tc_prepare_kernel<<<1, 256, 0, st>>>(e, K, (double)perms, NPAD, ws->k5tc_b_image, &ws->k5tc_consts, zero_flag, nullptr);
     EPI_CUDA(cudaGetLastError());
-    EPI_CUDA(cudaMemcpyToSymbolAsync(c_k5tc, consts, sizeof(K5TcConsts), 0, cudaMemcpyDeviceToDevice, st));
-    if (o64 != nullptr) return launch_k5_tc2<KT, KR, NWG, true>(cnt, bins, K, width, perms, ws, o32, o64, st);
-    return launch_k5_tc2<KT, KR, NWG, false>(cnt, bins, K, width, perms, ws, o32, o64, st);
+    EPI_CUDA(cudaMemcpyToSymbolAsync(c_k5tc, &ws->k5tc_consts, sizeof(K5TcConsts), 0, cudaMemcpyDeviceToDevice, st));
+    if (o64 != nullptr) return launch_k5_tc2<KT, KR, NWG, true>(cnt, bins, K, width, perms, ws->k5tc_b_image, o32, o64, st);
+    return launch_k5_tc2<KT, KR, NWG, false>(cnt, bins, K, width, perms, ws->k5tc_b_image, o32, o64, st);
 }
 
 // TABLE evaluation of the S2 scores on the tensor cores.  Writes *zero_flag (device int) = 1 and does nothing else when
 // the expected table has a zero entry; the caller queues the DIRECT kernel behind it, gated on that flag.
 int scores_s2_tc(const uint16_t* cnt, int64_t bins, int K, int width, int64_t perms, const float* e, int* zero_flag,
                  float* o32, double* o64, cudaStream_t st) {
-    // EPI_K5_F16=1 and width <= 1023: the kind::f16 form of this kernel (tc_scores_h.cu), kept for A/B runs
-    if (scores_s2_h_eligible(width)) return scores_s2_h(cnt, bins, K, width, perms, e, zero_flag, o32, o64, st);
     if (K == 18) return launch_k5_tc<18, 18, 3>(cnt, bins, K, width, perms, e, zero_flag, o32, o64, st);
     if (K == 15) return launch_k5_tc<16, 15, 4>(cnt, bins, K, width, perms, e, zero_flag, o32, o64, st);
     if (K <= 16) return launch_k5_tc<16, 0, 4>(cnt, bins, K, width, perms, e, zero_flag, o32, o64, st);
@@ -541,5 +527,20 @@ int scores_s2_tc(const uint16_t* cnt, int64_t bins, int K, int width, int64_t pe
 }
 
 bool scores_s2_tc_eligible(int width) { return width <= T5_MAX_WIDTH; }
+
+// the fixed-point image of -log2 E the kernel multiplies with, and F (diagnostic; used by the exactness test)
+int scores_s2_tc_fixed_point(const float* e, int K, int64_t perms, unsigned long long* mfix_dev, int* fbits_host,
+                             cudaStream_t st) {
+    DeviceWorkspace* ws = device_workspace();
+    EPI_REQUIRE(ws != nullptr, "could not allocate the per-device workspace");
+    k5tc_prepare_kernel<<<1, 256, 0, st>>>(e, K, (double)perms, 8 * EPI_MAX_STATES, ws->k5tc_b_image, &ws->k5tc_consts,
+                                           &ws->prep_flags.has_zero, mfix_dev);
+    EPI_CUDA(cudaGetLastError());
+    K5TcConsts host;
+    EPI_CUDA(cudaMemcpyAsync(&host, &ws->k5tc_consts, sizeof(host), cudaMemcpyDeviceToHost, st));
+    EPI_CUDA(cudaStreamSynchronize(st));
+    if (fbits_host) *fbits_host = host.fbits;
+    return 0;
+}
 
 }  // namespace epi

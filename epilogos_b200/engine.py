@@ -105,7 +105,8 @@ def scores_s2(cnt, width, exp2, perms=None, want64=False, mode=EPI_SCORE_TABLE, 
 
 
 def scores_s2_fixed_point(exp2, num_states, perms):
-    """(M int64 tensor [K, K] on the device, F): the fixed-point image of -log2 E2 used by the tensor-core S2 scores."""
+    """(M int64 tensor [K, K] on the device, F): M = round(-log2 E2 * 2^F), the 56-bit fixed-point table (seven base-256
+    digits, F = 56 - ib with -log2 E2 < 2^ib) that the tensor-core S2 scores multiply the counts with."""
     _require_cuda(exp2, torch.float32, "exp2")
     m = torch.empty((num_states, num_states), dtype=torch.int64, device=exp2.device)
     f = ctypes.c_int32(0)

@@ -79,10 +79,8 @@ int epi_scores_s1(const uint16_t* cnt_dev, int64_t bins, int32_t num_states, int
 int epi_scores_s2(const uint16_t* cnt_dev, int64_t bins, int32_t num_states, int32_t width, int64_t perms,
                   const float* exp2_dev, float* out32_dev, double* out64_dev, int32_t mode, void* stream);
 /* Diagnostic: the fixed-point image M[s][t] = round(-log2 E2[s][t] * 2^F) (uint64 [K][K], device) that the tensor-core
- * kind::f16 form of the TABLE evaluation of epi_scores_s2 (EPI_K5_F16=1, width <= 1023: 55-bit, five 11-bit fp16
- * digits) multiplies the counts with, and F.
- * With EPI_K5_DEBUG=1 / 2 in the environment, the float64 output of that kernel is replaced by the low / high part of
- * the integer sum_s c_s M[s][t] = L + 2^33 H exactly as assembled from the tensor-core accumulators (exactness tests). */
+ * TABLE evaluation of epi_scores_s2 (width <= 2047) multiplies the counts with, and F.  M is 56-bit, F = 56 - ib where
+ * -log2 E2 < 2^ib, and the kernel takes M as seven base-256 digits (kind::i8, exact int32 accumulation). */
 int epi_scores_s2_fixed_point(const float* exp2_dev, int32_t num_states, int64_t perms, uint64_t* mfix_dev,
                               int32_t* fraction_bits_out, void* stream);
 

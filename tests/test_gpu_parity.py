@@ -501,13 +501,12 @@ def test_s3_stage_drivers(eng, golden, tmp_path):
     assert np.max(np.abs(npz["scoreArr"] - g["s3_scores"])) < 2e-2
 
 
-def test_k5_tensor_core_matvec_is_exact(eng, monkeypatch):
-    """The S2 score kernel multiplies the count rows (uint16 counts read as fp16 SUBNORMALS) with the 11-bit digits of the
-    55-bit fixed-point image of -log2 E on the tensor cores (kind::f16, fp32 accumulators) and relies on that product being
-    EXACT integer arithmetic.  With EPI_K5_DEBUG=1 / 2 the kernel returns the two halves L, H of sum_s c_s M_st as assembled
-    from the accumulators; both must equal integer arithmetic on the same fixed-point table, for random, sparse and extreme
-    count rows (all 1023 labels in one state, counts 0 / 1 / 1023) and 18-, 15- and 7-state models."""
-    for k, width, seed in ((18, 833, 1), (15, 127, 2), (18, 1023, 3), (7, 500, 4), (16, 1000, 5)):
+def test_k5_tensor_core_fixed_point_table_and_scores(eng):
+    """The S2 score kernel multiplies the count bytes with the base-256 digits of the 56-bit fixed-point image M of -log2 E
+    on the tensor cores (kind::i8, int32 accumulators: exact).  The table it uses must be that image, F = 56 - ib fraction
+    bits with -log2 E < 2^ib, and the scores must match the oracle for random, sparse and extreme count rows (all labels in
+    one state, counts 0 / 1 / width - 1), for 18-, 16-, 15- and 7-state models up to the widest input of the kernel."""
+    for k, width, seed in ((18, 833, 1), (15, 127, 2), (18, 1023, 3), (7, 500, 4), (16, 1000, 5), (18, 2047, 6)):
         rng = np.random.default_rng(seed)
         bins = 3000
         # count rows that sum to `width`: multinomial with random sparsity, plus extremes
@@ -522,27 +521,13 @@ def test_k5_tensor_core_matvec_is_exact(eng, monkeypatch):
         perms = width * (width - 1)
         m, fbits = eng.scores_s2_fixed_point(ed, k, perms)
         m = m.cpu().numpy().astype(np.int64)
-        assert 40 <= fbits <= 54 and m.min() >= 0 and m.max() < 2 ** 55
+        assert 44 <= fbits <= 55 and m.min() >= 0 and m.max() < 2 ** 56
         want = np.rint(np.ldexp(-np.log2(e.astype(np.float64)), fbits))
         assert np.abs(m - want).max() <= 16                      # device log2 vs numpy log2: an ulp or two of a 53-bit value
-        monkeypatch.setenv("EPI_K5_F16", "1")                   # the kind::f16 kernel (opt-in)
-        digits = [(m >> (11 * d)) & 2047 for d in range(5)]      # [5][K][K]
-        n = [cnt @ dg for dg in digits]                          # N_d[b][t] = sum_s c_bs digit_d(M_st): exact in int64
-        want_l = n[0] + (n[1] << 11) + (n[2] << 22)
-        want_h = n[3] + (n[4] << 11)
         cd = torch.from_numpy(cnt.astype(np.uint16).view(np.int16)).cuda()
-        for dbg, ref in ((1, want_l), (2, want_h)):
-            monkeypatch.setenv("EPI_K5_DEBUG", str(dbg))
-            _, got = eng.scores_s2(cd, width, ed, perms=perms, want64=True)
-            assert np.array_equal(got.cpu().numpy(), ref.astype(np.float64)), (k, width, dbg)
-        monkeypatch.delenv("EPI_K5_DEBUG")
-        # and the scores themselves, against the oracle, with both tensor-core kernels (kind::f16 default, kind::i8)
         ref64 = orc.s2_scores_from_counts(cnt, perms, e, dtype=np.float64)
         _, s64 = eng.scores_s2(cd, width, ed, perms=perms, want64=True)
         np.testing.assert_allclose(s64.cpu().numpy(), ref64, rtol=RTOL, atol=ATOL)
-        monkeypatch.delenv("EPI_K5_F16")
-        _, s64b = eng.scores_s2(cd, width, ed, perms=perms, want64=True)
-        np.testing.assert_allclose(s64b.cpu().numpy(), ref64, rtol=RTOL, atol=ATOL)
 
 
 # ------------------------------------------------------------------------------------------------ paired

@@ -1,5 +1,4 @@
-"""One launch each of the score kernels at a benchmark shape (for ncu): S2 kind::f16, S2 kind::i8 (EPI_K5_I8), S1 table."""
-import os
+"""One launch each of the score kernels at a benchmark shape (for ncu): S2 kind::i8 (tensor cores), S1 table."""
 import sys
 from pathlib import Path
 
@@ -19,9 +18,6 @@ n1, n2 = engine.expected_tables(cnt, cols)
 e1, e2 = engine.normalize(n1), engine.normalize(n2)
 for _ in range(2):
     engine.scores_s2(cnt, cols, e2, out32=out)
-    os.environ["EPI_K5_F16"] = "1"
-    engine.scores_s2(cnt, cols, e2, out32=out)
-    del os.environ["EPI_K5_F16"]
     engine.scores_s1(cnt, cols, e1, out32=out)
 torch.cuda.synchronize()
 print("done")

@@ -3,7 +3,6 @@ compute-sanitizer runs:
     compute-sanitizer --tool memcheck  python tools/sanitize_small.py
     compute-sanitizer --tool racecheck python tools/sanitize_small.py --race      (fewer shapes: racecheck is slow)
 """
-import os
 import sys
 from pathlib import Path
 
@@ -25,9 +24,6 @@ for bins, cols, k in (shapes[:1] + shapes[3:4] if race else shapes):
     e1, e2 = engine.normalize(n1), engine.normalize(n2 + 1)                  # K4
     engine.scores_s1(cnt, cols, e1, want64=True)                             # K5-S1 value table + look-up
     engine.scores_s2(cnt, cols, e2, want64=True)                             # K5-S2 tensor cores (kind::i8)
-    os.environ["EPI_K5_F16"] = "1"
-    engine.scores_s2(cnt, cols, e2, want64=True)                             # K5-S2 tensor cores (kind::f16)
-    del os.environ["EPI_K5_F16"]
     engine.scores_s2(cnt, cols, engine.normalize(n2), want64=True, mode=1)   # DIRECT
     packed, bits = engine.pack_bits(xd, cols, k)                             # packed transport layout
     back = engine.unpack_bits(packed, cols, bits)
@@ -40,9 +36,6 @@ for bins, cols, k in (shapes[:1] + shapes[3:4] if race else shapes):
         counts, exp = engine.s3_finalize(tiles, cols, k, plan["mp"], bins)
         terms = engine.s3_terms(exp.reshape(-1), cols, k)
         engine.scores_s3(xd, cols, k, terms, want64=True)
-        os.environ["EPI_S3_GRAM1"] = "1"
-        engine.s3_expected_tiles(xd, cols, k)                                # one-CTA Gram
-        del os.environ["EPI_S3_GRAM1"]
         engine.s3_host(xh, cols, k)
     # paired
     c1 = cols // 2
