@@ -5,7 +5,7 @@ CPU fallback anywhere in this package: if the library is missing, or a compute e
 without a B200, the call raises.
 """
 import ctypes
-from ctypes import c_char_p, c_int, c_int32, c_int64, c_uint64, c_void_p, POINTER
+from ctypes import c_char_p, c_double, c_int, c_int32, c_int64, c_uint64, c_void_p, POINTER
 from pathlib import Path
 
 LIB_PATH = Path(__file__).resolve().parent / "libepilogos_b200.so"
@@ -72,6 +72,15 @@ PROTOTYPES = {
     "epi_roi_maxmean": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p, POINTER(c_int32)]),
     "epi_pairwise_real_reduce": (c_int, [c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
+    "epi_null_compact_workspace_size": (c_int, [c_int64, POINTER(c_int64)]),
+    "epi_null_compact": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+    "epi_null_subsample": (c_int, [c_void_p, c_int64, c_int32, c_int32, c_uint64, c_void_p, c_void_p, c_void_p]),
+    "epi_gennorm_fit": (c_int, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
+    "epi_gennorm_pvalues": (c_int, [c_void_p, c_int64, c_double, c_double, c_double, c_void_p, c_void_p]),
+    "epi_bh_workspace_size": (c_int, [c_int64, POINTER(c_int64)]),
+    "epi_bh_adjust": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p]),
+    "epi_write_metrics_gz": (c_int, [c_char_p, c_char_p, c_void_p, c_void_p, c_void_p, c_char_p, c_int32, c_void_p,
+                                     c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_int32]),
     "epi_single_host": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
     "epi_packed_bits": (c_int, [c_int32]),
     "epi_packed_pitch": (c_int64, [c_int32, c_int32]),

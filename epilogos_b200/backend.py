@@ -101,3 +101,23 @@ class CudaBackend:
 
     def quiescent_mask(self, cnt_a, cols_a, cnt_b, cols_b, quiescent_state):
         return engine.quiescent_mask(cnt_a, cols_a, cnt_b, cols_b, quiescent_state)
+
+    def pairwise_real_reduce(self, delta, text_round_trip=True):
+        return engine.pairwise_real_reduce(delta.to(self.device).contiguous(), text_round_trip)
+
+    # -- paired statistics (step 4) ---------------------------------------------------------------------
+    def null_pool(self, null_dist, quiescent):
+        return engine.null_compact(null_dist.to(self.device).contiguous(), quiescent.to(self.device).contiguous())
+
+    def null_subsample(self, pool, trials, size, seed):
+        return engine.null_subsample(pool, trials, size, seed)
+
+    def gennorm_fit(self, samples):
+        params, status = engine.gennorm_fit(samples)
+        return params.cpu().numpy(), status.cpu().numpy()
+
+    def gennorm_pvalues(self, x, beta, loc, scale):
+        return engine.gennorm_pvalues(x.to(self.device).contiguous(), beta, loc, scale)
+
+    def bh_adjust(self, p):
+        return engine.bh_adjust(p)

@@ -161,6 +161,38 @@ __device__ __forceinline__ uint32_t lop3_maj(uint32_t a, uint32_t b, uint32_t c)
     return r;
 }
 
+// Philox4x32-10 counter-based generator (paired null shuffles, pairwise.cu; null subsampling, pairwise_stats.cu)
+struct Philox {
+    uint32_t key0, key1;
+    uint32_t ctr[4];
+    uint32_t out[4];
+    int have;
+
+    __device__ __forceinline__ void round(uint32_t (&c)[4], uint32_t k0, uint32_t k1) const {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
+        const uint32_t n0 = hi1 ^ c[1] ^ k0, n1 = lo1, n2 = hi0 ^ c[3] ^ k1, n3 = lo0;
+        c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
+    }
+    __device__ __forceinline__ void refill() {
+        uint32_t c[4] = {ctr[0], ctr[1], ctr[2], ctr[3]};
+        uint32_t k0 = key0, k1 = key1;
+#pragma unroll
+        for (int r = 0; r < 10; ++r) {
+            round(c, k0, k1);
+            k0 += 0x9E3779B9u;
+            k1 += 0xBB67AE85u;
+        }
+        out[0] = c[0]; out[1] = c[1]; out[2] = c[2]; out[3] = c[3];
+        ++ctr[0];
+        have = 4;
+    }
+    __device__ __forceinline__ uint32_t next() {
+        if (have == 0) refill();
+        return out[--have];
+    }
+};
+
 #endif  // __CUDACC__
 
 }  // namespace epi

@@ -1008,24 +1008,14 @@ extern "C" int epi_scores_tsv_close(void* handle) {
     return 0;
 }
 
-extern "C" int epi_write_scores_gz(const char* path, const char* chrom_names, const int32_t* chrom_id,
-                                   const int64_t* starts, const int64_t* ends, const float* scores, int64_t rows,
-                                   int32_t K, int32_t level, int32_t threads) {
-    EPI_REQUIRE(path && chrom_names && starts && ends && (scores || rows == 0), "null pointer argument");
-    EPI_REQUIRE(rows >= 0 && K >= 1, "bad shape");
+namespace epi {
+// Rows formatted by `fmt(char* out, int64_t row) -> end` (at most row_bytes each) in blocks of 16384 rows, every block
+// deflated into its own gzip member on `threads` threads, the members written in order: one valid .gz file.
+template <typename Fmt>
+static int write_gz_rows(const char* path, int64_t rows, size_t row_bytes, int32_t level, int32_t threads, Fmt fmt) {
     if (level < 0 || level > 9) level = 6;
     if (threads <= 0) threads = (int)std::max(1u, std::thread::hardware_concurrency());
     if (threads > 64) threads = 64;
-    std::vector<const char*> names;
-    {
-        int max_id = 0;
-        for (int64_t r = 0; r < rows && chrom_id; ++r) max_id = std::max(max_id, (int)chrom_id[r]);
-        const char* p = chrom_names;
-        for (int i = 0; i <= max_id; ++i) {
-            names.push_back(p);
-            p += strlen(p) + 1;
-        }
-    }
     const int64_t block = 16384;
     const int64_t nblocks = (rows + block - 1) / block;
     std::vector<std::vector<unsigned char>> outs((size_t)nblocks);
@@ -1037,24 +1027,9 @@ extern "C" int epi_write_scores_gz(const char* path, const char* chrom_names, co
             const int64_t bi = next.fetch_add(1);
             if (bi >= nblocks) break;
             const int64_t lo = bi * block, hi = std::min(rows, lo + block);
-            text.resize((size_t)(hi - lo) * (64 + (size_t)K * 28));
+            text.resize((size_t)(hi - lo) * row_bytes);
             char* p = text.data();
-            for (int64_t r = lo; r < hi; ++r) {
-                const char* nm = names[chrom_id ? chrom_id[r] : 0];
-                const size_t nl = strlen(nm);
-                memcpy(p, nm, nl);
-                p += nl;
-                *p++ = '\t';
-                p = format_i64(p, starts[r]);
-                *p++ = '\t';
-                p = format_i64(p, ends[r]);
-                const float* row = scores + r * K;
-                for (int s = 0; s < K; ++s) {
-                    *p++ = '\t';
-                    p = format_5f(p, (double)row[s]);
-                }
-                *p++ = '\n';
-            }
+            for (int64_t r = lo; r < hi; ++r) p = fmt(p, r);
             const size_t tlen = (size_t)(p - text.data());
             z_stream zs;
             memset(&zs, 0, sizeof(zs));
@@ -1094,6 +1069,84 @@ extern "C" int epi_write_scores_gz(const char* path, const char* chrom_names, co
     ok = (fclose(f) == 0) && ok;
     EPI_REQUIRE(ok, "short write to %s", path);
     return 0;
+}
+
+// Pointers to `count` consecutive NUL-terminated strings.
+static std::vector<const char*> split_names(const char* p, int count) {
+    std::vector<const char*> names;
+    for (int i = 0; i < count; ++i) {
+        names.push_back(p);
+        p += strlen(p) + 1;
+    }
+    return names;
+}
+
+static int max_chrom_id(const int32_t* chrom_id, int64_t rows) {
+    int max_id = 0;
+    for (int64_t r = 0; r < rows && chrom_id; ++r) max_id = std::max(max_id, (int)chrom_id[r]);
+    return max_id;
+}
+
+// `chr \t start \t end` of row r
+static inline char* format_location(char* p, const char* nm, int64_t start, int64_t end) {
+    const size_t nl = strlen(nm);
+    memcpy(p, nm, nl);
+    p += nl;
+    *p++ = '\t';
+    p = format_i64(p, start);
+    *p++ = '\t';
+    return format_i64(p, end);
+}
+}  // namespace epi
+
+extern "C" int epi_write_scores_gz(const char* path, const char* chrom_names, const int32_t* chrom_id,
+                                   const int64_t* starts, const int64_t* ends, const float* scores, int64_t rows,
+                                   int32_t K, int32_t level, int32_t threads) {
+    EPI_REQUIRE(path && chrom_names && starts && ends && (scores || rows == 0), "null pointer argument");
+    EPI_REQUIRE(rows >= 0 && K >= 1, "bad shape");
+    const std::vector<const char*> names = split_names(chrom_names, max_chrom_id(chrom_id, rows) + 1);
+    return write_gz_rows(path, rows, 64 + (size_t)K * 28, level, threads, [&](char* p, int64_t r) {
+        p = format_location(p, names[chrom_id ? chrom_id[r] : 0], starts[r], ends[r]);
+        const float* row = scores + r * K;
+        for (int s = 0; s < K; ++s) {
+            *p++ = '\t';
+            p = format_5f(p, (double)row[s]);
+        }
+        *p++ = '\n';
+        return p;
+    });
+}
+
+extern "C" int epi_write_metrics_gz(const char* path, const char* chrom_names, const int32_t* chrom_id,
+                                    const int64_t* starts, const int64_t* ends, const char* state_names, int32_t K,
+                                    const int32_t* max_diff, const float* distance, const double* pval, const double* bh,
+                                    int64_t rows, int32_t level, int32_t threads) {
+    EPI_REQUIRE(path && chrom_names && starts && ends && state_names, "null pointer argument");
+    EPI_REQUIRE(rows == 0 || (max_diff && distance), "null pointer argument");
+    EPI_REQUIRE((pval == nullptr) == (bh == nullptr), "p-values and adjusted p-values go together");
+    EPI_REQUIRE(rows >= 0 && K >= 1 && K <= EPI_MAX_STATES, "bad shape");
+    for (int64_t r = 0; r < rows; ++r)
+        EPI_REQUIRE(max_diff[r] >= 1 && max_diff[r] <= K, "row %lld: state %d outside 1..%d", (long long)r, max_diff[r], K);
+    const std::vector<const char*> names = split_names(chrom_names, max_chrom_id(chrom_id, rows) + 1);
+    const std::vector<const char*> states = split_names(state_names, K);
+    size_t longest = 0;
+    for (const char* s : states) longest = std::max(longest, strlen(s));
+    return write_gz_rows(path, rows, 128 + longest + 64, level, threads, [&](char* p, int64_t r) {
+        p = format_location(p, names[chrom_id ? chrom_id[r] : 0], starts[r], ends[r]);
+        *p++ = '\t';
+        const char* st = states[max_diff[r] - 1];
+        const size_t sl = strlen(st);
+        memcpy(p, st, sl);
+        p += sl;
+        *p++ = '\t';
+        const float d = distance[r];
+        p = format_5f(p, (double)fabsf(d));
+        *p++ = '\t';
+        *p++ = d >= 0.f ? '+' : '-';
+        if (pval) p += sprintf(p, "\t%.5e\t%.5e", pval[r], bh[r]);
+        *p++ = '\n';
+        return p;
+    });
 }
 
 // ---- ChromHMM `-printstatebyline` files -> matrix: the native form of bin/preprocess_data_ChromHMM.sh (SURVEY.md 8f, row f3).

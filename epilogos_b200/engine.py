@@ -403,3 +403,61 @@ def pairwise_real_reduce(delta, text_round_trip=True):
     _lib.call("epi_pairwise_real_reduce", _ptr(delta), rows, k, 1 if text_round_trip else 0, _ptr(dist), _ptr(md),
               _stream())
     return dist, md
+
+
+# ------------------------------------------------------------------------------------------------ paired statistics
+def null_compact(null_dist, quiescent=None):
+    """Null distances float32 [bins] or [nperm, bins] -> the pool float32 [nperm * count] of the bins whose quiescent flag
+    (uint8 [bins]) is 0, permutation-major, bins in their order."""
+    _require_cuda(null_dist, torch.float32, "null_dist")
+    if quiescent is not None:
+        _require_cuda(quiescent, torch.uint8, "quiescent")
+    nperm, bins = (1, null_dist.shape[0]) if null_dist.dim() == 1 else tuple(null_dist.shape)
+    nbytes = ctypes.c_int64(0)
+    _lib.call("epi_null_compact_workspace_size", bins, ctypes.byref(nbytes))
+    ws = torch.empty(max(nbytes.value, 1), dtype=torch.uint8, device=null_dist.device)
+    pool = torch.empty(nperm * bins, dtype=torch.float32, device=null_dist.device)
+    count = torch.zeros(1, dtype=torch.int64, device=null_dist.device)
+    _lib.call("epi_null_compact", _ptr(null_dist), _ptr(quiescent), bins, nperm, _ptr(pool), _ptr(count), _ptr(ws),
+              nbytes.value, _stream())
+    return pool[: nperm * int(count.item())]
+
+
+def null_subsample(pool, trials, size, seed):
+    """(indices int32 [trials, size], samples float32 [trials, size]): trial t's keyed permutation of the pool."""
+    _require_cuda(pool, torch.float32, "pool")
+    idx = torch.empty((trials, size), dtype=torch.int32, device=pool.device)
+    samples = torch.empty((trials, size), dtype=torch.float32, device=pool.device)
+    _lib.call("epi_null_subsample", _ptr(pool), pool.numel(), int(trials), int(size),
+              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), _ptr(idx), _ptr(samples), _stream())
+    return idx, samples
+
+
+def gennorm_fit(samples):
+    """scipy.stats.gennorm.fit of every row of samples (float32 [trials, size]) -> (params float64 [trials, 4] = beta,
+    loc, scale, NLL; status int32 [trials, 2] = iterations, converged)."""
+    _require_cuda(samples, torch.float32, "samples")
+    trials, size = samples.shape
+    params = torch.empty((trials, 4), dtype=torch.float64, device=samples.device)
+    status = torch.empty((trials, 2), dtype=torch.int32, device=samples.device)
+    _lib.call("epi_gennorm_fit", _ptr(samples), int(trials), int(size), _ptr(params), _ptr(status), _stream())
+    return params, status
+
+
+def gennorm_pvalues(x, beta, loc, scale):
+    """Two-sided gennorm p-values float64 of the float32 values x."""
+    _require_cuda(x, torch.float32, "x")
+    p = torch.empty(x.shape, dtype=torch.float64, device=x.device)
+    _lib.call("epi_gennorm_pvalues", _ptr(x), x.numel(), float(beta), float(loc), float(scale), _ptr(p), _stream())
+    return p
+
+
+def bh_adjust(p):
+    """Benjamini-Hochberg adjusted p-values (statsmodels fdr_bh) of float64 p >= 0, in input order."""
+    _require_cuda(p, torch.float64, "p")
+    nbytes = ctypes.c_int64(0)
+    _lib.call("epi_bh_workspace_size", p.numel(), ctypes.byref(nbytes))
+    ws = torch.empty(max(nbytes.value, 1), dtype=torch.uint8, device=p.device)
+    q = torch.empty_like(p)
+    _lib.call("epi_bh_adjust", _ptr(p), p.numel(), _ptr(q), _ptr(ws), nbytes.value, _stream())
+    return q

@@ -2,7 +2,9 @@
 branches of s1Score / s2Score (scores.py:282-303, 319-322, 373-398, 414-421).
 
 Outputs (rank 0): `pairwiseDelta_<tag>_<file>.txt.gz`, `temp_nullDistances_<tag>_<file>.npz`
-{chrName, nullDistances float32[B]}, `temp_quiescence_<tag>_<file>.npz` {chrName, quiescenceArr bool[B]}.
+{chrName, nullDistances float32[B]}, `temp_quiescence_<tag>_<file>.npz` {chrName, quiescenceArr bool[B]}.  When the
+paired statistics stage (roi_pairwise) runs next in this process, the two temp files are not written: their content and
+the reduced real deltas are handed over in memory (session.handover).
 
 Null shuffles.  The reference shuffles each combined row once with the unseeded global numpy RNG
 (helpers.py:183-184).  Two modes are provided (environment variable EPILOGOS_B200_NULL or the `null_mode`
@@ -112,7 +114,16 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
         writer.write_scores_text(outputDirPath / "pairwiseDelta_{}_{}.txt.gz".format(fileTag, filename),
                                  delta.cpu().numpy(), loc)
         chrName = loc["chrom"][0] if len(loc["chrom"]) else ""
-        helpers.savez_level(outputDirPath / "temp_nullDistances_{}_{}.npz".format(fileTag, filename),
-                            chrName=np.array([chrName]), nullDistances=null_dist.cpu().numpy())
+        nullPath = outputDirPath / "temp_nullDistances_{}_{}.npz".format(fileTag, filename)
+        if session.handover_enabled and not os.environ.get("EPILOGOS_B200_KEEP_TEMP"):
+            # the paired statistics stage runs next, in this process: hand over what it reads, reduced on the device to
+            # the distance and the max-difference state of every bin (roi_pairwise.readInData)
+            distance, max_diff = be.pairwise_real_reduce(delta, text_round_trip=True)
+            session.handover[str(nullPath)] = dict(chrName=str(chrName), distance=distance, max_diff=max_diff,
+                                                   null=null_dist, quiescence=quies, chrom=loc["chrom"],
+                                                   start=np.asarray(loc["start"], dtype=np.int64),
+                                                   end=np.asarray(loc["end"], dtype=np.int64))
+            return
+        helpers.savez_level(nullPath, chrName=np.array([chrName]), nullDistances=null_dist.cpu().numpy())
         helpers.savez_level(outputDirPath / "temp_quiescence_{}_{}.npz".format(fileTag, filename),
                             chrName=np.array([chrName]), quiescenceArr=quies.cpu().numpy().astype(np.bool_))

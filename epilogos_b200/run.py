@@ -5,9 +5,9 @@ reference's.  What differs is the execution model: there is no SLURM fan-out (ru
 this process on the GPU, and across GPUs when the command is launched under torchrun
 (`torchrun --nproc-per-node 8 -m epilogos_b200.run -i ... -l`), where every stage shards the rows of each file over
 the ranks.  `-l` is therefore accepted but not required; `-x`, `-p` and the `--*-mem` options are accepted and
-ignored with a note.  Step 4 covers region-of-interest selection for single mode (epilogos_b200.roi); the paired
-statistics / plots of roiAndVisualPairwise.py are outside this package (their inputs -- pairwiseDelta,
-temp_nullDistances, temp_quiescence -- are written in the reference's formats).
+ignored with a note.  Step 4 selects the regions of interest: epilogos_b200.roi in single mode, and in paired mode
+epilogos_b200.roi_pairwise, which also fits the null distribution and writes p-values with -n (the statistics of
+roiAndVisualPairwise.py; its -d figures are not built).
 """
 import csv
 import errno
@@ -112,7 +112,8 @@ def deal_files(pairs, world):
 
 
 def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
-               groupSize, stateInfo, roiWidth, verbose, say, backend=None):
+               groupSize, stateInfo, roiWidth, verbose, say, backend=None, pvalBool=False, numTrials=101,
+               samplingSize=100000, diagnosticBool=False):
     """Steps 1-4 of run.main (run.py:193-303) in process.  Two ways to use several GPUs:
       rows  (default)  every file's rows are split over the ranks (helpers.splitRows); per-file tables are all-reduced and
                        score rows gathered on rank 0, which writes the files;
@@ -144,7 +145,7 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
     # temp_scores_*.npz (files written by other ranks, when whole files are dealt, are still read from disk)
     try:
         from . import roi as _roi_stage          # noqa: F401
-        roi_here = mode == "single" and dist.group_rank() == 0
+        roi_here = dist.group_rank() == 0
     except ImportError:
         roi_here = False
     session.handover_enabled = roi_here
@@ -167,9 +168,13 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
         elif dist.rank() == 0:
             roi.main(outputDirPath, stateInfo, fileTag, storedExpPath, roiWidth, verbose)
     else:
-        say("\nSTEP 4: p-values, regions of interest and figures are produced by the reference's "
-            "roiAndVisualPairwise from pairwiseDelta_*, temp_nullDistances_* and temp_quiescence_* in "
-            + str(outputDirPath))
+        from . import pairwise, roi_pairwise
+        seed = pairwise.run_seed() if pvalBool else None      # every rank takes part in drawing a fresh seed
+        say("\nSTEP 4: " + ("Fitting the null distribution, p-values and regions of interest" if pvalBool
+                            else "Pairwise metrics and regions of interest"))
+        if dist.rank() == 0:
+            roi_pairwise.main(outputDirPath, stateInfo, fileTag, storedExpPath, roiWidth, pvalBool, numTrials,
+                              samplingSize, diagnosticBool, verbose, backend=backend, seed=seed)
 
 
 @click.command(context_settings=dict(help_option_names=["-h", "--help"]))
@@ -190,11 +195,11 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
               help="Accepted for compatibility; parallelism comes from the GPUs of the torchrun launch")
 @click.option("-x", "--exit", "exitBool", is_flag=True, help="SLURM-only flag of the reference (ignored)")
 @click.option("-d", "--diagnostic-figures", "diagnosticBool", is_flag=True,
-              help="Paired mode diagnostic figures (produced by the reference's roiAndVisualPairwise, not here)")
+              help="Paired mode diagnostic figures (not built here: matplotlib is not a dependency; a note is printed)")
 @click.option("-t", "--num-trials", "numTrials", type=int, default=101, show_default=True,
-              help="The number of times subsamples of the scores are fit when using a null distribution")
+              help="Paired mode with -n: the number of subsamples of the null distances that are fit (the median fit is used)")
 @click.option("-z", "--sampling-size", "samplingSize", type=int, default=100000, show_default=True,
-              help="The size of the subsamples on which the scores are fit when using a null distribution")
+              help="Paired mode with -n: the size of each subsample of the null distances that is fit")
 @click.option("-q", "--quiescent-state", "quiescentState", type=int, default=-1,
               help="If a bin contains only states of this value, it is treated as quiescent and not factored into "
                    + "fitting. If set to 0, filtering is not done. [default: last state]")
@@ -204,7 +209,8 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
 @click.option("-v", "--version", "version", is_flag=True, help="Print the version number and exit")
 @click.option("-p", "--partition", "partition", type=str, help="SLURM-only option of the reference (ignored)")
 @click.option("-n", "--null-distribution", "pvalBool", is_flag=True,
-              help="Paired mode p-values (computed by the reference's roiAndVisualPairwise, not here)")
+              help="Paired mode: fit the null distribution and add p-values and Benjamini-Hochberg adjusted p-values to "
+                   + "pairwiseMetrics and regionsOfInterest")
 @click.option("-w", "--roi-width", "roiWidth", type=int, default=0,
               help="The number of bins in a region of interest [default: 50(single)/125(paired)]")
 @click.option("-f", "--file-tag", "fileTag", type=str, default="null",
@@ -277,7 +283,8 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
             pairs.append((f, match))
 
     run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
-               groupSize, stateInfo, roiWidth, verbose, say)
+               groupSize, stateInfo, roiWidth, verbose, say, pvalBool=pvalBool, numTrials=numTrials,
+               samplingSize=samplingSize, diagnosticBool=diagnosticBool)
     dist.barrier()
     if launched and td.is_initialized():
         td.destroy_process_group()

@@ -156,6 +156,37 @@ int epi_quiescent_mask(const uint16_t* cnt_a_dev, const uint16_t* cnt_b_dev, int
 int epi_pairwise_real_reduce(const float* delta_dev, int64_t rows, int32_t num_states, int32_t text_round_trip,
                              float* dist_out, int32_t* max_diff_out, void* stream);
 
+/* ---- paired statistics stage (roiAndVisualPairwise.py:177-242, csrc/pairwise_stats.cu) -----------------------
+ *   epi_null_compact       the null distances of the bins whose quiescent flag is 0 (all bins when quiescent_dev is NULL),
+ *                          stable order, every permutation: null_dev float32 [nperm][bins] -> pool_out [nperm][count]
+ *                          (sized nperm * bins by the caller), *count_out_dev (device int64) = count.  workspace_dev holds
+ *                          epi_null_compact_workspace_size(bins) bytes.
+ *   epi_null_subsample     trial t < trials takes the first `size` images of a keyed pseudo-random permutation of [0, n)
+ *                          (cycle-walking Feistel network, Philox4x32-10 rounds keyed by (seed, t)): size distinct indices
+ *                          per trial.  idx_out int32 [trials][size] and/or samples_out float32 [trials][size] = pool[idx].
+ *   epi_gennorm_fit        per trial, scipy.stats.gennorm.fit (rv_continuous.fit) of the `size` samples of that trial:
+ *                          optimize.fmin (Nelder-Mead, xatol = fatol = 1e-4, 600 iterations / evaluations) on
+ *                          _penalized_nnlf over (beta, loc, scale) from _fitstart (1, mean, std / sqrt(2)).  params_out
+ *                          float64 [trials][4] = beta, loc, scale, NLL of the best vertex (returned even when not converged);
+ *                          status_out int32 [trials][2] = iterations, converged (0/1).  Bit-reproducible run to run.
+ *   epi_gennorm_pvalues    p[i] = Q(1/beta, (|x[i] - loc| / scale)^beta), the regularized upper incomplete gamma in float64
+ *                          (= the two-sided 2 min(cdf, sf) of gennorm without the 1 - cdf cancellation); 1 at x == loc.
+ *   epi_bh_adjust          Benjamini-Hochberg (statsmodels multipletests fdr_bh): p sorted ascending (p >= 0), p_sorted /
+ *                          (rank / n), reverse cumulative minimum, clipped at 1, in input order.  workspace_dev holds
+ *                          epi_bh_workspace_size(n) bytes; n < 2^31. */
+int epi_null_compact_workspace_size(int64_t bins, int64_t* bytes_out);
+int epi_null_compact(const float* null_dev, const uint8_t* quiescent_dev, int64_t bins, int32_t nperm, float* pool_out,
+                     int64_t* count_out_dev, void* workspace_dev, int64_t workspace_bytes, void* stream);
+int epi_null_subsample(const float* pool_dev, int64_t n, int32_t trials, int32_t size, uint64_t seed, int32_t* idx_out,
+                       float* samples_out, void* stream);
+int epi_gennorm_fit(const float* samples_dev, int32_t trials, int32_t size, double* params_out, int32_t* status_out,
+                    void* stream);
+int epi_gennorm_pvalues(const float* x_dev, int64_t n, double beta, double loc, double scale, double* p_out,
+                        void* stream);
+int epi_bh_workspace_size(int64_t n, int64_t* bytes_out);
+int epi_bh_adjust(const double* p_dev, int64_t n, double* q_out, void* workspace_dev, int64_t workspace_bytes,
+                  void* stream);
+
 /* ---- whole path with HOST buffers (what expected.main -> expectedCombination.main -> scores.main
  *      compute for one in-memory matrix; run.py:196,231,246) ------------------------------------
  * x_host: int8 [bins][pitch] (any pitch >= cols; pinned memory makes the copies asynchronous).
@@ -254,6 +285,13 @@ int epi_scores_tsv_close(void* handle);
 int epi_write_scores_gz(const char* path, const char* chrom_names, const int32_t* chrom_id, const int64_t* starts,
                         const int64_t* ends, const float* scores, int64_t rows, int32_t num_states, int32_t level,
                         int32_t threads);
+/* pairwiseMetrics text through gzip, one line per bin: `chr \t start \t end \t <state name of max_diff (1-based)> \t
+ * "%.5f" of |distance| \t + or - (sign of distance) [\t "%.5e" p \t "%.5e" bh]`; the last two columns only when pval and
+ * bh are both given.  state_names: NUL-separated names of states 1..K.  Same deflate path as epi_write_scores_gz. */
+int epi_write_metrics_gz(const char* path, const char* chrom_names, const int32_t* chrom_id, const int64_t* starts,
+                         const int64_t* ends, const char* state_names, int32_t num_states, const int32_t* max_diff,
+                         const float* distance, const double* pval, const double* bh, int64_t rows, int32_t level,
+                         int32_t threads);
 /* ChromHMM `-printstatebyline` files (one per biosample and chromosome: `<biosample> <chr>`, `MaxState E`, then one label per
  * 200 bp bin) -> matrix: the native form of bin/preprocess_data_ChromHMM.sh:34-49, which pastes those files side by side.
  * epi_statebyline_read  parses ONE file into a column: out[r * stride] = label - 1 for bin r (out == NULL: count only);
