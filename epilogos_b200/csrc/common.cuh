@@ -79,7 +79,7 @@ typedef CUresult (*tensor_map_encode_fn)(CUtensorMap*, CUtensorMapDataType, cuui
 tensor_map_encode_fn get_tensor_map_encode();
 
 // tensor-core forms of the S2 table contractions (tc_tables.cu)
-int launch_k2_tc(const uint16_t* cnt, int64_t bins, int K, int width, int64_t* n1, int64_t* n2, cudaStream_t st);
+int launch_k2_tc(const uint16_t* cnt, int64_t bins, int K, int64_t* n1, int64_t* n2, cudaStream_t st);
 int scores_s2_tc(const uint16_t* cnt, int64_t bins, int K, int width, int64_t perms, const float* e, int* zero_flag,
                  float* o32, double* o64, cudaStream_t st);
 bool scores_s2_tc_eligible(int width);

@@ -22,8 +22,6 @@
 //    aliased states are separated exactly from sum(v) and sum(v^2), which cost one IDP4A each per
 //    4 bytes.  Models with more than 18 states use one-bit one-hot words (2 LOP3 per byte).
 //  * counts leave through shared memory as coalesced 16-byte stores of uint16 [bins][K].
-#include <stdlib.h>
-
 #include <utility>
 
 #include "common.cuh"
@@ -357,11 +355,9 @@ template <int BV, int MODE, bool SMALL = false>
 static int launch_k1(const CUtensorMap& tmap, int64_t bins, const K1Plan& pl, int num_states, uint16_t* cnt,
                           cudaStream_t stream) {
     constexpr int stage_bytes = (SMALL ? 8 : BV) * 16 * K1_ROWS;
-    int stages = (BV <= 3) ? 8 : (BV <= 9 ? 4 : 3);           // measured on B200 at 833 biosamples (tools/k1_sweep.py): 4 stages x 2 CTAs/SM: 2.22 ms;
+    const int stages = (BV <= 3) ? 8 : (BV <= 9 ? 4 : 3);     // measured on B200 at 833 biosamples: 4 stages x 2 CTAs/SM: 2.22 ms;
                                               // 3 x 2: 2.26, 5 x 2: 2.26, 3 x 3: 2.32, 2 x 4: 2.35, 6 x 1: 2.79
-    int ctas_per_sm = (BV <= 3 || SMALL) ? 3 : 2;           // small rows (127 x 15): 0.470 / 0.438 / 0.465 ms at 2 / 3 / 4 CTAs per SM
-    if (const char* e = getenv("EPI_K1_STAGES")) stages = atoi(e) > 0 ? atoi(e) : stages;      // tuning knobs
-    if (const char* e = getenv("EPI_K1_CTAS")) ctas_per_sm = atoi(e) > 0 ? atoi(e) : ctas_per_sm;
+    const int ctas_per_sm = (BV <= 3 || SMALL) ? 3 : 2;     // small rows (127 x 15): 0.470 / 0.438 / 0.465 ms at 2 / 3 / 4 CTAs per SM
     const size_t smem = (size_t)stages * stage_bytes + ((K1_ROWS * num_states * 2 + 15) & ~15) + 2 * stages * 8 +
                         (SMALL ? 1024 : 0);
     auto kern = k1_counts_kernel<BV, MODE, SMALL>;

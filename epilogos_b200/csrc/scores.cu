@@ -24,19 +24,16 @@
 //
 // Dispatch (dispatch_s2 below): with width <= 2047 the S2 TABLE evaluation runs on the tensor cores
 // (tc_tables.cu: the (LE c) mat-vec as an exact int8 tcgen05 product of the count bytes with base-256 digits
-// of -log2 E); the DFMA TABLE kernel in this file is the path for wider inputs and for EPI_K5_ALU=1, and the
-// DIRECT kernel is queued behind either, gated on the device-side "table has a zero" flag.
+// of -log2 E) and the DIRECT kernel is queued behind it, gated on the device-side "table has a zero" flag;
+// wider inputs take the DFMA TABLE kernel of this file, which switches to DIRECT itself on that flag.
 // S1 needs no re-association at all: its K x (width+1) value table is built with the reference expression
 // itself (k5_s1_table_kernel), so S1 scores are bit-equal to the float64 reference before the float32 cast.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace epi {
 
 constexpr int K5_THREADS = 256;
 constexpr int K5_WARPS = K5_THREADS / 32;
-constexpr int LC_MAX_WIDTH = 2047;        // log2(count) / count/width tables live in shared memory up to this width
 constexpr int KT_MAX = EPI_MAX_STATES;
 
 __constant__ __align__(16) double c_log2e[KT_MAX * KT_MAX];     // S2: log2 E[s][t], row stride KT; S1: log2 E[s]
@@ -198,7 +195,7 @@ __global__ void __launch_bounds__(K5_THREADS) k5_s1_direct_kernel(const uint16_t
 }
 
 // ---- S2 -----------------------------------------------------------------------------------------
-template <int KT, bool USE_LC>
+template <int KT>
 __global__ void __launch_bounds__(K5_THREADS) k5_s2_kernel(const uint16_t* __restrict__ cnt, long long bins, int K,
                                                            int width, double perms, const float* __restrict__ exp2,
                                                            const PrepFlags* __restrict__ flags, int force_direct,
@@ -209,15 +206,12 @@ __global__ void __launch_bounds__(K5_THREADS) k5_s2_kernel(const uint16_t* __res
     uint16_t* cslab = reinterpret_cast<uint16_t*>(smem_raw);                          // K5_WARPS * 2 * 32 * K u16
     float* fslab = reinterpret_cast<float*>(smem_raw + K5_WARPS * 32 * K * 4);        // K5_WARPS * 32 * K f32
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + K5_WARPS * 32 * K * 8);   // K5_WARPS * 2
-    double* lc = reinterpret_cast<double*>(bars + K5_WARPS * 2);                      // width + 1
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     if (tid == 0) {
         for (int i = 0; i < K5_WARPS * 2; ++i) mbar_init(&bars[i], 1);
         mbar_fence_init();
     }
-    if (USE_LC)
-        for (int i = tid; i <= width; i += K5_THREADS) lc[i] = i > 0 ? log2((double)i) : 0.0;
     __syncthreads();
     const double lp = log2(perms);
     const double inv_perms = 1.0 / perms;
@@ -258,7 +252,7 @@ __global__ void __launch_bounds__(K5_THREADS) k5_s2_kernel(const uint16_t* __res
                 for (int s = 0; s < KT; ++s) {
                     const int c = s < K ? row[s] : 0;
                     cd[s] = (double)c;
-                    const double l = USE_LC ? lc[c] : (c > 0 ? log2((double)c) : 0.0);
+                    const double l = c > 0 ? log2((double)c) : 0.0;
                     a = fma(cd[s], l, a);
                     w += cd[s];
                     mc[s] = 0.0;
@@ -279,8 +273,8 @@ __global__ void __launch_bounds__(K5_THREADS) k5_s2_kernel(const uint16_t* __res
                     if (q < K) {
                         const int c = row[q];
                         const int cm = c > 0 ? c - 1 : 0;
-                        const double lt = USE_LC ? lc[c] : (c > 0 ? log2((double)c) : 0.0);
-                        const double l1 = USE_LC ? lc[cm] : (cm > 0 ? log2((double)cm) : 0.0);
+                        const double lt = c > 0 ? log2((double)c) : 0.0;
+                        const double l1 = cm > 0 ? log2((double)cm) : 0.0;
                         double br = (a - mc[q]) + c_log2e[q * KT + q];
                         br = fma(lt - lp, wm1, br);
                         br = fma(-cd[q], lt, br);
@@ -300,11 +294,6 @@ __global__ void __launch_bounds__(K5_THREADS) k5_s2_kernel(const uint16_t* __res
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-static int k5_ctas_per_sm(int dflt) {
-    if (const char* e = getenv("EPI_K5_CTAS")) return atoi(e) > 0 ? atoi(e) : dflt;      // tuning knob
-    return dflt;
-}
-
 // builds the log2 table in the device workspace, copies it into constant memory (device-to-device, stream ordered)
 static int prepare_tables(const float* e, int rows, int cols, int kt, cudaStream_t st, const PrepFlags** flags_out) {
     DeviceWorkspace* ws = device_workspace();
@@ -348,26 +337,26 @@ static int launch_s1(const uint16_t* cnt, int64_t bins, int K, int width, const 
         auto kern = k5_s1_kernel<true, K5_THREADS>;
         EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(base + table)));
         const int per_sm = (int)((size_t)220 * 1024 / (base + table + 1024));
-        kern<<<persistent_grid(ntiles, k5_ctas_per_sm(per_sm < 1 ? 1 : (per_sm > 4 ? 4 : per_sm))), K5_THREADS, base + table, st>>>(
+        kern<<<persistent_grid(ntiles, per_sm < 1 ? 1 : (per_sm > 4 ? 4 : per_sm)), K5_THREADS, base + table, st>>>(
             cnt, bins, K, width, v32, v64, o32, o64);
     } else {
         auto kern = k5_s1_kernel<false, K5_THREADS>;
         EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)base));
-        kern<<<persistent_grid(ntiles, k5_ctas_per_sm(4)), K5_THREADS, base, st>>>(cnt, bins, K, width, v32, v64, o32, o64);
+        kern<<<persistent_grid(ntiles, 4), K5_THREADS, base, st>>>(cnt, bins, K, width, v32, v64, o32, o64);
     }
     EPI_CUDA(cudaGetLastError());
     return 0;
 }
 
-template <int KT, bool USE_LC>
+template <int KT>
 static int launch_s2(const uint16_t* cnt, int64_t bins, int K, int width, int64_t perms, const float* e,
                      const PrepFlags* flags, int direct, float* o32, double* o64, cudaStream_t st) {
-    auto kern = k5_s2_kernel<KT, USE_LC>;
-    const size_t smem = (size_t)K5_WARPS * 32 * K * 8 + K5_WARPS * 16 + (USE_LC ? (size_t)(width + 1) * 8 : 0);
+    auto kern = k5_s2_kernel<KT>;
+    const size_t smem = (size_t)K5_WARPS * 32 * K * 8 + K5_WARPS * 16;
     EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int64_t ntiles = (bins + K5_THREADS - 1) / K5_THREADS;
-    kern<<<persistent_grid(ntiles, k5_ctas_per_sm(3)), K5_THREADS, smem, st>>>(cnt, bins, K, width, (double)perms, e, flags, direct,
-                                                               o32, o64);
+    kern<<<persistent_grid(ntiles, 3), K5_THREADS, smem, st>>>(cnt, bins, K, width, (double)perms, e, flags, direct, o32,
+                                                                o64);
     EPI_CUDA(cudaGetLastError());
     return 0;
 }
@@ -376,18 +365,16 @@ template <int KT>
 static int dispatch_s2(const uint16_t* cnt, int64_t bins, int K, int width, int64_t perms, const float* e, float* o32,
                        double* o64, int mode, cudaStream_t st) {
     const PrepFlags* flags = nullptr;
-    if (mode == EPI_SCORE_TABLE && scores_s2_tc_eligible(width) && getenv("EPI_K5_ALU") == nullptr) {
+    if (mode == EPI_SCORE_TABLE && scores_s2_tc_eligible(width)) {
         // tensor-core mat-vec (tc_tables.cu); a table with zero entries makes it a no-op and un-gates the DIRECT kernel
         DeviceWorkspace* ws = device_workspace();
         EPI_REQUIRE(ws != nullptr, "could not allocate the per-device workspace");
         PrepFlags* fl = &ws->prep_flags;
         if (int rc = scores_s2_tc(cnt, bins, K, width, perms, e, &fl->has_zero, o32, o64, st)) return rc;
-        return launch_s2<KT, true>(cnt, bins, K, width, perms, e, fl, 2, o32, o64, st);
+        return launch_s2<KT>(cnt, bins, K, width, perms, e, fl, 2, o32, o64, st);
     }
     if (int rc = prepare_tables(e, K, K, KT, st, &flags)) return rc;
-    const int direct = mode == EPI_SCORE_DIRECT;
-    if (width <= LC_MAX_WIDTH) return launch_s2<KT, true>(cnt, bins, K, width, perms, e, flags, direct, o32, o64, st);
-    return launch_s2<KT, false>(cnt, bins, K, width, perms, e, flags, direct, o32, o64, st);
+    return launch_s2<KT>(cnt, bins, K, width, perms, e, flags, mode == EPI_SCORE_DIRECT, o32, o64, st);
 }
 
 }  // namespace epi

@@ -11,8 +11,6 @@
 //
 // Both replace ALU / fp64-pipe loops that were the limiters of K2 (IMAD) and K5 (324 DFMA per bin); what is left per
 // bin is byte shuffling for K2 and ~7 fp64 operations per state for K5.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tc05.cuh"
 #include "count_tile.cuh"
@@ -167,8 +165,7 @@ static int launch_k2_tc_impl(const uint16_t* cnt, int64_t bins, int K, int64_t* 
     auto kern = k2_tc_kernel<KT, KR>;
     EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int64_t ntiles = (bins + T2_BINS - 1) / T2_BINS;
-    int ctas = 4;          // measured at 15.5 M bins x 18 states: 0.33 / 0.22 / 0.19 ms at 1 / 2 / 3 CTAs per SM (6 stages), 0.185 at 4 (4 stages)
-    if (const char* e = getenv("EPI_K2TC_CTAS")) ctas = atoi(e) > 0 ? atoi(e) : ctas;      // tuning knob
+    const int ctas = 4;    // measured at 15.5 M bins x 18 states: 0.33 / 0.22 / 0.19 ms at 1 / 2 / 3 CTAs per SM (6 stages), 0.185 at 4 (4 stages)
     kern<<<persistent_grid(ntiles, ctas), T2_THREADS, smem, st>>>(cnt, (long long)bins, K,
                                                                 reinterpret_cast<unsigned long long*>(n1),
                                                                 reinterpret_cast<unsigned long long*>(n2));
@@ -176,8 +173,7 @@ static int launch_k2_tc_impl(const uint16_t* cnt, int64_t bins, int K, int64_t* 
     return 0;
 }
 
-int launch_k2_tc(const uint16_t* cnt, int64_t bins, int K, int width, int64_t* n1, int64_t* n2, cudaStream_t st) {
-    (void)width;
+int launch_k2_tc(const uint16_t* cnt, int64_t bins, int K, int64_t* n1, int64_t* n2, cudaStream_t st) {
     if (K == 18) return launch_k2_tc_impl<18, 18>(cnt, bins, K, n1, n2, st);
     if (K == 15) return launch_k2_tc_impl<16, 15>(cnt, bins, K, n1, n2, st);
     if (K <= 16) return launch_k2_tc_impl<16, 0>(cnt, bins, K, n1, n2, st);
