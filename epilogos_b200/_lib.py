@@ -13,6 +13,7 @@ LIB_PATH = Path(__file__).resolve().parent / "libepilogos_b200.so"
 EPI_SCORE_TABLE = 0
 EPI_SCORE_DIRECT = 1
 EPI_MAX_STATES = 32
+EPI_MAX_GROUPS = 64
 
 # name -> (restype, argtypes); mirrors include/epilogos_b200.h one to one
 PROTOTYPES = {
@@ -20,6 +21,9 @@ PROTOTYPES = {
     "epi_last_error": (c_char_p, []),
     "epi_device_info": (c_int, [POINTER(c_int), POINTER(c_int), POINTER(c_int)]),
     "epi_bin_counts": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_void_p, c_void_p]),
+    "epi_group_counts": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_void_p, c_void_p, c_int32, c_void_p,
+                                 c_void_p]),
+    "epi_gather_columns": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_void_p, c_int32, c_void_p, c_int64, c_void_p]),
     "epi_expected_s1s2": (c_int, [c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
     "epi_normalize_i64": (c_int, [c_void_p, c_int64, c_void_p, c_void_p]),
     "epi_scores_s1": (c_int, [c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),

@@ -40,6 +40,18 @@ class CudaBackend:
         with timing.stage("kernels", sync_cuda=True):
             return engine.bin_counts(x, states0.shape[1], num_states)
 
+    def group_counts(self, x_dev, cols, num_states, groups):
+        """Counts of every column group (lists of 0-based columns) of a device matrix, one pass: a list of [rows, K]
+        blocks.  The count kernels' consumers need 16-byte aligned counts, so a block that does not start on 16 bytes
+        (rows * K * 2 not a multiple of 16) is copied."""
+        with timing.stage("kernels", sync_cuda=True):
+            cnt = engine.group_counts(x_dev, cols, num_states, groups)
+        return [c if c.data_ptr() % 16 == 0 else c.clone() for c in cnt]
+
+    def gather_columns(self, x_dev, cols, idx):
+        """The matrix of the columns idx of a device matrix, on the device."""
+        return engine.gather_columns(x_dev, cols, idx)
+
     def add_counts(self, cnt_a, cnt_b):
         """Counts of the concatenated matrix [A | B] (helpers.py:173-179) = sum of the group counts."""
         return (cnt_a + cnt_b).contiguous()
@@ -69,7 +81,8 @@ class CudaBackend:
 
     # -- S3 ------------------------------------------------------------------------------------------
     def states_to_device(self, states0):
-        return self._upload(states0)
+        on_device = getattr(states0, "device_matrix", None)      # a group's columns, gathered on the device (groups.py)
+        return on_device() if on_device is not None else self._upload(states0)
 
     def s3_tiles(self, x_dev, width, num_states):
         """Upper-triangular tiles of the shard's one-hot Gram matrix (int32): the tensor that is all-reduced."""

@@ -24,20 +24,12 @@
 //  * counts leave through shared memory as coalesced 16-byte stores of uint16 [bins][K].
 #include <utility>
 
-#include "common.cuh"
+#include "count_planes.cuh"
 
 namespace epi {
 
 constexpr int K1_ROWS = 128;                 // bins per tile == consumer threads
 constexpr int K1_THREADS = K1_ROWS + 32;     // + producer warp
-
-enum { MODE_F2 = 0, MODE_F2M = 1, MODE_B1 = 2 };
-
-template <int MODE>
-struct PlaneCount {
-    static constexpr int N = (MODE == MODE_B1) ? 10 : 9;        // bit-sliced counter depth
-    static constexpr int CAP = (1 << N) - 1;                    // words that may be added before a flush
-};
 
 // Per-chunk register image of one row (the raw label words).  Pipe balance matters here: the kernel is bound
 // by the integer ALU pipe (SHF/LOP3/IADD3, 64 lanes/clk/SM), while the FMA pipe (IMAD/IDP, 128 lanes/clk/SM)
@@ -78,54 +70,6 @@ struct ChunkSrc {
     }
 };
 
-// Depth-first carry-save tree: Tree<L>::get<I> folds 2^L consecutive words into planes p[0..L-1] and
-// returns the carry word of weight 2^L.
-template <int L>
-struct Tree {
-    template <int I, class Src, int NP>
-    static __device__ __forceinline__ uint32_t get(const Src& src, uint32_t (&p)[NP]) {
-        uint32_t a = Tree<L - 1>::template get<2 * I>(src, p);
-        uint32_t b = Tree<L - 1>::template get<2 * I + 1>(src, p);
-        uint32_t s = lop3_xor3(p[L - 1], a, b);
-        uint32_t c = lop3_maj(p[L - 1], a, b);
-        p[L - 1] = s;
-        return c;
-    }
-};
-template <>
-struct Tree<0> {
-    template <int I, class Src, int NP>
-    static __device__ __forceinline__ uint32_t get(const Src& src, uint32_t (&)[NP]) {
-        return src.template tword<I>();
-    }
-};
-
-// Fold N words of weight 2^L into planes p[L..]; odd leftovers go through a half adder.
-template <int L, int N, int NP>
-struct Reduce {
-    static __device__ __forceinline__ void run(const uint32_t (&w)[N], uint32_t (&p)[NP]) {
-        if constexpr (L >= NP - 1) {
-#pragma unroll
-            for (int i = 0; i < N; ++i) p[NP - 1] ^= w[i];
-        } else {
-            constexpr int NPAIR = N / 2;
-            constexpr int NN = NPAIR + (N & 1);
-            uint32_t nx[NN];
-#pragma unroll
-            for (int i = 0; i < NPAIR; ++i) {
-                uint32_t s = lop3_xor3(p[L], w[2 * i], w[2 * i + 1]);
-                nx[i] = lop3_maj(p[L], w[2 * i], w[2 * i + 1]);
-                p[L] = s;
-            }
-            if constexpr (N & 1) {
-                nx[NPAIR] = p[L] & w[N - 1];
-                p[L] ^= w[N - 1];
-            }
-            Reduce<L + 1, NN, NP>::run(nx, p);
-        }
-    }
-};
-
 template <int BV, int MODE, int NP, int... G>
 __device__ __forceinline__ void fold_groups(const ChunkSrc<BV, MODE>& src, uint32_t (&p)[NP],
                                             std::integer_sequence<int, G...>) {
@@ -156,21 +100,6 @@ __device__ __forceinline__ void process_chunk(const uint4* __restrict__ row, uin
     }
     constexpr int NG = (MODE == MODE_B1) ? BV : BV / 3;      // groups of 16 words
     fold_groups<BV, MODE, NP>(src, p, std::make_integer_sequence<int, NG>{});
-}
-
-// bit-sliced planes -> packed 16-bit counters, then clear the planes
-template <int MODE, int NP, int NACC>
-__device__ __forceinline__ void flush_planes(uint32_t (&p)[NP], uint32_t (&acc)[NACC]) {
-#pragma unroll
-    for (int k = 0; k < NP; ++k) {
-#pragma unroll
-        for (int f = 0; f < NACC; ++f) {
-            // lo half: state/field f, hi half: state f+16 / field f+8.  acc += t * 2^k as one IMAD.
-            const uint32_t t = (MODE == MODE_B1) ? ((p[k] >> f) & 0x00010001u) : ((p[k] >> (2 * f)) & 0x00030003u);
-            asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(acc[f]) : "r"(t), "r"(1u << k));
-        }
-        p[k] = 0;
-    }
 }
 
 // SMALL (rows of at most 128 bytes, one chunk of BV = 9 vectors, two-bit modes): the box is 128 bytes wide and written by
@@ -263,39 +192,7 @@ k1_counts_kernel(const __grid_constant__ CUtensorMap tmap, long long bins, int n
 
         // ---- unpack the counters into per-state counts ----
         uint32_t cs[EPI_MAX_STATES];
-        if constexpr (MODE == MODE_B1) {
-#pragma unroll
-            for (int f = 0; f < 16; ++f) {
-                cs[f] = acc[f] & 0xffffu;
-                cs[f + 16] = acc[f] >> 16;
-            }
-            cs[0] -= (uint32_t)npad;
-        } else {
-#pragma unroll
-            for (int f = 0; f < 8; ++f) {
-                cs[f] = acc[f] & 0xffffu;
-                cs[f + 8] = acc[f] >> 16;
-            }
-#pragma unroll
-            for (int f = 16; f < EPI_MAX_STATES; ++f) cs[f] = 0;
-            if constexpr (MODE == MODE_F2M) {
-                // states 16 and 17 landed in fields 0 and 1; separate them with sum(v) and sum(v^2)
-                uint32_t m1 = 0, m2 = 0;
-#pragma unroll
-                for (int f = 1; f < 16; ++f) {
-                    m1 += f * cs[f];
-                    m2 += f * f * cs[f];
-                }
-                const uint32_t hi = (sum1 - m1) >> 4;                    // c16 + c17
-                const uint32_t c17 = ((sum2 - m2) - 256u * hi) >> 5;     // 256*c16 + 288*c17 - 256*(c16+c17)
-                const uint32_t c16 = hi - c17;
-                cs[16] = c16;
-                cs[17] = c17;
-                cs[0] -= c16;
-                cs[1] -= c17;
-            }
-            cs[0] -= (uint32_t)npad;
-        }
+        unpack_counts<MODE, NACC>(acc, sum1, sum2, npad, cs);
 
         // ---- stage the warp's 32 rows and write them with 16-byte stores ----
         uint16_t* wrow = out_stage + (size_t)tid * num_states;

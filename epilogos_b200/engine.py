@@ -56,6 +56,33 @@ def bin_counts(x, cols, num_states, out=None):
     return out
 
 
+def group_counts(x, cols, num_states, groups):
+    """Counts of column groups of one matrix, read once.  x: CUDA int8 [bins, pitch]; groups: sequences of 0-based column
+    indices.  Returns CUDA int16 [len(groups), bins, K] holding uint16 counts; block g is bin_counts of group g's columns."""
+    _require_cuda(x, torch.int8, "x")
+    bins, pitch = x.shape
+    lists = [np.asarray(g, dtype=np.int32).ravel() for g in groups]
+    offsets = np.concatenate(([0], np.cumsum([len(g) for g in lists]))).astype(np.int32)
+    flat = torch.from_numpy(np.concatenate(lists) if lists else np.zeros(0, np.int32)).to(x.device)
+    offs = torch.from_numpy(offsets).to(x.device)
+    out = torch.empty((len(lists), bins, num_states), dtype=torch.int16, device=x.device)
+    _lib.call("epi_group_counts", _ptr(x), bins, int(cols), pitch, int(num_states), _ptr(flat), _ptr(offs), len(lists),
+              _ptr(out), _stream())
+    return out
+
+
+def gather_columns(x, cols, idx):
+    """The columns idx (0-based, in the given order) of x (CUDA int8 [bins, pitch]) as a new CUDA int8
+    [bins, pitch_for(len(idx))] matrix with zero pad bytes."""
+    _require_cuda(x, torch.int8, "x")
+    bins, pitch = x.shape
+    idx_dev = torch.from_numpy(np.asarray(idx, dtype=np.int32).ravel()).to(x.device)
+    n = idx_dev.numel()
+    out = torch.empty((bins, pitch_for(max(n, 1))), dtype=torch.int8, device=x.device)
+    _lib.call("epi_gather_columns", _ptr(x), bins, int(cols), pitch, _ptr(idx_dev), n, _ptr(out), out.shape[1], _stream())
+    return out
+
+
 def expected_tables(cnt, width, want_s1=True, want_s2=True):
     """K2.  Returns (n1 int64[K] or None, n2 int64[K,K] or None) for this shard."""
     _require_cuda(cnt, torch.int16, "cnt")

@@ -17,7 +17,7 @@ import numpy as np
 from . import dist, helpers, session
 
 
-def main(file1, file2, numStates, saliency, outputDir, fileTag, numProcesses, verbose, backend=None):
+def main(file1, file2, numStates, saliency, outputDir, fileTag, numProcesses, verbose, backend=None, group=None):
     tTotal = time()
     file1Path, file2Path, outputDirPath = Path(file1), Path(file2), Path(outputDir)
     filename = file1Path.name.split(".")[0]                                         # expected.py:31
@@ -28,7 +28,7 @@ def main(file1, file2, numStates, saliency, outputDir, fileTag, numProcesses, ve
     if not verbose and dist.rank() == 0:
         print("    {}\t".format(filename), end="", flush=True)
 
-    shard = session.load_shard(file1Path, file2Path, numStates, backend)
+    shard = session.load_shard(file1Path, file2Path, numStates, backend, group=group)
     table = calculateExpected(saliency, shard, numStates, backend)
     if dist.rank() == 0:
         storeExpArray(table, outputDirPath, fileTag, filename)

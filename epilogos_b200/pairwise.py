@@ -63,14 +63,15 @@ def shuffled_widths(c1, c2, groupSize):
 
 
 def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDirPath, expFreqPath, fileTag, filename,
-                            quiescentState, groupSize, verbose, backend=None, null_mode=None, seed=None, nperm=1):
+                            quiescentState, groupSize, verbose, backend=None, null_mode=None, seed=None, nperm=1,
+                            group=None):
     if saliency not in (1, 2):
         raise ValueError("Please ensure that saliency metric is either 1 or 2 for Pairwise Epilogos")
     null_mode = null_mode or os.environ.get("EPILOGOS_B200_NULL", "device")
     if null_mode not in ("reference", "device"):
         raise ValueError("null_mode must be 'reference' or 'device'")
     be = session.get_backend(backend)
-    shard = session.load_shard(file1Path, file2Path, numStates, backend)
+    shard = session.load_shard(file1Path, file2Path, numStates, backend, group=group)
     c1, c2 = shard.states_a.shape[1], shard.states_b.shape[1]
     size_a, size_b = shuffled_widths(c1, c2, groupSize)                            # helpers.py:190-194
     exp = be.to_device(np.load(expFreqPath, allow_pickle=False))

@@ -61,6 +61,24 @@ def checkFlags(mode, commandLineBool, inputDirectory, inputDirectory1, inputDire
                 return
 
 
+def checkGroupFlags(mode, inputDirectory, inputDirectory1, inputDirectory2, fileTag, groupFile, comparisons):
+    """Flag rules of --groups / --compare (checked before checkFlags): first violated rule prints and exits."""
+    rules = [
+        (comparisons and not groupFile, "ERROR: [--compare] requires [--groups]"),
+        (groupFile and not inputDirectory, "ERROR: [--groups] requires [-i, --input-directory]"),
+        (groupFile and inputDirectory1, "ERROR: [--groups] not compatible with [-a, --directory-one] option"),
+        (groupFile and inputDirectory2, "ERROR: [--groups] not compatible with [-b, --directory-two] option"),
+        (groupFile and fileTag != "null", "ERROR: [--groups] not compatible with [-f, --file-tag] option"),
+        (comparisons and mode != "paired", "ERROR: [--compare] requires [-m, --mode] 'paired'"),
+        (groupFile and mode == "paired" and not comparisons,
+         "ERROR: [-m, --mode] 'paired' with [--groups] requires at least one [--compare]"),
+    ]
+    for bad, message in rules:
+        if bad:
+            _die(message)
+            return
+
+
 def checkArguments(mode, saliency, inputDirPath, inputDirPath2, outputDirPath, numProcesses, numStates, numTrials,
                    samplingSize, quiescentState, groupSize, roiWidth):
     """Value checks (run.py:378-451): same exceptions / messages."""
@@ -113,7 +131,7 @@ def deal_files(pairs, world):
 
 def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
                groupSize, stateInfo, roiWidth, verbose, say, backend=None, pvalBool=False, numTrials=101,
-               samplingSize=100000, diagnosticBool=False):
+               samplingSize=100000, diagnosticBool=False, groups=None):
     """Steps 1-4 of run.main (run.py:193-303) in process.  Two ways to use several GPUs:
       rows  (default)  every file's rows are split over the ranks (helpers.splitRows); per-file tables are all-reduced and
                        score rows gathered on rank 0, which writes the files;
@@ -121,7 +139,12 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
                        run the unsharded stages on them and write their own outputs; the ranks meet at the barriers between
                        the stages and the per-file count tables are combined from the files, as the reference's SLURM jobs
                        do.  No file is inflated or parsed by more than one rank, and the text is written in parallel.
-    Integer tables make both identical to a single-rank run."""
+    Integer tables make both identical to a single-rank run.
+    `groups` (a --groups run): a list of (outputDirPath, fileTag, storedExpPath, groups.Selection), one per group (single
+    mode) or comparison (paired mode), run on the column subsets of the files of `pairs`, which are (file, "null").  Every
+    stage keeps the reference's order: step 1 tables all groups of a file from the same counts, step 2 runs per group, step
+    3 scores all groups of a file, step 4 runs per group.  A comparison passes the file itself as the stage drivers'
+    second file, which the group view does not read."""
     from contextlib import nullcontext
     from . import dist, expected, expectedCombination, scores, session
     world = dist.world_size()
@@ -131,15 +154,25 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
     if by_file:
         say("        Input files dealt to the ranks: {} files over {} GPUs".format(len(pairs), world))
 
+    runs = groups or [(outputDirPath, fileTag, storedExpPath, None)]
+    for out, _, _, _ in runs:
+        Path(out).mkdir(parents=True, exist_ok=True)
+
+    def second(f, f2, sel):
+        return f if sel is not None and sel.paired else f2
+
     with alone():
         session.prefetch(mine, numStates, backend)       # parse all files concurrently, once (the stages re-use them)
     say("\nSTEP 1: Per data file background frequency calculation")
     with alone():
         for f, f2 in mine:
-            expected.main(f, f2, numStates, saliency, outputDirPath, fileTag, numProcesses, verbose, backend=backend)
+            for out, tag, _, sel in runs:
+                expected.main(f, second(f, f2, sel), numStates, saliency, out, tag, numProcesses, verbose, backend=backend,
+                              group=sel)
     dist.barrier()
     say("\nSTEP 2: Background frequency combination")
-    expectedCombination.main(outputDirPath, storedExpPath, fileTag, verbose, backend=backend)
+    for out, tag, exp_path, _ in runs:
+        expectedCombination.main(out, exp_path, tag, verbose, backend=backend)
     say("\nSTEP 3: Score calculation")
     # step 4 runs in this process right after: rank 0 hands its score arrays over in memory instead of through
     # temp_scores_*.npz (files written by other ranks, when whole files are dealt, are still read from disk)
@@ -152,8 +185,9 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
     try:
         with alone():
             for f, f2 in mine:
-                scores.main(f, f2, numStates, saliency, outputDirPath, storedExpPath, fileTag, numProcesses, quiescentState,
-                            groupSize, verbose, backend=backend)
+                for out, tag, exp_path, sel in runs:
+                    scores.main(f, second(f, f2, sel), numStates, saliency, out, exp_path, tag, numProcesses,
+                                quiescentState, groupSize, verbose, backend=backend, group=sel)
     finally:
         session.handover_enabled = False
     dist.barrier()
@@ -166,15 +200,17 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
         if roi is None:
             say("    (region-of-interest selection is not part of this build; temp_scores_*.npz kept for roiSingle)")
         elif dist.rank() == 0:
-            roi.main(outputDirPath, stateInfo, fileTag, storedExpPath, roiWidth, verbose)
+            for out, tag, exp_path, _ in runs:
+                roi.main(out, stateInfo, tag, exp_path, roiWidth, verbose)
     else:
         from . import pairwise, roi_pairwise
         seed = pairwise.run_seed() if pvalBool else None      # every rank takes part in drawing a fresh seed
         say("\nSTEP 4: " + ("Fitting the null distribution, p-values and regions of interest" if pvalBool
                             else "Pairwise metrics and regions of interest"))
         if dist.rank() == 0:
-            roi_pairwise.main(outputDirPath, stateInfo, fileTag, storedExpPath, roiWidth, pvalBool, numTrials,
-                              samplingSize, diagnosticBool, verbose, backend=backend, seed=seed)
+            for out, tag, exp_path, _ in runs:
+                roi_pairwise.main(out, stateInfo, tag, exp_path, roiWidth, pvalBool, numTrials, samplingSize,
+                                  diagnosticBool, verbose, backend=backend, seed=seed)
 
 
 @click.command(context_settings=dict(help_option_names=["-h", "--help"]))
@@ -215,21 +251,40 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
               help="The number of bins in a region of interest [default: 50(single)/125(paired)]")
 @click.option("-f", "--file-tag", "fileTag", type=str, default="null",
               help="Tag to be appended in output filenames [default: input-directory_saliency]")
+@click.option("--groups", "groupFile", type=str,
+              help="Tab-separated file of biosample groups, one per line: name<TAB>columns (1-based biosample numbers and "
+                   + "ranges a-b, comma-separated).  Runs every group (single mode) or every --compare (paired mode) on "
+                   + "the column subsets of the files of -i, parsing each file once; outputs go to OUT/<group> or "
+                   + "OUT/<A>_vs_<B>")
+@click.option("--compare", "comparisons", type=str, multiple=True,
+              help="Paired mode with --groups: compare group A with group B (A:B, repeatable)")
 @click.option("--exp-freq-mem", "expFreqMem", type=int, default=20000, help="SLURM-only (ignored)")
 @click.option("--exp-comb-mem", "expCombMem", type=int, default=8000, help="SLURM-only (ignored)")
 @click.option("--score-mem", "scoreMem", type=int, default=40000, help="SLURM-only (ignored)")
 @click.option("--roi-mem", "roiMem", type=int, default=-1, help="SLURM-only (ignored)")
 def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2, outputDirectory, stateInfo, saliency,
          numProcesses, exitBool, diagnosticBool, numTrials, samplingSize, quiescentState, groupSize, version, partition,
-         pvalBool, roiWidth, fileTag, expFreqMem, expCombMem, scoreMem, roiMem):
+         pvalBool, roiWidth, fileTag, groupFile, comparisons, expFreqMem, expCombMem, scoreMem, roiMem):
     """Information-theoretic navigation of multi-tissue functional genomic annotations (B200 scoring path)."""
     if version:
         from epilogos_b200 import __version__
         print("Version:", __version__)
         sys.exit()
 
+    checkGroupFlags(mode, inputDirectory, inputDirectory1, inputDirectory2, fileTag, groupFile, comparisons)
+    if groupFile and mode == "paired":       # both groups of a comparison come from the files of -i
+        inputDirectory, inputDirectory1, inputDirectory2 = None, inputDirectory, inputDirectory
     checkFlags(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2, outputDirectory, stateInfo,
                exitBool, diagnosticBool, partition, pvalBool)
+    groupSet, pairs_of_groups = None, []
+    if groupFile:
+        from . import groups as _groups
+        try:
+            groupSet = _groups.parseGroups(groupFile)
+            pairs_of_groups = _groups.parseComparisons(comparisons, groupSet)
+        except _groups.GroupFileError as exc:
+            _die(str(exc))
+            return
     verbose = False
     numStates = getNumStates(stateInfo)
     # user-facing quiescent state is 1-based, 0 = no filtering (run.py:112-113)
@@ -271,7 +326,17 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
 
     files = sorted(p for p in inputDirPath.glob("*"))
     pairs = []
+    runs = None
+    if groupSet is not None:
+        # every group / comparison behaves like a run on its column-subset files in a directory named after it
+        sel = ([(g, "{}_s{}".format(g, saliency), groupSet.select(g)) for g in groupSet.names] if mode == "single" else
+               [("{}_vs_{}".format(a, b), "{}_{}_s{}".format(a, b, saliency), groupSet.select(a, b))
+                for a, b in pairs_of_groups])
+        runs = [(outputDirPath / d, tag, outputDirPath / d / "exp_freq_{}.npy".format(tag), s) for d, tag, s in sel]
     for f in files:
+        if runs is not None:
+            pairs.append((f, "null"))
+            continue
         if mode == "single":
             pairs.append((f, "null"))
         else:
@@ -284,7 +349,7 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
 
     run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
                groupSize, stateInfo, roiWidth, verbose, say, pvalBool=pvalBool, numTrials=numTrials,
-               samplingSize=samplingSize, diagnosticBool=diagnosticBool)
+               samplingSize=samplingSize, diagnosticBool=diagnosticBool, groups=runs)
     dist.barrier()
     if launched and td.is_initialized():
         td.destroy_process_group()

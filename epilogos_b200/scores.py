@@ -18,7 +18,7 @@ from . import dist, helpers, session, writer
 
 
 def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, numProcesses, quiescentState, groupSize,
-         verbose, backend=None):
+         verbose, backend=None, group=None):
     tTotal = time()
     file1Path, file2Path, outputDirPath = Path(file1), Path(file2), Path(outputDir)
     filename = file1Path.name.split(".")[0]
@@ -26,22 +26,22 @@ def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, num
         print("    {}\t".format(filename), end="", flush=True)
     if str(file2) == "null":
         calculateScores(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
-                        backend)
+                        backend, group=group)
     else:
         from .pairwise import calculateScoresPairwise
         calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDirPath, expFreqPath, fileTag,
-                                filename, quiescentState, groupSize, verbose, backend)
+                                filename, quiescentState, groupSize, verbose, backend, group=group)
     if dist.rank() == 0:
         print("Total Time:", time() - tTotal, flush=True) if verbose else print("\t[Done]", flush=True)
     dist.barrier()
 
 
 def calculateScores(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
-                    backend=None):
+                    backend=None, group=None):
     if saliency not in (1, 2, 3):
         raise ValueError("Please ensure that saliency metric is either 1, 2, or 3")
     be = session.get_backend(backend)
-    shard = session.load_shard(file1Path, Path("null"), numStates, backend)
+    shard = session.load_shard(file1Path, Path("null"), numStates, backend, group=group)
     exp = be.to_device(np.load(expFreqPath, allow_pickle=False))
     if saliency in (1, 2):
         local = be.scores(shard.counts(), shard.width, saliency, exp)

@@ -94,8 +94,10 @@ class Shard:
             raise FileNotFoundError(str(file1))
         pinned = getattr(self.backend, "name", "") == "cuda"
         split = (rank, world) if world else (dist.rank(), dist.world_size())
+        self.file = Path(file1)
         self._counts = {}
         self._states_dev = None
+        self._views = {}              # groups.GroupView of this shard, by selection
         self.reader = None            # the rank that read the file when the rows were dealt (one_reader); else None
         self.loc_full = None          # locations of ALL rows, on rank 0, when the rows were dealt
         if split[1] > 1 and one_reader():
@@ -221,7 +223,12 @@ def _key(file1, file2):
 _keep = 4
 
 
-def load_shard(file1, file2, num_states, backend=None, keep=None):
+def load_shard(file1, file2, num_states, backend=None, keep=None, group=None):
+    """The cached Shard of a file (pair).  With `group` (a groups.Selection) the shard of file1 alone is loaded and the
+    view of that group, or of that comparison of two groups, is returned; file2 is then not read."""
+    if group is not None:
+        from . import groups
+        return groups.view(load_shard(file1, "null", num_states, backend, keep), group)
     key = _key(file1, file2)
     if key not in _cache:
         while len(_cache) >= (keep or _keep):

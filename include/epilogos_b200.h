@@ -46,6 +46,22 @@ int epi_device_info(int* sm_count, int* cc_major, int* cc_minor);
 int epi_bin_counts(const int8_t* x_dev, int64_t bins, int32_t cols, int64_t pitch, int32_t num_states,
                    uint16_t* cnt_dev, void* stream);
 
+/* ---- column groups: counts of many column subsets of one matrix (csrc/groups.cu) ----------------------------
+ * A group is a list of columns of x: group g lists group_cols[group_offsets[g] .. group_offsets[g+1]) (device int32
+ * arrays; offsets start at 0 and increase strictly, every column is in [0, cols); a column may appear in several groups).
+ *   epi_group_counts    cnt[g][b][s] = #{ listed columns j of group g : x[b][j] == s }, uint16 [groups][bins][num_states]:
+ *                       each group's block has the layout of epi_bin_counts.  The matrix is read once for all groups;
+ *                       pitch and base need no alignment (an unaligned matrix is repacked first, as in epi_bin_counts).
+ *   epi_gather_columns  out[b][j] = x[b][idx[j]] for j < n; bytes n .. out_pitch of a row are zero (out_pitch a
+ *                       multiple of 16): the matrix of a group's columns, in the layout the kernels consume.
+ * Both copy the (small) column lists to the host to validate them, which synchronises the stream. */
+#define EPI_MAX_GROUPS 64
+int epi_group_counts(const int8_t* x_dev, int64_t bins, int32_t cols, int64_t pitch, int32_t num_states,
+                     const int32_t* group_cols_dev, const int32_t* group_offsets_dev, int32_t groups, uint16_t* cnt_dev,
+                     void* stream);
+int epi_gather_columns(const int8_t* x_dev, int64_t bins, int32_t cols, int64_t pitch, const int32_t* idx_dev, int32_t n,
+                       int8_t* out_dev, int64_t out_pitch, void* stream);
+
 /* ---- K2: S1 / S2 expected count tables from the per-bin counts -------------------------------
  * n1[s]    += sum_b cnt[b][s]                                   (expected.py:106-113, s1Calc)
  * n2[s][t] += sum_b cnt[b][s]*cnt[b][t] - [s==t]*cnt[b][s]      (expected.py:146-158, s2Calc)
