@@ -42,6 +42,14 @@ PROTOTYPES = {
                                          c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
     "epi_shuffled_counts_philox": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_uint64,
                                            c_int64, c_int32, c_void_p, c_void_p, c_void_p]),
+    "epi_shuffled_counts_philox_range": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32,
+                                                 c_uint64, c_int64, c_int64, c_int32, c_void_p, c_void_p, c_void_p]),
+    "epi_null_exceedances": (c_int, [c_void_p, c_void_p, c_int32, c_int64, c_int32, c_void_p, c_void_p, c_void_p]),
+    "epi_permutation_exceedances_s1": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_uint64,
+                                               c_int64, c_int64, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_void_p,
+                                               c_void_p]),
+    "epi_write_permutations_gz": (c_int, [c_char_p, c_char_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                          c_int64, c_int32, c_int32]),
     "epi_pairwise_combine": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p,
                                      c_void_p]),
     "epi_quiescent_mask": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p,

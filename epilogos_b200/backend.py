@@ -109,6 +109,38 @@ class CudaBackend:
                                                bin_offset=bin_offset)
         return (oa[0], ob[0]) if nperm == 1 else (oa, ob)
 
+    def permutation_exceedances(self, cnt_a, cnt_b, dist, nperm, seed, size_a, size_b, width, bin_offset, saliency, exp,
+                                score_widths, perms, exact=False, workspace_bytes=1 << 30):
+        """Per-bin permutation counts k[b] = #{p < nperm : |null(b, p)| >= |dist[b]|} (int32 tensor holding uint32): the
+        null distances of permutations 0 .. nperm-1 drawn as shuffled_counts_device draws them, A' scored at
+        score_widths[0] with perms[0], B' at score_widths[1] with perms[1], in the run's score mode (`exact`).
+        S1 runs the fused kernel (its TABLE and DIRECT values are the same numbers); S2 and tables wider than the S1
+        value table loop over bin chunks x permutation blocks of draw + score + count, whose device buffers stay below
+        `workspace_bytes`.  The result does not depend on that cap."""
+        rows, k_states = cnt_a.shape
+        exp = exp.to(self.device).contiguous()
+        dist = dist.to(self.device).contiguous()
+        k = torch.zeros(rows, dtype=torch.int32, device=self.device)
+        if saliency == 1 and max(score_widths) <= engine.S1_TABLE_MAX_WIDTH:
+            with timing.stage("kernels", sync_cuda=True):
+                return engine.permutation_exceedances_s1(cnt_a, cnt_b, size_a, size_b, seed, 0, nperm, width, bin_offset,
+                                                         exp, score_widths[0], score_widths[1], dist, k)
+        pairs = max(1, int(workspace_bytes) // (12 * k_states))       # A', B' counts (uint16) and scores (float32)
+        chunk = max(1, min(rows, pairs))
+        block = max(1, min(nperm, pairs // chunk))
+        with timing.stage("kernels", sync_cuda=True):
+            for lo in range(0, rows, chunk):
+                hi = min(rows, lo + chunk)
+                for p0 in range(0, nperm, block):
+                    n = min(block, nperm - p0)
+                    oa, ob = engine.shuffled_counts_philox_range(cnt_a[lo:hi], cnt_b[lo:hi], size_a, size_b, seed, p0, n,
+                                                                 width, bin_offset=bin_offset + lo)
+                    sa = self.scores(oa.reshape(-1, k_states), score_widths[0], saliency, exp, perms=perms[0], exact=exact)
+                    sb = self.scores(ob.reshape(-1, k_states), score_widths[1], saliency, exp, perms=perms[1], exact=exact)
+                    engine.null_exceedances(sa.reshape(n, hi - lo, k_states), sb.reshape(n, hi - lo, k_states),
+                                            dist[lo:hi], k[lo:hi])
+        return k
+
     def pairwise_combine(self, score_a, score_b, null_a, null_b):
         return engine.pairwise_combine(score_a, score_b, null_a, null_b)
 

@@ -64,6 +64,7 @@ struct DeviceWorkspace {
     K5TcConsts k5tc_consts;
     alignas(8) double s1_v64[EPI_MAX_STATES * (S1_TABLE_MAX_WIDTH + 1)];   // S1 value table [K][width + 1]
     alignas(8) float s1_v32[EPI_MAX_STATES * (S1_TABLE_MAX_WIDTH + 1)];    // its float32 rounding
+    alignas(8) float perm_v32[2][EPI_MAX_STATES * (S1_TABLE_MAX_WIDTH + 1)];  // permutations.cu: the tables of A', B'
 };
 static_assert(offsetof(DeviceWorkspace, k5tc_b_image) % 16 == 0, "the B operand image is a bulk-copy source");
 static_assert(offsetof(DeviceWorkspace, s1_v64) % 8 == 0 && offsetof(DeviceWorkspace, s1_v32) % 8 == 0,
@@ -77,6 +78,10 @@ typedef CUresult (*tensor_map_encode_fn)(CUtensorMap*, CUtensorMapDataType, cuui
                                          CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
                                          CUtensorMapFloatOOBfill);
 tensor_map_encode_fn get_tensor_map_encode();
+
+// K5-S1 value table [K][width + 1] of the expected table e (scores.cu): the float64 reference expression and its float32
+// rounding, the values epi_scores_s1 looks up in TABLE mode; width <= S1_TABLE_MAX_WIDTH
+int s1_value_table(const float* e, int K, int width, float* v32, double* v64, cudaStream_t st);
 
 // tensor-core forms of the S2 table contractions (tc_tables.cu)
 int launch_k2_tc(const uint16_t* cnt, int64_t bins, int K, int64_t* n1, int64_t* n2, cudaStream_t st);

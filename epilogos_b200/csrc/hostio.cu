@@ -1149,6 +1149,23 @@ extern "C" int epi_write_metrics_gz(const char* path, const char* chrom_names, c
     });
 }
 
+extern "C" int epi_write_permutations_gz(const char* path, const char* chrom_names, const int32_t* chrom_id,
+                                         const int64_t* starts, const int64_t* ends, const uint32_t* k,
+                                         const double* pval, const double* bh, int64_t rows, int32_t level,
+                                         int32_t threads) {
+    EPI_REQUIRE(path && chrom_names && starts && ends, "null pointer argument");
+    EPI_REQUIRE(rows == 0 || (k && pval && bh), "null pointer argument");
+    EPI_REQUIRE(rows >= 0, "bad shape");
+    const std::vector<const char*> names = split_names(chrom_names, max_chrom_id(chrom_id, rows) + 1);
+    size_t longest = 0;
+    for (const char* s : names) longest = std::max(longest, strlen(s));
+    return write_gz_rows(path, rows, longest + 160, level, threads, [&](char* p, int64_t r) {
+        p = format_location(p, names[chrom_id ? chrom_id[r] : 0], starts[r], ends[r]);
+        p += sprintf(p, "\t%u\t%.5e\t%.5e\n", (unsigned)k[r], pval[r], bh[r]);
+        return p;
+    });
+}
+
 // ---- ChromHMM `-printstatebyline` files -> matrix: the native form of bin/preprocess_data_ChromHMM.sh (SURVEY.md 8f, row f3).
 //      One file per biosample and chromosome: line 1 `<biosample> <chr>`, line 2 `MaxState E`, then one state label per 200 bp
 //      bin.  The script pastes the files of a chromosome side by side and prefixes every row with `chr, start, end`

@@ -1,0 +1,138 @@
+// Device pieces shared by the paired-mode kernels: the shuffle sampler of epi_shuffled_counts_philox (pairwise.cu) and
+// numpy's float32 row summation of epi_pairwise_combine.  The fused permutation kernel (permutations.cu) draws and
+// reduces with these same functions, so its null distances are the composed path's bit for bit.
+#pragma once
+#include "common.cuh"
+
+namespace epi {
+
+// Hypergeometric variate by inversion from the mode (zig-zag search): number of "successes" among n draws without
+// replacement from a population of N holding K successes.  Everything is float64: the uniform has 53 random bits (two
+// Philox words), pmf(mode) comes from a shared-memory table of log(i!), the pmf ratios of the walk are products of exact
+// integers with a shared-memory table of reciprocals 1/i (relative error ~1e-16 per step), so every outcome whose
+// probability exceeds ~1e-16 is reachable with its own probability -- the resolution of the reference's
+// argsort(np.random.rand(...)) shuffle, whose uniforms carry 53 bits as well (helpers.py:183).  The walk visits
+// O(standard deviation) values; it can run out of outcomes only through accumulated rounding (total mass 1 - O(1e-13)),
+// and then the residual goes to the last outcome visited on the heavier side.  Used per state instead of walking every
+// label of the row (6x fewer operations than per-label selection sampling at 833 biosamples).
+__device__ __forceinline__ double uniform53(Philox& rng) {
+    const uint32_t hi = rng.next(), lo = rng.next();
+    // (0, 1): 53 random bits + one half
+    return ((double)(hi >> 5) * 67108864.0 + (double)(lo >> 6) + 0.5) * (1.0 / 9007199254740992.0);
+}
+
+__device__ __forceinline__ int hypergeometric(Philox& rng, int N, int K, int n, const double* __restrict__ lf,
+                                              const double* __restrict__ inv) {
+    const int lo = max(0, n - (N - K)), hi = min(n, K);
+    if (lo >= hi) return lo;
+    int mode = (int)(((long long)(n + 1) * (K + 1)) / (N + 2));
+    mode = min(max(mode, lo), hi);
+    const double logp = (lf[K] - lf[mode] - lf[K - mode]) + (lf[N - K] - lf[n - mode] - lf[N - K - n + mode]) -
+                        (lf[N] - lf[n] - lf[N - n]);
+    const double pm = exp(logp);
+    double u = uniform53(rng) - pm;
+    if (u <= 0.0) return mode;
+    int xu = mode, xd = mode;
+    double pu = pm, pd = pm;
+    const int off = N - K - n;                       // may be negative; off + x >= 0 for every feasible x
+    for (;;) {
+        const bool can_up = xu < hi, can_dn = xd > lo;
+        if (!can_up && !can_dn) return pu >= pd ? xu : xd;     // rounding residue (~1e-13 of the mass)
+        if (can_up) {
+            // p(x+1)/p(x) = (K-x)(n-x) / ((x+1)(N-K-n+x+1)): integer products are exact in float64
+            pu *= ((double)(K - xu) * (double)(n - xu)) * (inv[xu + 1] * inv[off + xu + 1]);
+            ++xu;
+            u -= pu;
+            if (u <= 0.0) return xu;
+        }
+        if (can_dn) {
+            // p(x-1)/p(x) = x (N-K-n+x) / ((K-x+1)(n-x+1))
+            pd *= ((double)xd * (double)(off + xd)) * (inv[K - xd + 1] * inv[n - xd + 1]);
+            --xd;
+            u -= pd;
+            if (u <= 0.0) return xd;
+        }
+    }
+}
+
+// The Philox stream of one shuffle, keyed by (seed; permutation p, GLOBAL bin index gb).
+__device__ __forceinline__ Philox shuffle_stream(unsigned long long seed, uint32_t p, unsigned long long gb) {
+    Philox rng;
+    rng.key0 = (uint32_t)seed;
+    rng.key1 = (uint32_t)(seed >> 32);
+    rng.ctr[0] = 0;
+    rng.ctr[1] = p;
+    rng.ctr[2] = (uint32_t)gb;
+    rng.ctr[3] = (uint32_t)(gb >> 32);
+    rng.have = 0;
+    return rng;
+}
+
+// One uniform shuffle of a bin's combined row split into A' (size_a labels) and B' (size_b labels).  For count-based
+// scores it is a multivariate hypergeometric draw: walking over the states,
+//   a'_s ~ HG(remaining labels, c_s, still needed by A'),  b'_s ~ HG(remaining - needed by A', c_s - a'_s, needed by B').
+// emit(s, a'_s, b'_s) is called for s = 0..K-1 in order.
+template <class Emit>
+__device__ __forceinline__ void draw_shuffle(Philox& rng, const uint16_t* __restrict__ ca, const uint16_t* __restrict__ cb,
+                                             int K, int size_a, int size_b, const double* __restrict__ lf,
+                                             const double* __restrict__ inv, Emit emit) {
+    int remaining = 0;
+    for (int s = 0; s < K; ++s) remaining += (int)ca[s] + (int)cb[s];
+    int need_a = min(size_a, remaining);
+    int need_b = min(size_b, remaining - need_a);
+    for (int s = 0; s < K; ++s) {
+        const int c = (int)ca[s] + (int)cb[s];
+        int ga = 0, gb2 = 0;
+        if (c > 0) {
+            ga = hypergeometric(rng, remaining, c, need_a, lf, inv);
+            gb2 = hypergeometric(rng, remaining - need_a, c - ga, need_b, lf, inv);
+        }
+        remaining -= c;
+        need_a -= ga;
+        need_b -= gb2;
+        emit(s, ga, gb2);
+    }
+}
+
+// shared-memory tables of the sampler: log(i!), i = 0..width, then 1/i, i = 0..width+1
+__device__ __forceinline__ void fill_draw_tables(double* lf, double* inv, int width) {
+    for (int i = threadIdx.x; i <= width; i += blockDim.x) lf[i] = lgamma((double)i + 1.0);
+    for (int i = threadIdx.x; i <= width + 1; i += blockDim.x) inv[i] = i > 0 ? 1.0 / (double)i : 0.0;
+}
+
+// numpy float32 pairwise summation of n < 128 contiguous values (what np.sum(axis=1) does per row):
+// n < 8: left to right from 0; else 8 running sums over blocks of 8, a fixed combination tree, then the tail.
+template <class F>
+__device__ __forceinline__ float numpy_rowsum_f32(int n, F at) {
+    if (n < 8) {
+        float res = 0.f;
+        for (int i = 0; i < n; ++i) res = __fadd_rn(res, at(i));
+        return res;
+    }
+    float r[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) r[k] = at(k);
+    int i = 8;
+    for (; i < n - (n % 8); i += 8) {
+#pragma unroll
+        for (int k = 0; k < 8; ++k) r[k] = __fadd_rn(r[k], at(i + k));
+    }
+    float res = __fadd_rn(__fadd_rn(__fadd_rn(r[0], r[1]), __fadd_rn(r[2], r[3])),
+                          __fadd_rn(__fadd_rn(r[4], r[5]), __fadd_rn(r[6], r[7])));
+    for (; i < n; ++i) res = __fadd_rn(res, at(i));
+    return res;
+}
+
+// sum_s d_s^2 * sign(sum_s d_s), float32 in numpy's order, of d_s = at(s) (scores.py:231-232)
+template <class F>
+__device__ __forceinline__ float signed_sq_distance(int K, F at) {
+    const float sum = numpy_rowsum_f32(K, at);
+    const float sq = numpy_rowsum_f32(K, [&](int i) {
+        const float d = at(i);
+        return __fmul_rn(d, d);
+    });
+    const float sign = sum > 0.f ? 1.f : (sum < 0.f ? -1.f : (sum == 0.f ? 0.f : sum));      // np.sign (nan stays nan)
+    return __fmul_rn(sq, sign);
+}
+
+}  // namespace epi

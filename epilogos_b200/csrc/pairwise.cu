@@ -15,10 +15,11 @@
 //   epi_shuffled_counts_philox  P independent uniform shuffles per bin drawn on the device: multivariate hypergeometric
 //                               draws from the combined counts with a counter-based Philox4x32-10 stream keyed by
 //                               (seed, global bin index, permutation) -- results do not depend on grid shape, on the
-//                               sharding of the bins or on the GPU count.
+//                               sharding of the bins or on the GPU count.  epi_shuffled_counts_philox_range draws
+//                               permutations from an offset on, so a caller can batch them.
 //   epi_pairwise_combine        delta and signed squared null distance from the four float32 score arrays.
 //   epi_quiescent_mask          from the group counts: cntA[q] == C1 and cntB[q] == C2.
-#include "common.cuh"
+#include "paired_draw.cuh"
 
 namespace epi {
 
@@ -45,126 +46,30 @@ __global__ void __launch_bounds__(128) shuffled_counts_perm_kernel(
     }
 }
 
-// Hypergeometric variate by inversion from the mode (zig-zag search): number of "successes" among n draws without
-// replacement from a population of N holding K successes.  Everything is float64: the uniform has 53 random bits (two
-// Philox words), pmf(mode) comes from a shared-memory table of log(i!), the pmf ratios of the walk are products of exact
-// integers with a shared-memory table of reciprocals 1/i (relative error ~1e-16 per step), so every outcome whose
-// probability exceeds ~1e-16 is reachable with its own probability -- the resolution of the reference's
-// argsort(np.random.rand(...)) shuffle, whose uniforms carry 53 bits as well (helpers.py:183).  The walk visits
-// O(standard deviation) values; it can run out of outcomes only through accumulated rounding (total mass 1 - O(1e-13)),
-// and then the residual goes to the last outcome visited on the heavier side.  Used per state instead of walking every
-// label of the row (6x fewer operations than per-label selection sampling at 833 biosamples).
-__device__ __forceinline__ double uniform53(Philox& rng) {
-    const uint32_t hi = rng.next(), lo = rng.next();
-    // (0, 1): 53 random bits + one half
-    return ((double)(hi >> 5) * 67108864.0 + (double)(lo >> 6) + 0.5) * (1.0 / 9007199254740992.0);
-}
-
-__device__ __forceinline__ int hypergeometric(Philox& rng, int N, int K, int n, const double* __restrict__ lf,
-                                              const double* __restrict__ inv) {
-    const int lo = max(0, n - (N - K)), hi = min(n, K);
-    if (lo >= hi) return lo;
-    int mode = (int)(((long long)(n + 1) * (K + 1)) / (N + 2));
-    mode = min(max(mode, lo), hi);
-    const double logp = (lf[K] - lf[mode] - lf[K - mode]) + (lf[N - K] - lf[n - mode] - lf[N - K - n + mode]) -
-                        (lf[N] - lf[n] - lf[N - n]);
-    const double pm = exp(logp);
-    double u = uniform53(rng) - pm;
-    if (u <= 0.0) return mode;
-    int xu = mode, xd = mode;
-    double pu = pm, pd = pm;
-    const int off = N - K - n;                       // may be negative; off + x >= 0 for every feasible x
-    for (;;) {
-        const bool can_up = xu < hi, can_dn = xd > lo;
-        if (!can_up && !can_dn) return pu >= pd ? xu : xd;     // rounding residue (~1e-13 of the mass)
-        if (can_up) {
-            // p(x+1)/p(x) = (K-x)(n-x) / ((x+1)(N-K-n+x+1)): integer products are exact in float64
-            pu *= ((double)(K - xu) * (double)(n - xu)) * (inv[xu + 1] * inv[off + xu + 1]);
-            ++xu;
-            u -= pu;
-            if (u <= 0.0) return xu;
-        }
-        if (can_dn) {
-            // p(x-1)/p(x) = x (N-K-n+x) / ((K-x+1)(n-x+1))
-            pd *= ((double)xd * (double)(off + xd)) * (inv[K - xd + 1] * inv[n - xd + 1]);
-            --xd;
-            u -= pd;
-            if (u <= 0.0) return xd;
-        }
-    }
-}
-
-// One thread per (bin, permutation).  A uniform shuffle of the combined row split into A' (size_a labels) and
-// B' (size_b labels) is, for count-based scores, a multivariate hypergeometric draw: walking over the states,
-//   a'_s ~ HG(remaining labels, c_s, still needed by A'),  b'_s ~ HG(remaining - needed by A', c_s - a'_s, needed by B').
-// The Philox stream of a draw is keyed by (seed; permutation, GLOBAL bin index = bin_offset + local index): the result
-// for a bin does not depend on how the bins are sharded over GPUs or on the launch geometry.
+// One thread per (bin, permutation); the draw is draw_shuffle (paired_draw.cuh).  The Philox stream of a draw is keyed by
+// (seed; permutation = perm_offset + local index, GLOBAL bin index = bin_offset + local index): the result for a bin
+// does not depend on how the bins are sharded over GPUs, on how the permutations are batched or on the launch geometry.
 __global__ void __launch_bounds__(256) shuffled_counts_philox_kernel(
     const uint16_t* __restrict__ cnt_a, const uint16_t* __restrict__ cnt_b, long long bins, int K, int size_a,
-    int size_b, int width, unsigned long long seed, long long bin_offset, int nperm, uint16_t* __restrict__ out_a,
-    uint16_t* __restrict__ out_b) {
+    int size_b, int width, unsigned long long seed, long long bin_offset, long long perm_offset, int nperm,
+    uint16_t* __restrict__ out_a, uint16_t* __restrict__ out_b) {
     extern __shared__ double lf[];                            // log(i!), i = 0..width, then 1/i, i = 0..width+1
     double* inv = lf + (width + 1);
-    for (int i = threadIdx.x; i <= width; i += blockDim.x) lf[i] = lgamma((double)i + 1.0);
-    for (int i = threadIdx.x; i <= width + 1; i += blockDim.x) inv[i] = i > 0 ? 1.0 / (double)i : 0.0;
+    fill_draw_tables(lf, inv, width);
     __syncthreads();
     const long long total = bins * nperm;
     for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
          idx += (long long)gridDim.x * blockDim.x) {
         const long long p = idx / bins, b = idx - p * bins;        // permutation-major output [P][bins][K]
-        const unsigned long long gb = (unsigned long long)(bin_offset + b);
-        Philox rng;
-        rng.key0 = (uint32_t)seed;
-        rng.key1 = (uint32_t)(seed >> 32);
-        rng.ctr[0] = 0;
-        rng.ctr[1] = (uint32_t)p;
-        rng.ctr[2] = (uint32_t)gb;
-        rng.ctr[3] = (uint32_t)(gb >> 32);
-        rng.have = 0;
-        int remaining = 0;
-        for (int s = 0; s < K; ++s) remaining += (int)cnt_a[b * K + s] + (int)cnt_b[b * K + s];
-        int need_a = min(size_a, remaining);
-        int need_b = min(size_b, remaining - need_a);
-        for (int s = 0; s < K; ++s) {
-            const int c = (int)cnt_a[b * K + s] + (int)cnt_b[b * K + s];
-            int ga = 0, gb2 = 0;
-            if (c > 0) {
-                ga = hypergeometric(rng, remaining, c, need_a, lf, inv);
-                gb2 = hypergeometric(rng, remaining - need_a, c - ga, need_b, lf, inv);
-            }
-            remaining -= c;
-            need_a -= ga;
-            need_b -= gb2;
+        Philox rng = shuffle_stream(seed, (uint32_t)(perm_offset + p), (unsigned long long)(bin_offset + b));
+        draw_shuffle(rng, cnt_a + b * K, cnt_b + b * K, K, size_a, size_b, lf, inv, [&](int s, int ga, int gb) {
             out_a[idx * K + s] = (uint16_t)ga;
-            out_b[idx * K + s] = (uint16_t)gb2;
-        }
+            out_b[idx * K + s] = (uint16_t)gb;
+        });
     }
 }
 
 // ---------------------------------------------------------------- delta / null distance
-// numpy float32 pairwise summation of n < 128 contiguous values (what np.sum(axis=1) does per row):
-// n < 8: left to right from 0; else 8 running sums over blocks of 8, a fixed combination tree, then the tail.
-template <class F>
-__device__ __forceinline__ float numpy_rowsum_f32(int n, F at) {
-    if (n < 8) {
-        float res = 0.f;
-        for (int i = 0; i < n; ++i) res = __fadd_rn(res, at(i));
-        return res;
-    }
-    float r[8];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) r[k] = at(k);
-    int i = 8;
-    for (; i < n - (n % 8); i += 8) {
-#pragma unroll
-        for (int k = 0; k < 8; ++k) r[k] = __fadd_rn(r[k], at(i + k));
-    }
-    float res = __fadd_rn(__fadd_rn(__fadd_rn(r[0], r[1]), __fadd_rn(r[2], r[3])),
-                          __fadd_rn(__fadd_rn(r[4], r[5]), __fadd_rn(r[6], r[7])));
-    for (; i < n; ++i) res = __fadd_rn(res, at(i));
-    return res;
-}
-
 __global__ void __launch_bounds__(256) pairwise_combine_kernel(const float* __restrict__ sa, const float* __restrict__ sb,
                                                                const float* __restrict__ na, const float* __restrict__ nb,
                                                                long long rows, int K, float* __restrict__ delta,
@@ -176,13 +81,7 @@ __global__ void __launch_bounds__(256) pairwise_combine_kernel(const float* __re
         if (null_dist != nullptr && na != nullptr) {
             const float* pa = na + r * K;
             const float* pb = nb + r * K;
-            const float sum = numpy_rowsum_f32(K, [&](int i) { return __fsub_rn(pa[i], pb[i]); });
-            const float sq = numpy_rowsum_f32(K, [&](int i) {
-                const float d = __fsub_rn(pa[i], pb[i]);
-                return __fmul_rn(d, d);
-            });
-            const float sign = sum > 0.f ? 1.f : (sum < 0.f ? -1.f : (sum == 0.f ? 0.f : sum));      // np.sign (nan stays nan)
-            null_dist[r] = __fmul_rn(sq, sign);
+            null_dist[r] = signed_sq_distance(K, [&](int i) { return __fsub_rn(pa[i], pb[i]); });
         }
     }
 }
@@ -285,15 +184,18 @@ extern "C" int epi_shuffled_counts_perm(const int8_t* xa_dev, int64_t pitch_a, i
     return 0;
 }
 
-extern "C" int epi_shuffled_counts_philox(const uint16_t* cnt_a_dev, const uint16_t* cnt_b_dev, int64_t bins,
-                                          int32_t K, int32_t width, int32_t size_a, int32_t size_b, uint64_t seed,
-                                          int64_t bin_offset, int32_t nperm,
-                                          uint16_t* cnt_a_out, uint16_t* cnt_b_out, void* stream_) {
+extern "C" int epi_shuffled_counts_philox_range(const uint16_t* cnt_a_dev, const uint16_t* cnt_b_dev, int64_t bins,
+                                                int32_t K, int32_t width, int32_t size_a, int32_t size_b, uint64_t seed,
+                                                int64_t bin_offset, int64_t perm_offset, int32_t nperm,
+                                                uint16_t* cnt_a_out, uint16_t* cnt_b_out, void* stream_) {
     cudaStream_t st = static_cast<cudaStream_t>(stream_);
     if (check_device()) return 3;
     EPI_REQUIRE(bins >= 0 && K >= 1 && K <= EPI_MAX_STATES && nperm >= 1, "bad paired shape");
     EPI_REQUIRE(size_a >= 0 && size_b >= 0, "negative group size");
     EPI_REQUIRE(bin_offset >= 0, "negative bin offset");
+    EPI_REQUIRE(perm_offset >= 0 && perm_offset + nperm <= (1ll << 32),
+                "permutations %lld..%lld outside the 32-bit stream key", (long long)perm_offset,
+                (long long)perm_offset + nperm - 1);
     if (bins == 0) return 0;
     EPI_REQUIRE(cnt_a_dev && cnt_b_dev && cnt_a_out && cnt_b_out, "null pointer argument");
     EPI_REQUIRE(width >= 1 && width <= 65535, "width=%d (combined biosamples) out of range [1, 65535]", width);
@@ -305,10 +207,18 @@ extern "C" int epi_shuffled_counts_philox(const uint16_t* cnt_a_dev, const uint1
     EPI_REQUIRE(smem <= 200 * 1024, "too many combined biosamples (%d) for the shuffle kernel", width);
     EPI_CUDA(cudaFuncSetAttribute(shuffled_counts_philox_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     shuffled_counts_philox_kernel<<<grid_for(bins * nperm, 256, 8), 256, smem, st>>>(
-        cnt_a_dev, cnt_b_dev, bins, K, size_a, size_b, width, (unsigned long long)seed, (long long)bin_offset, nperm, cnt_a_out,
-        cnt_b_out);
+        cnt_a_dev, cnt_b_dev, bins, K, size_a, size_b, width, (unsigned long long)seed, (long long)bin_offset,
+        (long long)perm_offset, nperm, cnt_a_out, cnt_b_out);
     EPI_CUDA(cudaGetLastError());
     return 0;
+}
+
+extern "C" int epi_shuffled_counts_philox(const uint16_t* cnt_a_dev, const uint16_t* cnt_b_dev, int64_t bins,
+                                          int32_t K, int32_t width, int32_t size_a, int32_t size_b, uint64_t seed,
+                                          int64_t bin_offset, int32_t nperm,
+                                          uint16_t* cnt_a_out, uint16_t* cnt_b_out, void* stream_) {
+    return epi_shuffled_counts_philox_range(cnt_a_dev, cnt_b_dev, bins, K, width, size_a, size_b, seed, bin_offset, 0,
+                                            nperm, cnt_a_out, cnt_b_out, stream_);
 }
 
 extern "C" int epi_pairwise_combine(const float* score_a, const float* score_b, const float* null_a,

@@ -305,6 +305,13 @@ static int prepare_tables(const float* e, int rows, int cols, int kt, cudaStream
     return 0;
 }
 
+int s1_value_table(const float* e, int K, int width, float* v32, double* v64, cudaStream_t st) {
+    const int n = K * (width + 1);
+    k5_s1_table_kernel<<<(n + 255) / 256, 256, 0, st>>>(e, K, width, v32, v64);
+    EPI_CUDA(cudaGetLastError());
+    return 0;
+}
+
 static int launch_s1(const uint16_t* cnt, int64_t bins, int K, int width, const float* e, int direct, float* o32,
                      double* o64, cudaStream_t st) {
     if (direct || width > S1_TABLE_MAX_WIDTH) {
@@ -321,8 +328,7 @@ static int launch_s1(const uint16_t* cnt, int64_t bins, int K, int width, const 
     double* v64 = ws->s1_v64;
     float* v32 = ws->s1_v32;
     const int n = K * (width + 1);
-    k5_s1_table_kernel<<<(n + 255) / 256, 256, 0, st>>>(e, K, width, v32, v64);
-    EPI_CUDA(cudaGetLastError());
+    if (int rc = s1_value_table(e, K, width, v32, v64, st)) return rc;
     const size_t base = (size_t)K5_WARPS * 32 * K * 8 + K5_WARPS * 16;
     const size_t table = (size_t)n * 4;
     const int64_t ntiles = (bins + K5_THREADS - 1) / K5_THREADS;

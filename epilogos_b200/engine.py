@@ -12,6 +12,8 @@ import torch
 from . import _lib
 from ._lib import EPI_SCORE_DIRECT, EPI_SCORE_TABLE  # noqa: F401
 
+S1_TABLE_MAX_WIDTH = 4095      # widest score width of the S1 value table (csrc/common.cuh)
+
 
 def _stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
@@ -397,6 +399,51 @@ def shuffled_counts_philox(cnt_a, cnt_b, size_a, size_b, seed, nperm=1, width=No
               int(width if width is not None else size_a + size_b), int(size_a), int(size_b),
               ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(nperm), _ptr(oa), _ptr(ob), _stream())
     return oa, ob
+
+
+def shuffled_counts_philox_range(cnt_a, cnt_b, size_a, size_b, seed, perm_offset, nperm, width, bin_offset=0):
+    """shuffled_counts_philox for permutations perm_offset .. perm_offset + nperm - 1: int16 tensors [nperm, bins, K]."""
+    _require_cuda(cnt_a, torch.int16, "cnt_a")
+    _require_cuda(cnt_b, torch.int16, "cnt_b")
+    bins, k = cnt_a.shape
+    oa = torch.empty((nperm, bins, k), dtype=torch.int16, device=cnt_a.device)
+    ob = torch.empty((nperm, bins, k), dtype=torch.int16, device=cnt_a.device)
+    _lib.call("epi_shuffled_counts_philox_range", _ptr(cnt_a), _ptr(cnt_b), bins, k, int(width), int(size_a), int(size_b),
+              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(perm_offset), int(nperm), _ptr(oa), _ptr(ob),
+              _stream())
+    return oa, ob
+
+
+def null_exceedances(null_a, null_b, dist, k):
+    """k[b] += #{p : |null distance of (null_a[p, b], null_b[p, b])| >= |dist[b]|}.  null_a, null_b: float32 score arrays
+    [nperm, bins, K]; dist: float32 [bins]; k: int32 [bins] holding uint32 counts (updated in place)."""
+    _require_cuda(null_a, torch.float32, "null_a")
+    _require_cuda(null_b, torch.float32, "null_b")
+    _require_cuda(dist, torch.float32, "dist")
+    _require_cuda(k, torch.int32, "k")
+    nperm, bins, K = null_a.shape
+    if tuple(null_b.shape) != (nperm, bins, K) or dist.numel() != bins or k.numel() != bins:
+        raise ValueError("null_a, null_b must be [nperm, bins, K] and dist, k [bins]")
+    _lib.call("epi_null_exceedances", _ptr(null_a), _ptr(null_b), int(nperm), bins, K, _ptr(dist), _ptr(k), _stream())
+    return k
+
+
+def permutation_exceedances_s1(cnt_a, cnt_b, size_a, size_b, seed, perm_offset, nperm, width, bin_offset, exp1, width_a,
+                               width_b, dist, k):
+    """Fused S1 permutation counts: k[b] += #{p : |null(b, p)| >= |dist[b]|} over permutations perm_offset ..
+    perm_offset + nperm - 1, A' scored at width_a and B' at width_b against exp1.  k: int32 [bins] (uint32 counts)."""
+    _require_cuda(cnt_a, torch.int16, "cnt_a")
+    _require_cuda(cnt_b, torch.int16, "cnt_b")
+    _require_cuda(exp1, torch.float32, "exp1")
+    _require_cuda(dist, torch.float32, "dist")
+    _require_cuda(k, torch.int32, "k")
+    bins, K = cnt_a.shape
+    if dist.numel() != bins or k.numel() != bins or exp1.numel() != K:
+        raise ValueError("dist and k must have one entry per bin, exp1 one per state")
+    _lib.call("epi_permutation_exceedances_s1", _ptr(cnt_a), _ptr(cnt_b), bins, K, int(width), int(size_a), int(size_b),
+              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(perm_offset), int(nperm), _ptr(exp1),
+              int(width_a), int(width_b), _ptr(dist), _ptr(k), _stream())
+    return k
 
 
 def pairwise_combine(score_a=None, score_b=None, null_a=None, null_b=None):

@@ -2,7 +2,8 @@
 branches of s1Score / s2Score (scores.py:282-303, 319-322, 373-398, 414-421).
 
 Outputs (rank 0): `pairwiseDelta_<tag>_<file>.txt.gz`, `temp_nullDistances_<tag>_<file>.npz`
-{chrName, nullDistances float32[B]}, `temp_quiescence_<tag>_<file>.npz` {chrName, quiescenceArr bool[B]}.  When the
+{chrName, nullDistances float32[B]}, `temp_quiescence_<tag>_<file>.npz` {chrName, quiescenceArr bool[B]}, and with
+--null-permutations `temp_permutations_<tag>_<file>.npz` {chrName, exceedances uint32[B], permutations}.  When the
 paired statistics stage (roi_pairwise) runs next in this process, the two temp files are not written: their content and
 the reduced real deltas are handed over in memory (session.handover).
 
@@ -64,7 +65,11 @@ def shuffled_widths(c1, c2, groupSize):
 
 def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDirPath, expFreqPath, fileTag, filename,
                             quiescentState, groupSize, verbose, backend=None, null_mode=None, seed=None, nperm=1,
-                            group=None):
+                            group=None, permutations=0):
+    """`permutations` P > 0: also count, for every bin, how many of P device-drawn null shuffles (permutations 0..P-1 of
+    the device sampler, scored like the run's null) are at least as far from 0 as the bin's real distance, and hand the
+    counts to step 4 (session.handover) or write them to temp_permutations_<tag>_<file>.npz {chrName, exceedances
+    uint32[B], permutations}.  Nothing else changes: in device mode permutation 0 is the run's own null."""
     if saliency not in (1, 2):
         raise ValueError("Please ensure that saliency metric is either 1 or 2 for Pairwise Epilogos")
     null_mode = null_mode or os.environ.get("EPILOGOS_B200_NULL", "device")
@@ -77,13 +82,14 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
     exp = be.to_device(np.load(expFreqPath, allow_pickle=False))
 
     cnt_a, cnt_b = shard.counts("a"), shard.counts("b")
+    draw_seed = file_seed(run_seed(seed), filename) if null_mode == "device" or permutations > 0 else None
     if null_mode == "reference":
         rows = shard.states_a.shape[0]
         perm = np.argsort(np.random.rand(rows, c1 + c2), axis=1)                     # helpers.py:183
         null_a, null_b = be.shuffled_counts_perm(shard.states_a, shard.states_b, perm, numStates, size_a, size_b)
     else:
-        null_a, null_b = be.shuffled_counts_device(cnt_a, cnt_b, size_a, size_b, file_seed(run_seed(seed), filename),
-                                                   nperm, width=c1 + c2, bin_offset=shard.lo)
+        null_a, null_b = be.shuffled_counts_device(cnt_a, cnt_b, size_a, size_b, draw_seed, nperm, width=c1 + c2,
+                                                   bin_offset=shard.lo)
 
     # S1 observes over the width of the array it is given (scores.py:343); S2 normalises the shuffled halves with
     # the ORIGINAL group widths even under -g (scores.py:397-398, 418-421)
@@ -100,6 +106,13 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
     if len(nshape) == 3:                # [nperm][rows] flat, permutation-major: row p = the p-th shuffle of every bin
         null_dist = null_dist.reshape(nshape[0], nshape[1])
     quies = be.quiescent_mask(cnt_a, c1, cnt_b, c2, quiescentState)
+    exceed = None
+    if permutations > 0:
+        # the real distance step 4 judges: the delta row after its "%.5f" text round trip
+        real_dist, _ = be.pairwise_real_reduce(delta, text_round_trip=True)
+        exceed = be.permutation_exceedances(cnt_a, cnt_b, real_dist, permutations, draw_seed, size_a, size_b, c1 + c2,
+                                            shard.lo, saliency, exp, (max(size_a, 1), max(size_b, 1)), (p1, p2),
+                                            exact=exact)
 
     total = shard.total_rows
     delta = dist.gather_rows(delta, total)
@@ -109,6 +122,8 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
         null_dist = None if parts[0] is None else __import__("torch").stack(parts, dim=0)
     else:
         null_dist = dist.gather_rows(null_dist, total)
+    if exceed is not None:
+        exceed = dist.gather_rows(exceed, total)
     loc = _gather_locations(shard)
     if dist.rank() == 0:
         outputDirPath = Path(outputDirPath)
@@ -124,7 +139,13 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
                                                    null=null_dist, quiescence=quies, chrom=loc["chrom"],
                                                    start=np.asarray(loc["start"], dtype=np.int64),
                                                    end=np.asarray(loc["end"], dtype=np.int64))
+            if exceed is not None:
+                session.handover[str(nullPath)].update(exceedances=exceed, permutations=int(permutations))
             return
         helpers.savez_level(nullPath, chrName=np.array([chrName]), nullDistances=null_dist.cpu().numpy())
         helpers.savez_level(outputDirPath / "temp_quiescence_{}_{}.npz".format(fileTag, filename),
                             chrName=np.array([chrName]), quiescenceArr=quies.cpu().numpy().astype(np.bool_))
+        if exceed is not None:
+            helpers.savez_level(outputDirPath / "temp_permutations_{}_{}.npz".format(fileTag, filename),
+                                chrName=np.array([chrName]), exceedances=exceed.cpu().numpy().view(np.uint32),
+                                permutations=np.array(int(permutations), dtype=np.int64))

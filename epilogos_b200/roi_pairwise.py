@@ -16,6 +16,9 @@ With -n (`pval`):
      a keyed permutation seeded by the run seed;
   3. scipy.stats.gennorm.fit of each subsample, on the device; the trial with the median NLL is kept;
   4. two-sided p-values of every bin's distance and their Benjamini-Hochberg adjustment over the genome.
+When the score stage counted null permutations (--null-permutations P: temp_permutations_<tag>_<file>.npz or the
+hand-over), pairwisePermutation_<tag>.txt.gz holds per bin (chrom, start, end, k, p, BH): k of the P shuffles of the bin
+whose |null distance| is at least |distance|, p = (1 + k) / (P + 1), and its Benjamini-Hochberg adjustment over all bins.
 Outputs: pairwiseMetrics_<tag>.txt.gz (chrom, start, end, max-difference state, |distance|, sign[, p, BH]) and
 regionsOfInterest_<tag>.txt (the 100 windows of largest max-mean |distance|; state and sign of the window's largest
 |distance| bin[, its p and BH]).  Without -n the reference writes z-scores instead, whose definition is not available to
@@ -51,6 +54,8 @@ def readInData(outputDirPath, fileTag, be):
     for key in [k for k in session.handover if Path(k).parent == outputDirPath
                 and Path(k).name.startswith("temp_nullDistances_{}_".format(fileTag))]:
         h = session.handover.pop(key)
+        if "exceedances" in h:
+            h["exceedances"] = h["exceedances"].cpu().numpy().view(np.uint32)
         chunks[h["chrName"]] = h
     nullFiles = sorted(outputDirPath.glob("temp_nullDistances_{}_*.npz".format(fileTag)))
     for nf in nullFiles:
@@ -67,6 +72,11 @@ def readInData(outputDirPath, fileTag, be):
                                null=be.to_device(np.ascontiguousarray(z["nullDistances"], dtype=np.float32)),
                                quiescence=be.to_device(q["quiescenceArr"].astype(np.uint8)),
                                chrom=loc["chrom"], start=loc["start"], end=loc["end"])
+        pf = outputDirPath / "temp_permutations_{}_{}.npz".format(fileTag, name)
+        if pf.exists():
+            zp = np.load(pf, allow_pickle=False)
+            chunks[chrName].update(exceedances=np.asarray(zp["exceedances"], dtype=np.uint32),
+                                   permutations=int(zp["permutations"]))
     if not chunks:
         raise FileNotFoundError("no paired score-stage outputs (temp_nullDistances_{}_*.npz) in {}"
                                 .format(fileTag, outputDirPath))
@@ -92,6 +102,22 @@ def fit_null(be, chunks, numTrials, samplingSize, seed):
                  iterations=status[:, 0].astype(np.int64), converged=status[:, 1].astype(bool), chosen=chosen,
                  pool_size=n, sample_size=size)
     return float(params[chosen, 0]), float(params[chosen, 1]), float(params[chosen, 2]), table
+
+
+def permutation_pvalues(be, chunks):
+    """(k uint32, p, BH) over the bins of all chunks, or None when the score stage counted no permutations: p = (1 + k) /
+    (P + 1), k = #{p < P : |null(b, p)| >= |distance(b)|}, and the Benjamini-Hochberg adjustment over the genome."""
+    perms = {c.get("permutations") for c in chunks}
+    if perms == {None}:
+        return None
+    if None in perms or len(perms) != 1:
+        raise ValueError("temp_permutations files are missing for some chromosomes or disagree on the number of "
+                         "permutations ({})".format(sorted(str(p) for p in perms)))
+    P = perms.pop()
+    k = np.concatenate([np.asarray(c["exceedances"], dtype=np.uint32) for c in chunks])
+    p = (k.astype(np.float64) + 1.0) / (P + 1.0)
+    bh = be.bh_adjust(be.to_device(p)).cpu().numpy()
+    return k, p, bh
 
 
 def roi_lines(chrom, starts, ends, distance, max_diff, names, roiWidth, pvals=None, bh=None):
@@ -147,11 +173,14 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, pval, numTrials=1
                               distance, pvals, bh)
     (outputDirPath / "regionsOfInterest_{}.txt".format(fileTag)).write_text(
         roi_lines(loc["chrom"], loc["start"], loc["end"], distance, max_diff, names, roiWidth, pvals, bh))
+    perm = permutation_pvalues(be, chunks)
+    if perm is not None:
+        writer.write_permutations_text(outputDirPath / "pairwisePermutation_{}.txt.gz".format(fileTag), loc, *perm)
     if not verbose:
         print("\t[Done]", flush=True)
     if diagnostic:
         print("    Diagnostic figures (-d) are not built: matplotlib is not a dependency of this package", flush=True)
-    pattern = re.compile(r"^temp_(nullDistances|quiescence)_{}_.*\.npz$".format(re.escape(fileTag)))
+    pattern = re.compile(r"^temp_(nullDistances|quiescence|permutations)_{}_.*\.npz$".format(re.escape(fileTag)))
     for f in outputDirPath.iterdir():
         if pattern.match(f.name):
             remove(f)

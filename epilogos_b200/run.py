@@ -115,6 +115,23 @@ def checkArguments(mode, saliency, inputDirPath, inputDirPath2, outputDirPath, n
             return
 
 
+MAX_NULL_PERMUTATIONS = 1000000
+
+
+def checkPermutationFlags(mode, nullPermutations):
+    """Rules of --null-permutations (checked after every other rule): first violated rule prints and exits."""
+    rules = [
+        (nullPermutations is not None and mode != "paired",
+         "ERROR: [--null-permutations] requires [-m, --mode] 'paired'"),
+        (nullPermutations is not None and not 1 <= nullPermutations <= MAX_NULL_PERMUTATIONS,
+         "ERROR: Number of null permutations must be between 1 and {}".format(MAX_NULL_PERMUTATIONS)),
+    ]
+    for bad, message in rules:
+        if bad:
+            _die(message)
+            return
+
+
 def deal_files(pairs, world):
     """Whole files dealt to the ranks, largest first to the least loaded rank (by size on disk): the same answer on every
     rank.  Returns a list of `world` lists of (file1, file2) pairs."""
@@ -131,7 +148,7 @@ def deal_files(pairs, world):
 
 def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
                groupSize, stateInfo, roiWidth, verbose, say, backend=None, pvalBool=False, numTrials=101,
-               samplingSize=100000, diagnosticBool=False, groups=None):
+               samplingSize=100000, diagnosticBool=False, groups=None, permutations=0):
     """Steps 1-4 of run.main (run.py:193-303) in process.  Two ways to use several GPUs:
       rows  (default)  every file's rows are split over the ranks (helpers.splitRows); per-file tables are all-reduced and
                        score rows gathered on rank 0, which writes the files;
@@ -144,7 +161,9 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
     mode) or comparison (paired mode), run on the column subsets of the files of `pairs`, which are (file, "null").  Every
     stage keeps the reference's order: step 1 tables all groups of a file from the same counts, step 2 runs per group, step
     3 scores all groups of a file, step 4 runs per group.  A comparison passes the file itself as the stage drivers'
-    second file, which the group view does not read."""
+    second file, which the group view does not read.
+    `permutations` P > 0 (paired mode): step 3 also counts P null shuffles per bin and step 4 writes
+    pairwisePermutation_<tag>.txt.gz."""
     from contextlib import nullcontext
     from . import dist, expected, expectedCombination, scores, session
     world = dist.world_size()
@@ -187,7 +206,8 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
             for f, f2 in mine:
                 for out, tag, exp_path, sel in runs:
                     scores.main(f, second(f, f2, sel), numStates, saliency, out, exp_path, tag, numProcesses,
-                                quiescentState, groupSize, verbose, backend=backend, group=sel)
+                                quiescentState, groupSize, verbose, backend=backend, group=sel,
+                                permutations=permutations)
     finally:
         session.handover_enabled = False
     dist.barrier()
@@ -258,13 +278,18 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
                    + "OUT/<A>_vs_<B>")
 @click.option("--compare", "comparisons", type=str, multiple=True,
               help="Paired mode with --groups: compare group A with group B (A:B, repeatable)")
+@click.option("--null-permutations", "nullPermutations", type=int, default=None,
+              help="Paired mode: draw P null shuffles of every bin on the GPU and write pairwisePermutation_<tag>.txt.gz "
+                   + "with each bin's count of shuffles at least as far apart as its groups, its permutation p-value "
+                   + "(1 + count) / (P + 1) and the Benjamini-Hochberg adjusted p-value (1 <= P <= 1000000)")
 @click.option("--exp-freq-mem", "expFreqMem", type=int, default=20000, help="SLURM-only (ignored)")
 @click.option("--exp-comb-mem", "expCombMem", type=int, default=8000, help="SLURM-only (ignored)")
 @click.option("--score-mem", "scoreMem", type=int, default=40000, help="SLURM-only (ignored)")
 @click.option("--roi-mem", "roiMem", type=int, default=-1, help="SLURM-only (ignored)")
 def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2, outputDirectory, stateInfo, saliency,
          numProcesses, exitBool, diagnosticBool, numTrials, samplingSize, quiescentState, groupSize, version, partition,
-         pvalBool, roiWidth, fileTag, groupFile, comparisons, expFreqMem, expCombMem, scoreMem, roiMem):
+         pvalBool, roiWidth, fileTag, groupFile, comparisons, nullPermutations, expFreqMem, expCombMem, scoreMem,
+         roiMem):
     """Information-theoretic navigation of multi-tissue functional genomic annotations (B200 scoring path)."""
     if version:
         from epilogos_b200 import __version__
@@ -297,6 +322,7 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
     outputDirPath = Path(outputDirectory).absolute()
     checkArguments(mode, saliency, inputDirPath, inputDirPath2, outputDirPath, numProcesses, numStates, numTrials,
                    samplingSize, quiescentState, groupSize, roiWidth)
+    checkPermutationFlags(mode, nullPermutations)
 
     import torch
     import torch.distributed as td
@@ -349,7 +375,8 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
 
     run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
                groupSize, stateInfo, roiWidth, verbose, say, pvalBool=pvalBool, numTrials=numTrials,
-               samplingSize=samplingSize, diagnosticBool=diagnosticBool, groups=runs)
+               samplingSize=samplingSize, diagnosticBool=diagnosticBool, groups=runs,
+               permutations=nullPermutations or 0)
     dist.barrier()
     if launched and td.is_initialized():
         td.destroy_process_group()

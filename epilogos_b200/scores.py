@@ -18,7 +18,7 @@ from . import dist, helpers, session, writer
 
 
 def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, numProcesses, quiescentState, groupSize,
-         verbose, backend=None, group=None):
+         verbose, backend=None, group=None, permutations=0):
     tTotal = time()
     file1Path, file2Path, outputDirPath = Path(file1), Path(file2), Path(outputDir)
     filename = file1Path.name.split(".")[0]
@@ -30,7 +30,8 @@ def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, num
     else:
         from .pairwise import calculateScoresPairwise
         calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDirPath, expFreqPath, fileTag,
-                                filename, quiescentState, groupSize, verbose, backend, group=group)
+                                filename, quiescentState, groupSize, verbose, backend, group=group,
+                                permutations=permutations)
     if dist.rank() == 0:
         print("Total Time:", time() - tTotal, flush=True) if verbose else print("\t[Done]", flush=True)
     dist.barrier()

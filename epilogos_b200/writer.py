@@ -64,6 +64,20 @@ def write_metrics_text(path, loc, state_names, max_diff, distance, pval=None, bh
               int(_gzip_level(level)), int(threads))
 
 
+def write_permutations_text(path, loc, k, pval, bh, level=None, threads=0):
+    """pairwisePermutation_<tag>.txt.gz through the native writer (epi_write_permutations_gz): per bin `chr \t start \t
+    end \t k \t "%.5e" p \t "%.5e" BH`."""
+    names, cid, starts, ends = _native_locations(loc)
+    k = np.ascontiguousarray(k, dtype=np.uint32)
+    pval = np.ascontiguousarray(pval, dtype=np.float64)
+    bh = np.ascontiguousarray(bh, dtype=np.float64)
+    if not (len(k) == len(pval) == len(bh) == len(starts)):
+        raise ValueError("one count, p-value and adjusted p-value per bin")
+    p = lambda a: ctypes.c_void_p(a.ctypes.data)
+    _lib.call("epi_write_permutations_gz", str(path).encode(), ctypes.c_char_p(names), p(cid), p(starts), p(ends), p(k),
+              p(pval), p(bh), len(k), int(_gzip_level(level)), int(threads))
+
+
 def location_array(loc):
     """object [rows, 3] array as produced by pd.read_table(...).to_numpy() in scores.py:161."""
     arr = np.empty((len(loc["chrom"]), 3), dtype=object)

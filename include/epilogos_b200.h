@@ -159,6 +159,13 @@ int epi_shuffled_counts_philox(const uint16_t* cnt_a_dev, const uint16_t* cnt_b_
                                int32_t num_states, int32_t width, int32_t size_a, int32_t size_b, uint64_t seed,
                                int64_t bin_offset, int32_t nperm,
                                uint16_t* cnt_a_out, uint16_t* cnt_b_out, void* stream);
+/* epi_shuffled_counts_philox_range  the same draws for permutations perm_offset .. perm_offset + nperm - 1 (outputs
+ *                                   [nperm][bins][K]): a caller batching the permutations continues one stream.
+ *                                   epi_shuffled_counts_philox is this with perm_offset 0.  perm_offset + nperm <= 2^32. */
+int epi_shuffled_counts_philox_range(const uint16_t* cnt_a_dev, const uint16_t* cnt_b_dev, int64_t bins,
+                                     int32_t num_states, int32_t width, int32_t size_a, int32_t size_b, uint64_t seed,
+                                     int64_t bin_offset, int64_t perm_offset, int32_t nperm,
+                                     uint16_t* cnt_a_out, uint16_t* cnt_b_out, void* stream);
 int epi_pairwise_combine(const float* score_a, const float* score_b, const float* null_a, const float* null_b,
                          int64_t rows, int32_t num_states, float* delta_out, float* null_dist_out, void* stream);
 int epi_quiescent_mask(const uint16_t* cnt_a_dev, const uint16_t* cnt_b_dev, int64_t bins, int32_t num_states,
@@ -171,6 +178,23 @@ int epi_quiescent_mask(const uint16_t* cnt_a_dev, const uint16_t* cnt_b_dev, int
  * pairwiseDelta_*.txt.gz (emulated arithmetically, bit-exact).  Either output may be NULL. */
 int epi_pairwise_real_reduce(const float* delta_dev, int64_t rows, int32_t num_states, int32_t text_round_trip,
                              float* dist_out, int32_t* max_diff_out, void* stream);
+
+/* ---- per-bin permutation tests of paired mode (csrc/permutations.cu) ----------------------------------------
+ * For every bin b: k[b] += #{p : |null(b, p)| >= |dist[b]|}, null(b, p) = sum_s d^2 * sign(sum_s d) with
+ * d = score(A'_p) - score(B'_p) (float32, numpy pairwise order: what epi_pairwise_combine computes).  k is ADDED to, so
+ * permutation blocks accumulate; no (bin, permutation) value is stored.
+ *   epi_null_exceedances            from the score arrays of A' and B' of nperm shuffles, [nperm][bins][K] float32.
+ *   epi_permutation_exceedances_s1  fused S1: draws permutations perm_offset .. perm_offset + nperm - 1 of every bin
+ *                                   exactly as epi_shuffled_counts_philox_range, scores A' at width_a and B' at width_b
+ *                                   against exp1 [K] with the values epi_scores_s1 gives in TABLE mode, and counts.
+ *                                   Equal bit for bit to the composed path; width_a, width_b <= 4095. */
+int epi_null_exceedances(const float* null_a_dev, const float* null_b_dev, int32_t nperm, int64_t bins,
+                         int32_t num_states, const float* dist_dev, uint32_t* k_inout, void* stream);
+int epi_permutation_exceedances_s1(const uint16_t* cnt_a_dev, const uint16_t* cnt_b_dev, int64_t bins,
+                                   int32_t num_states, int32_t width, int32_t size_a, int32_t size_b, uint64_t seed,
+                                   int64_t bin_offset, int64_t perm_offset, int32_t nperm, const float* exp1_dev,
+                                   int32_t width_a, int32_t width_b, const float* dist_dev, uint32_t* k_inout,
+                                   void* stream);
 
 /* ---- paired statistics stage (roiAndVisualPairwise.py:177-242, csrc/pairwise_stats.cu) -----------------------
  *   epi_null_compact       the null distances of the bins whose quiescent flag is 0 (all bins when quiescent_dev is NULL),
@@ -308,6 +332,12 @@ int epi_write_metrics_gz(const char* path, const char* chrom_names, const int32_
                          const int64_t* ends, const char* state_names, int32_t num_states, const int32_t* max_diff,
                          const float* distance, const double* pval, const double* bh, int64_t rows, int32_t level,
                          int32_t threads);
+/* pairwisePermutation text through gzip, one line per bin: `chr \t start \t end \t k \t "%.5e" p \t "%.5e" bh` (k the
+ * bin's exceedance count, p its permutation p-value, bh the Benjamini-Hochberg adjustment).  Same deflate path as
+ * epi_write_scores_gz. */
+int epi_write_permutations_gz(const char* path, const char* chrom_names, const int32_t* chrom_id, const int64_t* starts,
+                              const int64_t* ends, const uint32_t* k, const double* pval, const double* bh, int64_t rows,
+                              int32_t level, int32_t threads);
 /* ChromHMM `-printstatebyline` files (one per biosample and chromosome: `<biosample> <chr>`, `MaxState E`, then one label per
  * 200 bp bin) -> matrix: the native form of bin/preprocess_data_ChromHMM.sh:34-49, which pastes those files side by side.
  * epi_statebyline_read  parses ONE file into a column: out[r * stride] = label - 1 for bin r (out == NULL: count only);

@@ -50,6 +50,14 @@ for bins, cols, k in (shapes[:1] + shapes[3:4] if race else shapes):
     engine.quiescent_mask(ca, c1, cb, cols - c1, k - 1)
     engine.pairwise_real_reduce(delta)
     engine.paired_host(engine.pack_states(x[:, :c1]), c1, engine.pack_states(x[:, c1:]), cols - c1, k, 1, k - 1, nperm=2)
+    # permutation counts: range sampler, counting step, fused S1 kernel (1, 8 and 32 threads per bin)
+    dist, _ = engine.pairwise_real_reduce(delta)
+    pa, pb = engine.shuffled_counts_philox_range(ca, cb, c1, cols - c1, 3, 5, 3, cols, bin_offset=7)
+    kk = torch.zeros(bins, dtype=torch.int32, device="cuda")
+    engine.null_exceedances(engine.scores_s1(pa.reshape(-1, k), c1, e1).reshape(3, bins, k),
+                            engine.scores_s1(pb.reshape(-1, k), cols - c1, e1).reshape(3, bins, k), dist, kk)
+    for n in (3, 9, 40):
+        engine.permutation_exceedances_s1(ca, cb, c1, cols - c1, 3, 0, n, cols, 7, e1, c1, cols - c1, dist, kk)
     torch.cuda.synchronize()
     print("ok", bins, cols, k, flush=True)
 print("done")
