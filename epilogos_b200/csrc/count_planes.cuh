@@ -82,23 +82,35 @@ __device__ __forceinline__ void flush_planes(uint32_t (&p)[NP], uint32_t (&acc)[
     }
 }
 
-// packed counters -> per-state counts cs[0..EPI_MAX_STATES).  sum1 / sum2 (MODE_F2M only) are sum(v) and sum(v^2) over the
-// counted labels; npad zero labels that were counted but are not data are removed from state 0.
+// Zeroed counters, except that the low half of acc[0] starts at 0x10000 - npad: the npad zero labels that are counted but
+// are not data (the padding of a row or of a column list to whole chunks) carry it exactly once into the high half, so the
+// low half ends at the data's own count of field 0 however close the padded row comes to 65,535 labels or goes past it.
+// unpack_counts takes that one carry back out.
+template <int NACC>
+__device__ __forceinline__ void init_counters(uint32_t (&acc)[NACC], int npad) {
+    acc[0] = 0x10000u - (uint32_t)npad;
+#pragma unroll
+    for (int f = 1; f < NACC; ++f) acc[f] = 0;
+}
+
+// packed counters (started by init_counters) -> per-state counts cs[0..EPI_MAX_STATES).  sum1 / sum2 (MODE_F2M only) are
+// sum(v) and sum(v^2) over the counted labels.
 template <int MODE, int NACC>
-__device__ __forceinline__ void unpack_counts(const uint32_t (&acc)[NACC], uint32_t sum1, uint32_t sum2, int npad,
+__device__ __forceinline__ void unpack_counts(const uint32_t (&acc)[NACC], uint32_t sum1, uint32_t sum2,
                                               uint32_t (&cs)[EPI_MAX_STATES]) {
+    // the pad's carry leaves acc[0] modulo 2^32: a high-half count of 65,535 had wrapped to 0 and comes back
+    const auto word = [&](int f) { return f == 0 ? acc[0] - 0x10000u : acc[f]; };
     if constexpr (MODE == MODE_B1) {
 #pragma unroll
         for (int f = 0; f < 16; ++f) {
-            cs[f] = acc[f] & 0xffffu;
-            cs[f + 16] = acc[f] >> 16;
+            cs[f] = word(f) & 0xffffu;
+            cs[f + 16] = word(f) >> 16;
         }
-        cs[0] -= (uint32_t)npad;
     } else {
 #pragma unroll
         for (int f = 0; f < 8; ++f) {
-            cs[f] = acc[f] & 0xffffu;
-            cs[f + 8] = acc[f] >> 16;
+            cs[f] = word(f) & 0xffffu;
+            cs[f + 8] = word(f) >> 16;
         }
 #pragma unroll
         for (int f = 16; f < EPI_MAX_STATES; ++f) cs[f] = 0;
@@ -118,7 +130,6 @@ __device__ __forceinline__ void unpack_counts(const uint32_t (&acc)[NACC], uint3
             cs[0] -= c16;
             cs[1] -= c17;
         }
-        cs[0] -= (uint32_t)npad;
     }
 }
 

@@ -2,7 +2,7 @@
 // zero padded), 16-byte chunks XOR-swizzled by (b mod 8) -- the SWIZZLE_128B operand layout of tcgen05.mma.  Read K-major
 // it is a [128 bin] x [2K byte] A operand (S2 scores); read MN-major it is a [2K byte-index] x [128 bin] operand whose
 // contraction index is the bin, i.e. both operands of the Gram update G += T T^t that yields the S2 expected table
-// (expected.py:146-158).  Shared by tc_tables.cu (stand-alone K2 / K5) and counts.cu (K2 fused into the count kernel).
+// (expected.py:146-158).  Used by tc_tables.cu (K2 and K5).
 #pragma once
 #include "tc05.cuh"
 

@@ -9,8 +9,8 @@
 //    [128 bins x BV*16 bytes] boxes of the matrix into a shared-memory ring with 2D TMA
 //    (cp.async.bulk.tensor + mbarrier expect_tx).  The tensor map's inner extent is `cols`, so the
 //    padding of the last 16-byte vector of a row and rows beyond `bins` are zero-filled by the TMA
-//    unit (never read from HBM, never interpreted: the known number of zero pad bytes is subtracted
-//    from state 0).
+//    unit (never read from HBM, never interpreted: the known number of zero pad bytes is kept out of
+//    state 0 by the start value of its counter, init_counters).
 //  * BV (16-byte vectors per box row) is odd, so consecutive rows start in different 16-byte bank
 //    groups and the per-thread LDS.128 row reads are bank-conflict free without swizzling.
 //  * the ALU budget at HBM speed is ~3 integer-pipe instructions per input byte, far below a
@@ -79,7 +79,7 @@ __device__ __forceinline__ void fold_groups(const ChunkSrc<BV, MODE>& src, uint3
 }
 
 // SW: the row is a 128-byte TMA SWIZZLE_128B row (16-byte chunk v lives at chunk v ^ swz) that holds only BV - 1 vectors;
-// the last vector of the chunk is a virtual all-zero vector (label 0, removed again through npad).
+// the last vector of the chunk is a virtual all-zero vector (label 0, part of npad).
 template <int BV, int MODE, int NP, bool SW = false>
 __device__ __forceinline__ void process_chunk(const uint4* __restrict__ row, uint32_t (&p)[NP], uint32_t& sum1,
                                               uint32_t& sum2, uint32_t one, int swz = 0) {
@@ -167,8 +167,7 @@ k1_counts_kernel(const __grid_constant__ CUtensorMap tmap, long long bins, int n
         uint32_t acc[NACC];
 #pragma unroll
         for (int k = 0; k < NP; ++k) p[k] = 0;
-#pragma unroll
-        for (int f = 0; f < NACC; ++f) acc[f] = 0;
+        init_counters(acc, npad);
         uint32_t sum1 = 0, sum2 = 0;
         int pending = 0;
 
@@ -192,7 +191,7 @@ k1_counts_kernel(const __grid_constant__ CUtensorMap tmap, long long bins, int n
 
         // ---- unpack the counters into per-state counts ----
         uint32_t cs[EPI_MAX_STATES];
-        unpack_counts<MODE, NACC>(acc, sum1, sum2, npad, cs);
+        unpack_counts<MODE, NACC>(acc, sum1, sum2, cs);
 
         // ---- stage the warp's 32 rows and write them with 16-byte stores ----
         uint16_t* wrow = out_stage + (size_t)tid * num_states;

@@ -7,8 +7,8 @@
 //   different banks) and counts them with K1's arithmetic (count_planes.cuh): one-hot words, carry-save planes, the
 //   17/18-state separation and one-bit words for 19-32 states.  When a group's list ends the planes are flushed, the
 //   counts unpacked, and the 32 rows of a warp leave through shared memory as 16-byte stores.  Pad entries of a list point
-//   at a zero word behind the row and are removed from state 0, as K1 removes its zero padding.  No global atomics; each
-//   group's block has exactly the layout epi_bin_counts writes.
+//   at a zero word behind the row and are kept out of state 0 as K1 keeps its zero padding out (init_counters).  No global
+//   atomics; each group's block has exactly the layout epi_bin_counts writes.
 //   Per-bin work is one LDS.U8 and ~4 integer instructions per listed column, so the kernel is bound by shared-memory
 //   issue and the integer pipes rather than by HBM once the groups together list more columns than the matrix has.
 // epi_gather_columns -- out[b][j] = x[b][idx[j]], j < n, into a 16-byte pitched matrix (pad bytes zero).
@@ -102,8 +102,7 @@ group_counts_kernel(const int8_t* __restrict__ x, long long bins, long long pitc
                 uint32_t p[NP], acc[NACC];
 #pragma unroll
                 for (int k = 0; k < NP; ++k) p[k] = 0;
-#pragma unroll
-                for (int f = 0; f < NACC; ++f) acc[f] = 0;
+                init_counters(acc, npad[g]);
                 uint32_t sum1 = 0, sum2 = 0;
                 int pending = 0;
                 const int end = off[g + 1];
@@ -134,7 +133,7 @@ group_counts_kernel(const int8_t* __restrict__ x, long long bins, long long pitc
                     }
                 }
                 if (pending) flush_planes<MODE, NP, NACC>(p, acc);
-                unpack_counts<MODE, NACC>(acc, sum1, sum2, npad[g], cs);
+                unpack_counts<MODE, NACC>(acc, sum1, sum2, cs);
             }
             // ---- stage the warp's 32 rows and write them with 16-byte stores when the destination allows it ----
             uint16_t* wrow = out_stage + (size_t)tid * num_states;
@@ -201,7 +200,7 @@ static int launch_group_counts(const int8_t* x, int64_t bins, int32_t cols, int6
     for (int g = 0; g < groups; ++g) {
         const int n = offsets[g + 1] - offsets[g];
         const int padded = (n + CH - 1) / CH * CH;
-        EPI_REQUIRE(padded <= 65535, "group %d lists %d columns: at most %d fit the 16-bit counters", g, n, 65535 - CH + 1);
+        EPI_REQUIRE(padded <= 65535, "group %d lists %d columns: at most %d fit the 16-bit counters", g, n, 65535 / CH * CH);
         meta[g] = (int)meta.size() - head;
         meta[groups + 1 + g] = padded - n;
         meta.insert(meta.end(), list.begin() + offsets[g], list.begin() + offsets[g + 1]);

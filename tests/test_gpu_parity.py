@@ -204,7 +204,8 @@ def test_other_state_models(eng, k, cols):
 def test_tensor_core_tables_and_scores_edge_shapes(eng, bins, cols, k):
     """K2 / K5-S2 on the tensor cores at the edges of their tiling: fewer bins than one 128-bin tile, exact tile
     multiples, counts that do / do not need the high byte (255 / 256 biosamples), the widest table-driven width (2047) and
-    the first width that takes the per-bin path (2048), an accumulator drain in mid-run (33 000 bins), odd state counts."""
+    the first width that takes the per-bin path (2048), 258 tiles (33 000 bins, one tile per CTA), odd state counts.
+    Accumulator drains in mid-run need far more bins: test_limits_gpu.py."""
     rng = np.random.default_rng(bins * 7 + cols * 3 + k)
     x = rng.integers(0, k, size=(bins, cols)).astype(np.int8)
     if bins > 2:

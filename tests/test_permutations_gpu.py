@@ -72,6 +72,8 @@ CASES = [  # bins, c1, c2, K, -g, nperm, bin_offset
     (513, 400, 433, 18, 300, 1, 5),
     (999, 60, 67, 15, 50, 64, 3),
     (301, 60, 67, 18, 100, 7, (1 << 33) + 1),
+    (513, 700, 800, 18, -1, 33, 0),          # S1 value tables in global memory; 32-thread groups and one more permutation
+    (300, 4100, 4200, 15, -1, 7, 0),         # wider than the S1 value table: S1 takes the composed route too
 ]
 
 
