@@ -48,8 +48,20 @@ PROTOTYPES = {
     "epi_permutation_exceedances_s1": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_uint64,
                                                c_int64, c_int64, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_void_p,
                                                c_void_p]),
+    "epi_multigroup_stat": (c_int, [c_void_p, c_int32, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                    c_void_p]),
+    "epi_multigroup_shuffled_counts_range": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_void_p, c_uint64,
+                                                     c_int64, c_int64, c_int32, c_void_p, c_void_p]),
+    "epi_multigroup_null_exceedances": (c_int, [c_void_p, c_int32, c_int32, c_int64, c_int32, c_void_p, c_void_p,
+                                                c_void_p, c_void_p]),
+    "epi_multigroup_exceedances_s1": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_void_p, c_uint64, c_int64,
+                                              c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "epi_multigroup_s1_fused_fits": (c_int, [c_int32, c_int32, c_void_p]),
     "epi_write_permutations_gz": (c_int, [c_char_p, c_char_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                           c_int64, c_int32, c_int32]),
+    "epi_write_multigroup_gz": (c_int, [c_char_p, c_char_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                        c_void_p, c_char_p, c_int32, c_char_p, c_int32, c_void_p, c_void_p, c_void_p,
+                                        c_int64, c_int32, c_int32]),
     "epi_pairwise_combine": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p,
                                      c_void_p]),
     "epi_quiescent_mask": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_int32, c_int32, c_int32, c_void_p,

@@ -141,6 +141,82 @@ class CudaBackend:
                                             dist[lo:hi], k[lo:hi])
         return k
 
+    # -- multi-group comparisons ------------------------------------------------------------------------
+    def _group_scores(self, cnt, n, saliency, exp, exact, out=None):
+        """Scores of one group's counts [bins, K] at its own width n (S2 over its n (n - 1) ordered pairs), into `out`
+        when given.  The score kernels want 16-byte aligned counts and outputs; the callers keep their blocks aligned
+        except for a tail of fewer than 8 bins, whose blocks are copied."""
+        cnt = cnt if cnt.data_ptr() % 16 == 0 else cnt.clone()
+        direct = out is not None and out.data_ptr() % 16 != 0
+        o32 = None if out is None or direct else out
+        if saliency == 1:
+            sc = engine.scores_s1(cnt, n, exp, out32=o32)
+        else:
+            sc = engine.scores_s2(cnt, n, exp, perms=n * (n - 1), out32=o32,
+                                  mode=engine.EPI_SCORE_DIRECT if exact else engine.EPI_SCORE_TABLE)
+        if direct:
+            out.copy_(sc)
+        return sc if out is None else out
+
+    @staticmethod
+    def _bin_chunks(rows, chunk):
+        """[lo, hi) ranges of at most `chunk` bins whose lengths are multiples of 8, then the tail of rows % 8 bins: every
+        [G, hi - lo, K] block of uint16 counts or float32 scores then starts on 16 bytes, except in the tail."""
+        body = rows - rows % 8
+        step = max(8, chunk - chunk % 8)
+        edges = list(range(0, body, step)) + [body]
+        out = [(lo, hi) for lo, hi in zip(edges[:-1], edges[1:])]
+        return out + ([(body, rows)] if body < rows else [])
+
+    def multigroup_stat(self, cnt, sizes, saliency, exp, exact=False, workspace_bytes=1 << 30):
+        """(T float64, g* uint8, s* uint8, sign int8), each [bins], of the groups' counts cnt int16 [G, bins, K] (group g
+        of width sizes[g]) scored against exp in the run's score mode (`exact`).  Bins go in chunks whose G score arrays
+        stay below `workspace_bytes`."""
+        G, rows, k_states = cnt.shape
+        exp = exp.to(self.device).contiguous()
+        out = (torch.empty(rows, dtype=torch.float64, device=self.device),
+               torch.empty(rows, dtype=torch.uint8, device=self.device),
+               torch.empty(rows, dtype=torch.uint8, device=self.device),
+               torch.empty(rows, dtype=torch.int8, device=self.device))
+        chunk = max(1, int(workspace_bytes) // (4 * G * k_states))
+        with timing.stage("kernels", sync_cuda=True):
+            for lo, hi in self._bin_chunks(rows, chunk):
+                sc = torch.empty((G, hi - lo, k_states), dtype=torch.float32, device=self.device)
+                for g, n in enumerate(sizes):
+                    self._group_scores(cnt[g, lo:hi], n, saliency, exp, exact, out=sc[g])
+                for dst, src in zip(out, engine.multigroup_stat(sc, sizes)):
+                    dst[lo:hi] = src
+        return out
+
+    def multigroup_exceedances(self, cnt, sizes, t, nperm, seed, bin_offset, saliency, exp, exact=False,
+                               workspace_bytes=1 << 30):
+        """Per-bin permutation counts k[b] = #{p < nperm : T_null(b, p) >= t[b]} (int32 tensor holding uint32) of the
+        groups' counts cnt int16 [G, bins, K]: shuffle p drawn as engine.multigroup_shuffled_counts_range draws it, group
+        g scored at width sizes[g] in the run's score mode.  S1 runs the fused kernel where its tables fit; S2 and wider
+        S1 groups loop over bin chunks x permutation blocks of draw + score + count, whose device buffers (shuffled
+        counts and their scores) stay below `workspace_bytes`.  The result does not depend on that cap."""
+        G, rows, k_states = cnt.shape
+        exp = exp.to(self.device).contiguous()
+        t = t.to(self.device).contiguous()
+        k = torch.zeros(rows, dtype=torch.int32, device=self.device)
+        if saliency == 1 and engine.multigroup_s1_fused_fits(sizes, k_states):
+            with timing.stage("kernels", sync_cuda=True):
+                return engine.multigroup_exceedances_s1(cnt, sizes, seed, 0, nperm, bin_offset, exp, t, k)
+        cells = max(1, int(workspace_bytes) // (6 * G * k_states))     # shuffled counts (uint16) and scores (float32)
+        with timing.stage("kernels", sync_cuda=True):
+            for lo, hi in self._bin_chunks(rows, cells):
+                block = max(1, min(nperm, cells // (hi - lo)))
+                for p0 in range(0, nperm, block):
+                    n = min(block, nperm - p0)
+                    oc = engine.multigroup_shuffled_counts_range(cnt[:, lo:hi], sizes, seed, p0, n, bin_offset + lo)
+                    sc = torch.empty((n, G, hi - lo, k_states), dtype=torch.float32, device=self.device)
+                    for p in range(n):
+                        for g, size in enumerate(sizes):
+                            self._group_scores(oc[p, g], size, saliency, exp, exact, out=sc[p, g])
+                    del oc
+                    engine.multigroup_null_exceedances(sc, sizes, t[lo:hi], k[lo:hi])
+        return k
+
     def pairwise_combine(self, score_a, score_b, null_a, null_b):
         return engine.pairwise_combine(score_a, score_b, null_a, null_b)
 

@@ -1166,6 +1166,35 @@ extern "C" int epi_write_permutations_gz(const char* path, const char* chrom_nam
     });
 }
 
+extern "C" int epi_write_multigroup_gz(const char* path, const char* chrom_names, const int32_t* chrom_id,
+                                       const int64_t* starts, const int64_t* ends, const double* t, const uint8_t* group,
+                                       const uint8_t* state, const int8_t* sign, const char* group_names, int32_t groups,
+                                       const char* state_names, int32_t K, const uint32_t* k, const double* pval,
+                                       const double* bh, int64_t rows, int32_t level, int32_t threads) {
+    EPI_REQUIRE(path && chrom_names && starts && ends && group_names && state_names, "null pointer argument");
+    EPI_REQUIRE(rows == 0 || (t && group && state && sign), "null pointer argument");
+    EPI_REQUIRE((k == nullptr) == (pval == nullptr) && (pval == nullptr) == (bh == nullptr),
+                "counts, p-values and adjusted p-values go together");
+    EPI_REQUIRE(rows >= 0 && K >= 1 && K <= EPI_MAX_STATES && groups >= 1 && groups <= EPI_MAX_GROUPS, "bad shape");
+    for (int64_t r = 0; r < rows; ++r)
+        EPI_REQUIRE(group[r] < groups && state[r] < K, "row %lld: group %d or state %d outside 0..%d, 0..%d",
+                    (long long)r, group[r], state[r], groups - 1, K - 1);
+    const std::vector<const char*> names = split_names(chrom_names, max_chrom_id(chrom_id, rows) + 1);
+    const std::vector<const char*> gnames = split_names(group_names, groups);
+    const std::vector<const char*> states = split_names(state_names, K);
+    size_t longest = 0, gl = 0, sl = 0;
+    for (const char* s : names) longest = std::max(longest, strlen(s));
+    for (const char* s : gnames) gl = std::max(gl, strlen(s));
+    for (const char* s : states) sl = std::max(sl, strlen(s));
+    return write_gz_rows(path, rows, longest + gl + sl + 200, level, threads, [&](char* p, int64_t r) {
+        p = format_location(p, names[chrom_id ? chrom_id[r] : 0], starts[r], ends[r]);
+        p += sprintf(p, "\t%.5e\t%s\t%s\t%c", t[r], gnames[group[r]], states[state[r]], sign[r] < 0 ? '-' : '+');
+        if (k) p += sprintf(p, "\t%u\t%.5e\t%.5e", (unsigned)k[r], pval[r], bh[r]);
+        *p++ = '\n';
+        return p;
+    });
+}
+
 // ---- ChromHMM `-printstatebyline` files -> matrix: the native form of bin/preprocess_data_ChromHMM.sh (SURVEY.md 8f, row f3).
 //      One file per biosample and chromosome: line 1 `<biosample> <chr>`, line 2 `MaxState E`, then one state label per 200 bp
 //      bin.  The script pastes the files of a chromosome side by side and prefixes every row with `chr, start, end`

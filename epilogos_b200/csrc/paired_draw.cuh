@@ -94,6 +94,59 @@ __device__ __forceinline__ void draw_shuffle(Philox& rng, const uint16_t* __rest
     }
 }
 
+// One uniform shuffle of a bin's labels over G groups (multigroup.cu).  comb(s) is the bin's count of state s over the
+// union of the groups, size[g] the labels group g receives, and need(g) a per-thread int slot the draw keeps group g's
+// still-needed count in.  For every state s in order and every group g in order,
+//   x_gs ~ HG(labels still unassigned, labels of state s still unassigned, labels group g still needs);
+// emit(s, g, x_gs) is called in that order and end_state(s) after the last group of a state.  With G = 2 this uses the
+// same Philox words in the same order as draw_shuffle; the last group's draw is always deterministic (it consumes none).
+template <class Comb, class Need, class Emit, class EndState>
+__device__ __forceinline__ void draw_multigroup_shuffle(Philox& rng, int K, int G, const int* size, Comb comb, Need need,
+                                                        const double* __restrict__ lf, const double* __restrict__ inv,
+                                                        Emit emit, EndState end_state) {
+    int remaining = 0;
+    for (int s = 0; s < K; ++s) remaining += comb(s);
+    int left = remaining;
+    for (int g = 0; g < G; ++g) {
+        const int n = min(size[g], left);
+        need(g) = n;
+        left -= n;
+    }
+    for (int s = 0; s < K; ++s) {
+        const int c = comb(s);
+        int pop = remaining, succ = c;
+        for (int g = 0; g < G; ++g) {
+            const int ng = need(g);
+            const int x = succ > 0 ? hypergeometric(rng, pop, succ, ng, lf, inv) : 0;
+            pop -= ng;
+            succ -= x;
+            need(g) = ng - x;
+            emit(s, g, x);
+        }
+        remaining -= c;
+        end_state(s);
+    }
+}
+
+// The multi-group statistic, one state at a time, in float64 without contraction (the numpy oracle computes the same
+// numbers): m[s] = (sum_g n_g S_g[s]) / N, then t += n_g (S_g[s] - m[s])^2 for g in order, in one running sum over s
+// outer, g inner; T = t / N.  score(g) = S_g[s] of the state at hand.
+template <class F>
+__device__ __forceinline__ double multigroup_mean(int G, const int* n, double N, F score) {
+    double m = 0.0;
+    for (int g = 0; g < G; ++g) m = __dadd_rn(m, __dmul_rn((double)n[g], (double)score(g)));
+    return __ddiv_rn(m, N);
+}
+
+template <class F>
+__device__ __forceinline__ double multigroup_add_state(double t, int G, const int* n, double m, F score) {
+    for (int g = 0; g < G; ++g) {
+        const double d = __dsub_rn((double)score(g), m);
+        t = __dadd_rn(t, __dmul_rn((double)n[g], __dmul_rn(d, d)));
+    }
+    return t;
+}
+
 // shared-memory tables of the sampler: log(i!), i = 0..width, then 1/i, i = 0..width+1
 __device__ __forceinline__ void fill_draw_tables(double* lf, double* inv, int width) {
     for (int i = threadIdx.x; i <= width; i += blockDim.x) lf[i] = lgamma((double)i + 1.0);

@@ -446,6 +446,88 @@ def permutation_exceedances_s1(cnt_a, cnt_b, size_a, size_b, seed, perm_offset, 
     return k
 
 
+def _group_sizes(sizes):
+    arr = (ctypes.c_int32 * len(sizes))(*[int(n) for n in sizes])
+    return arr, ctypes.cast(arr, ctypes.c_void_p)
+
+
+def _group_blocks(cnt):
+    """(groups, bins, K, group stride) of a CUDA int16 [G, bins, K] tensor whose [bins, K] blocks are contiguous; the
+    blocks may be spaced further apart (a bin range of a larger [G, rows, K] tensor)."""
+    if not (isinstance(cnt, torch.Tensor) and cnt.is_cuda and cnt.dtype == torch.int16 and cnt.dim() == 3):
+        raise TypeError("cnt must be a CUDA int16 tensor [groups, bins, K]")
+    G, bins, K = cnt.shape
+    if cnt.stride(2) != 1 or (bins > 1 and cnt.stride(1) != K) or (G > 1 and cnt.stride(0) < bins * K):
+        raise TypeError("cnt must hold each group's [bins, K] counts contiguously")
+    return G, bins, K, cnt.stride(0) if G > 1 else bins * K
+
+
+def multigroup_stat(scores, sizes):
+    """Multi-group statistic of every bin: scores float32 [G, bins, K] (group g at width sizes[g]) -> (T float64 [bins],
+    g* uint8 [bins], s* uint8 [bins], sign int8 [bins]), see include/epilogos_b200.h."""
+    _require_cuda(scores, torch.float32, "scores")
+    G, bins, K = scores.shape
+    if len(sizes) != G:
+        raise ValueError("one size per group")
+    t = torch.empty(bins, dtype=torch.float64, device=scores.device)
+    g = torch.empty(bins, dtype=torch.uint8, device=scores.device)
+    s = torch.empty(bins, dtype=torch.uint8, device=scores.device)
+    sign = torch.empty(bins, dtype=torch.int8, device=scores.device)
+    _arr, sz = _group_sizes(sizes)
+    _lib.call("epi_multigroup_stat", _ptr(scores), G, bins, K, sz, _ptr(t), _ptr(g), _ptr(s), _ptr(sign), _stream())
+    return t, g, s, sign
+
+
+def multigroup_shuffled_counts_range(cnt, sizes, seed, perm_offset, nperm, bin_offset=0):
+    """Permutations perm_offset .. perm_offset + nperm - 1 of every bin of the groups' counts cnt [G, bins, K], drawn on
+    the device: int16 [nperm, G, bins, K]."""
+    G, bins, K, stride = _group_blocks(cnt)
+    if len(sizes) != G:
+        raise ValueError("one size per group")
+    out = torch.empty((nperm, G, bins, K), dtype=torch.int16, device=cnt.device)
+    _arr, sz = _group_sizes(sizes)
+    _lib.call("epi_multigroup_shuffled_counts_range", _ptr(cnt), stride, G, bins, K, sz,
+              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(perm_offset), int(nperm), _ptr(out),
+              _stream())
+    return out
+
+
+def multigroup_null_exceedances(null, sizes, t, k):
+    """k[b] += #{p : T of null[p, :, b] >= t[b]}.  null: float32 scores [nperm, G, bins, K]; t float64 [bins]; k int32
+    [bins] holding uint32 counts (updated in place)."""
+    _require_cuda(null, torch.float32, "null")
+    _require_cuda(t, torch.float64, "t")
+    _require_cuda(k, torch.int32, "k")
+    nperm, G, bins, K = null.shape
+    if len(sizes) != G or t.numel() != bins or k.numel() != bins:
+        raise ValueError("one size per group, and t, k with one entry per bin")
+    _arr, sz = _group_sizes(sizes)
+    _lib.call("epi_multigroup_null_exceedances", _ptr(null), G, int(nperm), bins, K, sz, _ptr(t), _ptr(k), _stream())
+    return k
+
+
+def multigroup_s1_fused_fits(sizes, num_states):
+    """Whether epi_multigroup_exceedances_s1 takes these group widths (value tables and sampler in shared memory)."""
+    arr, sz = _group_sizes(sizes)
+    return _lib.load().epi_multigroup_s1_fused_fits(len(sizes), int(num_states), sz) == 1
+
+
+def multigroup_exceedances_s1(cnt, sizes, seed, perm_offset, nperm, bin_offset, exp1, t, k):
+    """Fused S1 multi-group permutation counts: k[b] += #{p : T_null(b, p) >= t[b]} over permutations perm_offset ..
+    perm_offset + nperm - 1, group g scored at width sizes[g] against exp1.  cnt int16 [G, bins, K]; k int32 [bins]."""
+    G, bins, K, stride = _group_blocks(cnt)
+    _require_cuda(exp1, torch.float32, "exp1")
+    _require_cuda(t, torch.float64, "t")
+    _require_cuda(k, torch.int32, "k")
+    if len(sizes) != G or t.numel() != bins or k.numel() != bins or exp1.numel() != K:
+        raise ValueError("one size per group, t and k with one entry per bin, exp1 one per state")
+    _arr, sz = _group_sizes(sizes)
+    _lib.call("epi_multigroup_exceedances_s1", _ptr(cnt), stride, G, bins, K, sz,
+              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(perm_offset), int(nperm), _ptr(exp1),
+              _ptr(t), _ptr(k), _stream())
+    return k
+
+
 def pairwise_combine(score_a=None, score_b=None, null_a=None, null_b=None):
     """(delta float32 [rows, K] or None, null_dist float32 [rows] or None)."""
     ref = score_a if score_a is not None else null_a

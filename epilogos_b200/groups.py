@@ -48,14 +48,21 @@ class GroupSet:
         """One group (single mode) or the comparison a vs b (paired mode)."""
         return Selection(self, a, b)
 
+    def select_multi(self, names):
+        """The multi-group comparison of the named (disjoint) groups (paired mode, --multigroup)."""
+        return Selection(self, names[0], multi=tuple(names))
+
 
 class Selection:
-    def __init__(self, groupset, a, b=None):
-        self.groupset, self.a, self.b = groupset, a, b
+    """One group, a comparison a vs b, or a multi-group comparison of the groups `multi` (its first group is `a`)."""
+
+    def __init__(self, groupset, a, b=None, multi=None):
+        self.groupset, self.a, self.b, self.multi = groupset, a, b, multi
 
     @property
     def paired(self):
-        return self.b is not None
+        """Whether the selection compares groups: the stage drivers then take the file as their second file too."""
+        return self.b is not None or self.multi is not None
 
 
 def parseGroups(path):
@@ -103,6 +110,31 @@ def parseGroups(path):
     if not names:
         raise GroupFileError("ERROR: [--groups] no group in {}".format(path))
     return GroupSet(names, columns)
+
+
+def parseMultigroups(specs, groupset):
+    """`--multigroup A,B,C` values -> [(A, B, C)]; raises GroupFileError with the first problem, checked in this order
+    over all values: an unknown name, a name listed twice, fewer than 2 names, two groups sharing a biosample."""
+    lists = [[n.strip() for n in spec.split(",") if n.strip()] for spec in specs]
+    for names in lists:
+        for n in names:
+            if n not in groupset.index:
+                raise GroupFileError("ERROR: [--multigroup] group '{}' is not defined in the group file".format(n))
+    for spec, names in zip(specs, lists):
+        dup = [n for i, n in enumerate(names) if n in names[:i]]
+        if dup:
+            raise GroupFileError("ERROR: [--multigroup] {!r} lists group '{}' twice".format(spec, dup[0]))
+    for spec, names in zip(specs, lists):
+        if len(names) < 2:
+            raise GroupFileError("ERROR: [--multigroup] {!r} names fewer than 2 groups".format(spec))
+    for names in lists:
+        for i, a in enumerate(names):
+            for b in names[i + 1:]:
+                shared = np.intersect1d(groupset.columns[groupset.index[a]], groupset.columns[groupset.index[b]])
+                if len(shared):
+                    raise GroupFileError("ERROR: [--multigroup] groups '{}' and '{}' share biosample {}".format(
+                        a, b, int(shared[0]) + 1))
+    return [tuple(names) for names in lists]
 
 
 def parseComparisons(specs, groupset):
@@ -162,6 +194,13 @@ class GroupView:
         self._shard, self.selection = shard, selection
         gs = selection.groupset
         gs.check_width(shard.states_a.shape[1], shard.file)
+        if selection.multi is not None:
+            self._idx = [gs.index[n] for n in selection.multi]
+            self.sizes = [len(gs.columns[i]) for i in self._idx]
+            self.states_a = GroupColumns(shard, np.sort(np.concatenate([gs.columns[i] for i in self._idx])))
+            self.states_b = None
+            self._all = self._dev = None
+            return
         self._ia = gs.index[selection.a]
         self._ib = gs.index[selection.b] if selection.paired else None
         self.states_a = GroupColumns(shard, gs.columns[self._ia])
@@ -178,10 +217,24 @@ class GroupView:
 
     @property
     def width(self):
+        if self.selection.multi is not None:
+            return self.states_a.shape[1]
         return self.states_a.shape[1] + (self.states_b.shape[1] if self.paired else 0)
+
+    def group_blocks(self):
+        """Counts of the groups of a multi-group comparison, int16 [G, rows, K], in the order they were named."""
+        import torch
+        cnt = group_counts(self._shard, self.selection.groupset)
+        return torch.stack([cnt[i] for i in self._idx])
 
     def counts(self, which="all"):
         cnt = group_counts(self._shard, self.selection.groupset)
+        if self.selection.multi is not None:          # "all": the union of the groups, the background's counts
+            if self._all is None:
+                self._all = self._shard.backend.add_counts(cnt[self._idx[0]], cnt[self._idx[1]])
+                for i in self._idx[2:]:
+                    self._all = self._shard.backend.add_counts(self._all, cnt[i])
+            return self._all
         if which == "b":
             return cnt[self._ib]
         if which == "a" or not self.paired:
@@ -191,6 +244,8 @@ class GroupView:
         return self._all
 
     def combined(self):
+        if self.selection.multi is not None:
+            return self.states_a
         gs = self.selection.groupset
         cols = gs.columns[self._ia] if not self.paired else np.concatenate((gs.columns[self._ia], gs.columns[self._ib]))
         return GroupColumns(self._shard, cols)
@@ -203,7 +258,7 @@ class GroupView:
 
 def view(shard, selection):
     """The GroupView of a selection of a shard, kept with the shard (its gathered matrix is reused by later stages)."""
-    key = (selection.groupset.key, selection.a, selection.b)
+    key = (selection.groupset.key, selection.a, selection.b, selection.multi)
     if key not in shard._views:
         shard._views[key] = GroupView(shard, selection)
     return shard._views[key]

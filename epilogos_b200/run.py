@@ -61,7 +61,8 @@ def checkFlags(mode, commandLineBool, inputDirectory, inputDirectory1, inputDire
                 return
 
 
-def checkGroupFlags(mode, inputDirectory, inputDirectory1, inputDirectory2, fileTag, groupFile, comparisons):
+def checkGroupFlags(mode, inputDirectory, inputDirectory1, inputDirectory2, fileTag, groupFile, comparisons,
+                    multigroups=()):
     """Flag rules of --groups / --compare (checked before checkFlags): first violated rule prints and exits."""
     rules = [
         (comparisons and not groupFile, "ERROR: [--compare] requires [--groups]"),
@@ -70,7 +71,7 @@ def checkGroupFlags(mode, inputDirectory, inputDirectory1, inputDirectory2, file
         (groupFile and inputDirectory2, "ERROR: [--groups] not compatible with [-b, --directory-two] option"),
         (groupFile and fileTag != "null", "ERROR: [--groups] not compatible with [-f, --file-tag] option"),
         (comparisons and mode != "paired", "ERROR: [--compare] requires [-m, --mode] 'paired'"),
-        (groupFile and mode == "paired" and not comparisons,
+        (groupFile and mode == "paired" and not comparisons and not multigroups,
          "ERROR: [-m, --mode] 'paired' with [--groups] requires at least one [--compare]"),
     ]
     for bad, message in rules:
@@ -132,6 +133,33 @@ def checkPermutationFlags(mode, nullPermutations):
             return
 
 
+def checkMultigroupFlags(mode, groupFile, multigroups, groupSet, pvalBool, groupSize):
+    """Rules of --multigroup (checked after every other rule): first violated rule prints and exits.  Returns the
+    comparisons, each a tuple of group names."""
+    if not multigroups:
+        return []
+    rules = [
+        (not groupFile, "ERROR: [--multigroup] requires [--groups]"),
+        (mode != "paired", "ERROR: [--multigroup] requires [-m, --mode] 'paired'"),
+    ]
+    for bad, message in rules:
+        if bad:
+            _die(message)
+            return []
+    from . import groups as _groups
+    try:
+        out = _groups.parseMultigroups(multigroups, groupSet)
+    except _groups.GroupFileError as exc:
+        _die(str(exc))
+        return []
+    for bad, message in ((pvalBool, "ERROR: [--multigroup] not compatible with [-n, --null-distribution] flag"),
+                         (groupSize != -1, "ERROR: [--multigroup] not compatible with [-g, --group-size] option")):
+        if bad:
+            _die(message)
+            return []
+    return out
+
+
 def deal_files(pairs, world):
     """Whole files dealt to the ranks, largest first to the least loaded rank (by size on disk): the same answer on every
     rank.  Returns a list of `world` lists of (file1, file2) pairs."""
@@ -163,7 +191,9 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
     3 scores all groups of a file, step 4 runs per group.  A comparison passes the file itself as the stage drivers'
     second file, which the group view does not read.
     `permutations` P > 0 (paired mode): step 3 also counts P null shuffles per bin and step 4 writes
-    pairwisePermutation_<tag>.txt.gz."""
+    pairwisePermutation_<tag>.txt.gz.  A multi-group comparison (a Selection with `multi`, --multigroup) scores its groups
+    in step 3 (epilogos_b200.multigroup), counting P shuffles per bin when P > 0, and step 4 runs
+    epilogos_b200.roi_multigroup."""
     from contextlib import nullcontext
     from . import dist, expected, expectedCombination, scores, session
     world = dist.world_size()
@@ -223,12 +253,15 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
             for out, tag, exp_path, _ in runs:
                 roi.main(out, stateInfo, tag, exp_path, roiWidth, verbose)
     else:
-        from . import pairwise, roi_pairwise
+        from . import pairwise, roi_multigroup, roi_pairwise
         seed = pairwise.run_seed() if pvalBool else None      # every rank takes part in drawing a fresh seed
         say("\nSTEP 4: " + ("Fitting the null distribution, p-values and regions of interest" if pvalBool
                             else "Pairwise metrics and regions of interest"))
         if dist.rank() == 0:
-            for out, tag, exp_path, _ in runs:
+            for out, tag, exp_path, sel in runs:
+                if sel is not None and sel.multi is not None:
+                    roi_multigroup.main(out, stateInfo, tag, exp_path, roiWidth, verbose, backend=backend)
+                    continue
                 roi_pairwise.main(out, stateInfo, tag, exp_path, roiWidth, pvalBool, numTrials, samplingSize,
                                   diagnosticBool, verbose, backend=backend, seed=seed)
 
@@ -258,7 +291,8 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
               help="Paired mode with -n: the size of each subsample of the null distances that is fit")
 @click.option("-q", "--quiescent-state", "quiescentState", type=int, default=-1,
               help="If a bin contains only states of this value, it is treated as quiescent and not factored into "
-                   + "fitting. If set to 0, filtering is not done. [default: last state]")
+                   + "fitting. If set to 0, filtering is not done. [default: last state]  No effect on a --multigroup "
+                   + "comparison, which fits nothing")
 @click.option("-g", "--group-size", "groupSize", type=int, default=-1, show_default=True,
               help="In pairwise epilogos controls the sizes of the shuffled arrays. "
                    + "Default is sizes of the input groups")
@@ -278,6 +312,12 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
                    + "OUT/<A>_vs_<B>")
 @click.option("--compare", "comparisons", type=str, multiple=True,
               help="Paired mode with --groups: compare group A with group B (A:B, repeatable)")
+@click.option("--multigroup", "multigroups", type=str, multiple=True,
+              help="Paired mode with --groups: one test per bin across the disjoint groups A,B,C,... (2 to 64, "
+                   + "repeatable), written to OUT/A_B_C: multigroupMetrics_<tag>.txt.gz (per bin the size-weighted "
+                   + "between-group sum of squares T of the group scores, the group and state that drive it, the sign, "
+                   + "and with --null-permutations P the count of P label shuffles with a T as large, p and BH) and "
+                   + "regionsOfInterest_<tag>.txt.  Not with -n or -g")
 @click.option("--null-permutations", "nullPermutations", type=int, default=None,
               help="Paired mode: draw P null shuffles of every bin on the GPU and write pairwisePermutation_<tag>.txt.gz "
                    + "with each bin's count of shuffles at least as far apart as its groups, its permutation p-value "
@@ -288,15 +328,15 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
 @click.option("--roi-mem", "roiMem", type=int, default=-1, help="SLURM-only (ignored)")
 def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2, outputDirectory, stateInfo, saliency,
          numProcesses, exitBool, diagnosticBool, numTrials, samplingSize, quiescentState, groupSize, version, partition,
-         pvalBool, roiWidth, fileTag, groupFile, comparisons, nullPermutations, expFreqMem, expCombMem, scoreMem,
-         roiMem):
+         pvalBool, roiWidth, fileTag, groupFile, comparisons, multigroups, nullPermutations, expFreqMem, expCombMem,
+         scoreMem, roiMem):
     """Information-theoretic navigation of multi-tissue functional genomic annotations (B200 scoring path)."""
     if version:
         from epilogos_b200 import __version__
         print("Version:", __version__)
         sys.exit()
 
-    checkGroupFlags(mode, inputDirectory, inputDirectory1, inputDirectory2, fileTag, groupFile, comparisons)
+    checkGroupFlags(mode, inputDirectory, inputDirectory1, inputDirectory2, fileTag, groupFile, comparisons, multigroups)
     if groupFile and mode == "paired":       # both groups of a comparison come from the files of -i
         inputDirectory, inputDirectory1, inputDirectory2 = None, inputDirectory, inputDirectory
     checkFlags(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2, outputDirectory, stateInfo,
@@ -323,6 +363,7 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
     checkArguments(mode, saliency, inputDirPath, inputDirPath2, outputDirPath, numProcesses, numStates, numTrials,
                    samplingSize, quiescentState, groupSize, roiWidth)
     checkPermutationFlags(mode, nullPermutations)
+    multi_of_groups = checkMultigroupFlags(mode, groupFile, multigroups, groupSet, pvalBool, groupSize)
 
     import torch
     import torch.distributed as td
@@ -357,7 +398,8 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
         # every group / comparison behaves like a run on its column-subset files in a directory named after it
         sel = ([(g, "{}_s{}".format(g, saliency), groupSet.select(g)) for g in groupSet.names] if mode == "single" else
                [("{}_vs_{}".format(a, b), "{}_{}_s{}".format(a, b, saliency), groupSet.select(a, b))
-                for a, b in pairs_of_groups])
+                for a, b in pairs_of_groups] +
+               [("_".join(m), "{}_s{}".format("_".join(m), saliency), groupSet.select_multi(m)) for m in multi_of_groups])
         runs = [(outputDirPath / d, tag, outputDirPath / d / "exp_freq_{}.npy".format(tag), s) for d, tag, s in sel]
     for f in files:
         if runs is not None:

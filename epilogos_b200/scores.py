@@ -24,7 +24,11 @@ def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, num
     filename = file1Path.name.split(".")[0]
     if not verbose and dist.rank() == 0:
         print("    {}\t".format(filename), end="", flush=True)
-    if str(file2) == "null":
+    if group is not None and group.multi is not None:
+        from .multigroup import calculateScoresMultigroup
+        calculateScoresMultigroup(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
+                                  backend, group=group, permutations=permutations)
+    elif str(file2) == "null":
         calculateScores(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
                         backend, group=group)
     else:

@@ -78,6 +78,32 @@ def write_permutations_text(path, loc, k, pval, bh, level=None, threads=0):
               p(pval), p(bh), len(k), int(_gzip_level(level)), int(threads))
 
 
+def write_multigroup_text(path, loc, t, group, state, sign, group_names, state_names, k=None, pval=None, bh=None,
+                          level=None, threads=0):
+    """multigroupMetrics_<tag>.txt.gz through the native writer (epi_write_multigroup_gz): per bin `chr \t start \t end
+    \t "%.5e" T \t <driving group> \t <driving state> \t +/- [\t k \t "%.5e" p \t "%.5e" BH]`; group and state are
+    0-based indices into group_names and state_names."""
+    names, cid, starts, ends = _native_locations(loc)
+    t = np.ascontiguousarray(t, dtype=np.float64)
+    group = np.ascontiguousarray(group, dtype=np.uint8)
+    state = np.ascontiguousarray(state, dtype=np.uint8)
+    sign = np.ascontiguousarray(sign, dtype=np.int8)
+    if not (len(t) == len(group) == len(state) == len(sign) == len(starts)):
+        raise ValueError("one statistic, group, state and sign per bin")
+    if not ((k is None) == (pval is None) == (bh is None)):
+        raise ValueError("counts, p-values and adjusted p-values go together")
+    if k is not None:
+        k = np.ascontiguousarray(k, dtype=np.uint32)
+        pval = np.ascontiguousarray(pval, dtype=np.float64)
+        bh = np.ascontiguousarray(bh, dtype=np.float64)
+    p = lambda a: ctypes.c_void_p(0 if a is None else a.ctypes.data)
+    gnames = b"\0".join(str(n).encode() for n in group_names) + b"\0"
+    states = b"\0".join(str(n).encode() for n in state_names) + b"\0"
+    _lib.call("epi_write_multigroup_gz", str(path).encode(), ctypes.c_char_p(names), p(cid), p(starts), p(ends), p(t),
+              p(group), p(state), p(sign), ctypes.c_char_p(gnames), len(group_names), ctypes.c_char_p(states),
+              len(state_names), p(k), p(pval), p(bh), len(t), int(_gzip_level(level)), int(threads))
+
+
 def location_array(loc):
     """object [rows, 3] array as produced by pd.read_table(...).to_numpy() in scores.py:161."""
     arr = np.empty((len(loc["chrom"]), 3), dtype=object)

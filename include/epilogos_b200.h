@@ -196,6 +196,46 @@ int epi_permutation_exceedances_s1(const uint16_t* cnt_a_dev, const uint16_t* cn
                                    int32_t width_a, int32_t width_b, const float* dist_dev, uint32_t* k_inout,
                                    void* stream);
 
+/* ---- multi-group comparisons (csrc/multigroup.cu) ------------------------------------------------------------
+ * G = groups (2..EPI_MAX_GROUPS) disjoint groups of biosamples; sizes: HOST array of the G group widths n_g >= 1 with
+ * N = sum n_g <= 65535.  S_g [bins][K] float32 is group g's score at width n_g against the background of the union.  Per
+ * bin, in float64 without fused multiply-add:
+ *     m[s] = (sum_g n_g S_g[s]) / N,   T = (sum_s sum_g n_g (S_g[s] - m[s])^2) / N
+ * summed over g ascending for m, and in one running sum with s outer and g inner (both ascending) for T.
+ *   epi_multigroup_stat                   scores [G][bins][K] -> t_out [bins] = T, group_out = g* =
+ *                                         argmax_g n_g sum_s (S_g[s] - m[s])^2, state_out = s* = argmax_s
+ *                                         |S_g*[s] - m[s]| (first on ties; 0-based), sign_out = -1 if S_g*[s*] < m[s*]
+ *                                         else +1.
+ *   epi_multigroup_shuffled_counts_range  permutations perm_offset .. perm_offset + nperm - 1 of every bin, drawn from the
+ *                                         stream of epi_shuffled_counts_philox (seed, permutation, GLOBAL bin
+ *                                         bin_offset + b): for every state in order and every group in order, the
+ *                                         group's count is HG(labels unassigned, labels of the state unassigned, labels
+ *                                         the group still needs).  cnt [G] blocks of [bins][K], block g at
+ *                                         cnt_dev + g * group_stride; out [nperm][G][bins][K].  With G = 2 and
+ *                                         n_0 + n_1 the union's width, equal to epi_shuffled_counts_philox_range.
+ *   epi_multigroup_null_exceedances       k[b] += #{p < nperm : T of null[p][.][b][.] >= t[b]}; null [nperm][G][bins][K]
+ *                                         float32 scores of shuffled counts.
+ *   epi_multigroup_exceedances_s1         fused S1: draws as epi_multigroup_shuffled_counts_range, scores group g at
+ *                                         width n_g against exp1 [K] with the values epi_scores_s1 gives, and counts as
+ *                                         epi_multigroup_null_exceedances.  Equal bit for bit to that composed path.
+ *                                         Takes the shapes epi_multigroup_s1_fused_fits accepts.
+ *   epi_multigroup_s1_fused_fits          1 if the fused S1 kernel takes this shape (every n_g <= 4095 and its tables
+ *                                         fit in shared memory), else 0.  Needs no device.
+ * k is ADDED to, so permutation blocks accumulate; no (bin, permutation) value is stored by the fused path. */
+int epi_multigroup_stat(const float* scores_dev, int32_t groups, int64_t bins, int32_t num_states, const int32_t* sizes,
+                        double* t_out, uint8_t* group_out, uint8_t* state_out, int8_t* sign_out, void* stream);
+int epi_multigroup_shuffled_counts_range(const uint16_t* cnt_dev, int64_t group_stride, int32_t groups, int64_t bins,
+                                         int32_t num_states, const int32_t* sizes, uint64_t seed, int64_t bin_offset,
+                                         int64_t perm_offset, int32_t nperm, uint16_t* out_dev, void* stream);
+int epi_multigroup_null_exceedances(const float* null_dev, int32_t groups, int32_t nperm, int64_t bins,
+                                    int32_t num_states, const int32_t* sizes, const double* t_dev, uint32_t* k_inout,
+                                    void* stream);
+int epi_multigroup_exceedances_s1(const uint16_t* cnt_dev, int64_t group_stride, int32_t groups, int64_t bins,
+                                  int32_t num_states, const int32_t* sizes, uint64_t seed, int64_t bin_offset,
+                                  int64_t perm_offset, int32_t nperm, const float* exp1_dev, const double* t_dev,
+                                  uint32_t* k_inout, void* stream);
+int epi_multigroup_s1_fused_fits(int32_t groups, int32_t num_states, const int32_t* sizes);
+
 /* ---- paired statistics stage (roiAndVisualPairwise.py:177-242, csrc/pairwise_stats.cu) -----------------------
  *   epi_null_compact       the null distances of the bins whose quiescent flag is 0 (all bins when quiescent_dev is NULL),
  *                          stable order, every permutation: null_dev float32 [nperm][bins] -> pool_out [nperm][count]
@@ -338,6 +378,15 @@ int epi_write_metrics_gz(const char* path, const char* chrom_names, const int32_
 int epi_write_permutations_gz(const char* path, const char* chrom_names, const int32_t* chrom_id, const int64_t* starts,
                               const int64_t* ends, const uint32_t* k, const double* pval, const double* bh, int64_t rows,
                               int32_t level, int32_t threads);
+/* multigroupMetrics text through gzip, one line per bin: `chr \t start \t end \t "%.5e" T \t <name of group g*> \t
+ * <name of state s*> \t + or - [\t k \t "%.5e" p \t "%.5e" bh]` (group and state 0-based indices into the NUL-separated
+ * group_names and state_names; sign < 0 prints -); the last three columns only when k, pval and bh are all given.  Same
+ * deflate path as epi_write_scores_gz. */
+int epi_write_multigroup_gz(const char* path, const char* chrom_names, const int32_t* chrom_id, const int64_t* starts,
+                            const int64_t* ends, const double* t, const uint8_t* group, const uint8_t* state,
+                            const int8_t* sign, const char* group_names, int32_t groups, const char* state_names,
+                            int32_t num_states, const uint32_t* k, const double* pval, const double* bh, int64_t rows,
+                            int32_t level, int32_t threads);
 /* ChromHMM `-printstatebyline` files (one per biosample and chromosome: `<biosample> <chr>`, `MaxState E`, then one label per
  * 200 bp bin) -> matrix: the native form of bin/preprocess_data_ChromHMM.sh:34-49, which pastes those files side by side.
  * epi_statebyline_read  parses ONE file into a column: out[r * stride] = label - 1 for bin r (out == NULL: count only);
