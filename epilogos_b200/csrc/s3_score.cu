@@ -30,10 +30,12 @@
 namespace epi {
 
 constexpr int S3S_THREADS = 256;          // consumer threads (+ 32 producer threads)
+constexpr int S3S_JC = 8;                 // biosamples per j-block
 
 __host__ __device__ inline long long s3_block_stride(int K) { return ((long long)K * K + 1) & ~1ll; }   // 16-byte blocks
 
-// terms in padded block layout: block (i*C + j) holds K*K doubles [a][c] (+ pad), JC_MAX zero blocks at the end
+// terms in padded block layout: block (i*C + j) holds K*K doubles [a][c] (+ pad), S3S_JC zero blocks at the end
+// (the last slab of a row starts at most S3S_JC - 1 blocks before the end of the row)
 __global__ void __launch_bounds__(256) s3_terms_kernel(const float* __restrict__ e3, int cols, int K, double q,
                                                        double* __restrict__ terms, long long nblocks_total) {
     const long long blk = s3_block_stride(K);
@@ -293,15 +295,13 @@ static int launch_s3_score(const uint8_t* xt, int64_t bp, int64_t bins, int cols
     return 0;
 }
 
-constexpr int S3S_JC_MAX = 8;
-
 }  // namespace epi
 
 using namespace epi;
 
 extern "C" int epi_s3_terms_size(int32_t cols, int32_t K, int64_t* doubles_out) {
     EPI_REQUIRE(cols >= 2 && K >= 1 && K <= EPI_MAX_STATES && doubles_out != nullptr, "bad S3 shape");
-    *doubles_out = ((int64_t)cols * cols + S3S_JC_MAX) * s3_block_stride(K);
+    *doubles_out = ((int64_t)cols * cols + S3S_JC) * s3_block_stride(K);
     return 0;
 }
 
@@ -311,7 +311,7 @@ extern "C" int epi_s3_terms(const float* exp3_dev, int32_t cols, int32_t K, doub
     EPI_REQUIRE(cols >= 2 && K >= 1 && K <= EPI_MAX_STATES, "bad S3 shape (needs at least 2 biosamples)");
     EPI_REQUIRE(exp3_dev != nullptr && terms_dev != nullptr, "null pointer argument");
     EPI_REQUIRE((reinterpret_cast<uintptr_t>(terms_dev) & 15) == 0, "terms_dev must be 16-byte aligned");
-    const long long nblocks = (long long)cols * cols + S3S_JC_MAX;
+    const long long nblocks = (long long)cols * cols + S3S_JC;
     const long long n = nblocks * s3_block_stride(K);
     const double q = 1.0 / ((double)cols * (double)(cols - 1));
     long long blocks = (n + 255) / 256;
@@ -330,14 +330,14 @@ extern "C" int epi_scores_s3(const int8_t* x_dev, int64_t bins, int32_t cols, in
     if (bins == 0 || (out32_dev == nullptr && out64_dev == nullptr)) return 0;
     EPI_REQUIRE(x_dev != nullptr && terms_dev != nullptr, "null pointer argument");
     EPI_REQUIRE((reinterpret_cast<uintptr_t>(terms_dev) & 15) == 0, "terms_dev must be 16-byte aligned");
-    // choose the blocking that fits 227 KB of shared memory: score rows BC*K*8 + two slabs JC*blk*8
+    // choose the bins per thread so that score rows BC*K*8 + two slabs JC*blk*8 fit 220 KB of shared memory.  JC = 8 fits
+    // at BPT = 1 for every K <= 32 (66 KB of rows + 128 KB of slabs at K = 32); the check guards a larger EPI_MAX_STATES.
     const size_t blk8 = (size_t)s3_block_stride(K) * 8;
-    int bpt = 4, jc = 8;
-    auto fits = [&](int b, int j) { return (size_t)S3S_THREADS * b * (K | 1) * 8 + 2 * (size_t)j * blk8 + 256 <= 220 * 1024; };
+    int bpt = 4;
+    auto fits = [&](int b) { return (size_t)S3S_THREADS * b * (K | 1) * 8 + 2 * (size_t)S3S_JC * blk8 + 256 <= 220 * 1024; };
     if (bins <= S3S_THREADS * 2) bpt = bins <= S3S_THREADS ? 1 : 2;              // small inputs: more CTAs
-    while (!fits(bpt, jc) && bpt > 1) bpt >>= 1;
-    while (!fits(bpt, jc) && jc > 2) jc >>= 1;
-    EPI_REQUIRE(fits(bpt, jc), "S3 score blocking does not fit shared memory for K=%d", K);
+    while (!fits(bpt) && bpt > 1) bpt >>= 1;
+    EPI_REQUIRE(fits(bpt), "S3 score blocking does not fit shared memory for K=%d", K);
     DeviceWorkspace* ws = device_workspace();
     EPI_REQUIRE(ws != nullptr, "could not allocate the per-device workspace");
     const int64_t bc = (int64_t)S3S_THREADS * bpt;
@@ -351,9 +351,8 @@ extern "C" int epi_scores_s3(const int8_t* x_dev, int64_t bins, int32_t cols, in
     EPI_CUDA(cudaMemsetAsync(gate, 1, 4, st));
     s3_symmetry_kernel<<<sm_count() * 8, 256, 0, st>>>(terms_dev, cols, K, gate);
     int rc = 0;
-#define EPI_S3S_CASE(B, J) if (bpt == B && jc == J) rc = launch_s3_score<B, J>(xt, bp, bins, cols, K, terms_dev, gate, out32_dev, out64_dev, st); else
-    EPI_S3S_CASE(4, 8) EPI_S3S_CASE(2, 8) EPI_S3S_CASE(1, 8) EPI_S3S_CASE(4, 4) EPI_S3S_CASE(2, 4) EPI_S3S_CASE(1, 4)
-    EPI_S3S_CASE(1, 2) { set_error("no S3 score kernel for blocking %d x %d", bpt, jc); rc = 2; }
+#define EPI_S3S_CASE(B) if (bpt == B) rc = launch_s3_score<B, S3S_JC>(xt, bp, bins, cols, K, terms_dev, gate, out32_dev, out64_dev, st); else
+    EPI_S3S_CASE(4) EPI_S3S_CASE(2) EPI_S3S_CASE(1) { set_error("no S3 score kernel for %d bins per thread", bpt); rc = 2; }
 #undef EPI_S3S_CASE
     cudaFreeAsync(xt, st);
     return rc;

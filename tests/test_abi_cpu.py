@@ -49,6 +49,28 @@ def test_no_cpu_fallback(lib):
     assert "no CPU fallback" in msg or "CUDA" in msg
 
 
+@pytest.mark.parametrize("bins,cols,k", [(0, 2, 1), (1, 16, 16), (129, 17, 16), (300_001, 833, 18), (20_001, 1422, 18),
+                                         (50_001, 400, 25), (7, 4096, 32)])
+def test_s3_plan_closed_form(lib, bins, cols, k):
+    """epi_s3_plan (no device needed): one-hot rows padded to 256-row blocks, bins to 128-bin k-steps, the 128 x 256 tiles
+    of the blocks on or above the diagonal, and the tile buffer with its (row tile, block column) -> tile index behind.
+    C*K = 131,072 is the largest schedule (512 block columns in 64 raster groups)."""
+    from epilogos_b200 import engine
+    mp = -(-cols * k // 256) * 256
+    bp = -(-bins // 128) * 128
+    nt = mp // 256
+    ntiles = nt * (nt + 1)
+    assert engine.s3_plan(bins, cols, k) == dict(mp=mp, bp=bp, ntiles=ntiles, onehot_bytes=mp * bp,
+                                                 tile_bytes=ntiles * 128 * 256 * 4 + (mp // 128) * nt * 4)
+
+
+def test_s3_plan_refuses_a_schedule_past_64_raster_groups(lib):
+    from epilogos_b200 import _lib, engine
+    assert engine.s3_plan(1, 4096, 32)["mp"] == 131072
+    with pytest.raises(_lib.EpilogosB200Error, match="biosamples x states = 131073 is too large for the S3 tile schedule"):
+        engine.s3_plan(1, 43691, 3)
+
+
 def test_missing_library_fails_loudly(monkeypatch, tmp_path):
     """No silent fallback: if the shared library is absent the binding raises with build instructions."""
     from epilogos_b200 import _lib

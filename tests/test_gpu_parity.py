@@ -428,9 +428,8 @@ def test_s3_expected_and_scores_match_reference_goldens(eng, golden, name):
     ref_terms = orc.s3_pair_terms(c, g["s3_exp"], np.float64)
     np.testing.assert_allclose(eng.s3_terms_dense(terms, c, k).cpu().numpy(), ref_terms, rtol=1e-13, atol=0)
     s32, s64 = eng.scores_s3(xd, c, k, terms, want64=True)
-    sub = slice(0, 400)
-    ref64 = orc.s3_scores_f64(x[sub], k, g["s3_exp"])
-    np.testing.assert_allclose(s64.cpu().numpy()[sub], ref64, rtol=RTOL, atol=ATOL)
+    ref64 = orc.s3_scores_f64(x, k, g["s3_exp"])
+    np.testing.assert_allclose(s64.cpu().numpy(), ref64, rtol=RTOL, atol=ATOL)
     # the reference's own float32 result carries accumulation noise (SURVEY.md 8c): agree to 2e-2 absolute
     assert np.max(np.abs(s32.cpu().numpy() - g["s3_scores"])) < 2e-2
 
@@ -753,8 +752,9 @@ def test_paired_real_reductions_with_text_round_trip(eng):
 
 
 def test_s3_chr1_shape_properties(eng):
-    """BASELINE configs[2] at full size (1.25 M bins x 833 biosamples x 18 states): closed-form total, symmetry,
-    empty diagonal blocks of the tensor-core Gram table; scores of a sample against the float64 oracle."""
+    """BASELINE configs[2] at full size (1.25 M bins x 833 biosamples x 18 states): closed-form total, empty diagonal
+    blocks and one pair of the tensor-core Gram table; scores of a sample against the float64 oracle.  (The table is
+    symmetric by construction of epi_s3_finalize; tests/test_s3_gpu.py compares whole tables in steady state.)"""
     from epilogos_b200 import synth
     bins, cols, k = 1_250_000, 833, 18
     x = synth.synth_states_device(bins, cols, k, seed=22)
@@ -763,9 +763,6 @@ def test_s3_chr1_shape_properties(eng):
     assert int(counts.sum()) == bins * cols * (cols - 1)                         # SURVEY 8a closed form
     idx = torch.arange(cols, device="cuda")
     assert not bool(counts[idx, idx].any())                                      # i == j blocks stay empty
-    for lo in range(0, cols, 64):                                                # N3[i,j,a,c] == N3[j,i,c,a]
-        blk = counts[lo:lo + 64]
-        assert torch.equal(blk, counts[:, lo:lo + 64].permute(1, 0, 3, 2))
     # pair (0, 1): against a direct 2-D histogram of the two label columns
     pair = torch.bincount(x[:, 0].long() * k + x[:, 1].long(), minlength=k * k).reshape(k, k)
     assert torch.equal(counts[0, 1], pair)
