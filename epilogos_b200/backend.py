@@ -125,20 +125,15 @@ class CudaBackend:
             with timing.stage("kernels", sync_cuda=True):
                 return engine.permutation_exceedances_s1(cnt_a, cnt_b, size_a, size_b, seed, 0, nperm, width, bin_offset,
                                                          exp, score_widths[0], score_widths[1], dist, k)
-        pairs = max(1, int(workspace_bytes) // (12 * k_states))       # A', B' counts (uint16) and scores (float32)
-        chunk = max(1, min(rows, pairs))
-        block = max(1, min(nperm, pairs // chunk))
         with timing.stage("kernels", sync_cuda=True):
-            for lo in range(0, rows, chunk):
-                hi = min(rows, lo + chunk)
-                for p0 in range(0, nperm, block):
-                    n = min(block, nperm - p0)
-                    oa, ob = engine.shuffled_counts_philox_range(cnt_a[lo:hi], cnt_b[lo:hi], size_a, size_b, seed, p0, n,
-                                                                 width, bin_offset=bin_offset + lo)
-                    sa = self.scores(oa.reshape(-1, k_states), score_widths[0], saliency, exp, perms=perms[0], exact=exact)
-                    sb = self.scores(ob.reshape(-1, k_states), score_widths[1], saliency, exp, perms=perms[1], exact=exact)
-                    engine.null_exceedances(sa.reshape(n, hi - lo, k_states), sb.reshape(n, hi - lo, k_states),
-                                            dist[lo:hi], k[lo:hi])
+            # A', B' counts (uint16) and scores (float32)
+            for lo, hi, p0, n in self._blocks(rows, nperm, workspace_bytes, 12 * k_states):
+                oa, ob = engine.shuffled_counts_philox_range(cnt_a[lo:hi], cnt_b[lo:hi], size_a, size_b, seed, p0, n,
+                                                             width, bin_offset=bin_offset + lo)
+                sa = self.scores(oa.reshape(-1, k_states), score_widths[0], saliency, exp, perms=perms[0], exact=exact)
+                sb = self.scores(ob.reshape(-1, k_states), score_widths[1], saliency, exp, perms=perms[1], exact=exact)
+                engine.null_exceedances(sa.reshape(n, hi - lo, k_states), sb.reshape(n, hi - lo, k_states),
+                                        dist[lo:hi], k[lo:hi])
         return k
 
     # -- multi-group comparisons ------------------------------------------------------------------------
@@ -159,14 +154,19 @@ class CudaBackend:
         return sc if out is None else out
 
     @staticmethod
-    def _bin_chunks(rows, chunk):
-        """[lo, hi) ranges of at most `chunk` bins whose lengths are multiples of 8, then the tail of rows % 8 bins: every
-        [G, hi - lo, K] block of uint16 counts or float32 scores then starts on 16 bytes, except in the tail."""
+    def _blocks(rows, nperm, workspace_bytes, cell_bytes):
+        """(lo, hi, p0, n): bin chunks [lo, hi) x permutation blocks p0 .. p0 + n - 1 whose buffers, `cell_bytes` per
+        (bin, shuffle), stay below `workspace_bytes` (eight bins and one shuffle at the least).  Chunk lengths are
+        multiples of 8, then comes the tail of rows % 8 bins: every [.., hi - lo, K] block of uint16 counts or float32
+        scores then starts on 16 bytes, except in the tail."""
+        cells = max(1, int(workspace_bytes) // cell_bytes)
         body = rows - rows % 8
-        step = max(8, chunk - chunk % 8)
+        step = max(8, cells - cells % 8)
         edges = list(range(0, body, step)) + [body]
-        out = [(lo, hi) for lo, hi in zip(edges[:-1], edges[1:])]
-        return out + ([(body, rows)] if body < rows else [])
+        for lo, hi in list(zip(edges[:-1], edges[1:])) + ([(body, rows)] if body < rows else []):
+            block = max(1, min(nperm, cells // (hi - lo)))
+            for p0 in range(0, nperm, block):
+                yield lo, hi, p0, min(block, nperm - p0)
 
     def multigroup_stat(self, cnt, sizes, saliency, exp, exact=False, workspace_bytes=1 << 30):
         """(T float64, g* uint8, s* uint8, sign int8), each [bins], of the groups' counts cnt int16 [G, bins, K] (group g
@@ -178,9 +178,9 @@ class CudaBackend:
                torch.empty(rows, dtype=torch.uint8, device=self.device),
                torch.empty(rows, dtype=torch.uint8, device=self.device),
                torch.empty(rows, dtype=torch.int8, device=self.device))
-        chunk = max(1, int(workspace_bytes) // (4 * G * k_states))
         with timing.stage("kernels", sync_cuda=True):
-            for lo, hi in self._bin_chunks(rows, chunk):
+            # bin chunks only: with one "shuffle" every chunk is a single block
+            for lo, hi, _, _ in self._blocks(rows, 1, workspace_bytes, 4 * G * k_states):
                 sc = torch.empty((G, hi - lo, k_states), dtype=torch.float32, device=self.device)
                 for g, n in enumerate(sizes):
                     self._group_scores(cnt[g, lo:hi], n, saliency, exp, exact, out=sc[g])
@@ -202,19 +202,16 @@ class CudaBackend:
         if saliency == 1 and engine.multigroup_s1_fused_fits(sizes, k_states):
             with timing.stage("kernels", sync_cuda=True):
                 return engine.multigroup_exceedances_s1(cnt, sizes, seed, 0, nperm, bin_offset, exp, t, k)
-        cells = max(1, int(workspace_bytes) // (6 * G * k_states))     # shuffled counts (uint16) and scores (float32)
         with timing.stage("kernels", sync_cuda=True):
-            for lo, hi in self._bin_chunks(rows, cells):
-                block = max(1, min(nperm, cells // (hi - lo)))
-                for p0 in range(0, nperm, block):
-                    n = min(block, nperm - p0)
-                    oc = engine.multigroup_shuffled_counts_range(cnt[:, lo:hi], sizes, seed, p0, n, bin_offset + lo)
-                    sc = torch.empty((n, G, hi - lo, k_states), dtype=torch.float32, device=self.device)
-                    for p in range(n):
-                        for g, size in enumerate(sizes):
-                            self._group_scores(oc[p, g], size, saliency, exp, exact, out=sc[p, g])
-                    del oc
-                    engine.multigroup_null_exceedances(sc, sizes, t[lo:hi], k[lo:hi])
+            # shuffled counts (uint16) and scores (float32)
+            for lo, hi, p0, n in self._blocks(rows, nperm, workspace_bytes, 6 * G * k_states):
+                oc = engine.multigroup_shuffled_counts_range(cnt[:, lo:hi], sizes, seed, p0, n, bin_offset + lo)
+                sc = torch.empty((n, G, hi - lo, k_states), dtype=torch.float32, device=self.device)
+                for p in range(n):
+                    for g, size in enumerate(sizes):
+                        self._group_scores(oc[p, g], size, saliency, exp, exact, out=sc[p, g])
+                del oc
+                engine.multigroup_null_exceedances(sc, sizes, t[lo:hi], k[lo:hi])
         return k
 
     def pairwise_combine(self, score_a, score_b, null_a, null_b):

@@ -41,6 +41,14 @@ int sm_count() {
     return g_sm_count > 0 ? g_sm_count : 148;
 }
 
+unsigned grid_for(long long n, int per_block, int per_sm) {
+    long long blocks = (n + per_block - 1) / per_block;
+    const long long cap = (long long)sm_count() * per_sm;
+    if (blocks > cap) blocks = cap;
+    if (blocks < 1) blocks = 1;
+    return (unsigned)blocks;
+}
+
 tensor_map_encode_fn get_tensor_map_encode() {
     static tensor_map_encode_fn fn = nullptr;
     if (fn == nullptr) {

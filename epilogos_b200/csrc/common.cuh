@@ -34,6 +34,7 @@ int check_device();   // 0 if an sm_100 device is current, else sets the error a
     } while (0)
 
 int sm_count();
+unsigned grid_for(long long n, int per_block, int per_sm);   // min(ceil(n / per_block), SMs * per_sm), at least 1
 int persistent_grid(int64_t ntiles, int per_sm);   // min(ntiles, SMs * per_sm), at least 1
 
 // ---- per-device workspace ---------------------------------------------------------------------

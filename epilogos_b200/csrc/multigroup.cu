@@ -26,14 +26,6 @@ struct GroupSizes {
 constexpr int K10_THREADS = 256;
 constexpr int K10_STAT_THREADS = 128;
 
-static unsigned mg_grid(long long n, int per_block, int per_sm) {
-    long long blocks = (n + per_block - 1) / per_block;
-    const long long cap = (long long)sm_count() * per_sm;
-    if (blocks > cap) blocks = cap;
-    if (blocks < 1) blocks = 1;
-    return (unsigned)blocks;
-}
-
 // m[s] lives in shared memory, m[s * blockDim + thread]: the driver needs it after T is complete.
 __global__ void __launch_bounds__(K10_STAT_THREADS) multigroup_stat_kernel(const float* __restrict__ sc, int G,
                                                                            long long bins, int K, GroupSizes sz, int N,
@@ -162,8 +154,8 @@ __global__ void __launch_bounds__(K10_THREADS) multigroup_exceedances_s1_kernel(
     for (int i = threadIdx.x; i < nvt; i += blockDim.x) vt[i] = vt_g[i];
     __syncthreads();
     uint16_t* comb = comb_all + (threadIdx.x / T) * K;
-    const int lane = threadIdx.x & 31, t = threadIdx.x % T;
-    const unsigned gmask = T == 32 ? 0xffffffffu : (((1u << (T % 32)) - 1u) << (lane & ~(T - 1)));
+    const int t = threadIdx.x % T;
+    const unsigned gmask = group_mask<T>();
     const double dN = (double)N;
     for (long long b = blockIdx.x * (long long)SLOTS + threadIdx.x / T; b < bins; b += (long long)gridDim.x * SLOTS) {
         const double thr = tb[b];
@@ -195,8 +187,7 @@ __global__ void __launch_bounds__(K10_THREADS) multigroup_exceedances_s1_kernel(
                 });
             c += __ddiv_rn(tn, dN) >= thr ? 1u : 0u;
         }
-#pragma unroll
-        for (int off = T / 2; off > 0; off >>= 1) c += __shfl_xor_sync(gmask, c, off);
+        c = group_sum<T>(gmask, c);
         if (t == 0) k[b] += c;
     }
 }
@@ -221,14 +212,6 @@ static int read_sizes(const int32_t* sizes, int G, GroupSizes* sz, int* N) {
     return 0;
 }
 
-static int check_perm_range(int64_t bin_offset, int64_t perm_offset, int32_t nperm) {
-    EPI_REQUIRE(bin_offset >= 0, "negative bin offset");
-    EPI_REQUIRE(nperm >= 0 && perm_offset >= 0 && perm_offset + nperm <= (1ll << 32),
-                "permutations %lld..%lld outside the 32-bit stream key", (long long)perm_offset,
-                (long long)perm_offset + nperm - 1);
-    return 0;
-}
-
 extern "C" int epi_multigroup_stat(const float* scores_dev, int32_t groups, int64_t bins, int32_t num_states,
                                    const int32_t* sizes, double* t_out, uint8_t* group_out, uint8_t* state_out,
                                    int8_t* sign_out, void* stream_) {
@@ -242,7 +225,7 @@ extern "C" int epi_multigroup_stat(const float* scores_dev, int32_t groups, int6
     EPI_REQUIRE(scores_dev && t_out && group_out && state_out && sign_out, "null pointer argument");
     const size_t smem = (size_t)num_states * K10_STAT_THREADS * 8;
     EPI_CUDA(cudaFuncSetAttribute(multigroup_stat_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    multigroup_stat_kernel<<<mg_grid(bins, K10_STAT_THREADS, 8), K10_STAT_THREADS, smem, st>>>(
+    multigroup_stat_kernel<<<grid_for(bins, K10_STAT_THREADS, 8), K10_STAT_THREADS, smem, st>>>(
         scores_dev, groups, bins, num_states, sz, N, t_out, group_out, state_out, sign_out);
     EPI_CUDA(cudaGetLastError());
     return 0;
@@ -269,7 +252,7 @@ extern "C" int epi_multigroup_shuffled_counts_range(const uint16_t* cnt_dev, int
                                   (int)smem));
     int per_sm = 0;
     EPI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, multigroup_shuffled_counts_kernel, K10_THREADS, smem));
-    multigroup_shuffled_counts_kernel<<<mg_grid(bins * nperm, K10_THREADS, per_sm < 1 ? 1 : per_sm), K10_THREADS, smem,
+    multigroup_shuffled_counts_kernel<<<grid_for(bins * nperm, K10_THREADS, per_sm < 1 ? 1 : per_sm), K10_THREADS, smem,
                                         st>>>(cnt_dev, (long long)group_stride, groups, bins, num_states, sz, N,
                                               (unsigned long long)seed, (long long)bin_offset, (long long)perm_offset,
                                               nperm, out_dev);
@@ -288,7 +271,7 @@ extern "C" int epi_multigroup_null_exceedances(const float* null_dev, int32_t gr
     if (int rc = read_sizes(sizes, groups, &sz, &N)) return rc;
     if (bins == 0 || nperm == 0) return 0;
     EPI_REQUIRE(null_dev && t_dev && k_inout, "null pointer argument");
-    multigroup_null_exceedances_kernel<<<mg_grid(bins, K10_THREADS, 8), K10_THREADS, 0, st>>>(
+    multigroup_null_exceedances_kernel<<<grid_for(bins, K10_THREADS, 8), K10_THREADS, 0, st>>>(
         null_dev, groups, nperm, bins, num_states, sz, N, t_dev, k_inout);
     EPI_CUDA(cudaGetLastError());
     return 0;
@@ -310,22 +293,6 @@ extern "C" int epi_multigroup_s1_fused_fits(int32_t groups, int32_t num_states, 
     }
     // checked for one thread per bin, the launch with the most bin slots
     return n <= 65535 && mg_fused_smem(groups, num_states, n, nvt, 1) <= 200 * 1024 ? 1 : 0;
-}
-
-template <int T>
-static int launch_mg_fused(const uint16_t* cnt, int64_t gstride, int G, int64_t bins, int K, const GroupSizes& sz, int N,
-                           uint64_t seed, int64_t bin_offset, int64_t perm_offset, int nperm, const float* vt,
-                           const ValueOffsets& vo, int nvt, const double* tb, uint32_t* k, cudaStream_t st) {
-    auto kern = multigroup_exceedances_s1_kernel<T>;
-    const size_t smem = mg_fused_smem(G, K, N, nvt, T);
-    EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    EPI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, K10_THREADS, smem));
-    kern<<<mg_grid(bins, K10_THREADS / T, per_sm < 1 ? 1 : per_sm), K10_THREADS, smem, st>>>(
-        cnt, (long long)gstride, G, bins, K, sz, N, (unsigned long long)seed, (long long)bin_offset,
-        (long long)perm_offset, nperm, vt, vo, nvt, tb, k);
-    EPI_CUDA(cudaGetLastError());
-    return 0;
 }
 
 extern "C" int epi_multigroup_exceedances_s1(const uint16_t* cnt_dev, int64_t group_stride, int32_t groups,
@@ -363,12 +330,9 @@ extern "C" int epi_multigroup_exceedances_s1(const uint16_t* cnt_dev, int64_t gr
     float* vt = &ws->perm_v32[0][0];
     for (int g = 0; g < groups; ++g)
         if (int rc = s1_value_table(exp1_dev, K, sz.n[g], vt + vo.off[g], ws->s1_v64, st)) return rc;
-    if (nperm >= 32)
-        return launch_mg_fused<32>(cnt_dev, group_stride, groups, bins, K, sz, N, seed, bin_offset, perm_offset, nperm,
-                                   vt, vo, nvt, t_dev, k_inout, st);
-    if (nperm >= 8)
-        return launch_mg_fused<8>(cnt_dev, group_stride, groups, bins, K, sz, N, seed, bin_offset, perm_offset, nperm, vt,
-                                  vo, nvt, t_dev, k_inout, st);
-    return launch_mg_fused<1>(cnt_dev, group_stride, groups, bins, K, sz, N, seed, bin_offset, perm_offset, nperm, vt, vo,
-                              nvt, t_dev, k_inout, st);
+    return launch_fused(multigroup_exceedances_s1_kernel<32>, multigroup_exceedances_s1_kernel<8>,
+                        multigroup_exceedances_s1_kernel<1>, nperm, bins, K10_THREADS,
+                        [&](int T) { return mg_fused_smem(groups, K, N, nvt, T); }, st, cnt_dev, (long long)group_stride,
+                        groups, bins, K, sz, N, (unsigned long long)seed, (long long)bin_offset, (long long)perm_offset,
+                        nperm, vt, vo, nvt, t_dev, k_inout);
 }

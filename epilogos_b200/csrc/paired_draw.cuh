@@ -1,6 +1,8 @@
-// Device pieces shared by the paired-mode kernels: the shuffle sampler of epi_shuffled_counts_philox (pairwise.cu) and
-// numpy's float32 row summation of epi_pairwise_combine.  The fused permutation kernel (permutations.cu) draws and
-// reduces with these same functions, so its null distances are the composed path's bit for bit.
+// Pieces shared by the paired-mode and multi-group kernels: the shuffle samplers of epi_shuffled_counts_philox
+// (pairwise.cu) and epi_multigroup_shuffled_counts_range (multigroup.cu), numpy's float32 row summation of
+// epi_pairwise_combine, the multi-group statistic, and the thread groups and launch of the fused permutation kernels.
+// The fused kernels (permutations.cu, multigroup.cu) draw and reduce with these same functions, so their counts are the
+// composed paths' bit for bit.
 #pragma once
 #include "common.cuh"
 
@@ -71,7 +73,10 @@ __device__ __forceinline__ Philox shuffle_stream(unsigned long long seed, uint32
 // One uniform shuffle of a bin's combined row split into A' (size_a labels) and B' (size_b labels).  For count-based
 // scores it is a multivariate hypergeometric draw: walking over the states,
 //   a'_s ~ HG(remaining labels, c_s, still needed by A'),  b'_s ~ HG(remaining - needed by A', c_s - a'_s, needed by B').
-// emit(s, a'_s, b'_s) is called for s = 0..K-1 in order.
+// emit(s, a'_s, b'_s) is called for s = 0..K-1 in order.  draw_multigroup_shuffle at G = 2 with sizes {size_a, size_b}
+// and the combined row draws the same counts from the same Philox words (tests/test_multigroup_gpu.py checks it), but
+// with it the fused permutation kernel ran 1.0 % slower and the composed path 0.06 % slower on an NVIDIA B200 at 1000 W,
+// beyond the spread of alternated runs (profiles/r08_paired_draw_g2.jsonl), so the paired kernels keep this form.
 template <class Emit>
 __device__ __forceinline__ void draw_shuffle(Philox& rng, const uint16_t* __restrict__ ca, const uint16_t* __restrict__ cb,
                                              int K, int size_a, int size_b, const double* __restrict__ lf,
@@ -94,12 +99,13 @@ __device__ __forceinline__ void draw_shuffle(Philox& rng, const uint16_t* __rest
     }
 }
 
-// One uniform shuffle of a bin's labels over G groups (multigroup.cu).  comb(s) is the bin's count of state s over the
-// union of the groups, size[g] the labels group g receives, and need(g) a per-thread int slot the draw keeps group g's
-// still-needed count in.  For every state s in order and every group g in order,
+// One uniform shuffle of a bin's labels over G groups (multigroup.cu): a multivariate hypergeometric draw.  comb(s) is
+// the bin's count of state s over the row being shuffled, size[g] the labels group g receives, and need(g) a per-thread
+// int slot the draw keeps group g's still-needed count in.  For every state s in order and every group g in order,
 //   x_gs ~ HG(labels still unassigned, labels of state s still unassigned, labels group g still needs);
-// emit(s, g, x_gs) is called in that order and end_state(s) after the last group of a state.  With G = 2 this uses the
-// same Philox words in the same order as draw_shuffle; the last group's draw is always deterministic (it consumes none).
+// emit(s, g, x_gs) is called in that order and end_state(s) after the last group of a state.  When the sizes sum to
+// less than the row (-g), the labels no group takes are left out.  When they cover the row, the last group's draw is
+// deterministic and consumes no Philox word.
 template <class Comb, class Need, class Emit, class EndState>
 __device__ __forceinline__ void draw_multigroup_shuffle(Philox& rng, int K, int G, const int* size, Comb comb, Need need,
                                                         const double* __restrict__ lf, const double* __restrict__ inv,
@@ -151,6 +157,48 @@ __device__ __forceinline__ double multigroup_add_state(double t, int G, const in
 __device__ __forceinline__ void fill_draw_tables(double* lf, double* inv, int width) {
     for (int i = threadIdx.x; i <= width; i += blockDim.x) lf[i] = lgamma((double)i + 1.0);
     for (int i = threadIdx.x; i <= width + 1; i += blockDim.x) inv[i] = i > 0 ? 1.0 / (double)i : 0.0;
+}
+
+// The fused permutation kernels give each bin to a group of T threads (T divides 32: a group never straddles a warp);
+// thread t of the group takes permutations t, t + T, ...  group_mask is the calling thread's group, group_sum the sum of
+// c over it.
+template <int T>
+__device__ __forceinline__ unsigned group_mask() {
+    const int lane = threadIdx.x & 31;
+    return T == 32 ? 0xffffffffu : (((1u << (T % 32)) - 1u) << (lane & ~(T - 1)));
+}
+
+template <int T>
+__device__ __forceinline__ uint32_t group_sum(unsigned gmask, uint32_t c) {
+#pragma unroll
+    for (int off = T / 2; off > 0; off >>= 1) c += __shfl_xor_sync(gmask, c, off);
+    return c;
+}
+
+// Every entry point that draws permutations perm_offset .. perm_offset + nperm - 1 of the bins from bin_offset on: the
+// permutation word of the stream key (shuffle_stream) is 32 bits wide.
+static inline int check_perm_range(int64_t bin_offset, int64_t perm_offset, int32_t nperm) {
+    EPI_REQUIRE(bin_offset >= 0, "negative bin offset");
+    EPI_REQUIRE(nperm >= 0 && perm_offset >= 0 && perm_offset + nperm <= (1ll << 32),
+                "permutations %lld..%lld outside the 32-bit stream key", (long long)perm_offset,
+                (long long)perm_offset + nperm - 1);
+    return 0;
+}
+
+// Launches a fused permutation kernel with T = 32 / 8 / 1 threads per bin (k32, k8, k1) for nperm >= 32 / >= 8 / fewer,
+// in CTAs of `threads` threads with smem(T) bytes of dynamic shared memory, on no more CTAs than stay resident at once.
+template <class... P, class Smem, class... A>
+static int launch_fused(void (*k32)(P...), void (*k8)(P...), void (*k1)(P...), int nperm, long long bins, int threads,
+                        Smem smem, cudaStream_t st, A... args) {
+    const int T = nperm >= 32 ? 32 : (nperm >= 8 ? 8 : 1);
+    auto kern = T == 32 ? k32 : (T == 8 ? k8 : k1);
+    const size_t bytes = smem(T);
+    EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    int per_sm = 0;
+    EPI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, bytes));
+    kern<<<grid_for(bins, threads / T, per_sm < 1 ? 1 : per_sm), threads, bytes, st>>>(args...);
+    EPI_CUDA(cudaGetLastError());
+    return 0;
 }
 
 // numpy float32 pairwise summation of n < 128 contiguous values (what np.sum(axis=1) does per row):

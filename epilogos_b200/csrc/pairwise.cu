@@ -155,14 +155,6 @@ __global__ void __launch_bounds__(256) pairwise_real_reduce_kernel(const float* 
     }
 }
 
-static unsigned grid_for(long long n, int threads, int per_sm) {
-    long long blocks = (n + threads - 1) / threads;
-    const long long cap = (long long)sm_count() * per_sm;
-    if (blocks > cap) blocks = cap;
-    if (blocks < 1) blocks = 1;
-    return (unsigned)blocks;
-}
-
 }  // namespace epi
 
 using namespace epi;
@@ -192,10 +184,7 @@ extern "C" int epi_shuffled_counts_philox_range(const uint16_t* cnt_a_dev, const
     if (check_device()) return 3;
     EPI_REQUIRE(bins >= 0 && K >= 1 && K <= EPI_MAX_STATES && nperm >= 1, "bad paired shape");
     EPI_REQUIRE(size_a >= 0 && size_b >= 0, "negative group size");
-    EPI_REQUIRE(bin_offset >= 0, "negative bin offset");
-    EPI_REQUIRE(perm_offset >= 0 && perm_offset + nperm <= (1ll << 32),
-                "permutations %lld..%lld outside the 32-bit stream key", (long long)perm_offset,
-                (long long)perm_offset + nperm - 1);
+    if (int rc = check_perm_range(bin_offset, perm_offset, nperm)) return rc;
     if (bins == 0) return 0;
     EPI_REQUIRE(cnt_a_dev && cnt_b_dev && cnt_a_out && cnt_b_out, "null pointer argument");
     EPI_REQUIRE(width >= 1 && width <= 65535, "width=%d (combined biosamples) out of range [1, 65535]", width);

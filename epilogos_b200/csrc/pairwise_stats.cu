@@ -19,14 +19,6 @@
 
 namespace epi {
 
-static unsigned grid_for_n(long long n, int threads, int per_sm) {
-    long long blocks = (n + threads - 1) / threads;
-    const long long cap = (long long)sm_count() * per_sm;
-    if (blocks > cap) blocks = cap;
-    if (blocks < 1) blocks = 1;
-    return (unsigned)blocks;
-}
-
 static size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 // ---------------------------------------------------------------- block scans (blockDim.x a multiple of 32, <= 1024)
@@ -669,7 +661,7 @@ extern "C" int epi_gennorm_pvalues(const float* x_dev, int64_t n, double beta, d
                 "gennorm parameters out of range (beta=%g loc=%g scale=%g)", beta, loc, scale);
     if (n == 0) return 0;
     EPI_REQUIRE(x_dev && p_out, "null pointer argument");
-    gennorm_pvalues_kernel<<<grid_for_n(n, 256, 16), 256, 0, st>>>(x_dev, n, beta, loc, scale, p_out);
+    gennorm_pvalues_kernel<<<grid_for(n, 256, 16), 256, 0, st>>>(x_dev, n, beta, loc, scale, p_out);
     EPI_CUDA(cudaGetLastError());
     return 0;
 }

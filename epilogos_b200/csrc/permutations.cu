@@ -41,7 +41,7 @@ __global__ void __launch_bounds__(K9_THREADS) null_exceedances_kernel(const floa
     }
 }
 
-// T threads own one bin (T divides 32: a group never straddles a warp); thread t takes permutations t, t + T, ...
+// T threads own one bin (group_mask); thread t takes permutations t, t + T, ...
 // Shared memory: the sampler's tables (2 width + 3 doubles), then, when tables_in_smem, the value tables of A' and B'.
 template <int T>
 __global__ void __launch_bounds__(K9_THREADS) permutation_exceedances_s1_kernel(
@@ -61,8 +61,8 @@ __global__ void __launch_bounds__(K9_THREADS) permutation_exceedances_s1_kernel(
     __syncthreads();
     const float* va = tables_in_smem ? vs : va_g;
     const float* vb = tables_in_smem ? vs + na : vb_g;
-    const int lane = threadIdx.x & 31, t = threadIdx.x % T;
-    const unsigned gmask = T == 32 ? 0xffffffffu : (((1u << (T % 32)) - 1u) << (lane & ~(T - 1)));
+    const int t = threadIdx.x % T;
+    const unsigned gmask = group_mask<T>();
     constexpr int GROUPS = K9_THREADS / T;
     for (long long b = blockIdx.x * (long long)GROUPS + threadIdx.x / T; b < bins; b += (long long)gridDim.x * GROUPS) {
         const float thr = fabsf(dist[b]);
@@ -79,39 +79,9 @@ __global__ void __launch_bounds__(K9_THREADS) permutation_exceedances_s1_kernel(
             const float v = signed_sq_distance(K, [&](int i) { return d[i]; });
             c += fabsf(v) >= thr ? 1u : 0u;
         }
-#pragma unroll
-        for (int off = T / 2; off > 0; off >>= 1) c += __shfl_xor_sync(gmask, c, off);
+        c = group_sum<T>(gmask, c);
         if (t == 0) k[b] += c;
     }
-}
-
-static unsigned grid_for(long long n, int per_block, int per_sm) {
-    long long blocks = (n + per_block - 1) / per_block;
-    const long long cap = (long long)sm_count() * per_sm;
-    if (blocks > cap) blocks = cap;
-    if (blocks < 1) blocks = 1;
-    return (unsigned)blocks;
-}
-
-template <int T>
-static int launch_fused(const uint16_t* ca, const uint16_t* cb, int64_t bins, int K, int size_a, int size_b, int width,
-                        uint64_t seed, int64_t bin_offset, int64_t perm_offset, int nperm, const float* va, int wa,
-                        const float* vb, int wb, const float* dist, uint32_t* k, cudaStream_t st) {
-    auto kern = permutation_exceedances_s1_kernel<T>;
-    const size_t draw = (size_t)(2 * width + 3) * 8;
-    const size_t tables = (size_t)K * (wa + 1 + wb + 1) * 4;
-    // value tables in shared memory while two CTAs still fit on an SM; else they are read through L1
-    const bool in_smem = draw + tables <= (size_t)110 * 1024;
-    const size_t smem = draw + (in_smem ? tables : 0);
-    EPI_REQUIRE(smem <= 200 * 1024, "too many combined biosamples (%d) for the shuffle kernel", width);
-    EPI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    EPI_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, K9_THREADS, smem));
-    kern<<<grid_for(bins, K9_THREADS / T, per_sm < 1 ? 1 : per_sm), K9_THREADS, smem, st>>>(
-        ca, cb, bins, K, size_a, size_b, width, (unsigned long long)seed, (long long)bin_offset, (long long)perm_offset,
-        nperm, va, wa, vb, wb, in_smem ? 1 : 0, dist, k);
-    EPI_CUDA(cudaGetLastError());
-    return 0;
 }
 
 }  // namespace epi
@@ -140,10 +110,7 @@ extern "C" int epi_permutation_exceedances_s1(const uint16_t* cnt_a_dev, const u
     if (check_device()) return 3;
     EPI_REQUIRE(bins >= 0 && K >= 1 && K <= EPI_MAX_STATES && nperm >= 0, "bad paired shape");
     EPI_REQUIRE(size_a >= 0 && size_b >= 0, "negative group size");
-    EPI_REQUIRE(bin_offset >= 0, "negative bin offset");
-    EPI_REQUIRE(perm_offset >= 0 && perm_offset + nperm <= (1ll << 32),
-                "permutations %lld..%lld outside the 32-bit stream key", (long long)perm_offset,
-                (long long)perm_offset + nperm - 1);
+    if (int rc = check_perm_range(bin_offset, perm_offset, nperm)) return rc;
     EPI_REQUIRE(width >= 1 && width <= 65535, "width=%d (combined biosamples) out of range [1, 65535]", width);
     if (size_a + size_b > width) {
         set_error("group sizes %d + %d exceed the %d combined biosamples", size_a, size_b, width);
@@ -162,12 +129,15 @@ extern "C" int epi_permutation_exceedances_s1(const uint16_t* cnt_a_dev, const u
     if (int rc = s1_value_table(exp1_dev, K, width_a, ws->perm_v32[0], ws->s1_v64, st)) return rc;
     if (int rc = s1_value_table(exp1_dev, K, width_b, ws->perm_v32[1], ws->s1_v64, st)) return rc;
     const float *va = ws->perm_v32[0], *vb = ws->perm_v32[1];
-    if (nperm >= 32)
-        return launch_fused<32>(cnt_a_dev, cnt_b_dev, bins, K, size_a, size_b, width, seed, bin_offset, perm_offset, nperm,
-                                va, width_a, vb, width_b, dist_dev, k_inout, st);
-    if (nperm >= 8)
-        return launch_fused<8>(cnt_a_dev, cnt_b_dev, bins, K, size_a, size_b, width, seed, bin_offset, perm_offset, nperm,
-                               va, width_a, vb, width_b, dist_dev, k_inout, st);
-    return launch_fused<1>(cnt_a_dev, cnt_b_dev, bins, K, size_a, size_b, width, seed, bin_offset, perm_offset, nperm, va,
-                           width_a, vb, width_b, dist_dev, k_inout, st);
+    const size_t draw = (size_t)(2 * width + 3) * 8;
+    const size_t tables = (size_t)K * (width_a + 1 + width_b + 1) * 4;
+    // value tables in shared memory while two CTAs still fit on an SM; else they are read through L1
+    const bool in_smem = draw + tables <= (size_t)110 * 1024;
+    const size_t smem = draw + (in_smem ? tables : 0);
+    EPI_REQUIRE(smem <= 200 * 1024, "too many combined biosamples (%d) for the shuffle kernel", width);
+    return launch_fused(permutation_exceedances_s1_kernel<32>, permutation_exceedances_s1_kernel<8>,
+                        permutation_exceedances_s1_kernel<1>, nperm, bins, K9_THREADS, [&](int) { return smem; }, st,
+                        cnt_a_dev, cnt_b_dev, bins, K, size_a, size_b, width, (unsigned long long)seed,
+                        (long long)bin_offset, (long long)perm_offset, nperm, va, width_a, vb, width_b, in_smem ? 1 : 0,
+                        dist_dev, k_inout);
 }

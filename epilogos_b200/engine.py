@@ -23,6 +23,11 @@ def _ptr(t):
     return ctypes.c_void_p(t.data_ptr()) if t is not None else ctypes.c_void_p(0)
 
 
+def _seed(seed):
+    """A Python integer seed as the library's uint64 (taken modulo 2^64)."""
+    return ctypes.c_uint64(int(seed) & (2 ** 64 - 1))
+
+
 def _require_cuda(t, dtype, name):
     if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dtype and t.is_contiguous()):
         raise TypeError("%s must be a contiguous CUDA tensor of dtype %s" % (name, dtype))
@@ -273,7 +278,7 @@ def paired_host(xa_host, cols_a, xb_host, cols_b, num_states, saliency, quiescen
     quies = np.empty(bins, dtype=np.uint8)
     _lib.call("epi_paired_host", ctypes.c_void_p(xa_host.data_ptr()), xa_host.shape[1], int(cols_a),
               ctypes.c_void_p(xb_host.data_ptr()), xb_host.shape[1], int(cols_b), bins, int(num_states), int(saliency),
-              int(quiescent_state), int(group_size), ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(nperm),
+              int(quiescent_state), int(group_size), _seed(seed), int(bin_offset), int(nperm),
               ctypes.c_void_p(counts.ctypes.data), ctypes.c_void_p(exp.ctypes.data), ctypes.c_void_p(delta_out.data_ptr()),
               ctypes.c_void_p(null_out.data_ptr() if nperm > 0 else 0), ctypes.c_void_p(quies.ctypes.data))
     return dict(counts=counts, exp=exp, delta=delta_out.numpy(), null=null_out.numpy()[:nperm], quiescent=quies.astype(bool))
@@ -390,15 +395,8 @@ def shuffled_counts_philox(cnt_a, cnt_b, size_a, size_b, seed, nperm=1, width=No
     """nperm uniform shuffles per bin drawn on the device; returns int16 tensors [nperm, bins, K].
     `width` = combined number of biosamples (default: size_a + size_b, right unless -g shrinks the groups);
     `bin_offset` = global index of row 0 (the random stream of a bin is keyed by its global index)."""
-    _require_cuda(cnt_a, torch.int16, "cnt_a")
-    _require_cuda(cnt_b, torch.int16, "cnt_b")
-    bins, k = cnt_a.shape
-    oa = torch.empty((nperm, bins, k), dtype=torch.int16, device=cnt_a.device)
-    ob = torch.empty((nperm, bins, k), dtype=torch.int16, device=cnt_a.device)
-    _lib.call("epi_shuffled_counts_philox", _ptr(cnt_a), _ptr(cnt_b), bins, k,
-              int(width if width is not None else size_a + size_b), int(size_a), int(size_b),
-              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(nperm), _ptr(oa), _ptr(ob), _stream())
-    return oa, ob
+    return shuffled_counts_philox_range(cnt_a, cnt_b, size_a, size_b, seed, 0, nperm,
+                                        width if width is not None else size_a + size_b, bin_offset)
 
 
 def shuffled_counts_philox_range(cnt_a, cnt_b, size_a, size_b, seed, perm_offset, nperm, width, bin_offset=0):
@@ -409,8 +407,7 @@ def shuffled_counts_philox_range(cnt_a, cnt_b, size_a, size_b, seed, perm_offset
     oa = torch.empty((nperm, bins, k), dtype=torch.int16, device=cnt_a.device)
     ob = torch.empty((nperm, bins, k), dtype=torch.int16, device=cnt_a.device)
     _lib.call("epi_shuffled_counts_philox_range", _ptr(cnt_a), _ptr(cnt_b), bins, k, int(width), int(size_a), int(size_b),
-              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(perm_offset), int(nperm), _ptr(oa), _ptr(ob),
-              _stream())
+              _seed(seed), int(bin_offset), int(perm_offset), int(nperm), _ptr(oa), _ptr(ob), _stream())
     return oa, ob
 
 
@@ -441,8 +438,8 @@ def permutation_exceedances_s1(cnt_a, cnt_b, size_a, size_b, seed, perm_offset, 
     if dist.numel() != bins or k.numel() != bins or exp1.numel() != K:
         raise ValueError("dist and k must have one entry per bin, exp1 one per state")
     _lib.call("epi_permutation_exceedances_s1", _ptr(cnt_a), _ptr(cnt_b), bins, K, int(width), int(size_a), int(size_b),
-              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(perm_offset), int(nperm), _ptr(exp1),
-              int(width_a), int(width_b), _ptr(dist), _ptr(k), _stream())
+              _seed(seed), int(bin_offset), int(perm_offset), int(nperm), _ptr(exp1), int(width_a), int(width_b),
+              _ptr(dist), _ptr(k), _stream())
     return k
 
 
@@ -486,9 +483,8 @@ def multigroup_shuffled_counts_range(cnt, sizes, seed, perm_offset, nperm, bin_o
         raise ValueError("one size per group")
     out = torch.empty((nperm, G, bins, K), dtype=torch.int16, device=cnt.device)
     _arr, sz = _group_sizes(sizes)
-    _lib.call("epi_multigroup_shuffled_counts_range", _ptr(cnt), stride, G, bins, K, sz,
-              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(perm_offset), int(nperm), _ptr(out),
-              _stream())
+    _lib.call("epi_multigroup_shuffled_counts_range", _ptr(cnt), stride, G, bins, K, sz, _seed(seed), int(bin_offset),
+              int(perm_offset), int(nperm), _ptr(out), _stream())
     return out
 
 
@@ -522,9 +518,8 @@ def multigroup_exceedances_s1(cnt, sizes, seed, perm_offset, nperm, bin_offset, 
     if len(sizes) != G or t.numel() != bins or k.numel() != bins or exp1.numel() != K:
         raise ValueError("one size per group, t and k with one entry per bin, exp1 one per state")
     _arr, sz = _group_sizes(sizes)
-    _lib.call("epi_multigroup_exceedances_s1", _ptr(cnt), stride, G, bins, K, sz,
-              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), int(bin_offset), int(perm_offset), int(nperm), _ptr(exp1),
-              _ptr(t), _ptr(k), _stream())
+    _lib.call("epi_multigroup_exceedances_s1", _ptr(cnt), stride, G, bins, K, sz, _seed(seed), int(bin_offset),
+              int(perm_offset), int(nperm), _ptr(exp1), _ptr(t), _ptr(k), _stream())
     return k
 
 
@@ -584,8 +579,8 @@ def null_subsample(pool, trials, size, seed):
     _require_cuda(pool, torch.float32, "pool")
     idx = torch.empty((trials, size), dtype=torch.int32, device=pool.device)
     samples = torch.empty((trials, size), dtype=torch.float32, device=pool.device)
-    _lib.call("epi_null_subsample", _ptr(pool), pool.numel(), int(trials), int(size),
-              ctypes.c_uint64(int(seed) & (2 ** 64 - 1)), _ptr(idx), _ptr(samples), _stream())
+    _lib.call("epi_null_subsample", _ptr(pool), pool.numel(), int(trials), int(size), _seed(seed), _ptr(idx),
+              _ptr(samples), _stream())
     return idx, samples
 
 

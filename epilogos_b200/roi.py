@@ -46,6 +46,21 @@ def max_mean(starts, ends, score, window, max_regions=100):
     return dict(original_idx=out_i[:k], start=out_s[:k], end=out_e[:k], rolling_max=out_mx[:k], rolling_mean=out_mn[:k])
 
 
+def permutation_pvalues(be, chunks, mismatch):
+    """(k uint32, p, BH) over the bins of all chunks, or None when the score stage counted no permutations: k of the P
+    shuffles of a bin whose statistic is at least the bin's, p = (1 + k) / (P + 1), and the Benjamini-Hochberg adjustment
+    over all bins.  Chunks that disagree on P raise ValueError("<mismatch> on the number of permutations (...)")."""
+    perms = {c.get("permutations") for c in chunks}
+    if perms == {None}:
+        return None
+    if None in perms or len(perms) != 1:
+        raise ValueError("{} on the number of permutations ({})".format(mismatch, sorted(str(p) for p in perms)))
+    P = perms.pop()
+    k = np.concatenate([np.asarray(c["exceedances"], dtype=np.uint32) for c in chunks])
+    p = (k.astype(np.float64) + 1.0) / (P + 1.0)
+    return k, p, be.bh_adjust(be.to_device(p)).cpu().numpy()
+
+
 def readInData(outputDirPath):
     """All temp_scores_*.npz in chromosome order -> (chrom per row, starts, ends, scoreArr); temp files removed."""
     from . import session

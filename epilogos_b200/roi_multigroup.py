@@ -21,7 +21,7 @@ from sys import argv
 import numpy as np
 
 from . import session, writer
-from .roi import max_mean, orderChromosomes
+from .roi import max_mean, orderChromosomes, permutation_pvalues
 from .run import getStateNames
 
 
@@ -46,20 +46,6 @@ def readInData(outputDirPath, fileTag):
     if not chunks:
         raise FileNotFoundError("no multi-group score-stage outputs ({}*.npz) in {}".format(prefix, outputDirPath))
     return [chunks[c] for c in orderChromosomes(list(chunks))]
-
-
-def permutation_pvalues(be, chunks):
-    """(k, p, BH) over all bins, or (None, None, None) when no permutations were counted."""
-    perms = {c.get("permutations") for c in chunks}
-    if perms == {None}:
-        return None, None, None
-    if None in perms or len(perms) != 1:
-        raise ValueError("temp_multigroup files disagree on the number of permutations ({})".format(
-            sorted(str(p) for p in perms)))
-    P = perms.pop()
-    k = np.concatenate([np.asarray(c["exceedances"], dtype=np.uint32) for c in chunks])
-    p = (k.astype(np.float64) + 1.0) / (P + 1.0)
-    return k, p, be.bh_adjust(be.to_device(p)).cpu().numpy()
 
 
 def roi_lines(chrom, starts, ends, t, group, state, sign, group_names, state_names, roiWidth, pvals=None, bh=None):
@@ -88,7 +74,7 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, verbose=False, ba
     cat = lambda key, dtype: np.concatenate([np.asarray(c[key], dtype=dtype) for c in chunks])   # noqa: E731
     loc = dict(chrom=cat("chrom", object), start=cat("start", np.int64), end=cat("end", np.int64))
     t, group, state, sign = cat("t", np.float64), cat("group", np.uint8), cat("state", np.uint8), cat("sign", np.int8)
-    k, p, bh = permutation_pvalues(be, chunks)
+    k, p, bh = permutation_pvalues(be, chunks, "temp_multigroup files disagree") or (None, None, None)
     writer.write_multigroup_text(outputDirPath / "multigroupMetrics_{}.txt.gz".format(fileTag), loc, t, group, state,
                                  sign, group_names, names, k, p, bh)
     (outputDirPath / "regionsOfInterest_{}.txt".format(fileTag)).write_text(

@@ -34,7 +34,7 @@ import numpy as np
 
 from . import helpers, session, writer
 from .helpers import strToBool
-from .roi import max_mean, orderChromosomes
+from .roi import max_mean, orderChromosomes, permutation_pvalues
 from .run import getStateNames
 
 STATS_SEED_SALT = "epilogos_b200 paired statistics: null subsamples"
@@ -104,22 +104,6 @@ def fit_null(be, chunks, numTrials, samplingSize, seed):
     return float(params[chosen, 0]), float(params[chosen, 1]), float(params[chosen, 2]), table
 
 
-def permutation_pvalues(be, chunks):
-    """(k uint32, p, BH) over the bins of all chunks, or None when the score stage counted no permutations: p = (1 + k) /
-    (P + 1), k = #{p < P : |null(b, p)| >= |distance(b)|}, and the Benjamini-Hochberg adjustment over the genome."""
-    perms = {c.get("permutations") for c in chunks}
-    if perms == {None}:
-        return None
-    if None in perms or len(perms) != 1:
-        raise ValueError("temp_permutations files are missing for some chromosomes or disagree on the number of "
-                         "permutations ({})".format(sorted(str(p) for p in perms)))
-    P = perms.pop()
-    k = np.concatenate([np.asarray(c["exceedances"], dtype=np.uint32) for c in chunks])
-    p = (k.astype(np.float64) + 1.0) / (P + 1.0)
-    bh = be.bh_adjust(be.to_device(p)).cpu().numpy()
-    return k, p, bh
-
-
 def roi_lines(chrom, starts, ends, distance, max_diff, names, roiWidth, pvals=None, bh=None):
     """regionsOfInterest text: max-mean windows of |distance|, state and sign of the window's largest |distance| bin."""
     absd = np.abs(distance.astype(np.float32))
@@ -173,7 +157,8 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, pval, numTrials=1
                               distance, pvals, bh)
     (outputDirPath / "regionsOfInterest_{}.txt".format(fileTag)).write_text(
         roi_lines(loc["chrom"], loc["start"], loc["end"], distance, max_diff, names, roiWidth, pvals, bh))
-    perm = permutation_pvalues(be, chunks)
+    # k = #{p < P : |null(b, p)| >= |distance(b)|}
+    perm = permutation_pvalues(be, chunks, "temp_permutations files are missing for some chromosomes or disagree")
     if perm is not None:
         writer.write_permutations_text(outputDirPath / "pairwisePermutation_{}.txt.gz".format(fileTag), loc, *perm)
     if not verbose:
