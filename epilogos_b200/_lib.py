@@ -57,6 +57,9 @@ PROTOTYPES = {
     "epi_multigroup_exceedances_s1": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_void_p, c_uint64, c_int64,
                                               c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
     "epi_multigroup_s1_fused_fits": (c_int, [c_int32, c_int32, c_void_p]),
+    "epi_split_counts": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_void_p, c_int32, c_int32, c_void_p,
+                                 c_void_p]),
+    "epi_window_max": (c_int, [c_void_p, c_int32, c_int64, c_int64, c_int64, c_int32, c_void_p, c_void_p]),
     "epi_write_permutations_gz": (c_int, [c_char_p, c_char_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                           c_int64, c_int32, c_int32]),
     "epi_write_multigroup_gz": (c_int, [c_char_p, c_char_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,

@@ -214,6 +214,73 @@ class CudaBackend:
                 engine.multigroup_null_exceedances(sc, sizes, t[lo:hi], k[lo:hi])
         return k
 
+    # -- region null: whole-genome label permutations (epilogos_b200.region_null) ------------------------------------
+    def region_maxima_paired(self, x_dev, halo, sizes, num_states, window, nperm, seed, saliency, exp, exact=False,
+                             workspace_bytes=1 << 30):
+        """int64 [nperm] on the device: for split p of region_null.split_blocks, the largest sum of W = `window`
+        consecutive q(|distance|) of the rows of x_dev (the [A | B] label matrix, A of sizes[0] columns) followed by the
+        host rows `halo`.  Each permuted group is scored like its real counterpart (its width, S2 normaliser and score
+        mode) and reduced with the text round trip, so the identity split gives the real distances.  -1 where no window
+        fits."""
+        def stat(cnt, n0, out):
+            sa = self._group_scores(cnt[0], sizes[0], saliency, exp, exact)
+            sb = self._group_scores(cnt[1], sizes[1], saliency, exp, exact)
+            delta, _ = engine.pairwise_combine(sa, sb)
+            d, _ = engine.pairwise_real_reduce(delta, True)
+            torch.abs(d, out=out)
+        return self._region_maxima(x_dev, halo, sizes, num_states, window, nperm, seed, exp, torch.float32,
+                                   12 * num_states + 16, stat, workspace_bytes)
+
+    def region_maxima_multigroup(self, x_dev, halo, sizes, num_states, window, nperm, seed, saliency, exp, exact=False,
+                                 workspace_bytes=1 << 30):
+        """As region_maxima_paired for the multi-group statistic T of the groups, which are the consecutive column slices
+        of sizes[0], sizes[1], ... of x_dev."""
+        G = len(sizes)
+
+        def stat(cnt, n0, out):
+            sc = torch.empty((G, n0, num_states), dtype=torch.float32, device=self.device)
+            for g, n in enumerate(sizes):
+                self._group_scores(cnt[g], n, saliency, exp, exact, out=sc[g])
+            out.copy_(engine.multigroup_stat(sc, sizes)[0])
+        return self._region_maxima(x_dev, halo, sizes, num_states, window, nperm, seed, exp, torch.float64,
+                                   6 * G * num_states + 16, stat, workspace_bytes)
+
+    def _region_maxima(self, x_dev, halo, sizes, num_states, window, nperm, seed, exp, dtype, cell_bytes, stat,
+                       workspace_bytes):
+        """Split blocks (drawn in order, outer) x bin chunks (inner, overlapping by W - 1 rows): split counts, the
+        statistic of every split into one [splits, rows] array, its windowed maxima.  Buffers stay near
+        `workspace_bytes`; the result does not depend on it."""
+        from . import region_null
+        exp = exp.to(self.device).contiguous()
+        N, G = int(sum(sizes)), len(sizes)
+        x = x_dev
+        if halo is not None and len(halo):
+            h = np.zeros((len(halo), x_dev.shape[1]), dtype=np.int8)
+            h[:, :N] = halo
+            x = torch.cat([x_dev, torch.from_numpy(h).to(self.device)])
+        rows = x.shape[0]
+        maxima = torch.full((nperm,), -1, dtype=torch.int64, device=self.device)
+        starts = rows - window + 1
+        if starts <= 0:
+            return maxima
+        cells = max(1, int(workspace_bytes) // cell_bytes)
+        # long chunks, and as many splits per block as fit: the bitsets of a tile are built once per launch
+        chunk = min(starts, max(1 << 16, cells // nperm))
+        block = max(1, min(nperm, cells // (chunk + window - 1)))
+        with timing.stage("kernels", sync_cuda=True):
+            for p0, members in region_null.split_blocks(seed, sizes, nperm, block):
+                n = members.shape[0]
+                mem = torch.from_numpy(members.view(np.int64)).to(self.device)
+                for lo in range(0, starts, chunk):
+                    hi = min(rows, lo + chunk + window - 1)
+                    cnt = engine.split_counts(x[lo:hi], N, num_states, mem, G)
+                    vals = torch.empty((n, hi - lo), dtype=dtype, device=self.device)
+                    for p in range(n):
+                        stat(cnt[p], hi - lo, vals[p])
+                    del cnt
+                    engine.window_max(vals, window, maxima[p0:p0 + n])
+        return maxima
+
     def pairwise_combine(self, score_a, score_b, null_a, null_b):
         return engine.pairwise_combine(score_a, score_b, null_a, null_b)
 

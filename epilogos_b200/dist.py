@@ -54,6 +54,28 @@ def all_reduce_sum(t):
     return t
 
 
+def all_reduce_max(t):
+    """In-place maximum over ranks of an integer tensor (order independent => bit-exact for any world size)."""
+    if initialised() and dist.get_world_size() > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    return t
+
+
+def halo_rows(head, need):
+    """The first `need` rows that follow this rank's rows (ranks own consecutive row ranges): every rank passes its first
+    `need` host rows (numpy [<= need, ...]; fewer when it holds fewer) and gets the concatenation of those of the ranks
+    after it, cut to `need` rows.  Collective (an all-gather of at most world x need rows); None on a single rank."""
+    import numpy as np
+    if not initialised() or dist.get_world_size() == 1:
+        return None
+    parts = [None] * dist.get_world_size()
+    dist.all_gather_object(parts, np.ascontiguousarray(head[:need]))
+    after = parts[dist.get_rank() + 1:]
+    if not after:
+        return None
+    return np.concatenate(after, axis=0)[:need]
+
+
 def gather_rows(t, total_rows, dst=0):
     """Concatenate per-rank row blocks (ranks own consecutive row ranges) on rank `dst`; other ranks get None."""
     if not initialised() or dist.get_world_size() == 1:

@@ -523,6 +523,39 @@ def multigroup_exceedances_s1(cnt, sizes, seed, perm_offset, nperm, bin_offset, 
     return k
 
 
+def split_counts(x, cols, num_states, members, groups):
+    """Counts of the groups of column splits of x (CUDA int8 [bins, pitch]).  members: CUDA int64 [nsplit, groups - 1,
+    ceil(cols / 64)] column bitsets (uint64 bit patterns), the last group of a split being the complement.  Returns an int16
+    view [nsplit, groups, bins, K] holding uint16 counts whose [bins, K] blocks are contiguous and start on 16 bytes."""
+    _require_cuda(x, torch.int8, "x")
+    _require_cuda(members, torch.int64, "members")
+    bins, pitch = x.shape
+    words = (int(cols) + 63) // 64
+    if members.dim() != 3 or members.shape[1] != groups - 1 or members.shape[2] != words:
+        raise ValueError("members must be [nsplit, groups - 1, %d] column bitsets" % words)
+    nsplit = members.shape[0]
+    stride = (bins * num_states + 7) & ~7
+    buf = torch.empty(max(nsplit * groups * stride, 1), dtype=torch.int16, device=x.device)
+    _lib.call("epi_split_counts", _ptr(x), bins, int(cols), pitch, int(num_states), _ptr(members), nsplit, int(groups),
+              _ptr(buf), _stream())
+    return buf.as_strided((nsplit, groups, bins, num_states), (groups * stride, stride, num_states, 1))
+
+
+def window_max(stat, window, max_inout):
+    """max_inout[p] = max(max_inout[p], largest sum of `window` consecutive q(stat[p, i]) = rint(stat[p, i] * 2^24)).
+    stat: CUDA float32 or float64 [nrows, n] whose rows are contiguous; max_inout: CUDA int64 [nrows], updated in place."""
+    if not (isinstance(stat, torch.Tensor) and stat.is_cuda and stat.dtype in (torch.float32, torch.float64)
+            and stat.dim() == 2 and (stat.shape[1] <= 1 or stat.stride(1) == 1)):
+        raise TypeError("stat must be a CUDA float32 or float64 [nrows, n] tensor with contiguous rows")
+    _require_cuda(max_inout, torch.int64, "max_inout")
+    nrows, n = stat.shape
+    if max_inout.numel() != nrows:
+        raise ValueError("max_inout must have one entry per row")
+    _lib.call("epi_window_max", _ptr(stat), 0 if stat.dtype == torch.float32 else 1, nrows, stat.stride(0), n,
+              int(window), _ptr(max_inout), _stream())
+    return max_inout
+
+
 def pairwise_combine(score_a=None, score_b=None, null_a=None, null_b=None):
     """(delta float32 [rows, K] or None, null_dist float32 [rows] or None)."""
     ref = score_a if score_a is not None else null_a

@@ -166,6 +166,10 @@ class GroupColumns:
     def device_matrix(self):
         return group_matrix(self._shard, self._columns)
 
+    def head(self, n):
+        """The first n rows, on the host."""
+        return self._shard.states_a[:n][:, self._columns]
+
     def __array__(self, dtype=None, copy=None):
         m = self._shard.states_a[:, self._columns]
         return m if dtype is None else m.astype(dtype)
@@ -242,6 +246,12 @@ class GroupView:
         if self._all is None:
             self._all = self._shard.backend.add_counts(cnt[self._ia], cnt[self._ib])
         return self._all
+
+    def grouped(self):
+        """The columns of a multi-group comparison group after group, in the order the groups were named: the matrix
+        whose consecutive column slices of `sizes` are the groups (the region null's identity split)."""
+        gs = self.selection.groupset
+        return GroupColumns(self._shard, np.concatenate([gs.columns[i] for i in self._idx]))
 
     def combined(self):
         if self.selection.multi is not None:

@@ -22,9 +22,14 @@ from .scores import _gather_locations
 
 
 def calculateScoresMultigroup(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
-                              backend=None, group=None, permutations=0, seed=None):
+                              backend=None, group=None, permutations=0, seed=None, region_permutations=0,
+                              region_seed=None, roi_width=None):
+    """`region_permutations` P > 0: also the file's maxima of the region null over `region_seed`'s P label splits of the
+    groups' columns (epilogos_b200.region_null), handed to step 4 or written to temp_regionNull_<tag>_<file>.npz."""
     if saliency not in (1, 2):
         raise ValueError("Please ensure that saliency metric is either 1 or 2 for Pairwise Epilogos")
+    if region_permutations > 0 and region_seed is None:
+        raise ValueError("region permutations need the run's region seed (region_null.region_seed), drawn once per run")
     be = session.get_backend(backend)
     view = session.load_shard(file1Path, file1Path, numStates, backend, group=group)
     exp = be.to_device(np.load(expFreqPath, allow_pickle=False))
@@ -34,6 +39,12 @@ def calculateScoresMultigroup(saliency, file1Path, numStates, outputDirPath, exp
     if permutations > 0:
         exceed = be.multigroup_exceedances(cnt, sizes, t, permutations, file_seed(run_seed(seed), filename), view.lo,
                                            saliency, exp)
+    region = None
+    if region_permutations > 0:
+        from . import region_null
+        cols = view.grouped()
+        region = region_null.shard_maxima(be, "multigroup", cols.device_matrix(), cols.head, sizes, numStates, roi_width,
+                                          region_permutations, region_seed, saliency, exp)
     total = view.total_rows
     t, g, s, sign = (dist.gather_rows(a, total) for a in (t, g, s, sign))
     if exceed is not None:
@@ -41,6 +52,8 @@ def calculateScoresMultigroup(saliency, file1Path, numStates, outputDirPath, exp
     loc = _gather_locations(view)
     if dist.rank() != 0:
         return
+    if region is not None:
+        region_null.check_one_chromosome(loc["chrom"], file1Path)
     chrName = loc["chrom"][0] if len(loc["chrom"]) else ""
     out = dict(chrName=str(chrName), groups=list(group.multi), t=t.cpu().numpy(), group=g.cpu().numpy(),
                state=s.cpu().numpy(), sign=sign.cpu().numpy(), chrom=np.asarray(loc["chrom"], dtype=object),
@@ -50,7 +63,13 @@ def calculateScoresMultigroup(saliency, file1Path, numStates, outputDirPath, exp
     path = Path(outputDirPath) / "temp_multigroup_{}_{}.npz".format(fileTag, filename)
     if session.handover_enabled and not os.environ.get("EPILOGOS_B200_KEEP_TEMP"):
         session.handover[str(path)] = out          # step 4 runs next, in this process
+        if region is not None:
+            region_null.stage_output(outputDirPath, fileTag, filename, chrName, region.cpu().numpy(), roi_width,
+                                     region_permutations, out)
         return
+    if region is not None:
+        region_null.stage_output(Path(outputDirPath), fileTag, filename, chrName, region.cpu().numpy(), roi_width,
+                                 region_permutations, None)
     extra = {} if exceed is None else dict(exceedances=out["exceedances"],
                                            permutations=np.array(int(permutations), dtype=np.int64))
     helpers.savez_level(path, chrName=np.array([chrName]), groups=np.array(out["groups"]), t=out["t"],

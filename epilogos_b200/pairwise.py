@@ -65,13 +65,18 @@ def shuffled_widths(c1, c2, groupSize):
 
 def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDirPath, expFreqPath, fileTag, filename,
                             quiescentState, groupSize, verbose, backend=None, null_mode=None, seed=None, nperm=1,
-                            group=None, permutations=0):
+                            group=None, permutations=0, region_permutations=0, region_seed=None, roi_width=None):
     """`permutations` P > 0: also count, for every bin, how many of P device-drawn null shuffles (permutations 0..P-1 of
     the device sampler, scored like the run's null) are at least as far from 0 as the bin's real distance, and hand the
     counts to step 4 (session.handover) or write them to temp_permutations_<tag>_<file>.npz {chrName, exceedances
-    uint32[B], permutations}.  Nothing else changes: in device mode permutation 0 is the run's own null."""
+    uint32[B], permutations}.  Nothing else changes: in device mode permutation 0 is the run's own null.
+    `region_permutations` P > 0: also the file's maxima of the region null over `region_seed`'s P label splits of the
+    combined [A | B] matrix, windows of `roi_width` rows (epilogos_b200.region_null), handed to step 4 or written to
+    temp_regionNull_<tag>_<file>.npz."""
     if saliency not in (1, 2):
         raise ValueError("Please ensure that saliency metric is either 1 or 2 for Pairwise Epilogos")
+    if region_permutations > 0 and region_seed is None:
+        raise ValueError("region permutations need the run's region seed (region_null.region_seed), drawn once per run")
     null_mode = null_mode or os.environ.get("EPILOGOS_B200_NULL", "device")
     if null_mode not in ("reference", "device"):
         raise ValueError("null_mode must be 'reference' or 'device'")
@@ -113,6 +118,12 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
         exceed = be.permutation_exceedances(cnt_a, cnt_b, real_dist, permutations, draw_seed, size_a, size_b, c1 + c2,
                                             shard.lo, saliency, exp, (max(size_a, 1), max(size_b, 1)), (p1, p2),
                                             exact=exact)
+    region = None
+    if region_permutations > 0:
+        from . import region_null
+        region = region_null.shard_maxima(be, "paired", shard.states_device(), lambda n: _head(shard, n), (c1, c2),
+                                          numStates, roi_width, region_permutations, region_seed, saliency, exp,
+                                          exact=exact)
 
     total = shard.total_rows
     delta = dist.gather_rows(delta, total)
@@ -127,6 +138,9 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
     loc = _gather_locations(shard)
     if dist.rank() == 0:
         outputDirPath = Path(outputDirPath)
+        if region is not None:
+            from . import region_null
+            region_null.check_one_chromosome(loc["chrom"], file1Path)
         writer.write_scores_text(outputDirPath / "pairwiseDelta_{}_{}.txt.gz".format(fileTag, filename),
                                  delta.cpu().numpy(), loc)
         chrName = loc["chrom"][0] if len(loc["chrom"]) else ""
@@ -141,6 +155,9 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
                                                    end=np.asarray(loc["end"], dtype=np.int64))
             if exceed is not None:
                 session.handover[str(nullPath)].update(exceedances=exceed, permutations=int(permutations))
+            if region is not None:
+                region_null.stage_output(outputDirPath, fileTag, filename, chrName, region.cpu().numpy(), roi_width,
+                                         region_permutations, session.handover[str(nullPath)])
             return
         helpers.savez_level(nullPath, chrName=np.array([chrName]), nullDistances=null_dist.cpu().numpy())
         helpers.savez_level(outputDirPath / "temp_quiescence_{}_{}.npz".format(fileTag, filename),
@@ -149,3 +166,15 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
             helpers.savez_level(outputDirPath / "temp_permutations_{}_{}.npz".format(fileTag, filename),
                                 chrName=np.array([chrName]), exceedances=exceed.cpu().numpy().view(np.uint32),
                                 permutations=np.array(int(permutations), dtype=np.int64))
+        if region is not None:
+            region_null.stage_output(outputDirPath, fileTag, filename, chrName, region.cpu().numpy(), roi_width,
+                                     region_permutations, None)
+
+
+def _head(shard, n):
+    """The first n rows of the shard's combined [A | B] label matrix, on the host."""
+    a = shard.states_a.head(n) if hasattr(shard.states_a, "head") else np.asarray(shard.states_a[:n])
+    if not shard.paired:
+        return a
+    b = shard.states_b.head(n) if hasattr(shard.states_b, "head") else np.asarray(shard.states_b[:n])
+    return np.concatenate((a, b), axis=1)

@@ -11,6 +11,10 @@ Outputs, bins in chromosome order:
                                   p = (1 + k) / (P + 1) and BH its Benjamini-Hochberg adjustment over all bins;
   regionsOfInterest_<tag>.txt     the 100 windows of largest max-mean T (epi_roi_maxmean): chrom, start, end, then group,
                                   state, sign and "%.5e" T of the window's first bin of largest T [, its p and BH].
+With --roi-permutations P (temp_regionNull_<tag>_<file>.npz or the hand-over, epilogos_b200.region_null), also
+  regionPermutation_<tag>.txt     per region of regionsOfInterest, in its order: chrom, start, end, "%.5e" window mean of
+                                  T, k, "%.5e" family-wise p;
+  regionNullMaxima_<tag>.npz      {maxima int64 [P], window, permutations}: the genome-wide maxima of the window sums.
 The temp files and exp_freq_<tag>.npy are removed.
 """
 import re
@@ -20,7 +24,7 @@ from sys import argv
 
 import numpy as np
 
-from . import session, writer
+from . import region_null, session, writer
 from .roi import max_mean, orderChromosomes, permutation_pvalues
 from .run import getStateNames
 
@@ -79,7 +83,11 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, verbose=False, ba
                                  sign, group_names, names, k, p, bh)
     (outputDirPath / "regionsOfInterest_{}.txt".format(fileTag)).write_text(
         roi_lines(loc["chrom"], loc["start"], loc["end"], t, group, state, sign, group_names, names, roiWidth, p, bh))
-    pattern = re.compile(r"^temp_multigroup_{}_.*\.npz$".format(re.escape(fileTag)))
+    region_null.read_temps(outputDirPath, fileTag, chunks)
+    region = region_null.combine(chunks, "temp_regionNull files are missing for some chromosomes or disagree")
+    if region is not None:
+        region_null.write_outputs(outputDirPath, fileTag, loc["chrom"], loc["start"], loc["end"], t, region)
+    pattern = re.compile(r"^temp_(multigroup|regionNull)_{}_.*\.npz$".format(re.escape(fileTag)))
     for f in outputDirPath.iterdir():
         if pattern.match(f.name):
             remove(f)

@@ -16,6 +16,9 @@ With -n (`pval`):
      a keyed permutation seeded by the run seed;
   3. scipy.stats.gennorm.fit of each subsample, on the device; the trial with the median NLL is kept;
   4. two-sided p-values of every bin's distance and their Benjamini-Hochberg adjustment over the genome.
+With --roi-permutations P the score stage also found, per file, the P genome-wide maxima of the region null
+(temp_regionNull_<tag>_<file>.npz or the hand-over; epilogos_b200.region_null): regionPermutation_<tag>.txt gives every
+region of regionsOfInterest its family-wise p-value and regionNullMaxima_<tag>.npz keeps the maxima.
 When the score stage counted null permutations (--null-permutations P: temp_permutations_<tag>_<file>.npz or the
 hand-over), pairwisePermutation_<tag>.txt.gz holds per bin (chrom, start, end, k, p, BH): k of the P shuffles of the bin
 whose |null distance| is at least |distance|, p = (1 + k) / (P + 1), and its Benjamini-Hochberg adjustment over all bins.
@@ -32,7 +35,7 @@ from sys import argv
 
 import numpy as np
 
-from . import helpers, session, writer
+from . import helpers, region_null, session, writer
 from .helpers import strToBool
 from .roi import max_mean, orderChromosomes, permutation_pvalues
 from .run import getStateNames
@@ -161,11 +164,17 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, pval, numTrials=1
     perm = permutation_pvalues(be, chunks, "temp_permutations files are missing for some chromosomes or disagree")
     if perm is not None:
         writer.write_permutations_text(outputDirPath / "pairwisePermutation_{}.txt.gz".format(fileTag), loc, *perm)
+    # the region null (--roi-permutations): regionPermutation_<tag>.txt and regionNullMaxima_<tag>.npz
+    region_null.read_temps(outputDirPath, fileTag, chunks)
+    region = region_null.combine(chunks, "temp_regionNull files are missing for some chromosomes or disagree")
+    if region is not None:
+        region_null.write_outputs(outputDirPath, fileTag, loc["chrom"], loc["start"], loc["end"],
+                                  np.abs(distance.astype(np.float32)), region)
     if not verbose:
         print("\t[Done]", flush=True)
     if diagnostic:
         print("    Diagnostic figures (-d) are not built: matplotlib is not a dependency of this package", flush=True)
-    pattern = re.compile(r"^temp_(nullDistances|quiescence|permutations)_{}_.*\.npz$".format(re.escape(fileTag)))
+    pattern = re.compile(r"^temp_(nullDistances|quiescence|permutations|regionNull)_{}_.*\.npz$".format(re.escape(fileTag)))
     for f in outputDirPath.iterdir():
         if pattern.match(f.name):
             remove(f)

@@ -133,6 +133,25 @@ def checkPermutationFlags(mode, nullPermutations):
             return
 
 
+def checkRegionPermutationFlags(mode, roiPermutations, groupSize, roiWidth):
+    """Rules of --roi-permutations (checked after every other rule): first violated rule prints and exits."""
+    from .region_null import MAX_PERMUTATIONS, MAX_WINDOW
+    if roiPermutations is None:
+        return
+    rules = [
+        (mode != "paired", "ERROR: [--roi-permutations] requires [-m, --mode] 'paired'"),
+        (not 1 <= roiPermutations <= MAX_PERMUTATIONS,
+         "ERROR: Number of region permutations must be between 1 and {}".format(MAX_PERMUTATIONS)),
+        (groupSize != -1, "ERROR: [--roi-permutations] not compatible with [-g, --group-size] option"),
+        (roiWidth > MAX_WINDOW,
+         "ERROR: [--roi-permutations] needs a region width [-w, --roi-width] of at most {} bins".format(MAX_WINDOW)),
+    ]
+    for bad, message in rules:
+        if bad:
+            _die(message)
+            return
+
+
 def checkMultigroupFlags(mode, groupFile, multigroups, groupSet, pvalBool, groupSize):
     """Rules of --multigroup (checked after every other rule): first violated rule prints and exits.  Returns the
     comparisons, each a tuple of group names."""
@@ -176,7 +195,7 @@ def deal_files(pairs, world):
 
 def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
                groupSize, stateInfo, roiWidth, verbose, say, backend=None, pvalBool=False, numTrials=101,
-               samplingSize=100000, diagnosticBool=False, groups=None, permutations=0):
+               samplingSize=100000, diagnosticBool=False, groups=None, permutations=0, region_permutations=0):
     """Steps 1-4 of run.main (run.py:193-303) in process.  Two ways to use several GPUs:
       rows  (default)  every file's rows are split over the ranks (helpers.splitRows); per-file tables are all-reduced and
                        score rows gathered on rank 0, which writes the files;
@@ -193,7 +212,10 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
     `permutations` P > 0 (paired mode): step 3 also counts P null shuffles per bin and step 4 writes
     pairwisePermutation_<tag>.txt.gz.  A multi-group comparison (a Selection with `multi`, --multigroup) scores its groups
     in step 3 (epilogos_b200.multigroup), counting P shuffles per bin when P > 0, and step 4 runs
-    epilogos_b200.roi_multigroup."""
+    epilogos_b200.roi_multigroup.
+    `region_permutations` P > 0 (paired mode): step 3 also finds every file's maxima of the region null over P label
+    splits drawn from one seed per run, and step 4 writes regionPermutation_<tag>.txt and regionNullMaxima_<tag>.npz
+    (epilogos_b200.region_null)."""
     from contextlib import nullcontext
     from . import dist, expected, expectedCombination, scores, session
     world = dist.world_size()
@@ -222,6 +244,11 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
     say("\nSTEP 2: Background frequency combination")
     for out, tag, exp_path, _ in runs:
         expectedCombination.main(out, exp_path, tag, verbose, backend=backend)
+    region_seed = None
+    if region_permutations > 0:
+        # one seed for every file, rank and sharding mode: drawn here, by every rank together, outside dist.solo()
+        from . import pairwise, region_null
+        region_seed = region_null.region_seed(pairwise.run_seed())
     say("\nSTEP 3: Score calculation")
     # step 4 runs in this process right after: rank 0 hands its score arrays over in memory instead of through
     # temp_scores_*.npz (files written by other ranks, when whole files are dealt, are still read from disk)
@@ -237,7 +264,8 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
                 for out, tag, exp_path, sel in runs:
                     scores.main(f, second(f, f2, sel), numStates, saliency, out, exp_path, tag, numProcesses,
                                 quiescentState, groupSize, verbose, backend=backend, group=sel,
-                                permutations=permutations)
+                                permutations=permutations, region_permutations=region_permutations,
+                                region_seed=region_seed, roi_width=roiWidth)
     finally:
         session.handover_enabled = False
     dist.barrier()
@@ -322,14 +350,19 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
               help="Paired mode: draw P null shuffles of every bin on the GPU and write pairwisePermutation_<tag>.txt.gz "
                    + "with each bin's count of shuffles at least as far apart as its groups, its permutation p-value "
                    + "(1 + count) / (P + 1) and the Benjamini-Hochberg adjusted p-value (1 <= P <= 1000000)")
+@click.option("--roi-permutations", "roiPermutations", type=int, default=None,
+              help="Paired mode: permute the biosample labels P times over the whole genome on the GPU and give every "
+                   + "region of interest a family-wise p-value: the share of the P genome-wide maxima of the window sums "
+                   + "that reach its own (regionPermutation_<tag>.txt, regionNullMaxima_<tag>.npz; 1 <= P <= 100000; "
+                   + "not with -g)")
 @click.option("--exp-freq-mem", "expFreqMem", type=int, default=20000, help="SLURM-only (ignored)")
 @click.option("--exp-comb-mem", "expCombMem", type=int, default=8000, help="SLURM-only (ignored)")
 @click.option("--score-mem", "scoreMem", type=int, default=40000, help="SLURM-only (ignored)")
 @click.option("--roi-mem", "roiMem", type=int, default=-1, help="SLURM-only (ignored)")
 def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2, outputDirectory, stateInfo, saliency,
          numProcesses, exitBool, diagnosticBool, numTrials, samplingSize, quiescentState, groupSize, version, partition,
-         pvalBool, roiWidth, fileTag, groupFile, comparisons, multigroups, nullPermutations, expFreqMem, expCombMem,
-         scoreMem, roiMem):
+         pvalBool, roiWidth, fileTag, groupFile, comparisons, multigroups, nullPermutations, roiPermutations, expFreqMem,
+         expCombMem, scoreMem, roiMem):
     """Information-theoretic navigation of multi-tissue functional genomic annotations (B200 scoring path)."""
     if version:
         from epilogos_b200 import __version__
@@ -364,6 +397,7 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
                    samplingSize, quiescentState, groupSize, roiWidth)
     checkPermutationFlags(mode, nullPermutations)
     multi_of_groups = checkMultigroupFlags(mode, groupFile, multigroups, groupSet, pvalBool, groupSize)
+    checkRegionPermutationFlags(mode, roiPermutations, groupSize, roiWidth)
 
     import torch
     import torch.distributed as td
@@ -418,7 +452,7 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
     run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
                groupSize, stateInfo, roiWidth, verbose, say, pvalBool=pvalBool, numTrials=numTrials,
                samplingSize=samplingSize, diagnosticBool=diagnosticBool, groups=runs,
-               permutations=nullPermutations or 0)
+               permutations=nullPermutations or 0, region_permutations=roiPermutations or 0)
     dist.barrier()
     if launched and td.is_initialized():
         td.destroy_process_group()

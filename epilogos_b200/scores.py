@@ -18,7 +18,7 @@ from . import dist, helpers, session, writer
 
 
 def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, numProcesses, quiescentState, groupSize,
-         verbose, backend=None, group=None, permutations=0):
+         verbose, backend=None, group=None, permutations=0, region_permutations=0, region_seed=None, roi_width=None):
     tTotal = time()
     file1Path, file2Path, outputDirPath = Path(file1), Path(file2), Path(outputDir)
     filename = file1Path.name.split(".")[0]
@@ -27,7 +27,8 @@ def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, num
     if group is not None and group.multi is not None:
         from .multigroup import calculateScoresMultigroup
         calculateScoresMultigroup(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
-                                  backend, group=group, permutations=permutations)
+                                  backend, group=group, permutations=permutations,
+                                  region_permutations=region_permutations, region_seed=region_seed, roi_width=roi_width)
     elif str(file2) == "null":
         calculateScores(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
                         backend, group=group)
@@ -35,7 +36,8 @@ def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, num
         from .pairwise import calculateScoresPairwise
         calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDirPath, expFreqPath, fileTag,
                                 filename, quiescentState, groupSize, verbose, backend, group=group,
-                                permutations=permutations)
+                                permutations=permutations, region_permutations=region_permutations,
+                                region_seed=region_seed, roi_width=roi_width)
     if dist.rank() == 0:
         print("Total Time:", time() - tTotal, flush=True) if verbose else print("\t[Done]", flush=True)
     dist.barrier()

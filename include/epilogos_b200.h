@@ -236,6 +236,26 @@ int epi_multigroup_exceedances_s1(const uint16_t* cnt_dev, int64_t group_stride,
                                   uint32_t* k_inout, void* stream);
 int epi_multigroup_s1_fused_fits(int32_t groups, int32_t num_states, const int32_t* sizes);
 
+/* ---- whole-genome label permutations: the region null (csrc/label_permutations.cu) -----------------------------
+ *   epi_split_counts  counts of the groups of nsplit column splits of one matrix x (cols <= 65535, any pitch and
+ *                     alignment).  members_dev (device) holds nsplit x (groups - 1) column bitsets of ceil(cols / 64)
+ *                     uint64 words (column j is bit j % 64 of word j / 64); group groups - 1 of a split is the complement
+ *                     of the others.  cnt[p][g][b][s] = #{ columns j of group g of split p : x[b][j] == s }, uint16: block
+ *                     (p, g) starts at cnt_dev + (p * groups + g) * stride, stride = bins * num_states rounded up to a
+ *                     multiple of 8, and has the layout of epi_bin_counts, 16-byte aligned (cnt_dev must be).  groups in
+ *                     [2, EPI_MAX_GROUPS].  The bitsets are copied to the host and validated (which synchronises the
+ *                     stream): a bit at or above cols, or a column in two groups of a split, is rejected.
+ *   epi_window_max    for each row p < nrows of stat (dtype 0: float32, 1: float64; row p at stat_dev + p * row_stride
+ *                     elements, n values): max_inout[p] = max(max_inout[p], max_{0 <= i <= n - W} sum_{j < W}
+ *                     q(stat[p][i + j])) with q(x) = rint(x * 2^24) (round half to even) as int64 and W = window in
+ *                     [1, 16384].  Rows with n < W are left unchanged.  Every value must be finite with 0 <= x < 2^24
+ *                     (-0.0 included); otherwise return code 2 and a message naming one offending (row, index).
+ *                     Synchronises the stream. */
+int epi_split_counts(const int8_t* x_dev, int64_t bins, int32_t cols, int64_t pitch, int32_t num_states,
+                     const uint64_t* members_dev, int32_t nsplit, int32_t groups, uint16_t* cnt_dev, void* stream);
+int epi_window_max(const void* stat_dev, int32_t dtype, int64_t nrows, int64_t row_stride, int64_t n, int32_t window,
+                   int64_t* max_inout_dev, void* stream);
+
 /* ---- paired statistics stage (roiAndVisualPairwise.py:177-242, csrc/pairwise_stats.cu) -----------------------
  *   epi_null_compact       the null distances of the bins whose quiescent flag is 0 (all bins when quiescent_dev is NULL),
  *                          stable order, every permutation: null_dev float32 [nperm][bins] -> pool_out [nperm][count]
