@@ -4,8 +4,8 @@ branches of s1Score / s2Score (scores.py:282-303, 319-322, 373-398, 414-421).
 Outputs (rank 0): `pairwiseDelta_<tag>_<file>.txt.gz`, `temp_nullDistances_<tag>_<file>.npz`
 {chrName, nullDistances float32[B]}, `temp_quiescence_<tag>_<file>.npz` {chrName, quiescenceArr bool[B]}, and with
 --null-permutations `temp_permutations_<tag>_<file>.npz` {chrName, exceedances uint32[B], permutations}.  When the
-paired statistics stage (roi_pairwise) runs next in this process, the two temp files are not written: their content and
-the reduced real deltas are handed over in memory (session.handover).
+paired statistics stage (roi_pairwise) runs next in this process, the temp files are not written: their content and
+the reduced real deltas are handed over in memory (epilogos_b200.handoff).
 
 Null shuffles.  The reference shuffles each combined row once with the unseeded global numpy RNG
 (helpers.py:183-184).  Two modes are provided (environment variable EPILOGOS_B200_NULL or the `null_mode`
@@ -29,7 +29,7 @@ from pathlib import Path
 
 import numpy as np
 
-from . import dist, helpers, session, writer
+from . import dist, handoff, region_null, session, writer
 from .scores import _gather_locations
 
 
@@ -68,15 +68,14 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
                             group=None, permutations=0, region_permutations=0, region_seed=None, roi_width=None):
     """`permutations` P > 0: also count, for every bin, how many of P device-drawn null shuffles (permutations 0..P-1 of
     the device sampler, scored like the run's null) are at least as far from 0 as the bin's real distance, and hand the
-    counts to step 4 (session.handover) or write them to temp_permutations_<tag>_<file>.npz {chrName, exceedances
+    counts to step 4 (epilogos_b200.handoff) or write them to temp_permutations_<tag>_<file>.npz {chrName, exceedances
     uint32[B], permutations}.  Nothing else changes: in device mode permutation 0 is the run's own null.
     `region_permutations` P > 0: also the file's maxima of the region null over `region_seed`'s P label splits of the
     combined [A | B] matrix, windows of `roi_width` rows (epilogos_b200.region_null), handed to step 4 or written to
     temp_regionNull_<tag>_<file>.npz."""
     if saliency not in (1, 2):
         raise ValueError("Please ensure that saliency metric is either 1 or 2 for Pairwise Epilogos")
-    if region_permutations > 0 and region_seed is None:
-        raise ValueError("region permutations need the run's region seed (region_null.region_seed), drawn once per run")
+    region_null.check_seed(region_permutations, region_seed)
     null_mode = null_mode or os.environ.get("EPILOGOS_B200_NULL", "device")
     if null_mode not in ("reference", "device"):
         raise ValueError("null_mode must be 'reference' or 'device'")
@@ -120,7 +119,6 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
                                             exact=exact)
     region = None
     if region_permutations > 0:
-        from . import region_null
         region = region_null.shard_maxima(be, "paired", shard.states_device(), lambda n: _head(shard, n), (c1, c2),
                                           numStates, roi_width, region_permutations, region_seed, saliency, exp,
                                           exact=exact)
@@ -133,42 +131,17 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
         null_dist = None if parts[0] is None else __import__("torch").stack(parts, dim=0)
     else:
         null_dist = dist.gather_rows(null_dist, total)
-    if exceed is not None:
-        exceed = dist.gather_rows(exceed, total)
     loc = _gather_locations(shard)
+    extra = handoff.optional_parts(file1Path, loc, total, exceed, permutations, region, roi_width, region_permutations)
     if dist.rank() == 0:
-        outputDirPath = Path(outputDirPath)
-        if region is not None:
-            from . import region_null
-            region_null.check_one_chromosome(loc["chrom"], file1Path)
-        writer.write_scores_text(outputDirPath / "pairwiseDelta_{}_{}.txt.gz".format(fileTag, filename),
+        writer.write_scores_text(Path(outputDirPath) / "pairwiseDelta_{}_{}.txt.gz".format(fileTag, filename),
                                  delta.cpu().numpy(), loc)
-        chrName = loc["chrom"][0] if len(loc["chrom"]) else ""
-        nullPath = outputDirPath / "temp_nullDistances_{}_{}.npz".format(fileTag, filename)
-        if session.handover_enabled and not os.environ.get("EPILOGOS_B200_KEEP_TEMP"):
-            # the paired statistics stage runs next, in this process: hand over what it reads, reduced on the device to
-            # the distance and the max-difference state of every bin (roi_pairwise.readInData)
-            distance, max_diff = be.pairwise_real_reduce(delta, text_round_trip=True)
-            session.handover[str(nullPath)] = dict(chrName=str(chrName), distance=distance, max_diff=max_diff,
-                                                   null=null_dist, quiescence=quies, chrom=loc["chrom"],
-                                                   start=np.asarray(loc["start"], dtype=np.int64),
-                                                   end=np.asarray(loc["end"], dtype=np.int64))
-            if exceed is not None:
-                session.handover[str(nullPath)].update(exceedances=exceed, permutations=int(permutations))
-            if region is not None:
-                region_null.stage_output(outputDirPath, fileTag, filename, chrName, region.cpu().numpy(), roi_width,
-                                         region_permutations, session.handover[str(nullPath)])
-            return
-        helpers.savez_level(nullPath, chrName=np.array([chrName]), nullDistances=null_dist.cpu().numpy())
-        helpers.savez_level(outputDirPath / "temp_quiescence_{}_{}.npz".format(fileTag, filename),
-                            chrName=np.array([chrName]), quiescenceArr=quies.cpu().numpy().astype(np.bool_))
-        if exceed is not None:
-            helpers.savez_level(outputDirPath / "temp_permutations_{}_{}.npz".format(fileTag, filename),
-                                chrName=np.array([chrName]), exceedances=exceed.cpu().numpy().view(np.uint32),
-                                permutations=np.array(int(permutations), dtype=np.int64))
-        if region is not None:
-            region_null.stage_output(outputDirPath, fileTag, filename, chrName, region.cpu().numpy(), roi_width,
-                                     region_permutations, None)
+        # step 4 takes the distance and the max-difference state of every bin: handed over, reduced here on the device;
+        # from files, reduced from the delta text
+        handoff.publish("paired", outputDirPath, fileTag, filename,
+                        handoff.record(loc, null=null_dist, quiescence=quies, **extra),
+                        in_memory=lambda: dict(zip(("distance", "max_diff"),
+                                                   be.pairwise_real_reduce(delta, text_round_trip=True))))
 
 
 def _head(shard, n):

@@ -69,6 +69,11 @@ def shard_maxima(be, kind, x_dev, head, sizes, num_states, window, nperm, seed, 
     return dist.all_reduce_max(m)
 
 
+def check_seed(nperm, seed):
+    if nperm > 0 and seed is None:
+        raise ValueError("region permutations need the run's region seed (region_null.region_seed), drawn once per run")
+
+
 def check_one_chromosome(chrom, path):
     """The region null keys a file's maxima by its chromosome: one chromosome per input file."""
     names = np.unique(np.asarray(chrom, dtype=object).astype(str))
@@ -115,29 +120,3 @@ def write_outputs(outputDirPath, fileTag, chrom, starts, ends, x, combined):
         region_lines(chrom, starts, ends, x, window, maxima))
     np.savez(outputDirPath / "regionNullMaxima_{}.npz".format(fileTag), maxima=maxima.astype(np.int64),
              window=np.array(window, dtype=np.int64), permutations=np.array(P, dtype=np.int64))
-
-
-def stage_output(outputDirPath, fileTag, filename, chrName, maxima, window, nperm, handover):
-    """Step 3's result of one file: into `handover` (a dict step 4 of this process reads) or written as
-    temp_regionNull_<tag>_<file>.npz {chrName, maxima, window, permutations}."""
-    from . import helpers
-    out = dict(region_maxima=np.asarray(maxima, dtype=np.int64), region_window=int(window),
-               region_permutations=int(nperm))
-    if handover is not None:
-        handover.update(out)
-        return
-    helpers.savez_level(outputDirPath / "temp_regionNull_{}_{}.npz".format(fileTag, filename),
-                        chrName=np.array([chrName]), maxima=out["region_maxima"],
-                        window=np.array(window, dtype=np.int64), permutations=np.array(nperm, dtype=np.int64))
-
-
-def read_temps(outputDirPath, fileTag, chunks):
-    """Add the maxima of temp_regionNull_<tag>_<file>.npz to the step-4 chunks of their chromosomes (chunks handed over
-    in memory already carry theirs)."""
-    by_name = {c["chrName"]: c for c in chunks}
-    for f in sorted(outputDirPath.glob("temp_regionNull_{}_*.npz".format(fileTag))):
-        z = np.load(f, allow_pickle=False)
-        c = by_name.get(str(z["chrName"][0]))
-        if c is not None and "region_maxima" not in c:
-            c.update(region_maxima=np.asarray(z["maxima"], dtype=np.int64), region_window=int(z["window"]),
-                     region_permutations=int(z["permutations"]))

@@ -2,7 +2,8 @@
 
     main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, verbose)                     (roiSingle.py:10)
 
-Reads every `temp_scores_*.npz`, orders the chromosomes (helpers.orderChromosomes, helpers.py:224-250), selects the
+Reads the score stage's results (every `temp_scores_*.npz`, or what the score stage of this process handed over in
+memory: epilogos_b200.handoff), orders the chromosomes (helpers.orderChromosomes, helpers.py:224-250), selects the
 top 100 non-overlapping windows with the max-mean rule (native epi_roi_maxmean), names the strongest state of each
 window, writes `regionsOfInterest_<tag>.txt` and removes the temp score files and the expected-frequency file exactly
 as the reference does (roiSingle.py:40, 73-74).
@@ -14,7 +15,7 @@ from sys import argv
 
 import numpy as np
 
-from . import _lib
+from . import _lib, handoff
 from .helpers import strToBool
 from .run import getStateNames
 
@@ -61,28 +62,11 @@ def permutation_pvalues(be, chunks, mismatch):
     return k, p, be.bh_adjust(be.to_device(p)).cpu().numpy()
 
 
-def readInData(outputDirPath):
-    """All temp_scores_*.npz in chromosome order -> (chrom per row, starts, ends, scoreArr); temp files removed."""
-    from . import session
-    outputDirPath = Path(outputDirPath)
-    files = list(outputDirPath.glob("temp_scores_*.npz"))
-    chunks = {}
-    for f in files:
-        z = np.load(f, allow_pickle=True)
-        loc = z["locationArr"]
-        chunks[str(z["chrName"][0])] = (z["scoreArr"], loc[:, 0], loc[:, 1].astype(np.int64), loc[:, 2].astype(np.int64))
-    # files of this directory that the score stage of this process handed over in memory instead of writing them
-    for key in [k for k in session.handover if Path(k).parent == outputDirPath and Path(k).name.startswith("temp_scores_")]:
-        h = session.handover.pop(key)
-        chunks[h["chrName"]] = (h["scoreArr"], h["chrom"], h["start"], h["end"])
-    order = orderChromosomes(list(chunks))
-    scoreArr = np.concatenate([chunks[c][0] for c in order])
-    chrom = np.concatenate([np.asarray(chunks[c][1], dtype=object) for c in order])
-    starts = np.concatenate([chunks[c][2] for c in order])
-    ends = np.concatenate([chunks[c][3] for c in order])
-    for f in files:
-        remove(f)
-    return chrom, starts, ends, scoreArr
+def readInData(outputDirPath, fileTag):
+    """The score stage's results in chromosome order -> (chrom per row, starts, ends, scoreArr); temp files removed."""
+    chunks = handoff.collect("scores", outputDirPath, fileTag)
+    handoff.remove_temps("scores", outputDirPath, fileTag)
+    return tuple(np.concatenate([c[k] for c in chunks]) for k in ("chrom", "start", "end", "scoreArr"))
 
 
 def createTopScoresTxt(filePath, chrom, starts, ends, scoreArr, nameArr, roiWidth):
@@ -108,7 +92,7 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, verbose):
     names = getStateNames(stateInfo)
     if not verbose:
         print("    Reading in files\t", end="", flush=True)
-    chrom, starts, ends, scoreArr = readInData(outputDirPath)
+    chrom, starts, ends, scoreArr = readInData(outputDirPath, fileTag)
     if not verbose:
         print("\t[Done]\n    Regions of interest txt\t", end="", flush=True)
     createTopScoresTxt(outputDirPath / "regionsOfInterest_{}.txt".format(fileTag), chrom, starts, ends, scoreArr, names,

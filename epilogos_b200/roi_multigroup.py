@@ -3,9 +3,10 @@
     main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, verbose)
     python -m epilogos_b200.roi_multigroup OUTPUT_DIR STATE_INFO FILE_TAG EXP_FREQ_PATH ROI_WIDTH
 
-Inputs per chromosome, from the score stage of this process (session.handover) or from temp_multigroup_<tag>_<file>.npz
-(epilogos_b200.multigroup): the statistic T of every bin, the group g* and state s* that drive it, the sign of
-S_g*[s*] - m[s*], and with --null-permutations P the count k of the P shuffles whose T is at least as large.
+Inputs per chromosome, from the score stage of this process (epilogos_b200.handoff) or from
+temp_multigroup_<tag>_<file>.npz (epilogos_b200.multigroup): the statistic T of every bin, the group g* and state s* that
+drive it, the sign of S_g*[s*] - m[s*], and with --null-permutations P the count k of the P shuffles whose T is at least
+as large.
 Outputs, bins in chromosome order:
   multigroupMetrics_<tag>.txt.gz  chrom, start, end, "%.5e" T, group, state, +/- [, k, "%.5e" p, "%.5e" BH], with
                                   p = (1 + k) / (P + 1) and BH its Benjamini-Hochberg adjustment over all bins;
@@ -17,39 +18,15 @@ With --roi-permutations P (temp_regionNull_<tag>_<file>.npz or the hand-over, ep
   regionNullMaxima_<tag>.npz      {maxima int64 [P], window, permutations}: the genome-wide maxima of the window sums.
 The temp files and exp_freq_<tag>.npy are removed.
 """
-import re
 from os import remove
 from pathlib import Path
 from sys import argv
 
 import numpy as np
 
-from . import region_null, session, writer
-from .roi import max_mean, orderChromosomes, permutation_pvalues
+from . import handoff, region_null, session, writer
+from .roi import max_mean, permutation_pvalues
 from .run import getStateNames
-
-
-def readInData(outputDirPath, fileTag):
-    """The score stage's results for this directory, in chromosome order: a list of dicts (chrName, groups, t, group,
-    state, sign, chrom, start, end[, exceedances, permutations])."""
-    chunks = {}
-    prefix = "temp_multigroup_{}_".format(fileTag)
-    for key in [k for k in session.handover if Path(k).parent == outputDirPath and Path(k).name.startswith(prefix)]:
-        h = session.handover.pop(key)
-        chunks[h["chrName"]] = h
-    for f in sorted(outputDirPath.glob(prefix + "*.npz")):
-        z = np.load(f, allow_pickle=False)
-        chrName = str(z["chrName"][0])
-        if chrName in chunks:
-            continue
-        c = dict(chrName=chrName, groups=[str(g) for g in z["groups"]], t=z["t"], group=z["group"], state=z["state"],
-                 sign=z["sign"], chrom=z["chrom"].astype(object), start=z["start"], end=z["end"])
-        if "exceedances" in z.files:
-            c.update(exceedances=z["exceedances"], permutations=int(z["permutations"]))
-        chunks[chrName] = c
-    if not chunks:
-        raise FileNotFoundError("no multi-group score-stage outputs ({}*.npz) in {}".format(prefix, outputDirPath))
-    return [chunks[c] for c in orderChromosomes(list(chunks))]
 
 
 def roi_lines(chrom, starts, ends, t, group, state, sign, group_names, state_names, roiWidth, pvals=None, bh=None):
@@ -73,7 +50,7 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, verbose=False, ba
     be = session.get_backend(backend)
     if not verbose:
         print("    Multi-group metrics and regions of interest\t", end="", flush=True)
-    chunks = readInData(outputDirPath, fileTag)
+    chunks = handoff.collect("multigroup", outputDirPath, fileTag)
     group_names = chunks[0]["groups"]
     cat = lambda key, dtype: np.concatenate([np.asarray(c[key], dtype=dtype) for c in chunks])   # noqa: E731
     loc = dict(chrom=cat("chrom", object), start=cat("start", np.int64), end=cat("end", np.int64))
@@ -83,14 +60,10 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, verbose=False, ba
                                  sign, group_names, names, k, p, bh)
     (outputDirPath / "regionsOfInterest_{}.txt".format(fileTag)).write_text(
         roi_lines(loc["chrom"], loc["start"], loc["end"], t, group, state, sign, group_names, names, roiWidth, p, bh))
-    region_null.read_temps(outputDirPath, fileTag, chunks)
     region = region_null.combine(chunks, "temp_regionNull files are missing for some chromosomes or disagree")
     if region is not None:
         region_null.write_outputs(outputDirPath, fileTag, loc["chrom"], loc["start"], loc["end"], t, region)
-    pattern = re.compile(r"^temp_(multigroup|regionNull)_{}_.*\.npz$".format(re.escape(fileTag)))
-    for f in outputDirPath.iterdir():
-        if pattern.match(f.name):
-            remove(f)
+    handoff.remove_temps("multigroup", outputDirPath, fileTag)
     if Path(expFreqPath).exists():
         remove(Path(expFreqPath))
     if not verbose:

@@ -7,7 +7,7 @@ the reference's roiAndVisualPairwise.py (:177-242, 339-354), without its figures
 
 Inputs per chromosome: the distance (sum_s d^2 * sign(sum_s d) of the delta row after its "%.5f" text round trip) and
 the max-difference state of every bin, the null distances and the quiescence mask.  They come from the score stage of
-this process (session.handover: already reduced on the device) or from its files: pairwiseDelta_<tag>_<file>.txt.gz,
+this process (epilogos_b200.handoff: already reduced on the device) or from its files: pairwiseDelta_<tag>_<file>.txt.gz,
 temp_nullDistances_<tag>_<file>.npz and temp_quiescence_<tag>_<file>.npz.  Both routes give the same bits.
 
 With -n (`pval`):
@@ -28,16 +28,15 @@ regionsOfInterest_<tag>.txt (the 100 windows of largest max-mean |distance|; sta
 this package; the six-column files are written.  -d figures are not built (matplotlib is not a dependency).  The temp
 files and exp_freq_<tag>.npy are removed, as the reference does (roiAndVisualPairwise.py:172, 343-344).
 """
-import re
 from os import remove
 from pathlib import Path
 from sys import argv
 
 import numpy as np
 
-from . import helpers, region_null, session, writer
+from . import handoff, helpers, region_null, session, writer
 from .helpers import strToBool
-from .roi import max_mean, orderChromosomes, permutation_pvalues
+from .roi import max_mean, permutation_pvalues
 from .run import getStateNames
 
 STATS_SEED_SALT = "epilogos_b200 paired statistics: null subsamples"
@@ -51,40 +50,16 @@ def stats_seed(run_seed):
 
 
 def readInData(outputDirPath, fileTag, be):
-    """{chrName: dict(distance, max_diff, null, quiescence, chrom, start, end)}: the score stage's hand-over for this
-    directory, then the files of chromosomes not handed over."""
-    chunks = {}
-    for key in [k for k in session.handover if Path(k).parent == outputDirPath
-                and Path(k).name.startswith("temp_nullDistances_{}_".format(fileTag))]:
-        h = session.handover.pop(key)
-        if "exceedances" in h:
-            h["exceedances"] = h["exceedances"].cpu().numpy().view(np.uint32)
-        chunks[h["chrName"]] = h
-    nullFiles = sorted(outputDirPath.glob("temp_nullDistances_{}_*.npz".format(fileTag)))
-    for nf in nullFiles:
-        name = nf.name[len("temp_nullDistances_{}_".format(fileTag)):-len(".npz")]
-        z = np.load(nf, allow_pickle=False)
-        chrName = str(z["chrName"][0])
-        if chrName in chunks:
-            continue
-        q = np.load(outputDirPath / "temp_quiescence_{}_{}.npz".format(fileTag, name), allow_pickle=False)
+    """The score stage's results in chromosome order: dicts (chrName, distance, max_diff, null, quiescence, chrom, start,
+    end[, exceedances, permutations][, region_maxima, region_window, region_permutations]), arrays on the device."""
+    def from_files(c, name):
         loc, delta = helpers.read_scores(outputDirPath / "pairwiseDelta_{}_{}.txt.gz".format(fileTag, name))
         # the text already went through "%.5f": the reduction takes the parsed values as they are
-        dist, md = be.pairwise_real_reduce(be.to_device(delta.astype(np.float32)), text_round_trip=False)
-        chunks[chrName] = dict(chrName=chrName, distance=dist, max_diff=md,
-                               null=be.to_device(np.ascontiguousarray(z["nullDistances"], dtype=np.float32)),
-                               quiescence=be.to_device(q["quiescenceArr"].astype(np.uint8)),
-                               chrom=loc["chrom"], start=loc["start"], end=loc["end"])
-        pf = outputDirPath / "temp_permutations_{}_{}.npz".format(fileTag, name)
-        if pf.exists():
-            zp = np.load(pf, allow_pickle=False)
-            chunks[chrName].update(exceedances=np.asarray(zp["exceedances"], dtype=np.uint32),
-                                   permutations=int(zp["permutations"]))
-    if not chunks:
-        raise FileNotFoundError("no paired score-stage outputs (temp_nullDistances_{}_*.npz) in {}"
-                                .format(fileTag, outputDirPath))
-    order = orderChromosomes(list(chunks))
-    return [chunks[c] for c in order]
+        distance, max_diff = be.pairwise_real_reduce(be.to_device(delta.astype(np.float32)), text_round_trip=False)
+        c.update(distance=distance, max_diff=max_diff, chrom=loc["chrom"], start=loc["start"], end=loc["end"],
+                 null=be.to_device(np.ascontiguousarray(c["null"], dtype=np.float32)),
+                 quiescence=be.to_device(c["quiescence"].astype(np.uint8)))
+    return handoff.collect("paired", outputDirPath, fileTag, from_files=from_files)
 
 
 def fit_null(be, chunks, numTrials, samplingSize, seed):
@@ -165,7 +140,6 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, pval, numTrials=1
     if perm is not None:
         writer.write_permutations_text(outputDirPath / "pairwisePermutation_{}.txt.gz".format(fileTag), loc, *perm)
     # the region null (--roi-permutations): regionPermutation_<tag>.txt and regionNullMaxima_<tag>.npz
-    region_null.read_temps(outputDirPath, fileTag, chunks)
     region = region_null.combine(chunks, "temp_regionNull files are missing for some chromosomes or disagree")
     if region is not None:
         region_null.write_outputs(outputDirPath, fileTag, loc["chrom"], loc["start"], loc["end"],
@@ -174,10 +148,7 @@ def main(outputDir, stateInfo, fileTag, expFreqPath, roiWidth, pval, numTrials=1
         print("\t[Done]", flush=True)
     if diagnostic:
         print("    Diagnostic figures (-d) are not built: matplotlib is not a dependency of this package", flush=True)
-    pattern = re.compile(r"^temp_(nullDistances|quiescence|permutations|regionNull)_{}_.*\.npz$".format(re.escape(fileTag)))
-    for f in outputDirPath.iterdir():
-        if pattern.match(f.name):
-            remove(f)
+    handoff.remove_temps("paired", outputDirPath, fileTag)
     if Path(expFreqPath).exists():
         remove(Path(expFreqPath))
     return result

@@ -14,7 +14,7 @@ from time import time
 
 import numpy as np
 
-from . import dist, helpers, session, writer
+from . import dist, handoff, helpers, session, writer
 
 
 def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, numProcesses, quiescentState, groupSize,
@@ -61,16 +61,7 @@ def calculateScores(saliency, file1Path, numStates, outputDirPath, expFreqPath, 
         with timing.stage("device -> host", sync_cuda=True):
             scoreArr = scoreArr.cpu().numpy()
         writer.write_scores_text(outputDirPath / "scores_{}_{}.txt.gz".format(fileTag, filename), scoreArr, loc)
-        chrName = loc["chrom"][0] if len(loc["chrom"]) else ""
-        npz = outputDirPath / "temp_scores_{}_{}.npz".format(fileTag, filename)
-        import os
-        if session.handover_enabled and not os.environ.get("EPILOGOS_B200_KEEP_TEMP"):
-            # the ROI stage runs next, in this process: hand the arrays over in memory (session.handover)
-            session.handover[str(npz)] = dict(chrName=str(chrName), scoreArr=scoreArr, chrom=loc["chrom"],
-                                              start=np.asarray(loc["start"], dtype=np.int64),
-                                              end=np.asarray(loc["end"], dtype=np.int64))
-        else:
-            helpers.savez_level(npz, chrName=np.array([chrName]), scoreArr=scoreArr, locationArr=writer.location_array(loc))
+        handoff.publish("scores", outputDirPath, fileTag, filename, handoff.record(loc, scoreArr=scoreArr))
 
 
 def _gather_locations(shard):

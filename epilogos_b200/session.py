@@ -15,12 +15,12 @@ from . import dist, helpers
 _backend = None
 _cache = {}
 
-# In-process hand-over of the score stage to the region-of-interest stage.  The reference passes the scores of every file
-# through temp_scores_<tag>_<file>.npz (scores.py:166-169), which the ROI stage reads and deletes (roiSingle.py:43-76).  When
-# both stages run in THIS process (the CLI, run.run_stages) the arrays are handed over in memory instead: the file would
-# be written, read back and removed within seconds (0.3-0.6 s of a 2 s run at 400 k bins x 833).  Stand-alone calls of
-# scores.main still write the file, and EPILOGOS_B200_KEEP_TEMP=1 forces it everywhere.
-handover = {}              # str(path of the temp_scores npz that was not written) -> dict(chrName, scoreArr, chrom, start, end)
+# In-process hand-over of the score stage to the region-of-interest stage (epilogos_b200.handoff).  The reference passes
+# the results of every file through temp_*_<tag>_<file>.npz files, which the ROI stage reads and deletes.  When both stages
+# run in THIS process (the CLI, run.run_stages) the records are handed over in memory instead: the files would be written,
+# read back and removed within seconds (0.3-0.6 s of a 2 s run at 400 k bins x 833).  Stand-alone calls of scores.main
+# still write the files, and EPILOGOS_B200_KEEP_TEMP=1 forces them everywhere.
+handover = {}              # (kind, output directory, tag, file) -> the record handoff.publish did not write
 handover_enabled = False
 
 
