@@ -19,7 +19,8 @@ namespace epi {
 // label of the row (6x fewer operations than per-label selection sampling at 833 biosamples).
 __device__ __forceinline__ double uniform53(Philox& rng) {
     const uint32_t hi = rng.next(), lo = rng.next();
-    // (0, 1): 53 random bits + one half
+    // 53 random bits + one half, in float64: (0, 1], since the + 0.5 rounds to even once the integer part reaches 2^52,
+    // so U = 1.0 occurs with probability 2^-53 (tests/sampler_oracle.py restates this expression)
     return ((double)(hi >> 5) * 67108864.0 + (double)(lo >> 6) + 0.5) * (1.0 / 9007199254740992.0);
 }
 

@@ -4,6 +4,7 @@ product never imports this, and epilogos_b200 itself has no CPU path."""
 import numpy as np
 import torch
 
+import sampler_oracle as so
 from oracle import epilogos_oracle as orc
 
 
@@ -47,23 +48,14 @@ class OracleBackend:
         return self.counts(sa, num_states), self.counts(sb, num_states)
 
     def shuffled_counts_device(self, cnt_a, cnt_b, size_a, size_b, seed, nperm=1, width=None, bin_offset=0):
-        """numpy multivariate hypergeometric draws keyed like the device kernel: (seed, permutation, GLOBAL bin)."""
+        """The device's draws (sampler_oracle.draw_shuffle): permutation p of row r from the stream keyed by (seed, p,
+        GLOBAL bin bin_offset + r)."""
         a, b = self._cnt(cnt_a), self._cnt(cnt_b)
         rows, k = a.shape
-        oa = np.zeros((nperm, rows, k), dtype=np.int64)
-        ob = np.zeros_like(oa)
-        for p in range(nperm):
-            for r in range(rows):
-                rng = np.random.default_rng([int(seed) & (2 ** 63 - 1), p, bin_offset + r])
-                comb = a[r] + b[r]
-                na = min(size_a, int(comb.sum()))
-                ga = rng.multivariate_hypergeometric(comb, na) if na else np.zeros(k, dtype=np.int64)
-                rest = comb - ga
-                nb = min(size_b, int(rest.sum()))
-                gb = rng.multivariate_hypergeometric(rest, nb) if nb else np.zeros(k, dtype=np.int64)
-                oa[p, r], ob[p, r] = ga, gb
-        ta = torch.from_numpy(oa.astype(np.uint16).view(np.int16))
-        tb = torch.from_numpy(ob.astype(np.uint16).view(np.int16))
+        r = so.draw_shuffle(seed, np.repeat(np.arange(nperm), rows), bin_offset + np.tile(np.arange(rows), nperm),
+                            np.tile(a, (nperm, 1)), np.tile(b, (nperm, 1)), size_a, size_b)
+        ta = torch.from_numpy(r["a"].reshape(nperm, rows, k).astype(np.uint16).view(np.int16))
+        tb = torch.from_numpy(r["b"].reshape(nperm, rows, k).astype(np.uint16).view(np.int16))
         return (ta[0], tb[0]) if nperm == 1 else (ta, tb)
 
     def pairwise_combine(self, score_a, score_b, null_a, null_b):

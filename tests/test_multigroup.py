@@ -3,6 +3,7 @@ kernels are covered by test_multigroup_gpu.py."""
 import numpy as np
 
 import multigroup_oracle as mgo
+import sampler_oracle as so
 
 
 def scores(rng, G, bins, K):
@@ -86,22 +87,14 @@ STATE_NAMES = ["S%d" % i for i in range(1, K + 1)]
 
 
 def draw_exceedances(cnt, sizes, t, nperm, seed, bin_offset, saliency, exp, score):
-    """k per bin from numpy G-way draws keyed like the device (seed, permutation, GLOBAL bin): for every group in order,
-    its counts are a multivariate hypergeometric draw from the labels the earlier groups left."""
+    """k per bin from the device's G-way draws (sampler_oracle.draw_multigroup_shuffle): permutation p of row r from the
+    stream keyed by (seed, p, GLOBAL bin bin_offset + r)."""
     G, rows, k = cnt.shape
-    k_out = np.zeros(rows, dtype=np.int64)
-    for r in range(rows):
-        comb = cnt[:, r].sum(axis=0)
-        null = np.zeros((nperm, G, 1, k), dtype=np.float32)
-        for p in range(nperm):
-            rng = np.random.default_rng([int(seed) & (2 ** 63 - 1), p, bin_offset + r])
-            rest = comb.copy()
-            for g, n in enumerate(sizes):
-                x = rng.multivariate_hypergeometric(rest, n) if g < G - 1 else rest.copy()
-                rest = rest - x
-                null[p, g, 0] = score(x[None, :], n)[0]
-        k_out[r] = mgo.exceedances(null, sizes, np.asarray(t[r:r + 1]))[0]
-    return k_out
+    comb = cnt.sum(axis=0)
+    x = so.draw_multigroup_shuffle(seed, np.repeat(np.arange(nperm), rows), bin_offset + np.tile(np.arange(rows), nperm),
+                                   np.tile(comb, (nperm, 1)), sizes)["x"].reshape(nperm, rows, G, k)
+    null = np.stack([np.stack([score(x[p, :, g], n) for g, n in enumerate(sizes)]) for p in range(nperm)])
+    return mgo.exceedances(null.astype(np.float32), sizes, np.asarray(t))
 
 
 class MultiBackend(PermBackend):

@@ -13,6 +13,7 @@ import scipy.stats
 import torch
 from click.testing import CliRunner
 
+import sampler_oracle as so
 from fake_backend import OracleBackend
 from oracle import epilogos_oracle as orc
 from oracle import pairwise_stats_oracle as pso
@@ -21,8 +22,8 @@ from test_host_stages import ROOT, write_tsv
 
 
 class StatsBackend(OracleBackend):
-    """OracleBackend plus the paired statistics, answered with numpy / scipy (the subsamples come from numpy's generator,
-    not from the device's keyed permutation)."""
+    """OracleBackend plus the paired statistics, answered with numpy / scipy; the subsamples are the device's keyed
+    permutation (sampler_oracle.null_subsample)."""
 
     def pairwise_real_reduce(self, delta, text_round_trip=True):
         d, md = orc.paired_real_reductions(np.asarray(delta, dtype=np.float32), text_round_trip)
@@ -32,9 +33,7 @@ class StatsBackend(OracleBackend):
         return torch.from_numpy(pso.null_pool([null_dist.numpy()], [quiescent.numpy()]))
 
     def null_subsample(self, pool, trials, size, seed):
-        n = pool.numel()
-        idx = np.stack([np.random.default_rng([int(seed) & (2 ** 63 - 1), t]).permutation(n)[:size]
-                        for t in range(trials)]).astype(np.int32)
+        idx = so.null_subsample(pool.numel(), trials, size, seed)
         return torch.from_numpy(idx), torch.from_numpy(pool.numpy()[idx])
 
     def gennorm_fit(self, samples):

@@ -10,6 +10,7 @@ import pytest
 import torch
 from click.testing import CliRunner
 
+import sampler_oracle as so
 from oracle import epilogos_oracle as orc
 from oracle import pairwise_stats_oracle as pso
 from test_cli import META
@@ -77,7 +78,8 @@ def test_flag_rules_and_their_precedence(tmp_path, monkeypatch, golden):
 
 
 def test_permutation_file_against_numpy(tmp_path, golden, monkeypatch):
-    """Steps 1-4 on one file with the temp files kept between steps 3 and 4: the counts against numpy draws and scores,
+    """Steps 1-4 on one file with the temp files kept between steps 3 and 4: the counts against the device's draws
+    (sampler_oracle) and numpy scores,
     the file's columns against (1 + k) / (P + 1) and its Benjamini-Hochberg adjustment."""
     from epilogos_b200 import expected, expectedCombination, roi_pairwise, scores, session
     from epilogos_b200.pairwise import file_seed
@@ -99,15 +101,12 @@ def test_permutation_file_against_numpy(tmp_path, golden, monkeypatch):
     xa, xb = golden("paired_synth_c30_c25_k18")["xa"], golden("paired_synth_c30_c25_k18")["xb"]
     ca, cb = orc.bin_counts(xa, 18).astype(np.int64), orc.bin_counts(xb, 18).astype(np.int64)
     seed = file_seed(11, "epilogos_matrix_chr1")
+    rows = len(ca)
+    draws = so.draw_shuffle(seed, np.repeat(np.arange(P), rows), np.tile(np.arange(rows), P), np.tile(ca, (P, 1)),
+                            np.tile(cb, (P, 1)), 30, 25)
     nulls = []
     for p in range(P):
-        ga = np.zeros_like(ca); gb = np.zeros_like(cb)
-        for r in range(len(ca)):
-            rng = np.random.default_rng([seed & (2 ** 63 - 1), p, r])
-            comb = ca[r] + cb[r]
-            ga[r] = rng.multivariate_hypergeometric(comb, min(30, int(comb.sum())))
-            rest = comb - ga[r]
-            gb[r] = rng.multivariate_hypergeometric(rest, min(25, int(rest.sum())))
+        ga, gb = draws["a"][p * rows:(p + 1) * rows], draws["b"][p * rows:(p + 1) * rows]
         d = orc.s1_scores_from_counts(ga, 30, exp) - orc.s1_scores_from_counts(gb, 25, exp)
         nulls.append(np.sum(np.square(d), axis=1) * np.sign(np.sum(d, axis=1)))
     nulls = np.array(nulls, dtype=np.float32)
