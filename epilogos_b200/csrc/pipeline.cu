@@ -343,13 +343,13 @@ extern "C" int epi_paired_host(const int8_t* xa_host, int64_t pitch_a, int32_t c
         if (int rc = na.alloc((size_t)batch * bins * K * 4)) return rc;
         if (int rc = nb.alloc((size_t)batch * bins * K * 4)) return rc;
         if (int rc = nd.alloc((size_t)nperm * bins * 4)) return rc;
-        // the philox counter carries the permutation index: batches continue the numbering through a seed-independent offset
+        // the philox counter carries the permutation index: batch [done, done + nbatch) draws permutations done .. done +
+        // nbatch - 1 of the one (seed, global bin) stream, so null row p does not depend on the batch size (nor on bins)
         for (int done = 0; done < nperm; done += batch) {
             const int nbatch = (nperm - done) < batch ? (nperm - done) : batch;
-            // permutations [done, done + nbatch): one launch draws them all; key the batch by mixing its start into the seed
-            const uint64_t bseed = seed + 0x9E3779B97F4A7C15ull * (uint64_t)done;
-            if (int rc = epi_shuffled_counts_philox(ca.as<uint16_t>(), cb.as<uint16_t>(), bins, K, n, size_a, size_b, bseed,
-                                                    bin_offset, nbatch, oa.as<uint16_t>(), ob.as<uint16_t>(), st))
+            if (int rc = epi_shuffled_counts_philox_range(ca.as<uint16_t>(), cb.as<uint16_t>(), bins, K, n, size_a, size_b,
+                                                          seed, bin_offset, done, nbatch, oa.as<uint16_t>(),
+                                                          ob.as<uint16_t>(), st))
                 return rc;
             if (int rc = score(oa.as<uint16_t>(), (int64_t)nbatch * bins, size_a, p1, na.as<float>())) return rc;
             if (int rc = score(ob.as<uint16_t>(), (int64_t)nbatch * bins, size_b, p2, nb.as<float>())) return rc;

@@ -327,7 +327,9 @@ int epi_single_host_packed(const uint8_t* packed_host, int64_t bins, int32_t col
  *                  device-drawn null shuffles per bin (the reference draws one) with their signed squared distances.
  *                  group_size -1 = the groups' own widths, else -g (clipped like the reference's slices, helpers.py:190-194);
  *                  bin_offset = global index of row 0 (keys the random streams).  Outputs (any may be NULL): counts int64 /
- *                  exp float32 [K] or [K][K], delta float32 [bins][K], null float32 [nperm][bins], quiescent uint8 [bins]. */
+ *                  exp float32 [K] or [K][K], delta float32 [bins][K], null float32 [nperm][bins], quiescent uint8 [bins].
+ *                  Null row p of a bin is permutation p of the stream keyed by (seed, bin_offset + row), the draw
+ *                  epi_shuffled_counts_philox_range makes, whatever batches the call splits the permutations into. */
 int epi_s3_host(const int8_t* x_host, int64_t bins, int32_t cols, int64_t pitch, int32_t num_states, float* exp_host,
                 float* scores_host);
 int epi_paired_host(const int8_t* xa_host, int64_t pitch_a, int32_t cols_a, const int8_t* xb_host, int64_t pitch_b,
