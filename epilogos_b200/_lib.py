@@ -14,6 +14,7 @@ EPI_SCORE_TABLE = 0
 EPI_SCORE_DIRECT = 1
 EPI_MAX_STATES = 32
 EPI_MAX_GROUPS = 64
+EPI_MAX_STRATA = 64
 
 # name -> (restype, argtypes); mirrors include/epilogos_b200.h one to one
 PROTOTYPES = {
@@ -57,6 +58,11 @@ PROTOTYPES = {
     "epi_multigroup_exceedances_s1": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_void_p, c_uint64, c_int64,
                                               c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
     "epi_multigroup_s1_fused_fits": (c_int, [c_int32, c_int32, c_void_p]),
+    "epi_stratified_shuffled_counts_range": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_void_p, c_int32,
+                                                     c_uint64, c_int64, c_int64, c_int32, c_void_p, c_void_p]),
+    "epi_stratified_exceedances_s1": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_int64, c_int32,
+                                              c_uint64, c_int64, c_int64, c_int32, c_void_p, c_int32, c_int32, c_void_p,
+                                              c_void_p, c_void_p]),
     "epi_split_counts": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int32, c_void_p, c_int32, c_int32, c_void_p,
                                  c_void_p]),
     "epi_window_max": (c_int, [c_void_p, c_int32, c_int64, c_int64, c_int64, c_int32, c_void_p, c_void_p]),

@@ -48,6 +48,12 @@ class CudaBackend:
             cnt = engine.group_counts(x_dev, cols, num_states, groups)
         return [c if c.data_ptr() % 16 == 0 else c.clone() for c in cnt]
 
+    def stratum_counts(self, x_dev, cols, num_states, columns):
+        """Counts of every stratum's row (lists of 0-based columns, a column listed twice counted twice) of a device
+        matrix, one epi_group_counts pass: int16 [H, rows, K]."""
+        with timing.stage("kernels", sync_cuda=True):
+            return engine.group_counts(x_dev, cols, num_states, columns)
+
     def gather_columns(self, x_dev, cols, idx):
         """The matrix of the columns idx of a device matrix, on the device."""
         return engine.gather_columns(x_dev, cols, idx)
@@ -104,23 +110,36 @@ class CudaBackend:
         return engine.shuffled_counts_perm(xa, states_a.shape[1], xb, states_b.shape[1], p.contiguous(), num_states,
                                            size_a, size_b)
 
-    def shuffled_counts_device(self, cnt_a, cnt_b, size_a, size_b, seed, nperm=1, width=None, bin_offset=0):
+    def shuffled_counts_device(self, cnt_a, cnt_b, size_a, size_b, seed, nperm=1, width=None, bin_offset=0, strata=None):
+        """`strata` (groups.StrataLayout): the labels are shuffled within strata (engine.stratified_shuffled_counts_range
+        on the per-stratum counts); the sizes of A' and B' are then the strata's."""
+        if strata is not None:
+            oc = engine.stratified_shuffled_counts_range(strata.counts, strata.sizes, seed, 0, nperm, bin_offset)
+            if nperm > 1:
+                return oc[:, 0].contiguous(), oc[:, 1].contiguous()
+            # the score kernels want 16-byte aligned counts
+            return tuple(c if c.data_ptr() % 16 == 0 else c.clone() for c in (oc[0, 0], oc[0, 1]))
         oa, ob = engine.shuffled_counts_philox(cnt_a, cnt_b, size_a, size_b, seed, nperm, width=width,
                                                bin_offset=bin_offset)
         return (oa[0], ob[0]) if nperm == 1 else (oa, ob)
 
     def permutation_exceedances(self, cnt_a, cnt_b, dist, nperm, seed, size_a, size_b, width, bin_offset, saliency, exp,
-                                score_widths, perms, exact=False, workspace_bytes=1 << 30):
+                                score_widths, perms, exact=False, workspace_bytes=1 << 30, strata=None):
         """Per-bin permutation counts k[b] = #{p < nperm : |null(b, p)| >= |dist[b]|} (int32 tensor holding uint32): the
         null distances of permutations 0 .. nperm-1 drawn as shuffled_counts_device draws them, A' scored at
         score_widths[0] with perms[0], B' at score_widths[1] with perms[1], in the run's score mode (`exact`).
         S1 runs the fused kernel (its TABLE and DIRECT values are the same numbers); S2 and tables wider than the S1
         value table loop over bin chunks x permutation blocks of draw + score + count, whose device buffers stay below
-        `workspace_bytes`.  The result does not depend on that cap."""
+        `workspace_bytes`.  The result does not depend on that cap.
+        `strata` (groups.StrataLayout): the shuffles keep to the strata, drawn as shuffled_counts_device draws them with
+        strata; S1 runs the fused stratified kernel, the rest the same loops with the stratified sampler."""
         rows, k_states = cnt_a.shape
         exp = exp.to(self.device).contiguous()
         dist = dist.to(self.device).contiguous()
         k = torch.zeros(rows, dtype=torch.int32, device=self.device)
+        if strata is not None:
+            return self._stratified_exceedances(cnt_a, cnt_b, dist, nperm, seed, bin_offset, saliency, exp, score_widths,
+                                                perms, exact, workspace_bytes, strata, k)
         if saliency == 1 and max(score_widths) <= engine.S1_TABLE_MAX_WIDTH:
             with timing.stage("kernels", sync_cuda=True):
                 return engine.permutation_exceedances_s1(cnt_a, cnt_b, size_a, size_b, seed, 0, nperm, width, bin_offset,
@@ -136,10 +155,30 @@ class CudaBackend:
                                         dist[lo:hi], k[lo:hi])
         return k
 
+    def _stratified_exceedances(self, cnt_a, cnt_b, dist, nperm, seed, bin_offset, saliency, exp, score_widths, perms,
+                                exact, workspace_bytes, strata, k):
+        rows, k_states = cnt_a.shape
+        if saliency == 1 and max(score_widths) <= engine.S1_TABLE_MAX_WIDTH:
+            with timing.stage("kernels", sync_cuda=True):
+                return engine.stratified_exceedances_s1(strata.counts, strata.sizes, cnt_a, cnt_b, seed, 0, nperm,
+                                                        bin_offset, exp, score_widths[0], score_widths[1], dist, k)
+        with timing.stage("kernels", sync_cuda=True):
+            # A', B' counts (uint16) and scores (float32)
+            for lo, hi, p0, n in self._blocks(rows, nperm, workspace_bytes, 12 * k_states):
+                oc = engine.stratified_shuffled_counts_range(strata.counts[:, lo:hi], strata.sizes, seed, p0, n,
+                                                             bin_offset + lo)
+                sc = torch.empty((2, n, hi - lo, k_states), dtype=torch.float32, device=self.device)
+                for p in range(n):
+                    for g in range(2):
+                        self._group_scores(oc[p, g], score_widths[g], saliency, exp, exact, out=sc[g, p], perms=perms[g])
+                del oc
+                engine.null_exceedances(sc[0], sc[1], dist[lo:hi], k[lo:hi])
+        return k
+
     # -- multi-group comparisons ------------------------------------------------------------------------
-    def _group_scores(self, cnt, n, saliency, exp, exact, out=None):
-        """Scores of one group's counts [bins, K] at its own width n (S2 over its n (n - 1) ordered pairs), into `out`
-        when given.  The score kernels want 16-byte aligned counts and outputs; the callers keep their blocks aligned
+    def _group_scores(self, cnt, n, saliency, exp, exact, out=None, perms=None):
+        """Scores of one group's counts [bins, K] at its own width n (S2 over its n (n - 1) ordered pairs, or `perms`),
+        into `out` when given.  The score kernels want 16-byte aligned counts and outputs; the callers keep their blocks aligned
         except for a tail of fewer than 8 bins, whose blocks are copied."""
         cnt = cnt if cnt.data_ptr() % 16 == 0 else cnt.clone()
         direct = out is not None and out.data_ptr() % 16 != 0
@@ -147,7 +186,7 @@ class CudaBackend:
         if saliency == 1:
             sc = engine.scores_s1(cnt, n, exp, out32=o32)
         else:
-            sc = engine.scores_s2(cnt, n, exp, perms=n * (n - 1), out32=o32,
+            sc = engine.scores_s2(cnt, n, exp, perms=n * (n - 1) if perms is None else perms, out32=o32,
                                   mode=engine.EPI_SCORE_DIRECT if exact else engine.EPI_SCORE_TABLE)
         if direct:
             out.copy_(sc)
@@ -189,23 +228,32 @@ class CudaBackend:
         return out
 
     def multigroup_exceedances(self, cnt, sizes, t, nperm, seed, bin_offset, saliency, exp, exact=False,
-                               workspace_bytes=1 << 30):
+                               workspace_bytes=1 << 30, strata=None):
         """Per-bin permutation counts k[b] = #{p < nperm : T_null(b, p) >= t[b]} (int32 tensor holding uint32) of the
         groups' counts cnt int16 [G, bins, K]: shuffle p drawn as engine.multigroup_shuffled_counts_range draws it, group
         g scored at width sizes[g] in the run's score mode.  S1 runs the fused kernel where its tables fit; S2 and wider
         S1 groups loop over bin chunks x permutation blocks of draw + score + count, whose device buffers (shuffled
-        counts and their scores) stay below `workspace_bytes`.  The result does not depend on that cap."""
+        counts and their scores) stay below `workspace_bytes`.  The result does not depend on that cap.
+        `strata` (groups.StrataLayout): the shuffles keep to the strata (engine.stratified_shuffled_counts_range), in the
+        loops of draw + score + count for every score mode."""
         G, rows, k_states = cnt.shape
         exp = exp.to(self.device).contiguous()
         t = t.to(self.device).contiguous()
         k = torch.zeros(rows, dtype=torch.int32, device=self.device)
-        if saliency == 1 and engine.multigroup_s1_fused_fits(sizes, k_states):
+        if strata is None:
+            def draw(lo, hi, p0, n):
+                return engine.multigroup_shuffled_counts_range(cnt[:, lo:hi], sizes, seed, p0, n, bin_offset + lo)
+        else:
+            def draw(lo, hi, p0, n):
+                return engine.stratified_shuffled_counts_range(strata.counts[:, lo:hi], strata.sizes, seed, p0, n,
+                                                               bin_offset + lo)
+        if strata is None and saliency == 1 and engine.multigroup_s1_fused_fits(sizes, k_states):
             with timing.stage("kernels", sync_cuda=True):
                 return engine.multigroup_exceedances_s1(cnt, sizes, seed, 0, nperm, bin_offset, exp, t, k)
         with timing.stage("kernels", sync_cuda=True):
             # shuffled counts (uint16) and scores (float32)
             for lo, hi, p0, n in self._blocks(rows, nperm, workspace_bytes, 6 * G * k_states):
-                oc = engine.multigroup_shuffled_counts_range(cnt[:, lo:hi], sizes, seed, p0, n, bin_offset + lo)
+                oc = draw(lo, hi, p0, n)
                 sc = torch.empty((n, G, hi - lo, k_states), dtype=torch.float32, device=self.device)
                 for p in range(n):
                     for g, size in enumerate(sizes):
@@ -216,12 +264,12 @@ class CudaBackend:
 
     # -- region null: whole-genome label permutations (epilogos_b200.region_null) ------------------------------------
     def region_maxima_paired(self, x_dev, halo, sizes, num_states, window, nperm, seed, saliency, exp, exact=False,
-                             workspace_bytes=1 << 30):
+                             workspace_bytes=1 << 30, strata=None):
         """int64 [nperm] on the device: for split p of region_null.split_blocks, the largest sum of W = `window`
         consecutive q(|distance|) of the rows of x_dev (the [A | B] label matrix, A of sizes[0] columns) followed by the
         host rows `halo`.  Each permuted group is scored like its real counterpart (its width, S2 normaliser and score
         mode) and reduced with the text round trip, so the identity split gives the real distances.  -1 where no window
-        fits."""
+        fits.  `strata` (groups.StrataLayout): the splits keep to the strata (region_null.split_blocks)."""
         def stat(cnt, n0, out):
             sa = self._group_scores(cnt[0], sizes[0], saliency, exp, exact)
             sb = self._group_scores(cnt[1], sizes[1], saliency, exp, exact)
@@ -229,10 +277,10 @@ class CudaBackend:
             d, _ = engine.pairwise_real_reduce(delta, True)
             torch.abs(d, out=out)
         return self._region_maxima(x_dev, halo, sizes, num_states, window, nperm, seed, exp, torch.float32,
-                                   12 * num_states + 16, stat, workspace_bytes)
+                                   12 * num_states + 16, stat, workspace_bytes, strata)
 
     def region_maxima_multigroup(self, x_dev, halo, sizes, num_states, window, nperm, seed, saliency, exp, exact=False,
-                                 workspace_bytes=1 << 30):
+                                 workspace_bytes=1 << 30, strata=None):
         """As region_maxima_paired for the multi-group statistic T of the groups, which are the consecutive column slices
         of sizes[0], sizes[1], ... of x_dev."""
         G = len(sizes)
@@ -243,10 +291,10 @@ class CudaBackend:
                 self._group_scores(cnt[g], n, saliency, exp, exact, out=sc[g])
             out.copy_(engine.multigroup_stat(sc, sizes)[0])
         return self._region_maxima(x_dev, halo, sizes, num_states, window, nperm, seed, exp, torch.float64,
-                                   6 * G * num_states + 16, stat, workspace_bytes)
+                                   6 * G * num_states + 16, stat, workspace_bytes, strata)
 
     def _region_maxima(self, x_dev, halo, sizes, num_states, window, nperm, seed, exp, dtype, cell_bytes, stat,
-                       workspace_bytes):
+                       workspace_bytes, strata=None):
         """Split blocks (drawn in order, outer) x bin chunks (inner, overlapping by W - 1 rows): split counts, the
         statistic of every split into one [splits, rows] array, its windowed maxima.  Buffers stay near
         `workspace_bytes`; the result does not depend on it."""
@@ -268,7 +316,8 @@ class CudaBackend:
         chunk = min(starts, max(1 << 16, cells // nperm))
         block = max(1, min(nperm, cells // (chunk + window - 1)))
         with timing.stage("kernels", sync_cuda=True):
-            for p0, members in region_null.split_blocks(seed, sizes, nperm, block):
+            by_strata = {} if strata is None else {"strata": (strata.positions, strata.sizes)}
+            for p0, members in region_null.split_blocks(seed, sizes, nperm, block, **by_strata):
                 n = members.shape[0]
                 mem = torch.from_numpy(members.view(np.int64)).to(self.device)
                 for lo in range(0, starts, chunk):

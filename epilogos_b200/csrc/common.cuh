@@ -66,6 +66,7 @@ struct DeviceWorkspace {
     alignas(8) double s1_v64[EPI_MAX_STATES * (S1_TABLE_MAX_WIDTH + 1)];   // S1 value table [K][width + 1]
     alignas(8) float s1_v32[EPI_MAX_STATES * (S1_TABLE_MAX_WIDTH + 1)];    // its float32 rounding
     alignas(8) float perm_v32[2][EPI_MAX_STATES * (S1_TABLE_MAX_WIDTH + 1)];  // permutations.cu: the tables of A', B'
+    int strata_sizes[EPI_MAX_STRATA * EPI_MAX_GROUPS];             // strata.cu: the group sizes of every stratum
 };
 static_assert(offsetof(DeviceWorkspace, k5tc_b_image) % 16 == 0, "the B operand image is a bulk-copy source");
 static_assert(offsetof(DeviceWorkspace, s1_v64) % 8 == 0 && offsetof(DeviceWorkspace, s1_v32) % 8 == 0,

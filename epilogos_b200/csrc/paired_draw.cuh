@@ -135,6 +135,21 @@ __device__ __forceinline__ void draw_multigroup_shuffle(Philox& rng, int K, int 
     }
 }
 
+// One stratified shuffle (strata.cu): labels move only within their stratum.  comb(h, s) is stratum h's count of state s
+// over the row being shuffled and size + h * G its G group sizes, which cover the stratum's row.  draw_multigroup_shuffle
+// runs once per stratum h = 0 .. H-1 in order, on the stream as the previous stratum left it, and emit(h, s, g, x) gets
+// stratum h's draws; a group's null counts are their sums over the strata.  With H = 1 this is draw_multigroup_shuffle,
+// word for word.
+template <class Comb, class Need, class Emit>
+__device__ __forceinline__ void draw_stratified_shuffle(Philox& rng, int H, int K, int G, const int* size, Comb comb,
+                                                        Need need, const double* __restrict__ lf,
+                                                        const double* __restrict__ inv, Emit emit) {
+    for (int h = 0; h < H; ++h)
+        draw_multigroup_shuffle(
+            rng, K, G, size + h * G, [&](int s) { return comb(h, s); }, need, lf, inv,
+            [&](int s, int g, int x) { emit(h, s, g, x); }, [](int) {});
+}
+
 // The multi-group statistic, one state at a time, in float64 without contraction (the numpy oracle computes the same
 // numbers): m[s] = (sum_g n_g S_g[s]) / N, then t += n_g (S_g[s] - m[s])^2 for g in order, in one running sum over s
 // outer, g inner; T = t / N.  score(g) = S_g[s] of the state at hand.

@@ -523,6 +523,53 @@ def multigroup_exceedances_s1(cnt, sizes, seed, perm_offset, nperm, bin_offset, 
     return k
 
 
+def _strata_sizes(sizes, groups=None):
+    """(H, G, ctypes array) of the sizes [H][G] (a sequence of per-stratum group sizes)."""
+    rows = [[int(v) for v in r] for r in sizes]
+    G = len(rows[0]) if rows else 0
+    if any(len(r) != G for r in rows) or (groups is not None and G != groups):
+        raise ValueError("the strata sizes must be [strata][groups]%s" % ("" if groups is None else " with %d groups" % groups))
+    flat = [v for r in rows for v in r]
+    arr = (ctypes.c_int32 * max(len(flat), 1))(*flat)
+    return len(rows), G, arr
+
+
+def stratified_shuffled_counts_range(cnt, sizes, seed, perm_offset, nperm, bin_offset=0):
+    """Permutations perm_offset .. perm_offset + nperm - 1 of every bin shuffled within strata: cnt int16 [H, bins, K]
+    holds each stratum's counts over the row being shuffled (blocks may be spaced further apart), sizes [H][G] the groups'
+    biosamples in each stratum.  Returns int16 [nperm, G, bins, K], the groups' counts summed over the strata."""
+    H, bins, K, stride = _group_blocks(cnt)
+    h, G, arr = _strata_sizes(sizes)
+    if h != H:
+        raise ValueError("one row of sizes per stratum")
+    out = torch.empty((nperm, G, bins, K), dtype=torch.int16, device=cnt.device)
+    _lib.call("epi_stratified_shuffled_counts_range", _ptr(cnt), stride, H, bins, K, ctypes.cast(arr, ctypes.c_void_p), G,
+              _seed(seed), int(bin_offset), int(perm_offset), int(nperm), _ptr(out), _stream())
+    return out
+
+
+def stratified_exceedances_s1(cnt, sizes, cnt_a, cnt_b, seed, perm_offset, nperm, bin_offset, exp1, width_a, width_b,
+                              dist, k):
+    """Fused stratified S1 permutation counts of a paired comparison: k[b] += #{p : |null(b, p)| >= |dist[b]|} over
+    permutations perm_offset .. perm_offset + nperm - 1 drawn as stratified_shuffled_counts_range draws them (sizes
+    [H][2]), A' scored at width_a and B' = cnt_a + cnt_b - A' at width_b against exp1.  k: int32 [bins] (uint32 counts)."""
+    H, bins, K, stride = _group_blocks(cnt)
+    h, _, arr = _strata_sizes(sizes, groups=2)
+    for t, name in ((cnt_a, "cnt_a"), (cnt_b, "cnt_b")):
+        _require_cuda(t, torch.int16, name)
+    _require_cuda(exp1, torch.float32, "exp1")
+    _require_cuda(dist, torch.float32, "dist")
+    _require_cuda(k, torch.int32, "k")
+    if h != H or tuple(cnt_a.shape) != (bins, K) or tuple(cnt_b.shape) != (bins, K):
+        raise ValueError("one row of sizes per stratum, and cnt_a, cnt_b [bins, K]")
+    if dist.numel() != bins or k.numel() != bins or exp1.numel() != K:
+        raise ValueError("dist and k must have one entry per bin, exp1 one per state")
+    _lib.call("epi_stratified_exceedances_s1", _ptr(cnt), stride, H, ctypes.cast(arr, ctypes.c_void_p), _ptr(cnt_a),
+              _ptr(cnt_b), bins, K, _seed(seed), int(bin_offset), int(perm_offset), int(nperm), _ptr(exp1), int(width_a),
+              int(width_b), _ptr(dist), _ptr(k), _stream())
+    return k
+
+
 def split_counts(x, cols, num_states, members, groups):
     """Counts of the groups of column splits of x (CUDA int8 [bins, pitch]).  members: CUDA int64 [nsplit, groups - 1,
     ceil(cols / 64)] column bitsets (uint64 bit patterns), the last group of a split being the complement.  Returns an int16

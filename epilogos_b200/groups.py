@@ -65,13 +65,14 @@ class Selection:
         return self.b is not None or self.multi is not None
 
 
-def parseGroups(path):
-    """The GroupSet of a group file; raises GroupFileError with the message of the first problem."""
+def parseGroups(path, flag="--groups"):
+    """The GroupSet of a group file; raises GroupFileError with the message of the first problem.  `flag` is the option
+    the messages name (the strata file of --strata has the same format)."""
     path = Path(path)
     try:
         text = path.read_text()
     except OSError as exc:
-        raise GroupFileError("ERROR: [--groups] cannot read {}: {}".format(path, exc.strerror or exc))
+        raise GroupFileError("ERROR: [{}] cannot read {}: {}".format(flag, path, exc.strerror or exc))
     names, columns = [], []
     for n, raw in enumerate(text.splitlines(), start=1):
         line = raw.rstrip("\r")
@@ -79,36 +80,36 @@ def parseGroups(path):
             continue
         fields = line.split("\t")
         if len(fields) != 2:
-            raise GroupFileError("ERROR: [--groups] line {}: expected 'name<TAB>columns', got {!r}".format(n, line))
+            raise GroupFileError("ERROR: [{}] line {}: expected 'name<TAB>columns', got {!r}".format(flag, n, line))
         name, spec = fields[0].strip(), fields[1].strip()
         if not _NAME.match(name):
-            raise GroupFileError("ERROR: [--groups] line {}: group name {!r} must match [A-Za-z0-9._-]+".format(n, name))
+            raise GroupFileError("ERROR: [{}] line {}: group name {!r} must match [A-Za-z0-9._-]+".format(flag, n, name))
         if name in names:
-            raise GroupFileError("ERROR: [--groups] line {}: group name '{}' is used twice".format(n, name))
+            raise GroupFileError("ERROR: [{}] line {}: group name '{}' is used twice".format(flag, n, name))
         cols = []
         for tok in (t.strip() for t in spec.split(",")):
             if tok == "":
                 continue
             m = _TOKEN.match(tok)
             if not m or int(m.group(1)) < 1 or (m.group(2) is not None and int(m.group(2)) < int(m.group(1))):
-                raise GroupFileError("ERROR: [--groups] line {}: {!r} is not a biosample number (from 1) or a range a-b "
-                                     "with a <= b".format(n, tok))
+                raise GroupFileError("ERROR: [{}] line {}: {!r} is not a biosample number (from 1) or a range a-b "
+                                     "with a <= b".format(flag, n, tok))
             lo = int(m.group(1))
             hi = int(m.group(2)) if m.group(2) is not None else lo
             cols.extend(range(lo, hi + 1))
         if not cols:
-            raise GroupFileError("ERROR: [--groups] line {}: group '{}' has no columns".format(n, name))
+            raise GroupFileError("ERROR: [{}] line {}: group '{}' has no columns".format(flag, n, name))
         ordered = np.sort(np.asarray(cols, dtype=np.int64))
         dup = ordered[1:][ordered[1:] == ordered[:-1]]
         if len(dup):
-            raise GroupFileError("ERROR: [--groups] line {}: group '{}' lists biosample {} more than once".format(
-                n, name, int(dup[0])))
+            raise GroupFileError("ERROR: [{}] line {}: group '{}' lists biosample {} more than once".format(
+                flag, n, name, int(dup[0])))
         if len(names) == MAX_GROUPS:
-            raise GroupFileError("ERROR: [--groups] more than {} groups in {}".format(MAX_GROUPS, path))
+            raise GroupFileError("ERROR: [{}] more than {} groups in {}".format(flag, MAX_GROUPS, path))
         names.append(name)
         columns.append(ordered - 1)
     if not names:
-        raise GroupFileError("ERROR: [--groups] no group in {}".format(path))
+        raise GroupFileError("ERROR: [{}] no group in {}".format(flag, path))
     return GroupSet(names, columns)
 
 
@@ -272,3 +273,98 @@ def view(shard, selection):
     if key not in shard._views:
         shard._views[key] = GroupView(shard, selection)
     return shard._views[key]
+
+
+# ---- strata (--strata): null shuffles that move labels only within strata ------------------------------------------------
+
+class Strata:
+    """The strata of a run, in file order (a GroupSet of disjoint column sets), and the file they came from."""
+
+    def __init__(self, groupset, path):
+        self.groupset, self.path = groupset, str(path)
+
+    def __len__(self):
+        return len(self.groupset)
+
+    def summary(self):
+        """The CLI header line."""
+        sizes = ", ".join(str(len(c)) for c in self.groupset.columns)
+        return "Strata = {} (biosamples per stratum: {})".format(len(self), sizes)
+
+    def layout(self, group_cols, comparison, cols, file, null_mode=None):
+        """The StrataLayout of one comparison whose groups are the column lists `group_cols` of a matrix of `cols`
+        columns (`file`); raises ValueError naming the file for the load-time rules, in their order."""
+        gs = self.groupset
+        for name, c in zip(gs.names, gs.columns):
+            if len(c) and c[-1] >= cols:
+                raise ValueError("[--strata] {}: stratum '{}' uses biosample {}, but {} has {} biosamples".format(
+                    self.path, name, int(c[-1]) + 1, file, cols))
+        stratum_of = np.full(cols, -1, dtype=np.int64)
+        for h, c in enumerate(gs.columns):
+            stratum_of[c] = h
+        group_cols = [np.asarray(c, dtype=np.int64) for c in group_cols]
+        compared = np.concatenate(group_cols)
+        missing = compared[stratum_of[compared] < 0]
+        if len(missing):
+            raise ValueError("[--strata] {}: biosample {} of the comparison {} is in no stratum".format(
+                self.path, int(missing[0]) + 1, comparison))
+        held = [h for h in range(len(gs)) if np.any(stratum_of[compared] == h)]
+        sizes = [[int(np.count_nonzero(stratum_of[c] == h)) for c in group_cols] for h in held]
+        if not any(sum(1 for n in row if n > 0) >= 2 for row in sizes):
+            raise ValueError("[--strata] {}: no stratum holds biosamples of two groups of the comparison {}, so no "
+                             "shuffle can move a label".format(self.path, comparison))
+        if null_mode == "reference":
+            raise ValueError("[--strata] {}: EPILOGOS_B200_NULL=reference replays the reference's unstratified shuffle; "
+                             "stratified nulls are drawn on the device".format(self.path))
+        return StrataLayout([gs.names[h] for h in held], sizes,
+                            [np.concatenate([c[stratum_of[c] == h] for c in group_cols]) for h in held],
+                            [np.flatnonzero(stratum_of[compared] == h) for h in held])
+
+
+class StrataLayout:
+    """The strata of one comparison that hold at least one compared biosample, in file order:
+      sizes      [H][G] n[h][g], group g's biosamples in stratum h (a biosample of two groups counts in both);
+      columns    [H] the matrix columns of stratum h's row, group after group (such a biosample listed twice);
+      positions  [H] the same biosamples as ascending positions in the compared matrix, whose columns are the groups'
+                 one group after the other (the region null's splits);
+      counts     int16 [H, rows, K], each stratum's counts over the shard's rows (set by stratify)."""
+
+    def __init__(self, names, sizes, columns, positions):
+        self.names, self.sizes, self.columns, self.positions = names, sizes, columns, positions
+        self.counts = None
+        self.key = tuple((n, tuple(int(v) for v in c)) for n, c in zip(names, columns))
+
+
+def parseStrata(path):
+    """The Strata of a --strata file (the group-file format); raises GroupFileError with the message of the first
+    problem: those of parseGroups naming [--strata], then two strata sharing a biosample."""
+    gs = parseGroups(path, flag="--strata")
+    for i in range(len(gs)):
+        for j in range(i + 1, len(gs)):
+            shared = np.intersect1d(gs.columns[i], gs.columns[j])
+            if len(shared):
+                raise GroupFileError("ERROR: [--strata] strata '{}' and '{}' share biosample {}".format(
+                    gs.names[i], gs.names[j], int(shared[0]) + 1))
+    return Strata(gs, path)
+
+
+def stratify(view, strata, null_mode=None):
+    """The StrataLayout of the comparison of a paired shard (-a/-b: columns numbered over [A | B]) or of a group view
+    (--compare, --multigroup: the numbering of the -i matrix), with its per-stratum counts: one epi_group_counts pass
+    over the shard's device matrix, kept with the shard's counts."""
+    base = getattr(view, "_shard", view)             # the session.Shard whose device matrix holds the columns
+    sel = getattr(view, "selection", None)
+    if sel is None:
+        c1 = view.states_a.shape[1]
+        group_cols, comparison = [np.arange(c1), c1 + np.arange(view.states_b.shape[1])], "[-a] vs [-b]"
+    else:
+        gs = sel.groupset
+        names = list(sel.multi) if sel.multi is not None else [sel.a, sel.b]
+        group_cols = [gs.columns[gs.index[n]] for n in names]
+        comparison = ",".join(names) if sel.multi is not None else "{}:{}".format(sel.a, sel.b)
+    lay = strata.layout(group_cols, comparison, base.width, base.file, null_mode)
+    key = ("strata", lay.key)
+    if key not in base._counts:
+        base._counts[key] = base.backend.stratum_counts(base.states_device(), base.width, base.num_states, lay.columns)
+    lay.counts = base._counts[key]
+    return lay

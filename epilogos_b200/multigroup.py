@@ -20,9 +20,10 @@ from .scores import _gather_locations
 
 def calculateScoresMultigroup(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
                               backend=None, group=None, permutations=0, seed=None, region_permutations=0,
-                              region_seed=None, roi_width=None):
+                              region_seed=None, roi_width=None, strata=None):
     """`region_permutations` P > 0: also the file's maxima of the region null over `region_seed`'s P label splits of the
-    groups' columns (epilogos_b200.region_null), handed to step 4 or written to temp_regionNull_<tag>_<file>.npz."""
+    groups' columns (epilogos_b200.region_null), handed to step 4 or written to temp_regionNull_<tag>_<file>.npz.
+    `strata` (groups.Strata, --strata): the permutations and the region splits shuffle labels only within strata."""
     if saliency not in (1, 2):
         raise ValueError("Please ensure that saliency metric is either 1 or 2 for Pairwise Epilogos")
     region_null.check_seed(region_permutations, region_seed)
@@ -30,16 +31,20 @@ def calculateScoresMultigroup(saliency, file1Path, numStates, outputDirPath, exp
     view = session.load_shard(file1Path, file1Path, numStates, backend, group=group)
     exp = be.to_device(np.load(expFreqPath, allow_pickle=False))
     cnt, sizes = view.group_blocks(), view.sizes
+    by_strata = {}
+    if strata is not None:
+        from . import groups
+        by_strata = {"strata": groups.stratify(view, strata)}
     t, g, s, sign = be.multigroup_stat(cnt, sizes, saliency, exp)
     exceed = None
     if permutations > 0:
         exceed = be.multigroup_exceedances(cnt, sizes, t, permutations, file_seed(run_seed(seed), filename), view.lo,
-                                           saliency, exp)
+                                           saliency, exp, **by_strata)
     region = None
     if region_permutations > 0:
         cols = view.grouped()
         region = region_null.shard_maxima(be, "multigroup", cols.device_matrix(), cols.head, sizes, numStates, roi_width,
-                                          region_permutations, region_seed, saliency, exp)
+                                          region_permutations, region_seed, saliency, exp, **by_strata)
     total = view.total_rows
     t, g, s, sign = (dist.gather_rows(a, total) for a in (t, g, s, sign))
     loc = _gather_locations(view)

@@ -65,14 +65,18 @@ def shuffled_widths(c1, c2, groupSize):
 
 def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDirPath, expFreqPath, fileTag, filename,
                             quiescentState, groupSize, verbose, backend=None, null_mode=None, seed=None, nperm=1,
-                            group=None, permutations=0, region_permutations=0, region_seed=None, roi_width=None):
+                            group=None, permutations=0, region_permutations=0, region_seed=None, roi_width=None,
+                            strata=None):
     """`permutations` P > 0: also count, for every bin, how many of P device-drawn null shuffles (permutations 0..P-1 of
     the device sampler, scored like the run's null) are at least as far from 0 as the bin's real distance, and hand the
     counts to step 4 (epilogos_b200.handoff) or write them to temp_permutations_<tag>_<file>.npz {chrName, exceedances
     uint32[B], permutations}.  Nothing else changes: in device mode permutation 0 is the run's own null.
     `region_permutations` P > 0: also the file's maxima of the region null over `region_seed`'s P label splits of the
     combined [A | B] matrix, windows of `roi_width` rows (epilogos_b200.region_null), handed to step 4 or written to
-    temp_regionNull_<tag>_<file>.npz."""
+    temp_regionNull_<tag>_<file>.npz.
+    `strata` (groups.Strata, --strata): every null of the file -- the run's own, the P permutations and the region splits
+    -- shuffles labels only within strata (groups.stratify numbers the columns over [A | B], or over the -i matrix with
+    `group`).  Device null mode only."""
     if saliency not in (1, 2):
         raise ValueError("Please ensure that saliency metric is either 1 or 2 for Pairwise Epilogos")
     region_null.check_seed(region_permutations, region_seed)
@@ -84,6 +88,10 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
     c1, c2 = shard.states_a.shape[1], shard.states_b.shape[1]
     size_a, size_b = shuffled_widths(c1, c2, groupSize)                            # helpers.py:190-194
     exp = be.to_device(np.load(expFreqPath, allow_pickle=False))
+    by_strata = {}
+    if strata is not None:
+        from . import groups
+        by_strata = {"strata": groups.stratify(shard, strata, null_mode)}
 
     cnt_a, cnt_b = shard.counts("a"), shard.counts("b")
     draw_seed = file_seed(run_seed(seed), filename) if null_mode == "device" or permutations > 0 else None
@@ -93,7 +101,7 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
         null_a, null_b = be.shuffled_counts_perm(shard.states_a, shard.states_b, perm, numStates, size_a, size_b)
     else:
         null_a, null_b = be.shuffled_counts_device(cnt_a, cnt_b, size_a, size_b, draw_seed, nperm, width=c1 + c2,
-                                                   bin_offset=shard.lo)
+                                                   bin_offset=shard.lo, **by_strata)
 
     # S1 observes over the width of the array it is given (scores.py:343); S2 normalises the shuffled halves with
     # the ORIGINAL group widths even under -g (scores.py:397-398, 418-421)
@@ -116,12 +124,12 @@ def calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDir
         real_dist, _ = be.pairwise_real_reduce(delta, text_round_trip=True)
         exceed = be.permutation_exceedances(cnt_a, cnt_b, real_dist, permutations, draw_seed, size_a, size_b, c1 + c2,
                                             shard.lo, saliency, exp, (max(size_a, 1), max(size_b, 1)), (p1, p2),
-                                            exact=exact)
+                                            exact=exact, **by_strata)
     region = None
     if region_permutations > 0:
         region = region_null.shard_maxima(be, "paired", shard.states_device(), lambda n: _head(shard, n), (c1, c2),
                                           numStates, roi_width, region_permutations, region_seed, saliency, exp,
-                                          exact=exact)
+                                          exact=exact, **by_strata)
 
     total = shard.total_rows
     delta = dist.gather_rows(delta, total)

@@ -41,9 +41,12 @@ def quantise(x):
     return np.rint(np.ldexp(x, 24)).astype(np.int64)
 
 
-def split_blocks(seed, sizes, nperm, block):
+def split_blocks(seed, sizes, nperm, block, strata=None):
     """(p0, members): the splits p0 .. p0 + n - 1 in blocks of at most `block`, drawn in order; members uint64
-    [n, G - 1, ceil(N / 64)] holds the column bitsets of the first G - 1 groups (the last group is the rest)."""
+    [n, G - 1, ceil(N / 64)] holds the column bitsets of the first G - 1 groups (the last group is the rest).
+    strata = (positions, n) (groups.StrataLayout): split p permutes, for every stratum h in order, the stratum's positions
+    (ascending) with rng.permutation(N_h) and gives the first n[h][0] of them to group 0, the next n[h][1] to group 1, ...
+    so every group keeps its make-up in every stratum; the identity permutation is the real split."""
     rng = np.random.Generator(np.random.Philox(key=int(seed)))
     N, G = int(sum(sizes)), len(sizes)
     words = (N + 63) // 64
@@ -52,20 +55,28 @@ def split_blocks(seed, sizes, nperm, block):
         n = min(block, nperm - p0)
         members = np.zeros((n, G - 1, words * 64), dtype=np.uint8)
         for i in range(n):
-            perm = rng.permutation(N)
-            for g in range(G - 1):
-                members[i, g, perm[edges[g]:edges[g + 1]]] = 1
+            if strata is None:
+                perm = rng.permutation(N)
+                for g in range(G - 1):
+                    members[i, g, perm[edges[g]:edges[g + 1]]] = 1
+                continue
+            for pos, nh in zip(*strata):
+                moved = np.asarray(pos)[rng.permutation(len(pos))]
+                cuts = np.cumsum([0] + [int(v) for v in nh])
+                for g in range(G - 1):
+                    members[i, g, moved[cuts[g]:cuts[g + 1]]] = 1
         yield p0, np.packbits(members, axis=2, bitorder="little").view(np.uint64)
 
 
-def shard_maxima(be, kind, x_dev, head, sizes, num_states, window, nperm, seed, saliency, exp, exact=False):
+def shard_maxima(be, kind, x_dev, head, sizes, num_states, window, nperm, seed, saliency, exp, exact=False, strata=None):
     """int64 [P] maxima of this file on every rank.  x_dev: the shard's rows of the compared matrix on the device; head(n):
     its first n rows on the host.  In rows mode the windows that start in a rank's rows may end in the rows of the ranks
     after it: each rank gets up to W - 1 such rows (dist.halo_rows), evaluates the windows starting in its own rows, and
-    the ranks take the maximum."""
+    the ranks take the maximum.  `strata` (groups.StrataLayout): the splits keep to the strata (split_blocks)."""
     halo = dist.halo_rows(head(window - 1), window - 1)
     fn = be.region_maxima_paired if kind == "paired" else be.region_maxima_multigroup
-    m = fn(x_dev, halo, sizes, num_states, window, nperm, seed, saliency, exp, exact=exact)
+    extra = {} if strata is None else {"strata": strata}
+    m = fn(x_dev, halo, sizes, num_states, window, nperm, seed, saliency, exp, exact=exact, **extra)
     return dist.all_reduce_max(m)
 
 

@@ -179,6 +179,24 @@ def checkMultigroupFlags(mode, groupFile, multigroups, groupSet, pvalBool, group
     return out
 
 
+def checkStrataFlags(mode, strataFile, groupSize):
+    """Rules of --strata (checked after every other rule): first violated rule prints and exits.  Returns the
+    groups.Strata of the file, or None without --strata."""
+    if not strataFile:
+        return None
+    for bad, message in ((mode != "paired", "ERROR: [--strata] requires [-m, --mode] 'paired'"),
+                         (groupSize != -1, "ERROR: [--strata] not compatible with [-g, --group-size] option")):
+        if bad:
+            _die(message)
+            return None
+    from . import groups as _groups
+    try:
+        return _groups.parseStrata(strataFile)
+    except _groups.GroupFileError as exc:
+        _die(str(exc))
+        return None
+
+
 def deal_files(pairs, world):
     """Whole files dealt to the ranks, largest first to the least loaded rank (by size on disk): the same answer on every
     rank.  Returns a list of `world` lists of (file1, file2) pairs."""
@@ -195,7 +213,7 @@ def deal_files(pairs, world):
 
 def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
                groupSize, stateInfo, roiWidth, verbose, say, backend=None, pvalBool=False, numTrials=101,
-               samplingSize=100000, diagnosticBool=False, groups=None, permutations=0, region_permutations=0):
+               samplingSize=100000, diagnosticBool=False, groups=None, permutations=0, region_permutations=0, strata=None):
     """Steps 1-4 of run.main (run.py:193-303) in process.  Two ways to use several GPUs:
       rows  (default)  every file's rows are split over the ranks (helpers.splitRows); per-file tables are all-reduced and
                        score rows gathered on rank 0, which writes the files;
@@ -215,7 +233,8 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
     epilogos_b200.roi_multigroup.
     `region_permutations` P > 0 (paired mode): step 3 also finds every file's maxima of the region null over P label
     splits drawn from one seed per run, and step 4 writes regionPermutation_<tag>.txt and regionNullMaxima_<tag>.npz
-    (epilogos_b200.region_null)."""
+    (epilogos_b200.region_null).
+    `strata` (groups.Strata, paired mode): every null of step 3 shuffles biosample labels only within strata."""
     from contextlib import nullcontext
     from . import dist, expected, expectedCombination, scores, session
     world = dist.world_size()
@@ -265,7 +284,7 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
                     scores.main(f, second(f, f2, sel), numStates, saliency, out, exp_path, tag, numProcesses,
                                 quiescentState, groupSize, verbose, backend=backend, group=sel,
                                 permutations=permutations, region_permutations=region_permutations,
-                                region_seed=region_seed, roi_width=roiWidth)
+                                region_seed=region_seed, roi_width=roiWidth, strata=strata)
     finally:
         session.handover_enabled = False
     dist.barrier()
@@ -355,14 +374,20 @@ def run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedE
                    + "region of interest a family-wise p-value: the share of the P genome-wide maxima of the window sums "
                    + "that reach its own (regionPermutation_<tag>.txt, regionNullMaxima_<tag>.npz; 1 <= P <= 100000; "
                    + "not with -g)")
+@click.option("--strata", "strataFile", type=str,
+              help="Paired mode: tab-separated file of strata (tissue, donor, batch, ...) in the --groups format, "
+                   + "name<TAB>columns; columns are numbered over [A | B] with -a/-b and as in the group file with "
+                   + "--groups.  Every null (-n, --null-permutations, --multigroup p-values, --roi-permutations) then "
+                   + "shuffles biosample labels only within strata, so each group keeps its make-up in every stratum.  "
+                   + "Not with -g")
 @click.option("--exp-freq-mem", "expFreqMem", type=int, default=20000, help="SLURM-only (ignored)")
 @click.option("--exp-comb-mem", "expCombMem", type=int, default=8000, help="SLURM-only (ignored)")
 @click.option("--score-mem", "scoreMem", type=int, default=40000, help="SLURM-only (ignored)")
 @click.option("--roi-mem", "roiMem", type=int, default=-1, help="SLURM-only (ignored)")
 def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2, outputDirectory, stateInfo, saliency,
          numProcesses, exitBool, diagnosticBool, numTrials, samplingSize, quiescentState, groupSize, version, partition,
-         pvalBool, roiWidth, fileTag, groupFile, comparisons, multigroups, nullPermutations, roiPermutations, expFreqMem,
-         expCombMem, scoreMem, roiMem):
+         pvalBool, roiWidth, fileTag, groupFile, comparisons, multigroups, nullPermutations, roiPermutations, strataFile,
+         expFreqMem, expCombMem, scoreMem, roiMem):
     """Information-theoretic navigation of multi-tissue functional genomic annotations (B200 scoring path)."""
     if version:
         from epilogos_b200 import __version__
@@ -398,6 +423,7 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
     checkPermutationFlags(mode, nullPermutations)
     multi_of_groups = checkMultigroupFlags(mode, groupFile, multigroups, groupSet, pvalBool, groupSize)
     checkRegionPermutationFlags(mode, roiPermutations, groupSize, roiWidth)
+    strata = checkStrataFlags(mode, strataFile, groupSize)
 
     import torch
     import torch.distributed as td
@@ -424,6 +450,8 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
     say("        Saliency level =", saliency, "  States =", numStates, "  Output =", str(outputDirPath))
     if mode == "paired":
         say("        Quiescent State =", "No quiescent filtering" if quiescentState == -1 else quiescentState + 1)
+    if strata is not None:
+        say("        " + strata.summary())
 
     files = sorted(p for p in inputDirPath.glob("*"))
     pairs = []
@@ -452,7 +480,7 @@ def main(mode, commandLineBool, inputDirectory, inputDirectory1, inputDirectory2
     run_stages(pairs, mode, numStates, saliency, outputDirPath, fileTag, storedExpPath, numProcesses, quiescentState,
                groupSize, stateInfo, roiWidth, verbose, say, pvalBool=pvalBool, numTrials=numTrials,
                samplingSize=samplingSize, diagnosticBool=diagnosticBool, groups=runs,
-               permutations=nullPermutations or 0, region_permutations=roiPermutations or 0)
+               permutations=nullPermutations or 0, region_permutations=roiPermutations or 0, strata=strata)
     dist.barrier()
     if launched and td.is_initialized():
         td.destroy_process_group()

@@ -18,7 +18,8 @@ from . import dist, handoff, helpers, session, writer
 
 
 def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, numProcesses, quiescentState, groupSize,
-         verbose, backend=None, group=None, permutations=0, region_permutations=0, region_seed=None, roi_width=None):
+         verbose, backend=None, group=None, permutations=0, region_permutations=0, region_seed=None, roi_width=None,
+         strata=None):
     tTotal = time()
     file1Path, file2Path, outputDirPath = Path(file1), Path(file2), Path(outputDir)
     filename = file1Path.name.split(".")[0]
@@ -28,7 +29,8 @@ def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, num
         from .multigroup import calculateScoresMultigroup
         calculateScoresMultigroup(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
                                   backend, group=group, permutations=permutations,
-                                  region_permutations=region_permutations, region_seed=region_seed, roi_width=roi_width)
+                                  region_permutations=region_permutations, region_seed=region_seed, roi_width=roi_width,
+                                  strata=strata)
     elif str(file2) == "null":
         calculateScores(saliency, file1Path, numStates, outputDirPath, expFreqPath, fileTag, filename, verbose,
                         backend, group=group)
@@ -37,7 +39,8 @@ def main(file1, file2, numStates, saliency, outputDir, expFreqPath, fileTag, num
         calculateScoresPairwise(saliency, file1Path, file2Path, numStates, outputDirPath, expFreqPath, fileTag,
                                 filename, quiescentState, groupSize, verbose, backend, group=group,
                                 permutations=permutations, region_permutations=region_permutations,
-                                region_seed=region_seed, roi_width=roi_width)
+                                region_seed=region_seed, roi_width=roi_width,
+                                strata=strata)
     if dist.rank() == 0:
         print("Total Time:", time() - tTotal, flush=True) if verbose else print("\t[Done]", flush=True)
     dist.barrier()

@@ -236,6 +236,38 @@ int epi_multigroup_exceedances_s1(const uint16_t* cnt_dev, int64_t group_stride,
                                   uint32_t* k_inout, void* stream);
 int epi_multigroup_s1_fused_fits(int32_t groups, int32_t num_states, const int32_t* sizes);
 
+/* ---- stratified permutations (csrc/strata.cu) -----------------------------------------------------------------
+ * Labels are shuffled only within strata.  H = strata (1..EPI_MAX_STRATA) and G = groups (2..EPI_MAX_GROUPS); sizes: HOST
+ * array [H][G] of n[h][g] >= 0, the biosamples of group g in stratum h, every stratum holding at least one, and
+ * N = sum of all n[h][g] <= 65535.  cnt [H] blocks of [bins][K] uint16, block h at cnt_dev + h * stratum_stride (>= bins *
+ * K): stratum h's counts over the row being shuffled.  The draw of (bin b, permutation p) takes the stream of
+ * epi_shuffled_counts_philox (seed, p, GLOBAL bin bin_offset + b) and runs, for h = 0 .. H-1 in order on that stream, the
+ * draw of epi_multigroup_shuffled_counts_range on stratum h's counts with sizes n[h][.]; group g's count is the sum over
+ * the strata.  With H = 1 both entry points equal their unstratified counterparts bit for bit.  perm_offset + nperm <=
+ * 2^32.  The sizes reach the device by one cudaMemcpyAsync (from the caller's pageable array) or in the kernel's
+ * parameters.
+ *   epi_stratified_shuffled_counts_range  out [nperm][G][bins][K] uint16.  Return code 2 when the largest stratum's
+ *                                         sampler tables exceed shared memory (about 12,600 biosamples in one stratum
+ *                                         at G = 2).
+ *   epi_stratified_exceedances_s1         fused paired S1 (G = 2, sizes [H][2]): per (bin, permutation) A' = the group-0
+ *                                         counts of the draw summed over the strata, B' = cnt_a + cnt_b - A', scored at
+ *                                         width_a / width_b (covering sum_h n[h][0] / sum_h n[h][1], at most 4095) against
+ *                                         exp1 [K] with the values epi_scores_s1 gives in TABLE mode;
+ *                                         k[b] += #{p : |null(b, p)| >= |dist[b]|}, as epi_permutation_exceedances_s1.
+ *                                         cnt_a + cnt_b must equal the sum of the strata's counts.  Equal bit for bit to
+ *                                         the composed path (epi_stratified_shuffled_counts_range, epi_scores_s1,
+ *                                         epi_null_exceedances). */
+#define EPI_MAX_STRATA 64
+int epi_stratified_shuffled_counts_range(const uint16_t* cnt_dev, int64_t stratum_stride, int32_t strata, int64_t bins,
+                                         int32_t num_states, const int32_t* sizes, int32_t groups, uint64_t seed,
+                                         int64_t bin_offset, int64_t perm_offset, int32_t nperm, uint16_t* out_dev,
+                                         void* stream);
+int epi_stratified_exceedances_s1(const uint16_t* cnt_dev, int64_t stratum_stride, int32_t strata, const int32_t* sizes,
+                                  const uint16_t* cnt_a_dev, const uint16_t* cnt_b_dev, int64_t bins, int32_t num_states,
+                                  uint64_t seed, int64_t bin_offset, int64_t perm_offset, int32_t nperm,
+                                  const float* exp1_dev, int32_t width_a, int32_t width_b, const float* dist_dev,
+                                  uint32_t* k_inout, void* stream);
+
 /* ---- whole-genome label permutations: the region null (csrc/label_permutations.cu) -----------------------------
  *   epi_split_counts  counts of the groups of nsplit column splits of one matrix x (cols <= 65535, any pitch and
  *                     alignment).  members_dev (device) holds nsplit x (groups - 1) column bitsets of ceil(cols / 64)
